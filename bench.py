@@ -21,6 +21,10 @@ config 2, the configuration that fits one GPU and that the metric is quoted on.
 --impl reference times the CPU path the reference drives (one single-threaded `dashing sketch`
 per (genome, k), floor(0.95*cores) at a time -- lib/huffman_dandd.py:217) using the oracle port,
 because neither Dashing nor GNU parallel exists here (see oracle/dandd_oracle.c header).
+
+--dump-outputs DIR writes what the last step of each timed loop computed (leaf and prefix-union
+cardinalities, a fixed sample of the registers) as DIR/<name>.npy.  The inputs are generated from
+fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -243,6 +247,31 @@ def _profile_json(name):
         return {}
 
 
+# ------------------------------------------------------------------------------------ --dump-outputs
+DUMP_LIMIT_BYTES = 64 << 20
+REGISTER_SAMPLE = 1 << 20
+
+
+def register_sample(regs):
+    """A fixed, seeded sample of a register array (12 x 23 x 2^20 bytes per step at config 2, too large to
+    write whole), as float32: distinct positions, the same on every run, so two builds can be compared."""
+    import torch
+    idx = np.sort(np.random.default_rng(0).choice(regs.numel(), min(REGISTER_SAMPLE, regs.numel()), replace=False))
+    return regs.reshape(-1)[torch.from_numpy(idx).to(regs.device)].float()
+
+
+def write_outputs(directory, arrays):
+    """Write each array (tensor or numpy) as <directory>/<name>.npy; float32 / float64 only, 64 MiB in all."""
+    arrays = {name: a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a) for name, a in arrays.items()}
+    bad = [name for name, a in arrays.items() if a.dtype not in (np.float32, np.float64)]
+    total = sum(a.nbytes for a in arrays.values())
+    if bad or total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes, non-float arrays {bad}")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(args):
     if args.config == 3:
         return run_ours_config3(args)
@@ -411,6 +440,12 @@ def run_ours(args):
     ms_step, res = timed(lambda: step_resident(time_k2=True), args.steps)
     launches_timed = eng.lib.dd_kernel_launches() - launches0     # counted inside the library, not a formula
     sampler.active = False
+    outputs = {}
+    if args.dump_outputs:     # the last timed step's results, taken before the serialized K2 pass below rewrites regs
+        leaf_cards, (prog, full) = res
+        outputs = {"leaf_cards": leaf_cards, "prefix_union_cards": prog, "registers_sample": register_sample(regs)}
+        if full is not None:
+            outputs["union_cards"] = full
     # K2's own duration: with several streams in flight the per-launch events above include time shared
     # with the other stream's kernels, so the roofline uses a serialized pass over the same 12
     # genomes taken right after the timed region (same clocks, L2 displaced by the other genomes).
@@ -430,13 +465,17 @@ def run_ours(args):
     for _ in range(max(args.warmup, 3)):
         step_e2e()
     sampler.active = True
-    ms_e2e, _ = timed(step_e2e, args.steps)
+    ms_e2e, res_e2e = timed(step_e2e, args.steps)
     sampler.stop_flag = True
+    if args.dump_outputs:
+        outputs.update(zip(("e2e_leaf_cards", "e2e_prefix_union_cards", "e2e_union_cards"), res_e2e))
 
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
 
     total_bases = bases * world  # every rank holds the same number of genomes; sizes differ by < 0.1 %
     value = total_bases / (ms_step / 1e3) / 1e9
@@ -649,19 +688,26 @@ def run_ours_config3(args):
     k2_events.clear()
     sampler.active = True
     launches0 = eng.lib.dd_kernel_launches()
-    ms_step, _ = timed(step_resident, args.steps)
+    ms_step, res = timed(step_resident, args.steps)
     launches_timed = eng.lib.dd_kernel_launches() - launches0
     sampler.active = False
+    outputs = {}
+    if args.dump_outputs:     # the last timed step's results, taken before the e2e steps below rewrite regs
+        outputs = {"leaf_cards": res[0], "prefix_union_cards": res[1], "registers_sample": register_sample(regs)}
     k2_ms = [a.elapsed_time(b) for a, b in k2_events]
     for _ in range(max(args.warmup, 3)):
         step_e2e()
     sampler.active = True
-    ms_e2e, _ = timed(step_e2e, args.steps)
+    ms_e2e, res_e2e = timed(step_e2e, args.steps)
     sampler.stop_flag = True
+    if args.dump_outputs:
+        outputs.update(e2e_leaf_cards=res_e2e[0], e2e_prefix_union_cards=res_e2e[1])
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     total_bases = bases * world
     peaks = {}
     try:
@@ -718,7 +764,15 @@ def main():
                     help="BASELINE.json workload: 2 = 12 x 5 Mbp per GPU (default, the metric's configuration), "
                          "3 = one 3.1 Gbp assembly per GPU, k = 2..32")
     ap.add_argument("--bases", type=float, default=3.1e9, help="config 3: bases per genome")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy: "
+                         "float64 cardinalities and a fixed sample of the registers as float32 (rank 0).  Only with "
+                         "--impl ours: it compares builds of this project, and the CPU arm keeps no results")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     _claim_stdout()
     if args.impl == "reference":
         run_reference(args)

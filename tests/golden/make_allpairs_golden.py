@@ -5,11 +5,11 @@ The reference's `go()` cannot run as shipped (undefined `args.name`, helpers/all
 `run_fneighbor`, :418), so this script replays the part of it that can -- the command list (:356-370),
 `mp_runner` on every command with the oracle-backed `dashing` stand-in first on PATH (oracle/shims),
 `delta_summarize`, `kij_summarize`, `j_summarize` and `summ_to_phylip` (:381-432) -- calling the
-reference's own functions, imported from /root/reference.  The fixtures pin the HOST LOGIC of
+reference's own functions, imported from the checkout DANDD_REFERENCE names.  The fixtures pin the HOST LOGIC of
 dandd_b200/helpers/allpairs.py to the reference's behaviour; the cardinalities are the oracle's, printed
 by the stand-in with six decimals as `dashing hll` text output is parsed (parity unpinned, see
-oracle/dandd_oracle.c).  Run from the repository root (build container only):
-    python tests/golden/make_allpairs_golden.py
+oracle/dandd_oracle.c).  Run from the repository root:
+    DANDD_REFERENCE=<checkout of the reference> python tests/golden/make_allpairs_golden.py
 """
 import importlib.util
 import json
@@ -20,9 +20,9 @@ import tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import pyoracle  # noqa: E402
-from tests.util import make_dataset  # noqa: E402
+from tests.util import make_dataset, reference_path  # noqa: E402
 
-REF = "/root/reference/helpers/allpairs.py"
+REF = reference_path("helpers", "allpairs.py")
 CASES = {
     # name: (genomes, length, seed, substitution rate, klist, nest, extra)
     "six_p12": (6, 20000, 71, 0.05, list(range(8, 21)), 4096, ""),
@@ -68,6 +68,8 @@ def run_case(ref, work, case):
 
 
 def main():
+    if not REF:
+        sys.exit("set DANDD_REFERENCE to a checkout of the reference")
     ref = load_reference()
     work = tempfile.mkdtemp(prefix="allpairs_golden_")
     bindir = pyoracle.install_shims(os.path.join(work, "bin"))

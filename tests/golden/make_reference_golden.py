@@ -1,4 +1,4 @@
-"""Runs the UNMODIFIED reference Python (/root/reference/lib/dandd) on small synthetic datasets
+"""Runs the UNMODIFIED reference Python (lib/dandd of the checkout DANDD_REFERENCE names) on small synthetic datasets
 with oracle-backed stand-ins for dashing / kmc / kmc_tools / parallel first on PATH
 (oracle/shims, SURVEY.md Appendix C technique) and records what it produced -- deltas, argmax k,
 cardinalities, sketchdb layout, progressive and KIJ tables -- as tests/golden/reference_runs.json.
@@ -7,9 +7,8 @@ These fixtures pin the HOST LOGIC of the drop-in layer (dandd_b200/lib/*) to the
 behaviour: the tests re-create the same inputs and require the same outputs.  They cannot pin the
 arithmetic to real Dashing/KMC (absent here; parity unpinned, see oracle/dandd_oracle.c).
 
-The reference can only be imported in the build container (/root/reference is not on the GPU
-box), hence committed fixtures.  Run from the repository root:
-    python tests/golden/make_reference_golden.py
+The reference is not part of this repository, hence committed fixtures.  Run from the repository root:
+    DANDD_REFERENCE=<checkout of the reference> python tests/golden/make_reference_golden.py
 """
 import csv
 import json
@@ -23,9 +22,9 @@ import tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import pyoracle  # noqa: E402
-from tests.util import make_dataset  # noqa: E402
+from tests.util import make_dataset, reference_path  # noqa: E402
 
-REF = "/root/reference/lib"
+REF = reference_path("lib")
 
 # --exact is broken as shipped (KMCSketchObj.sketch_check <-> check_cardinality recurse forever,
 # SURVEY.md App. B).  The golden for exact mode is produced with that ONE method replaced at run
@@ -164,6 +163,8 @@ def exact_runs(work, bindir, data5, gold):
 
 
 def main():
+    if not REF:
+        sys.exit("set DANDD_REFERENCE to a checkout of the reference")
     work = tempfile.mkdtemp(prefix="dandd_golden_")
     bindir = pyoracle.install_shims(os.path.join(work, "bin"))
     gold = {"generator": "tests/golden/make_reference_golden.py", "runs": {}}

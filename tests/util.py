@@ -109,6 +109,15 @@ def kmask_of(ks):
     return m
 
 
+def reference_path(*parts):
+    """A path inside the checkout of the reference project (github.com/jessicabonnie/dandd) that the
+    DANDD_REFERENCE environment variable names, or None without one: the tests that run the reference
+    beside the drop-in skip then, and the fixtures under tests/golden/ hold what it produced."""
+    import os
+    root = os.environ.get("DANDD_REFERENCE")
+    return os.path.join(root, *parts) if root else None
+
+
 def make_dataset(directory, n_genomes, length, seed, sub=0.03, indel=0.002, prefix="g"):
     """n mutated copies of one random ancestor, written as <prefix><i>.fasta (multi-record, odd line
     width).  Deterministic: the golden generator and the tests call this with the same arguments."""

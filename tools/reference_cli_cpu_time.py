@@ -3,7 +3,7 @@
 behind stand-in `dashing` / `parallel` executables (oracle/shims) -- the "reference-equivalent CPU
 proxy" of SURVEY.md 8(d): same process topology as the reference (one single-threaded process per
 (file, k), floor(0.95 * cores) at a time, genomes sequential, one `dashing union` + `dashing card`
-process per prefix union).  Only runs where /root/reference exists (the build container); the
+process per prefix union).  Needs DANDD_REFERENCE to name a checkout of the reference; the
 result is committed under profiles/.   usage: reference_cli_cpu_time.py [n_orderings] [out.json]"""
 import json
 import os
@@ -19,11 +19,14 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bench  # noqa: E402
 from oracle import pyoracle  # noqa: E402
+from tests.util import reference_path  # noqa: E402
 
-REF = "/root/reference/lib"
+REF = reference_path("lib")
 
 
 def main():
+    if not REF:
+        sys.exit("set DANDD_REFERENCE to a checkout of the reference")
     n_ord = int(sys.argv[1]) if len(sys.argv) > 1 else 30
     out_json = sys.argv[2] if len(sys.argv) > 2 else None
     cores = os.cpu_count() or 1
