@@ -436,6 +436,70 @@ int dd_exact_count(void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64
     return DD_OK;
 }
 
+// ---- K7 ------------------------------------------------------------------------------------------
+static int sm_count_now() {
+    int dev = 0, sms = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+        return 148;
+    return sms > 0 ? sms : 148;
+}
+static int pairs_check(int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams, const void *ws, size_t ws_bytes,
+                       const char *fn) {
+    if (!ws) return fail(DD_ERR_ARG, "%s: null workspace", fn);
+    if (k < 1 || k > DD_EXACT_MAXK) return fail(DD_ERR_ARG, "%s: k=%d outside [1,%d]", fn, k, DD_EXACT_MAXK);
+    if (capacity < 1024 || (capacity & (capacity - 1))) return fail(DD_ERR_ARG, "%s: capacity must be a power of two >= 1024", fn);
+    if (max_nodes >= 0xFFFFFFFFull) return fail(DD_ERR_ARG, "%s: max_nodes must be below 2^32 - 1", fn);
+    if (k > 64 && (max_streams < 1 || max_streams > 65536))   // an entry keeps the stream index in 16 bits
+        return fail(DD_ERR_ARG, "%s: k > 64 needs 1 <= max_streams <= 65536", fn);
+    if (ws_bytes < dd::exact_pairs_workspace_bytes(k, capacity, max_nodes, max_streams))
+        return fail(DD_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, ws_bytes,
+                    dd::exact_pairs_workspace_bytes(k, capacity, max_nodes, max_streams));
+    return DD_OK;
+}
+size_t dd_exact_pairs_workspace_bytes(int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams) {
+    return dd::exact_pairs_workspace_bytes(k, capacity, max_nodes, max_streams);
+}
+int dd_exact_pairs_begin(void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams,
+                         dd_stream stream) {
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, "dd_exact_pairs_begin")) return rc;
+    DD_CUDA(dd::exact_pairs_begin(d_ws, k, capacity, max_streams, S(stream)), "dd_exact_pairs_begin");
+    return DD_OK;
+}
+int dd_exact_pairs_insert_shard(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end, int k,
+                                int canon, uint32_t genome, void *d_ws, size_t ws_bytes, uint64_t capacity, uint64_t max_nodes,
+                                uint32_t max_streams, uint32_t shard_rank, uint32_t shard_world, dd_stream stream) {
+    if (!d_codes || !d_invalid) return fail(DD_ERR_ARG, "dd_exact_pairs_insert: null pointer");
+    if (genome == 0xFFFFFFFFu) return fail(DD_ERR_ARG, "dd_exact_pairs_insert: genome index out of range");
+    if (shard_world < 1 || shard_rank >= shard_world || shard_world > 65536)
+        return fail(DD_ERR_ARG, "dd_exact_pairs_insert: shard %u of %u", shard_rank, shard_world);
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, "dd_exact_pairs_insert")) return rc;
+    DD_CUDA(dd::exact_pairs_insert(d_codes, d_invalid, sym_begin, sym_end, k, canon, genome, d_ws, capacity, max_nodes,
+                                   max_streams, shard_rank, shard_world, S(stream)),
+            "dd_exact_pairs_insert");
+    return DD_OK;
+}
+int dd_exact_pairs_accumulate(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                              uint32_t max_streams, int64_t n_genomes, uint64_t *d_inter, dd_stream stream) {
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, "dd_exact_pairs_accumulate")) return rc;
+    if (n_genomes < 0 || n_genomes > 0xFFFFFFFFll) return fail(DD_ERR_ARG, "dd_exact_pairs_accumulate: n_genomes=%lld", (long long)n_genomes);
+    if (n_genomes > 1 && !d_inter) return fail(DD_ERR_ARG, "dd_exact_pairs_accumulate: null output");
+    DD_CUDA(dd::exact_pairs_accumulate(d_ws, k, capacity, max_streams, (uint64_t)n_genomes, d_inter, sm_count_now(), S(stream)),
+            "dd_exact_pairs_accumulate");
+    return DD_OK;
+}
+int dd_exact_pair_popc(const void *d_row_ws, int64_t row0, int nr, const void *d_col_ws, int64_t col0, int nc, size_t ws_stride,
+                       int k, int64_t n_genomes, uint64_t *d_inter, dd_stream stream) {
+    if (!d_row_ws || !d_col_ws || !d_inter) return fail(DD_ERR_ARG, "dd_exact_pair_popc: null pointer");
+    if (k < 1 || k > DD_EXACT_BITMAP_MAXK) return fail(DD_ERR_ARG, "dd_exact_pair_popc: k=%d outside [1,%d]", k, DD_EXACT_BITMAP_MAXK);
+    if (ws_stride < dd::exact_workspace_bytes(k, 0) || ws_stride % 16)
+        return fail(DD_ERR_WORKSPACE, "dd_exact_pair_popc: stride %zu below the K5 workspace of k=%d or not 16-byte aligned", ws_stride, k);
+    if (nr < 0 || nc < 0 || row0 < 0 || col0 < 0 || row0 + nr > n_genomes || col0 + nc > n_genomes)
+        return fail(DD_ERR_ARG, "dd_exact_pair_popc: genome block outside [0,%lld)", (long long)n_genomes);
+    DD_CUDA(dd::exact_pair_popc(d_row_ws, row0, nr, d_col_ws, col0, nc, ws_stride, k, n_genomes, d_inter, sm_count_now(), S(stream)),
+            "dd_exact_pair_popc");
+    return DD_OK;
+}
+
 // ---- host-buffer path -----------------------------------------------------------------------------
 namespace {
 constexpr size_t kHostChunk = (size_t)32 << 20;  // text bytes per H2D / pack / sketch round

@@ -55,14 +55,50 @@ __device__ __forceinline__ bool mine(uint64_t h, uint32_t shard_rank, uint32_t s
     return shard_world <= 1u || (uint32_t)(h >> 40) % shard_world == shard_rank;
 }
 
-template <bool kBitmap>
+// What an insert kernel does once it has found or claimed the slot of a k-mer.  The probe loops are
+// shared; K5 counts the keys it claimed, K7 (pair intersections) records which genome holds the key.
+struct CountFresh {  // K5: distinct keys
+    unsigned long long fresh = 0;
+    __device__ __forceinline__ void key(uint64_t, bool claimed) { fresh += claimed; }
+    __device__ __forceinline__ void ones(ExactWsHeader *hdr) { if (atomicExch(&hdr->saw_ones, 1ull) == 0ull) ++fresh; }
+    __device__ __forceinline__ void finish(ExactWsHeader *hdr) {   // one global add per warp
+        fresh = __reduce_add_sync(0xffffffffu, (unsigned)fresh);
+        if ((threadIdx.x & 31) == 0 && fresh) atomicAdd(&hdr->count, fresh);
+    }
+};
+
+constexpr uint32_t kNil = 0xFFFFFFFFu;
+struct PairNode {
+    uint32_t genome, next;
+};
+// K7: slot s keeps (last genome pushed, head of its node list) in lh[s]; the all-ones key, which cannot
+// live in the table, uses the extra slot lh[capacity].  Genomes are inserted one after another, so the
+// first thread of genome g to reach a slot is the one whose exchange returns something other than g.
+struct PushGenome {
+    uint2 *lh;
+    PairNode *nodes;
+    uint64_t max_nodes, capacity;
+    uint32_t genome;
+    ExactWsHeader *hdr;
+    __device__ __forceinline__ void push(uint64_t slot) {
+        if (atomicExch(&lh[slot].x, genome) == genome) return;
+        const unsigned long long n = atomicAdd(&hdr->n_nodes, 1ull);
+        if (n >= max_nodes) { hdr->overflow = 1; return; }
+        nodes[n].genome = genome;
+        nodes[n].next = atomicExch(&lh[slot].y, (uint32_t)n);
+    }
+    __device__ __forceinline__ void key(uint64_t slot, bool) { push(slot); }
+    __device__ __forceinline__ void ones(ExactWsHeader *) { push(capacity); }
+    __device__ __forceinline__ void finish(ExactWsHeader *) {}
+};
+
+template <bool kBitmap, class Action>
 __global__ void __launch_bounds__(kExactThreads)
 exact_insert_kernel(const uint32_t *__restrict__ codes, const uint32_t *__restrict__ invalid, uint64_t sym_begin,
                     uint64_t sym_end, int k, int canon, ExactWsHeader *hdr, void *table, uint64_t capacity,
-                    uint32_t shard_rank, uint32_t shard_world) {
+                    uint32_t shard_rank, uint32_t shard_world, Action act) {
     const uint64_t w = (sym_begin >> 4) + (uint64_t)blockIdx.x * kExactThreads + threadIdx.x;
     const uint64_t s0 = w << 4;
-    unsigned long long fresh = 0;
     if (s0 < sym_end) {
         const uint32_t w0 = __ldg(codes + w);
         const uint32_t w1 = w >= 1 ? __ldg(codes + w - 1) : 0u;
@@ -86,7 +122,7 @@ exact_insert_kernel(const uint32_t *__restrict__ codes, const uint32_t *__restri
                 if (!(__ldcg(word) & bit)) atomicOr(word, bit);
             } else {
                 if (v == kEmptyKey) {  // cannot be stored: it is the empty marker
-                    if (atomicExch(&hdr->saw_ones, 1ull) == 0ull) ++fresh;
+                    act.ones(hdr);
                     continue;
                 }
                 unsigned long long *tab = static_cast<unsigned long long *>(table);
@@ -96,19 +132,15 @@ exact_insert_kernel(const uint32_t *__restrict__ codes, const uint32_t *__restri
                 for (;;) {
                     unsigned long long cur = __ldcg(tab + slot);
                     if (cur == kEmptyKey) cur = atomicCAS(tab + slot, kEmptyKey, (unsigned long long)v);
-                    if (cur == kEmptyKey) { ++fresh; break; }
-                    if (cur == v) break;
+                    if (cur == kEmptyKey) { act.key(slot, true); break; }
+                    if (cur == v) { act.key(slot, false); break; }
                     slot = (slot + 1) & mask;
                     if (++probes > mask) { hdr->overflow = 1; break; }
                 }
             }
         }
     }
-    if (!kBitmap) {
-        // one global add per warp
-        fresh = __reduce_add_sync(0xffffffffu, (unsigned)fresh);
-        if ((threadIdx.x & 31) == 0 && fresh) atomicAdd(&hdr->count, fresh);
-    }
+    if (!kBitmap) act.finish(hdr);
 }
 
 // ---- k = 33..64: 128-bit keys ---------------------------------------------------------------------
@@ -123,13 +155,13 @@ __device__ __forceinline__ ulonglong2 cas128(ulonglong2 *addr, ulonglong2 cmp, u
     return old;
 }
 
+template <class Action>
 __global__ void __launch_bounds__(kExactThreads)
 exact_insert_wide_kernel(const uint32_t *__restrict__ codes, const uint32_t *__restrict__ invalid, uint64_t sym_begin,
                          uint64_t sym_end, int k, int canon, ExactWsHeader *hdr, ulonglong2 *tab, uint64_t capacity,
-                         uint32_t shard_rank, uint32_t shard_world) {
+                         uint32_t shard_rank, uint32_t shard_world, Action act) {
     const uint64_t w = (sym_begin >> 4) + (uint64_t)blockIdx.x * kExactThreads + threadIdx.x;
     const uint64_t s0 = w << 4;
-    unsigned long long fresh = 0;
     if (s0 < sym_end) {
         uint32_t c[5], I[5];
         const uint64_t iw = w >> 1;
@@ -147,7 +179,7 @@ exact_insert_wide_kernel(const uint32_t *__restrict__ codes, const uint32_t *__r
             if (valid_run_long(I, sm_base + (uint32_t)j) < k) continue;
             const U128 v = kmer128_at(c, j, k, canon != 0);
             if (v.lo == kEmptyKey && v.hi == kEmptyKey) {  // cannot be stored: it is the empty marker (rank 0's)
-                if (shard_rank == 0u && atomicExch(&hdr->saw_ones, 1ull) == 0ull) ++fresh;
+                if (shard_rank == 0u) act.ones(hdr);
                 continue;
             }
             const uint64_t hv = slot_hash(v.lo ^ slot_hash(v.hi));
@@ -158,28 +190,28 @@ exact_insert_wide_kernel(const uint32_t *__restrict__ codes, const uint32_t *__r
             for (;;) {
                 // a matching read settles it; anything else is decided by the CAS result alone
                 const ulonglong2 seen = __ldcg(tab + slot);
-                if (seen.x == key.x && seen.y == key.y) break;
+                if (seen.x == key.x && seen.y == key.y) { act.key(slot, false); break; }
                 const ulonglong2 old = cas128(tab + slot, empty, key);
-                if (old.x == kEmptyKey && old.y == kEmptyKey) { ++fresh; break; }
-                if (old.x == key.x && old.y == key.y) break;
+                if (old.x == kEmptyKey && old.y == kEmptyKey) { act.key(slot, true); break; }
+                if (old.x == key.x && old.y == key.y) { act.key(slot, false); break; }
                 slot = (slot + 1) & mask;
                 if (++probes > mask) { hdr->overflow = 1; break; }
             }
         }
     }
-    fresh = __reduce_add_sync(0xffffffffu, (unsigned)fresh);
-    if ((threadIdx.x & 31) == 0 && fresh) atomicAdd(&hdr->count, fresh);
+    act.finish(hdr);
 }
 
 // ---- k = 65..256: (fingerprint, reference) entries ------------------------------------------------
 constexpr int kRefPosBits = 48;
 
 // one thread: find or append `codes` in the set's stream table; publish its index for the insert kernel
-__global__ void exact_register_stream_kernel(ExactWsHeader *hdr, const uint32_t **streams, const uint32_t *codes) {
+__global__ void exact_register_stream_kernel(ExactWsHeader *hdr, const uint32_t **streams, const uint32_t *codes,
+                                             unsigned max_streams) {
     unsigned long long n = hdr->n_streams, i = 0;
     while (i < n && streams[i] != codes) ++i;
     if (i == n) {
-        if (n >= kMaxStreams) {
+        if (n >= max_streams) {
             hdr->overflow = 1;
             i = 0;
         } else {
@@ -190,13 +222,13 @@ __global__ void exact_register_stream_kernel(ExactWsHeader *hdr, const uint32_t 
     hdr->cur_stream = i;
 }
 
+template <class Action>
 __global__ void __launch_bounds__(kExactThreads)
 exact_insert_long_kernel(const uint32_t *__restrict__ codes, const uint32_t *__restrict__ invalid, uint64_t sym_begin,
                          uint64_t sym_end, int k, int canon, ExactWsHeader *hdr, ulonglong2 *tab, uint64_t capacity,
-                         const uint32_t *const *streams, uint32_t shard_rank, uint32_t shard_world) {
+                         const uint32_t *const *streams, uint32_t shard_rank, uint32_t shard_world, Action act) {
     const uint64_t w = (sym_begin >> 4) + (uint64_t)blockIdx.x * kExactThreads + threadIdx.x;
     const uint64_t s0 = w << 4;
-    unsigned long long fresh = 0;
     if (s0 < sym_end) {
         const int j_lo = sym_begin > s0 ? (int)(sym_begin - s0) : 0;
         const int j_hi = sym_end - s0 < 16 ? (int)(sym_end - s0) : 16;
@@ -227,22 +259,21 @@ exact_insert_long_kernel(const uint32_t *__restrict__ codes, const uint32_t *__r
                 ulonglong2 seen = __ldcg(tab + slot);
                 if (seen.x == kEmptyKey && seen.y == kEmptyKey) {
                     seen = cas128(tab + slot, empty, entry);
-                    if (seen.x == kEmptyKey && seen.y == kEmptyKey) { ++fresh; break; }
+                    if (seen.x == kEmptyKey && seen.y == kEmptyKey) { act.key(slot, true); break; }
                 }
                 if (seen.x == h) {   // same fingerprint: the k-mer at the referenced occurrence decides
                     uint64_t other[kLongWords];
                     kmer_long_at(streams[seen.y >> kRefPosBits], seen.y & ((1ull << kRefPosBits) - 1ull), k, canon != 0, other);
                     bool same = true;
                     for (int t = 0; t < W; ++t) same = same && other[t] == key[t];
-                    if (same) break;
+                    if (same) { act.key(slot, false); break; }
                 }
                 slot = (slot + 1) & mask;
                 if (++probes > mask) { hdr->overflow = 1; break; }
             }
         }
     }
-    fresh = __reduce_add_sync(0xffffffffu, (unsigned)fresh);
-    if ((threadIdx.x & 31) == 0 && fresh) atomicAdd(&hdr->count, fresh);
+    act.finish(hdr);
 }
 
 __global__ void __launch_bounds__(256) bitmap_count_kernel(const uint32_t *__restrict__ bm, size_t nwords,
@@ -269,31 +300,41 @@ cudaError_t exact_begin(void *d_ws, int k, uint64_t capacity, cudaStream_t strea
     return cudaSuccess;
 }
 
-cudaError_t exact_insert(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end,
-                         int k, int canon, void *d_ws, uint64_t capacity, uint32_t shard_rank, uint32_t shard_world,
-                         cudaStream_t stream) {
+// The probe loops of the three key layouts, for either action.  kBitmap: k <= DD_EXACT_BITMAP_MAXK sets of K5.
+template <class Action>
+static cudaError_t insert_with(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end,
+                               int k, int canon, ExactWsHeader *hdr, void *table, uint64_t capacity, const uint32_t **streams,
+                               unsigned max_streams, bool bitmap, uint32_t shard_rank, uint32_t shard_world, Action act,
+                               cudaStream_t stream) {
     if (sym_end <= sym_begin) return cudaSuccess;
     const size_t nwords = (size_t)((sym_end - sym_begin + 15) / 16 + 2);  // +2: the range need not start on a word boundary
     const unsigned grid = (unsigned)((nwords + kExactThreads - 1) / kExactThreads);
     if (k > 64) {
         if (sym_end >> kRefPosBits) return cudaErrorInvalidValue;
-        const uint32_t **streams = reinterpret_cast<const uint32_t **>(static_cast<uint8_t *>(ex_tab(d_ws)) + exact_table_bytes(k, capacity));
-        DD_COUNT_LAUNCH(), exact_register_stream_kernel<<<1, 1, 0, stream>>>(ex_hdr(d_ws), streams, d_codes);
+        DD_COUNT_LAUNCH(), exact_register_stream_kernel<<<1, 1, 0, stream>>>(hdr, streams, d_codes, max_streams);
         DD_COUNT_LAUNCH(), exact_insert_long_kernel<<<grid, kExactThreads, 0, stream>>>(d_codes, d_invalid, sym_begin, sym_end, k, canon,
-                                                                    ex_hdr(d_ws), static_cast<ulonglong2 *>(ex_tab(d_ws)),
-                                                                    capacity, streams, shard_rank, shard_world);
+                                                                    hdr, static_cast<ulonglong2 *>(table),
+                                                                    capacity, streams, shard_rank, shard_world, act);
     } else if (k > 32)
         DD_COUNT_LAUNCH(), exact_insert_wide_kernel<<<grid, kExactThreads, 0, stream>>>(d_codes, d_invalid, sym_begin, sym_end, k, canon,
-                                                                    ex_hdr(d_ws), static_cast<ulonglong2 *>(ex_tab(d_ws)),
-                                                                    capacity, shard_rank, shard_world);
-    else if (k <= DD_EXACT_BITMAP_MAXK)
+                                                                    hdr, static_cast<ulonglong2 *>(table),
+                                                                    capacity, shard_rank, shard_world, act);
+    else if (bitmap)
         DD_COUNT_LAUNCH(), exact_insert_kernel<true><<<grid, kExactThreads, 0, stream>>>(d_codes, d_invalid, sym_begin, sym_end, k, canon,
-                                                                     ex_hdr(d_ws), ex_tab(d_ws), capacity, shard_rank, shard_world);
+                                                                     hdr, table, capacity, shard_rank, shard_world, act);
     else
         DD_COUNT_LAUNCH(), exact_insert_kernel<false><<<grid, kExactThreads, 0, stream>>>(d_codes, d_invalid, sym_begin, sym_end, k,
-                                                                      canon, ex_hdr(d_ws), ex_tab(d_ws), capacity, shard_rank,
-                                                                      shard_world);
+                                                                      canon, hdr, table, capacity, shard_rank,
+                                                                      shard_world, act);
     return cudaGetLastError();
+}
+
+cudaError_t exact_insert(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end,
+                         int k, int canon, void *d_ws, uint64_t capacity, uint32_t shard_rank, uint32_t shard_world,
+                         cudaStream_t stream) {
+    const uint32_t **streams = reinterpret_cast<const uint32_t **>(static_cast<uint8_t *>(ex_tab(d_ws)) + exact_table_bytes(k, capacity));
+    return insert_with(d_codes, d_invalid, sym_begin, sym_end, k, canon, ex_hdr(d_ws), ex_tab(d_ws), capacity, streams,
+                       kMaxStreams, k <= DD_EXACT_BITMAP_MAXK, shard_rank, shard_world, CountFresh{}, stream);
 }
 
 cudaError_t exact_count(void *d_ws, int k, uint64_t capacity, uint64_t *d_count, cudaStream_t stream) {
@@ -311,6 +352,231 @@ cudaError_t exact_count(void *d_ws, int k, uint64_t capacity, uint64_t *d_count,
         DD_COUNT_LAUNCH(), exact_publish_kernel<<<1, 1, 0, stream>>>(ex_hdr(d_ws), reinterpret_cast<unsigned long long *>(d_count));
     }
     return cudaGetLastError();
+}
+
+// ---- K7: |A n B| for every pair of genomes ------------------------------------------------------
+// Sparse path.  Workspace = [header | K5 key table (hash layout at every k) | k > 64: stream table |
+// (last, head) u32 pairs for capacity + 1 slots | node array].  Each genome's insert pushes one node
+// {genome, next} per key it holds onto that key's list; the accumulate kernel then adds 1 to pair (a, b)
+// for every two genomes on one list -- sum over keys of occ(occ-1)/2 increments.
+static size_t pairs_key_bytes(int k, uint64_t capacity) { return (size_t)capacity * (k > 32 ? 2 : 1) * sizeof(unsigned long long); }
+static size_t pairs_stream_bytes(int k, unsigned max_streams) { return k > 64 ? (size_t)max_streams * sizeof(const uint32_t *) : 0; }
+static size_t pairs_lh_offset(int k, uint64_t capacity, unsigned max_streams) {
+    return 256 + pairs_key_bytes(k, capacity) + pairs_stream_bytes(k, max_streams);
+}
+static size_t pairs_node_offset(int k, uint64_t capacity, unsigned max_streams) {
+    return pairs_lh_offset(k, capacity, max_streams) + (size_t)(capacity + 1) * sizeof(uint2);
+}
+size_t exact_pairs_workspace_bytes(int k, uint64_t capacity, uint64_t max_nodes, unsigned max_streams) {
+    return pairs_node_offset(k, capacity, max_streams) + (size_t)max_nodes * sizeof(PairNode);
+}
+
+cudaError_t exact_pairs_begin(void *d_ws, int k, uint64_t capacity, unsigned max_streams, cudaStream_t stream) {
+    uint8_t *ws = static_cast<uint8_t *>(d_ws);
+    cudaError_t e = cudaMemsetAsync(ws, 0, 256, stream);
+    if (e != cudaSuccess) return e;
+    if ((e = cudaMemsetAsync(ws + 256, 0xff, pairs_key_bytes(k, capacity), stream)) != cudaSuccess) return e;
+    if (k > 64 && (e = cudaMemsetAsync(ws + 256 + pairs_key_bytes(k, capacity), 0, pairs_stream_bytes(k, max_streams), stream)) != cudaSuccess)
+        return e;
+    return cudaMemsetAsync(ws + pairs_lh_offset(k, capacity, max_streams), 0xff, (size_t)(capacity + 1) * sizeof(uint2), stream);
+}
+
+cudaError_t exact_pairs_insert(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end, int k,
+                               int canon, uint32_t genome, void *d_ws, uint64_t capacity, uint64_t max_nodes,
+                               unsigned max_streams, uint32_t shard_rank, uint32_t shard_world, cudaStream_t stream) {
+    uint8_t *ws = static_cast<uint8_t *>(d_ws);
+    PushGenome act;
+    act.lh = reinterpret_cast<uint2 *>(ws + pairs_lh_offset(k, capacity, max_streams));
+    act.nodes = reinterpret_cast<PairNode *>(ws + pairs_node_offset(k, capacity, max_streams));
+    act.max_nodes = max_nodes;
+    act.capacity = capacity;
+    act.genome = genome;
+    act.hdr = ex_hdr(d_ws);
+    const uint32_t **streams = reinterpret_cast<const uint32_t **>(ws + 256 + pairs_key_bytes(k, capacity));
+    return insert_with(d_codes, d_invalid, sym_begin, sym_end, k, canon, ex_hdr(d_ws), ws + 256, capacity, streams,
+                       max_streams, /*bitmap=*/false, shard_rank, shard_world, act, stream);
+}
+
+__device__ __forceinline__ uint64_t pair_row(uint64_t a, uint64_t b, uint64_t n) {  // a < b
+    return a * (2 * n - a - 1) / 2 + (b - a - 1);
+}
+
+// Each warp takes 32 slots at a time (grid-stride) and walks the list of every occupied one in turn.  A
+// list is read 32 nodes at a time, every lane loading the
+// same node (one broadcast transaction); lane j keeps the j-th genome of the chunk.  Pairs inside a
+// chunk come from shuffles; a chunk is then paired with every later chunk of the list.  kSmem: the
+// pair counters of the whole job fit in shared memory, and each CTA adds its counters to the output
+// once at the end.
+template <bool kSmem>
+__global__ void __launch_bounds__(256)
+exact_pairs_accumulate_kernel(const ExactWsHeader *__restrict__ hdr, const uint2 *__restrict__ lh,
+                              const PairNode *__restrict__ nodes, uint64_t n_slots, uint64_t n_genomes,
+                              unsigned long long *out, uint64_t n_pairs) {
+    extern __shared__ uint32_t sm_count[];
+    if (hdr->overflow) {   // a full table or node array: the marker, never a count
+        for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_pairs; i += (uint64_t)gridDim.x * blockDim.x)
+            out[i] = kEmptyKey;
+        return;
+    }
+    if (kSmem) {
+        for (uint64_t i = threadIdx.x; i < n_pairs; i += blockDim.x) sm_count[i] = 0;
+        __syncthreads();
+    }
+    const unsigned lane = threadIdx.x & 31;
+    auto add = [&](uint32_t a, uint32_t b) {
+        if (a >= n_genomes || b >= n_genomes) return;   // outside the caller's genome range: never written out of bounds
+        const uint64_t r = a < b ? pair_row(a, b, n_genomes) : pair_row(b, a, n_genomes);
+        if (kSmem) atomicAdd(&sm_count[r], 1u);
+        else atomicAdd(&out[r], 1ull);
+    };
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    for (uint64_t base = ((uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 32; base < n_slots; base += warps * 32) {
+        // 32 slots per coalesced load; the warp then walks the lists of the occupied ones one by one
+        const uint32_t head = base + lane < n_slots ? __ldg(&lh[base + lane].y) : kNil;
+        for (unsigned occ = __ballot_sync(0xffffffffu, head != kNil); occ; occ &= occ - 1) {
+            uint32_t a_at = __shfl_sync(0xffffffffu, head, __ffs(occ) - 1);
+            while (a_at != kNil) {
+                uint32_t ga = 0, cur = a_at;
+                int na = 0;
+                for (; na < 32 && cur != kNil; ++na) {
+                    const PairNode nd = nodes[cur];
+                    if (lane == (unsigned)na) ga = nd.genome;
+                    cur = nd.next;
+                }
+                a_at = cur;
+                for (int d = 1; d < na; ++d) {
+                    const uint32_t gb = __shfl_down_sync(0xffffffffu, ga, d);
+                    if ((int)lane + d < na) add(ga, gb);
+                }
+                for (uint32_t b_at = a_at; b_at != kNil;) {
+                    uint32_t gb = 0;
+                    int nb = 0;
+                    for (; nb < 32 && b_at != kNil; ++nb) {
+                        const PairNode nd = nodes[b_at];
+                        if (lane == (unsigned)nb) gb = nd.genome;
+                        b_at = nd.next;
+                    }
+                    for (int i = 0; i < na; ++i) {
+                        const uint32_t g = __shfl_sync(0xffffffffu, ga, i);
+                        if ((int)lane < nb) add(g, gb);
+                    }
+                }
+            }
+        }
+    }
+    if (kSmem) {
+        __syncthreads();
+        for (uint64_t i = threadIdx.x; i < n_pairs; i += blockDim.x)
+            if (sm_count[i]) atomicAdd(&out[i], (unsigned long long)sm_count[i]);
+    }
+}
+
+constexpr size_t kPairSmemBytes = 96 * 1024;
+
+cudaError_t exact_pairs_accumulate(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
+                                   uint64_t *d_inter, int sm_count, cudaStream_t stream) {
+    const uint8_t *ws = static_cast<const uint8_t *>(d_ws);
+    const uint64_t n_pairs = n_genomes * (n_genomes - 1) / 2;
+    if (n_pairs == 0) return cudaSuccess;
+    const ExactWsHeader *hdr = static_cast<const ExactWsHeader *>(d_ws);
+    const uint2 *lh = reinterpret_cast<const uint2 *>(ws + pairs_lh_offset(k, capacity, max_streams));
+    const PairNode *nodes = reinterpret_cast<const PairNode *>(ws + pairs_node_offset(k, capacity, max_streams));
+    unsigned long long *out = reinterpret_cast<unsigned long long *>(d_inter);
+    const uint64_t n_slots = capacity + 1;
+    const size_t smem = (size_t)n_pairs * sizeof(uint32_t);
+    if (smem <= kPairSmemBytes) {
+        cudaError_t e = cudaFuncSetAttribute(exact_pairs_accumulate_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             (int)kPairSmemBytes);
+        if (e != cudaSuccess) return e;
+        // few CTAs: every CTA pays one pass over the counters at the start and one at the end
+        const unsigned grid = (unsigned)(sm_count * 2);
+        DD_COUNT_LAUNCH(), exact_pairs_accumulate_kernel<true><<<grid, 256, smem, stream>>>(hdr, lh, nodes, n_slots, n_genomes, out, n_pairs);
+    } else {
+        const uint64_t want = (n_slots + 255) / 256;   // one 32-slot group per warp
+        const unsigned grid = (unsigned)(want < (uint64_t)sm_count * 16 ? (want ? want : 1) : (uint64_t)sm_count * 16);
+        DD_COUNT_LAUNCH(), exact_pairs_accumulate_kernel<false><<<grid, 256, 0, stream>>>(hdr, lh, nodes, n_slots, n_genomes, out, n_pairs);
+    }
+    return cudaGetLastError();
+}
+
+// Dense path: popc(A & B) over K5 presence bitmaps.  A CTA owns a tile of 8 row genomes x 8 column
+// genomes and a slice of the bitmap words: each word range of the 16 bitmaps is read once per tile
+// (from L2 when other tiles have just read it) and feeds 64 pair counters.
+constexpr int kPopcTile = 8;
+__global__ void __launch_bounds__(256)
+exact_pair_popc_kernel(const uint8_t *__restrict__ rows, int64_t row0, int nr, const uint8_t *__restrict__ cols, int64_t col0,
+                       int nc, size_t ws_stride, size_t nwords, int64_t n_genomes, int col_tiles, int64_t tile0,
+                       unsigned long long *out) {
+    const int64_t t = tile0 + blockIdx.y;
+    const int tr = (int)(t / col_tiles), tc = (int)(t % col_tiles);
+    const int r_lo = tr * kPopcTile, c_lo = tc * kPopcTile;
+    const int c_hi = min(nc, c_lo + kPopcTile);
+    if (row0 + r_lo >= col0 + c_hi - 1) return;   // no pair a < b in this tile
+    const uint32_t *ra[kPopcTile], *cb[kPopcTile];
+#pragma unroll
+    for (int i = 0; i < kPopcTile; ++i) {
+        const int r = min(r_lo + i, nr - 1), c = min(c_lo + i, nc - 1);   // clamped rows/columns are never counted
+        ra[i] = reinterpret_cast<const uint32_t *>(rows + (size_t)r * ws_stride + 256);
+        cb[i] = reinterpret_cast<const uint32_t *>(cols + (size_t)c * ws_stride + 256);
+    }
+    uint32_t acc[kPopcTile][kPopcTile];
+#pragma unroll
+    for (int i = 0; i < kPopcTile; ++i)
+#pragma unroll
+        for (int j = 0; j < kPopcTile; ++j) acc[i][j] = 0;
+    for (size_t w = (size_t)blockIdx.x * blockDim.x + threadIdx.x; w < nwords; w += (size_t)gridDim.x * blockDim.x) {
+        uint32_t a[kPopcTile], b[kPopcTile];
+#pragma unroll
+        for (int i = 0; i < kPopcTile; ++i) {
+            a[i] = __ldg(ra[i] + w);
+            b[i] = __ldg(cb[i] + w);
+        }
+#pragma unroll
+        for (int i = 0; i < kPopcTile; ++i)
+#pragma unroll
+            for (int j = 0; j < kPopcTile; ++j) acc[i][j] += __popc(a[i] & b[j]);
+    }
+    __shared__ unsigned long long tile[kPopcTile * kPopcTile];
+    if (threadIdx.x < kPopcTile * kPopcTile) tile[threadIdx.x] = 0;
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < kPopcTile; ++i)
+#pragma unroll
+        for (int j = 0; j < kPopcTile; ++j) {
+            const uint32_t v = __reduce_add_sync(0xffffffffu, acc[i][j]);
+            if ((threadIdx.x & 31) == 0 && v) atomicAdd(&tile[i * kPopcTile + j], (unsigned long long)v);
+        }
+    __syncthreads();
+    if (threadIdx.x < kPopcTile * kPopcTile) {
+        const int i = threadIdx.x / kPopcTile, j = threadIdx.x % kPopcTile;
+        const int64_t a = row0 + r_lo + i, b = col0 + c_lo + j;
+        if (r_lo + i < nr && c_lo + j < nc && a < b && tile[threadIdx.x])
+            atomicAdd(&out[pair_row((uint64_t)a, (uint64_t)b, (uint64_t)n_genomes)], tile[threadIdx.x]);
+    }
+}
+
+cudaError_t exact_pair_popc(const void *d_rows, int64_t row0, int nr, const void *d_cols, int64_t col0, int nc,
+                            size_t ws_stride, int k, int64_t n_genomes, uint64_t *d_inter, int sm_count, cudaStream_t stream) {
+    if (nr <= 0 || nc <= 0) return cudaSuccess;
+    const size_t nwords = exact_table_bytes(k, 0) / 4;
+    const int row_tiles = (nr + kPopcTile - 1) / kPopcTile, col_tiles = (nc + kPopcTile - 1) / kPopcTile;
+    const uint64_t tiles = (uint64_t)row_tiles * col_tiles;
+    // enough word slices to give every SM a few CTAs, none shorter than 4 words per thread
+    uint64_t slices = ((uint64_t)sm_count * 8 + tiles - 1) / tiles;
+    const uint64_t most = (nwords + 256 * 4 - 1) / (256 * 4);
+    if (slices > most) slices = most;
+    if (slices < 1) slices = 1;
+    for (uint64_t t0 = 0; t0 < tiles; t0 += 65535) {   // grid.y holds at most 65535 tiles per launch
+        const uint64_t nt = tiles - t0 < 65535 ? tiles - t0 : 65535;
+        const dim3 grid((unsigned)slices, (unsigned)nt);
+        DD_COUNT_LAUNCH(), exact_pair_popc_kernel<<<grid, 256, 0, stream>>>(static_cast<const uint8_t *>(d_rows), row0, nr,
+                                                                         static_cast<const uint8_t *>(d_cols), col0, nc, ws_stride,
+                                                                         nwords, n_genomes, col_tiles, (int64_t)t0,
+                                                                         reinterpret_cast<unsigned long long *>(d_inter));
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 }  // namespace dd

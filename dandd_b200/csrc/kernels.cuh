@@ -78,6 +78,7 @@ struct ExactWsHeader {
     unsigned long long saw_ones;  // the all-ones key (== the empty marker) was inserted
     unsigned long long cur_stream;  // k > 64: index (in the stream table) of the stream being inserted
     unsigned long long n_streams;   // k > 64: streams registered so far
+    unsigned long long n_nodes;     // K7: co-occurrence nodes pushed so far
 };
 size_t exact_workspace_bytes(int k, uint64_t capacity);
 cudaError_t exact_begin(void *d_ws, int k, uint64_t capacity, cudaStream_t stream);
@@ -85,5 +86,17 @@ cudaError_t exact_insert(const uint32_t *d_codes, const uint32_t *d_invalid, uin
                          int k, int canon, void *d_ws, uint64_t capacity, uint32_t shard_rank, uint32_t shard_world,
                          cudaStream_t stream);
 cudaError_t exact_count(void *d_ws, int k, uint64_t capacity, uint64_t *d_count, cudaStream_t stream);
+
+// ---- K7 (exact.cu): pair intersections.  Sparse: [ExactWsHeader | key table | streams | (last, head) | nodes]
+size_t exact_pairs_workspace_bytes(int k, uint64_t capacity, uint64_t max_nodes, unsigned max_streams);
+cudaError_t exact_pairs_begin(void *d_ws, int k, uint64_t capacity, unsigned max_streams, cudaStream_t stream);
+cudaError_t exact_pairs_insert(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end, int k,
+                               int canon, uint32_t genome, void *d_ws, uint64_t capacity, uint64_t max_nodes,
+                               unsigned max_streams, uint32_t shard_rank, uint32_t shard_world, cudaStream_t stream);
+cudaError_t exact_pairs_accumulate(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
+                                   uint64_t *d_inter, int sm_count, cudaStream_t stream);
+// Dense: K5 bitmap workspaces, ws_stride bytes apart, for genomes row0.. and col0..
+cudaError_t exact_pair_popc(const void *d_rows, int64_t row0, int nr, const void *d_cols, int64_t col0, int nc,
+                            size_t ws_stride, int k, int64_t n_genomes, uint64_t *d_inter, int sm_count, cudaStream_t stream);
 
 }  // namespace dd

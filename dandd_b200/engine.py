@@ -423,6 +423,151 @@ class Engine:
             raise DandDError("exact k-mer table overflowed; pass a larger capacity")
         return [int(v) for v in out]
 
+    # ---- K7 ---------------------------------------------------------------------------------
+    def exact_pair_intersections(self, seqs: Sequence[PackedSeq], k: int, canon: bool = True,
+                                 singles: Optional[Sequence[int]] = None, shard: Optional[tuple] = None) -> np.ndarray:
+        """|A n B| for every pair of `seqs` at k: uint64 [n(n-1)/2], pairs (0,1), (0,2) .. (n-2,n-1).
+        `singles` = |A| per sequence (exact_counts; with `shard`, this rank's shard of them) sizes the job
+        and picks the path: presence bitmaps and a popcount per pair where almost every genome holds
+        almost every k-mer (dense_pairs), else co-occurrence lists (sparse).  shard=(rank, world): only
+        this rank's key range, the ranks' results add up (dandd_b200.dist.sum_counts)."""
+        world = int(shard[1]) if shard is not None else 1
+        if singles is None:
+            singles = [self.exact_counts([s], k, canon, shard=shard)[0] for s in seqs]
+        if dense_pairs(k, singles, world):
+            return self.exact_pairs_dense(seqs, k, canon, shard=shard)
+        return self.exact_pairs_sparse(seqs, k, canon, singles, shard=shard)
+
+    def _pairs_budget(self) -> int:
+        """Share of the device memory a pass may take: what is free plus what torch holds cached but unused."""
+        free, _ = torch.cuda.mem_get_info(self.device)
+        cached = torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        return int((free + cached) * PAIR_BUDGET_SHARE)
+
+    def exact_pairs_sparse(self, seqs: Sequence[PackedSeq], k: int, canon: bool, singles: Sequence[int],
+                           shard: Optional[tuple] = None, passes: Optional[int] = None) -> np.ndarray:
+        """The co-occurrence-list path of exact_pair_intersections, in `passes` key-range passes (default:
+        as few as fit the memory budget, plan_pair_passes)."""
+        n = len(seqs)
+        out = np.zeros(n * (n - 1) // 2, dtype=np.uint64)
+        if n < 2:
+            return out
+        if k > 64 and n > 65536:
+            raise DandDError("exact pairs above k = 64 take at most 65536 genomes per job")
+        srank, sworld = (int(shard[0]), int(shard[1])) if shard is not None else (0, 1)
+        nsyms = [s.nsym for s in seqs]
+        plan = plan_pair_passes(singles, k, lambda c, m: int(self.lib.dd_exact_pairs_workspace_bytes(k, c, m, n)),
+                                self._pairs_budget(), passes)
+        self.last_pair_plan = dict(plan, path="sparse")
+        cap, nodes = plan["capacity"], plan["max_nodes"]
+        ws = self._buf(plan["ws_bytes"], "exact_pairs")
+        part = torch.zeros(len(out), dtype=torch.int64, device=self.device)
+        st = self.stream
+        for p in range(plan["passes"]):
+            sr, sw = pass_shard(srank, sworld, p, plan["passes"])
+            check(self.lib.dd_exact_pairs_begin(ws.data_ptr(), ws.numel(), k, cap, nodes, n, st), "dd_exact_pairs_begin")
+            for g, (s, ns) in enumerate(zip(seqs, nsyms)):
+                check(self.lib.dd_exact_pairs_insert_shard(s.codes.data_ptr(), s.invalid.data_ptr(), 0, ns, k, int(canon), g,
+                                                           ws.data_ptr(), ws.numel(), cap, nodes, n, sr, sw, st),
+                      "dd_exact_pairs_insert_shard")
+            part.zero_()
+            check(self.lib.dd_exact_pairs_accumulate(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part.data_ptr(), st),
+                  "dd_exact_pairs_accumulate")
+            got = part.cpu().numpy().view(np.uint64)
+            if (got == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
+                raise DandDError("exact pair table or node array overflowed; the single counts given understate the genomes")
+            out += got
+        del ws
+        self._ws.pop("exact_pairs", None)     # a pass may take half the device: not kept for later stages
+        return out
+
+    def exact_pairs_dense(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
+                          block: Optional[int] = None) -> np.ndarray:
+        """The bitmap path of exact_pair_intersections (k <= DD_EXACT_BITMAP_MAXK): one K5 presence bitmap
+        per genome, popc(A & B) per pair.  Genomes go through in blocks of `block` (default: as many as
+        two blocks of bitmaps fit the memory budget)."""
+        n = len(seqs)
+        if n < 2:
+            return np.zeros(n * (n - 1) // 2, dtype=np.uint64)
+        srank, sworld = (int(shard[0]), int(shard[1])) if shard is not None else (0, 1)
+        stride = (int(self.lib.dd_exact_workspace_bytes(k, 0)) + 255) // 256 * 256
+        if block is None:
+            block = max(1, min(n, self._pairs_budget() // (2 * stride)))
+        block = min(int(block), n)
+        nb = (n + block - 1) // block
+        self.last_pair_plan = {"path": "dense", "passes": 1, "block": block, "bitmap_bytes": stride}
+        rows = self._buf(block * stride, "pairs_rows")
+        cols = self._buf(block * stride, "pairs_cols") if nb > 1 else rows
+        out = torch.zeros(n * (n - 1) // 2, dtype=torch.int64, device=self.device)
+        st = self.stream
+
+        def fill(buf, g0):
+            for i, g in enumerate(range(g0, min(n, g0 + block))):
+                ws = buf.data_ptr() + i * stride
+                s = seqs[g]
+                check(self.lib.dd_exact_begin(ws, stride, k, 0, st), "dd_exact_begin")
+                check(self.lib.dd_exact_insert_shard(s.codes.data_ptr(), s.invalid.data_ptr(), 0, s.nsym, k, int(canon), ws, stride,
+                                                     0, srank, sworld, st), "dd_exact_insert_shard")
+
+        for bi in range(nb):
+            r0 = bi * block
+            fill(rows, r0)
+            nr = min(n, r0 + block) - r0
+            for bj in range(bi, nb):
+                c0 = bj * block
+                if bj != bi:
+                    fill(cols, c0)
+                cbuf = rows if bj == bi else cols
+                check(self.lib.dd_exact_pair_popc(rows.data_ptr(), r0, nr, cbuf.data_ptr(), c0, min(n, c0 + block) - c0, stride, k, n,
+                                                  out.data_ptr(), st), "dd_exact_pair_popc")
+        result = out.cpu().numpy().view(np.uint64).copy()
+        del rows, cols
+        for tag in ("pairs_rows", "pairs_cols"):
+            self._ws.pop(tag, None)
+        return result
+
+
+# Exact all pairs (K7): the bitmap path wins where 4^k bits per genome are cheap next to the number of k-mers a
+# genome holds -- then almost every genome holds almost every k-mer and the co-occurrence lists would hold
+# sum(occ^2) ~ n^2 4^k / 2 entries.  DENSE_BITS_PER_KMER is the crossover: 4^k / DENSE_BITS_PER_KMER <= mean |A|.
+DENSE_BITS_PER_KMER = 32
+PAIR_BUDGET_SHARE = 0.5      # share of the free device memory one pass of the pair job may take
+
+
+def dense_pairs(k: int, singles: Sequence[int], world: int = 1) -> bool:
+    """Whether exact_pair_intersections takes the bitmap path.  `singles` may be one key-range shard of the
+    counts (shard world `world`): the rule looks at whole genomes."""
+    if k > _lib.DD_EXACT_BITMAP_MAXK or not len(singles):
+        return False
+    mean = float(np.mean(np.asarray(singles, dtype=np.float64))) * world
+    return 4 ** k / DENSE_BITS_PER_KMER <= mean
+
+
+def pass_shard(rank: int, world: int, p: int, passes: int) -> tuple:
+    """Key range of pass p of rank `rank`: the ranks split the keys, every rank splits its range again over its
+    passes -- shard (rank + world * p) of (world * passes), so every key is handled by exactly one (rank, pass)."""
+    return rank + world * p, world * passes
+
+
+def plan_pair_passes(singles: Sequence[int], k: int, ws_bytes, budget: int, passes: Optional[int] = None) -> dict:
+    """Table capacity, node count and number of key-range passes for the sparse pair job.  singles: |A| per
+    genome in the key range to cover; ws_bytes(capacity, max_nodes) -> workspace bytes.  A pass holds about
+    1/passes of the keys: the table must take every distinct key of its range (at most sum |A|, at most 4^k)
+    at load <= 1/2, the node array one node per (genome, key).  Hash shares fluctuate: a margin is added."""
+    total = int(sum(int(s) for s in singles))
+    distinct = min(total, 4 ** k) if k < 32 else total
+    p = int(passes) if passes else 1
+    while True:
+        keys = -(-distinct // p)
+        capacity = 1024
+        while capacity < 2 * (keys + keys // 16) + 1024:
+            capacity *= 2
+        max_nodes = -(-total // p) + total // (16 * p) + 4096
+        need = ws_bytes(capacity, max_nodes)
+        if passes or (need <= budget and max_nodes < 0xFFFFFFFE) or p >= 1 << 16:   # (node indices are u32)
+            return {"passes": p, "capacity": capacity, "max_nodes": max_nodes, "ws_bytes": need}
+        p *= 2
+
 
 _default_engine = None
 

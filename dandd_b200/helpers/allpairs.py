@@ -22,7 +22,8 @@ deliberate differences (the reference's `go()` cannot run as shipped: it reads a
     matrices they would be built from are the last product;
   * `--write-commands` defaults to "" -- no commands are run, so the list is only written on request;
   * `--tool kmc` counts the union of a pair exactly (the reference's kmc command line for a pair is
-    malformed: it passes "A B" where kmc expects one input, :38-44);
+    malformed: it passes "A B" where kmc expects one input, :38-44), all pairs of one k in one device
+    job (K7, `store.exact_pair_cards`) that reads every FASTA once;
   * `--extra` understands `--no-canon` (the only sketching flag DandD itself ever passes).
 Under torchrun / several ranks the FASTAs are sharded over the GPUs for sketching, the registers
 are all-gathered and the pair list is split over the ranks; rank 0 writes the files."""
@@ -201,7 +202,8 @@ def card_table(tool: str, inputs: Sequence[str], names: Sequence[str], klist: Se
     if tool == "dashing" and (nest < 1 or nest & (nest - 1)):
         raise RuntimeError("--nest must be a power of 2 for dashing (got %d)" % nest)
     from dandd_b200 import ingest, timing
-    ingest.prefetch([inputs[g] for g in owners[rank]], want_digest=False)    # file i+1.. are read while the GPU works on file i
+    batched_exact = tool == "kmc" and hasattr(store, "exact_pair_cards")        # every rank reads every FASTA
+    ingest.prefetch(list(inputs) if batched_exact else [inputs[g] for g in owners[rank]], want_digest=False)   # file i+1.. are read while the GPU works on file i
     if tool == "dashing":
         p = int(math.log2(nest))
         uniq = sorted(set(ks))
@@ -219,6 +221,17 @@ def card_table(tool: str, inputs: Sequence[str], names: Sequence[str], klist: Se
             part = store.pair_cards(regs, mine, p, tile_pairs)
         col = [uniq.index(k) for k in ks]
         single, part = single[:, col], part[:, col]
+    elif batched_exact:
+        # one batched job per k; under several ranks every rank counts its key range of the same job and
+        # the integer counts are summed (each k-mer belongs to exactly one rank's range)
+        with timing.span("allpairs_exact"):
+            single, pair = store.exact_pair_cards(inputs, ks, canon, shard=(rank, world) if world > 1 else None)
+            if world > 1:
+                dev = getattr(getattr(store, "engine", None), "device", "cpu")
+                both = torch.as_tensor(np.concatenate([single, pair]).astype(np.int64), device=dev)
+                both = dd_dist.sum_counts(both).cpu().numpy().astype(np.float64)
+                single, pair = both[:n], both[n:]
+        return CardTable(tool, names, ks, single, pair)
     else:
         with timing.span("allpairs_exact"):
             single_mine = np.array([[store.exact_count([inputs[g]], k, canon) for k in ks] for g in owners[rank]],

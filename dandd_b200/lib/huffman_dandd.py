@@ -40,6 +40,7 @@ def get_store():
 
 
 HLL_MAX_K = 32      # "maxk<=32 for estimation" (reference README.md:82, lib/huffman_dandd.py:109-110)
+EXACT_MAX_K = 256   # KMC's own k limit
 MIN_KSLOTS = 100    # default length of DeltaTreeNode.ksketches (index = k, slot 0 = sweep template)
 
 
@@ -660,7 +661,7 @@ class DeltaTree:
                 if table is not None:
                     rows = self._pair_from_table(first, second, table, pair_index, pair_experiment, jaccard, mink, maxk)
                 pair_index += 1
-                if rows is None:         # exact mode, --safe, or a k outside the batched table: one SubSpider per pair
+                if rows is None:         # --safe, no batched job in this store, or a k outside the table: one SubSpider per pair
                     pair = SubSpider(leafnodes=[first, second], speciesinfo=self.speciesinfo, experiment=pair_experiment)
                     pair.root.find_delta(self.root_k())
                     krow, jrows = pair.kij_summarize(), []
@@ -684,6 +685,8 @@ class DeltaTree:
         spec, exp = self.speciesinfo, pair_experiment
         col = table.col
         registers, canon = exp["registers"], exp["canonicalize"]
+        exact = exp["tool"] == "kmc"
+        limit = EXACT_MAX_K if exact else HLL_MAX_K
         files = sorted(os.path.basename(f) for f in (first.fastas[0], second.fastas[0]))
         set_key = "".join(files)
         stored = spec.fastahex.get(set_key)
@@ -702,8 +705,8 @@ class DeltaTree:
             then evaluates every pair x every k at once)."""
             hit = cells.get(k)
             if hit is None:
-                path = os.path.join(spec.sketchdir, "ngen2", "k" + str(k), stem + str(k) + nc) + ".hll"
-                there = os.path.exists(path) and os.path.getsize(path) > 0
+                path = os.path.join(spec.sketchdir, "ngen2", "k" + str(k), stem + str(k) + nc) + ("" if exact else ".hll")
+                there = all(nonempty_file(path + ext) for ext in ((".kmc_pre", ".kmc_suf") if exact else ("",)))
                 card = float(spec.cardkey.get(path) or 0) if there else 0.0
                 if not card > 0:
                     card = float(table.cards()[row, col[k]])
@@ -711,14 +714,14 @@ class DeltaTree:
             return hit
 
         def touch(lo, hi):
-            for k in range(max(1, lo), min(hi, HLL_MAX_K) + 1):
+            for k in range(max(1, lo), min(hi, limit) + 1):
                 if k not in col:
                     raise KeyError(k)
                 if k not in visited:
                     visited.append(k)
 
         def helper(k, direction):
-            if k > HLL_MAX_K:
+            if not exact and k > HLL_MAX_K:
                 raise ValueError("Exploratory k value is too high for dashing. Either something is amiss with your data "
                                  "or you need to be using --exact mode")
             touch(k - 1, k + 1)
@@ -757,7 +760,9 @@ class DeltaTree:
             if k == 0:
                 continue
             path, there, card = cell(k)
-            if not there:
+            if not there and exact:        # the descriptor pair the union's KMCSketchObj would write
+                KMCSketchObj.write_db(path, k, bool(canon), [first.fastas[0], second.fastas[0]], int(card), spec.cardkey)
+            elif not there:
                 ensure_dir(os.path.dirname(path))
                 get_store().materialize_union(path, int(registers), card, [leaf_sketch[first][k].sketch, leaf_sketch[second][k].sketch])
             if not float(spec.cardkey.get(path) or 0):
@@ -771,22 +776,22 @@ class DeltaTree:
             for k in range(mink, maxk + 1):
                 jr = {"A": first.fastas[0], "B": second.fastas[0], "Atitle": first.node_title, "Btitle": second.node_title,
                       "kval": k, "Acard": _card_at(first, k), "Bcard": _card_at(second, k),
-                      "ABcard": cell(k)[2] if k <= HLL_MAX_K else 0.0}
+                      "ABcard": cell(k)[2] if k <= limit else 0.0}
                 jr["jaccard"] = (jr["Acard"] + jr["Bcard"] - jr["ABcard"]) / jr["ABcard"]
                 jrows.append(jr)
         return kij, jrows
 
     def _prefetch_pair_unions(self, leaves):
-        """K6: the union cardinality of every pair of leaves at every k the leaves hold is computed by
-        ONE batched device job (sketches transposed once, pair matrix tiled) and kept by the store;
-        the per-pair SubSpiders below then find every two-leaf union already evaluated and issue no
-        device work of their own.  HLL mode only; exact mode goes pair by pair (k-mer sets are not
-        mergeable sketches)."""
-        if (self.experiment["tool"] != "dashing" or len(leaves) < 3 or self.experiment["safety"] or self.experiment["lowmem"]
+        """The union cardinality of every pair of leaves at every k the leaves hold, computed by ONE
+        batched device job and kept by the store: K6 on the HLL sketches (transposed once, pair matrix
+        tiled), or in exact mode K7 (one pair-intersection job per k, every FASTA read once per k).  The
+        pairs below are then replayed on that table and issue no device work of their own."""
+        tool = self.experiment["tool"]
+        if (tool not in ("dashing", "kmc") or len(leaves) < 3 or self.experiment["safety"] or self.experiment["lowmem"]
                 or os.environ.get("DANDD_B200_PAIR_TABLE", "1") == "0"
                 or not all(hasattr(leaf, "ksketches") for leaf in leaves)):
             return None
-        ks = [k for k in range(1, HLL_MAX_K + 1)
+        ks = [k for k in range(1, (EXACT_MAX_K if tool == "kmc" else HLL_MAX_K) + 1)
               if all(k < len(leaf.ksketches) and leaf.ksketches[k] is not None for leaf in leaves)]
         if not ks:
             return None
@@ -794,6 +799,11 @@ class DeltaTree:
 
         def compute():
             store = get_store()
+            if tool == "kmc":
+                if not hasattr(store, "exact_pair_cards"):
+                    raise KeyError("this store has no batched exact pair job")     # -> the object path
+                return store.exact_pair_cards([leaf.fastas[0] for leaf in leaves], ks, bool(self.experiment["canonicalize"]),
+                                              remember=True)[1]
             if not hasattr(store, "pair_unions"):
                 raise KeyError("this store has no batched pair job")       # -> the object path, pair by pair
             return store.pair_unions({k: [leaf.ksketches[k].sketch for leaf in leaves] for k in ks}, registers)

@@ -377,6 +377,13 @@ class KMCSketchObj(SketchObj):
         `full` + .kmc_pre/.kmc_suf and cache the count -- `kmc` (one FASTA) or `kmc_tools complex`
         (several) followed by `kmc_tools info`, in one step."""
         count = get_store().exact_count(list(fastas), kval, canon)
+        cls.write_db(full, kval, canon, fastas, count, cardkey)
+        return count
+
+    @classmethod
+    def write_db(cls, full: str, kval: int, canon: bool, fastas, count: int, cardkey) -> None:
+        """Write the descriptor pair of a set whose count is known at `full` + .kmc_pre/.kmc_suf and cache
+        the count (build_db, and the pairs a batched all-pairs job has already counted)."""
         ensure_dir(os.path.dirname(full))
         body = (cls.MAGIC + f"k={kval}\ncanonical={int(canon)}\ntotal k-mers={count}\n".encode()
                 + "".join(f"input={f}\n" for f in fastas).encode())
@@ -384,7 +391,6 @@ class KMCSketchObj(SketchObj):
             with open(full + ext, "wb") as fh:
                 fh.write(body)
         cardkey[full] = float(count)
-        return count
 
     def _run_leaf(self) -> None:
         self.build_db(self.sfp.full, self.kval, bool(self.experiment["canonicalize"]), self.sfp.ffiles,

@@ -10,6 +10,7 @@ progressive prefix unions and pairwise unions never re-read a file or re-sketch 
     dashing union  (x nk via parallel)  -> union_sketches()     one batched max+histogram+MLE launch
     dashing card                        -> card_of_file()
     kmc + kmc_tools info / complex      -> exact_count()        GPU k-mer set (bitmap / hash set)
+    kmc_tools complex over all pairs    -> exact_pair_cards()   one pair-intersection job per k
 
 One store per process; it talks to one Engine (one GPU).  There is no CPU path here.
 """
@@ -52,6 +53,7 @@ class GpuSketchStore:
         self._cost: Dict[tuple, int] = {}
         self._bytes = 0
         self.pair_table = None   # cardinalities of every two-leaf union, filled by one batched K6 job (pair_unions)
+        self.exact_pair_table = None   # exact counts of every leaf and two-leaf union (exact_pair_cards, remember=True)
         self.stats = {"leaf_passes": 0, "union_launches": 0, "files_written": 0, "files_read": 0, "exact_calls": 0}
         self.exact_workers = None   # set by start_exact_workers() for `--exact` under torchrun
         self.stream_stats: List[dict] = []   # per streamed FASTA: stage times (read, blake2b, GPU span, wall)
@@ -445,6 +447,9 @@ class GpuSketchStore:
     # ------------------------------------------------------------------ kmc / kmc_tools
     def exact_count(self, fastas: Sequence[str], k: int, canon: bool) -> int:
         """Number of distinct (canonical) k-mers in the union of the FASTAs (KMC semantics)."""
+        known = self._exact_from_table(fastas, k, canon)
+        if known is not None:
+            return known
         return self.exact_prefix_counts(fastas, k, canon)[-1]
 
     def exact_prefix_counts(self, fastas: Sequence[str], k: int, canon: bool) -> List[int]:
@@ -452,6 +457,51 @@ class GpuSketchStore:
         if self.exact_workers is not None:
             return self.exact_workers.counts(list(fastas), int(k), bool(canon))
         return self._exact_shard_counts(fastas, k, canon, None)
+
+    def exact_pair_cards(self, fastas: Sequence[str], ks: Sequence[int], canon: bool, shard: Optional[Tuple[int, int]] = None,
+                         remember: bool = False) -> Tuple[np.ndarray, np.ndarray]:
+        """Exact counts of every FASTA and of the union of every pair, at every k: (singles [n, nk],
+        unions [n(n-1)/2, nk]) float64, pairs (0,1), (0,2) .. (n-2,n-1).  One batched device job per k
+        (K7: every genome read once per k, |A u B| = |A| + |B| - |A n B| in integers).  shard=(rank, world):
+        this rank's key range only; the ranks' results add up to the whole counts.  An engine without
+        the batched job answers pair by pair through exact_count.  With `remember`, later exact_count
+        calls for one or two of these FASTAs at these k are answered from the table."""
+        n, ks = len(fastas), [int(k) for k in ks]
+        singles = np.zeros((n, len(ks)), dtype=np.int64)
+        unions = np.zeros((n * (n - 1) // 2, len(ks)), dtype=np.int64)
+        batched = getattr(self.engine, "exact_pair_intersections", None)
+        if batched is None:
+            if shard is not None and shard[0] != 0:     # (the per-pair path counts whole sets: rank 0 holds them)
+                return singles.astype(np.float64), unions.astype(np.float64)
+            for c, k in enumerate(ks):
+                singles[:, c] = [self.exact_count([f], k, canon) for f in fastas]
+                unions[:, c] = [self.exact_count([fastas[a], fastas[b]], k, canon) for a, b in zip(*np.triu_indices(n, 1))]
+        else:
+            seqs = [self.packed(f) for f in fastas]
+            iu = np.triu_indices(n, 1)
+            for c, k in enumerate(ks):
+                self.stats["exact_calls"] += 1
+                singles[:, c] = [self.engine.exact_counts([s], k, canon, shard=shard)[0] for s in seqs]
+                inter = batched(seqs, k, canon, singles[:, c].tolist(), shard=shard).astype(np.int64)
+                unions[:, c] = singles[iu[0], c] + singles[iu[1], c] - inter
+        if remember:
+            self.exact_pair_table = {"n": n, "canon": bool(canon), "col": {k: c for c, k in enumerate(ks)},
+                                     "row": {f: g for g, f in enumerate(fastas)}, "singles": singles, "unions": unions}
+        return singles.astype(np.float64), unions.astype(np.float64)
+
+    def _exact_from_table(self, fastas, k, canon):
+        tab = getattr(self, "exact_pair_table", None)
+        if tab is None or tab["canon"] != bool(canon) or int(k) not in tab["col"] or not 1 <= len(fastas) <= 2:
+            return None
+        rows = [tab["row"].get(f) for f in fastas]
+        if None in rows:
+            return None
+        c = tab["col"][int(k)]
+        if len(rows) == 1 or rows[0] == rows[1]:
+            return int(tab["singles"][rows[0], c])
+        i, j = sorted(rows)
+        n = tab["n"]
+        return int(tab["unions"][i * n - i * (i + 1) // 2 + (j - i - 1), c])
 
     def _exact_shard_counts(self, fastas, k, canon, shard):
         return self.engine.exact_counts([self.packed(f) for f in fastas], int(k), canon, shard=shard)

@@ -266,6 +266,43 @@ DD_API int dd_exact_insert_shard(const uint32_t *d_codes, const uint32_t *d_inva
 DD_API int dd_exact_count(void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t *d_count, dd_stream stream);
 
 /* ===========================================================================================
+ * K7  --exact all pairs: |A n B| for every unordered pair of n_genomes genomes at one k, added into
+ * d_inter [n_genomes(n_genomes-1)/2] u64, rows in the order (0,1), (0,2) .. (n-2,n-1); the caller forms
+ * |A u B| = |A| + |B| - |A n B|.  Replaces the pair unions of `kmc_tools complex` that an exact all-pairs
+ * run asks for, one pair and one k at a time (helpers/allpairs.py:38-44,360-370; the SubSpider of each
+ * pair in lib/huffman_dandd.py:666-695), with one job that reads every genome once.
+ *
+ * Sparse path (any k <= DD_EXACT_MAXK): the K5 open-addressing key table (64-bit keys to k = 32, 128-bit
+ * to k = 64, verified references above; at every k, no bitmap), plus a (last genome, list head) pair per
+ * slot and `max_nodes` list nodes.  dd_exact_pairs_insert pushes `genome` once onto the list of every key
+ * of [sym_begin, sym_end) it holds: all ranges of one genome must be inserted before the next genome's
+ * (a genome may come in several ranges or streams); `genome` must be below the n_genomes later passed to
+ * dd_exact_pairs_accumulate (other indices are not counted).  dd_exact_pairs_accumulate then adds 1 to
+ * every pair on a list.  `capacity` (power of two >= 1024) must exceed the distinct keys of the job, `max_nodes`
+ * (< 2^32 - 1) the sum over genomes of their distinct keys; `max_streams` (k > 64 only, at most 65536) bounds
+ * the distinct streams inserted.  A full table or node array makes dd_exact_pairs_accumulate write all-ones
+ * into every row of d_inter: a count is never silently wrong.  _shard restricts the job to key range
+ * shard_rank of shard_world exactly as dd_exact_insert_shard does: the shards' results add up.
+ *
+ * Dense path: dd_exact_pair_popc adds popc(A & B) over K5 presence bitmaps (k <= DD_EXACT_BITMAP_MAXK,
+ * filled with dd_exact_begin / dd_exact_insert[_shard]).  d_row_ws points at nr K5 workspaces, ws_stride
+ * bytes apart, holding genomes row0 .. row0+nr-1; d_col_ws likewise for col0 .. col0+nc-1 (it may be
+ * d_row_ws).  Every pair a < b with a a row and b a column genome is counted; blocks of genomes that do
+ * not fit in memory together are covered by calling it for every (row block, column block).
+ * =========================================================================================== */
+DD_API size_t dd_exact_pairs_workspace_bytes(int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams);
+DD_API int dd_exact_pairs_begin(void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                                uint32_t max_streams, dd_stream stream);
+DD_API int dd_exact_pairs_insert_shard(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end,
+                                       int k, int canon, uint32_t genome, void *d_ws, size_t ws_bytes, uint64_t capacity,
+                                       uint64_t max_nodes, uint32_t max_streams, uint32_t shard_rank, uint32_t shard_world,
+                                       dd_stream stream);
+DD_API int dd_exact_pairs_accumulate(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                                     uint32_t max_streams, int64_t n_genomes, uint64_t *d_inter, dd_stream stream);
+DD_API int dd_exact_pair_popc(const void *d_row_ws, int64_t row0, int nr, const void *d_col_ws, int64_t col0, int nc,
+                              size_t ws_stride, int k, int64_t n_genomes, uint64_t *d_inter, dd_stream stream);
+
+/* ===========================================================================================
  * Host-buffer convenience path (what bench.py's e2e number times): one FASTA held in host memory
  * -> H2D copy -> K1 -> K2 -> K4 -> D2H of cardinalities (and registers if h_regs != NULL);
  * synchronises the stream before returning.  Equivalent to the reference running
