@@ -487,6 +487,20 @@ int dd_exact_pairs_accumulate(const void *d_ws, size_t ws_bytes, int k, uint64_t
             "dd_exact_pairs_accumulate");
     return DD_OK;
 }
+// ---- K8 ------------------------------------------------------------------------------------------
+int dd_exact_first_rank_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams,
+                             int64_t n_genomes, const uint16_t *d_ranks, int64_t n_rows, uint64_t *d_hist, dd_stream stream) {
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, "dd_exact_first_rank_hist")) return rc;
+    if (n_genomes < 0 || n_genomes > 0xFFFF)   // ranks are u16 below n_genomes; 0xFFFF means "not in the row"
+        return fail(DD_ERR_ARG, "dd_exact_first_rank_hist: n_genomes=%lld outside [0,65535]", (long long)n_genomes);
+    if (n_rows < 0 || n_rows > 0x7FFFFFFFll) return fail(DD_ERR_ARG, "dd_exact_first_rank_hist: n_rows=%lld", (long long)n_rows);
+    if (n_genomes > 0 && n_rows > 0 && (!d_ranks || !d_hist)) return fail(DD_ERR_ARG, "dd_exact_first_rank_hist: null pointer");
+    DD_CUDA(dd::exact_first_rank_hist(d_ws, k, capacity, max_streams, (uint64_t)n_genomes, d_ranks, (uint64_t)n_rows, d_hist,
+                                      sm_count_now(), S(stream)),
+            "dd_exact_first_rank_hist");
+    return DD_OK;
+}
+
 int dd_exact_pair_popc(const void *d_row_ws, int64_t row0, int nr, const void *d_col_ws, int64_t col0, int nc, size_t ws_stride,
                        int k, int64_t n_genomes, uint64_t *d_inter, dd_stream stream) {
     if (!d_row_ws || !d_col_ws || !d_inter) return fail(DD_ERR_ARG, "dd_exact_pair_popc: null pointer");

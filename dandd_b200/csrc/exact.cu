@@ -499,6 +499,129 @@ cudaError_t exact_pairs_accumulate(const void *d_ws, int k, uint64_t capacity, u
     return cudaGetLastError();
 }
 
+// ---- K8: first-rank histograms over the K7 lists ---------------------------------------------------
+// Row r of the rank table gives every genome a rank (ties allowed, 0xFFFF = not in the row's family);
+// hist[r][m] counts the keys whose minimum rank over the genomes on their list is m.  A progressive
+// ordering is a row of positions (prefix i holds the keys of bins < i), a set a row of zeros (its union
+// is bin 0).  The work per slot is occ x ceil(R / 32): linear in the list, so no bitmap path is needed.
+//
+// Row blocks are the outer loop: lane j owns row rb*32 + j for a whole pass over the slots, so bin 0 --
+// where almost every key of a progressive row or a set lands -- is a register counter, flushed once per
+// lane and row block.  kSmemHist: the other bins count in shared memory (u32, row stride odd so that 32
+// rows hitting one bin hit 32 banks); kSmemRanks: the table sits transposed in shared memory, [genome][row],
+// so the 32 lanes of a row block read 32 adjacent entries.
+constexpr uint16_t kNoRank = 0xFFFF;
+
+template <bool kSmemHist, bool kSmemRanks>
+__global__ void __launch_bounds__(256)
+exact_first_rank_kernel(const ExactWsHeader *__restrict__ hdr, const uint2 *__restrict__ lh, const PairNode *__restrict__ nodes,
+                        uint64_t n_slots, uint32_t n_genomes, const uint16_t *__restrict__ ranks, uint32_t n_rows,
+                        uint32_t hist_stride, uint32_t rank_stride, unsigned long long *out) {
+    extern __shared__ uint32_t smem[];
+    const uint64_t n_cells = (uint64_t)n_rows * n_genomes;
+    if (hdr->overflow) {   // a full table or node array: the marker, never a count
+        for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_cells; i += (uint64_t)gridDim.x * blockDim.x)
+            out[i] = kEmptyKey;
+        return;
+    }
+    uint32_t *sm_hist = smem;
+    uint16_t *sm_rank = reinterpret_cast<uint16_t *>(smem + (kSmemHist ? (size_t)n_rows * hist_stride : 0));
+    if (kSmemHist)
+        for (uint64_t i = threadIdx.x; i < (uint64_t)n_rows * hist_stride; i += blockDim.x) sm_hist[i] = 0;
+    if (kSmemRanks)
+        for (uint64_t i = threadIdx.x; i < (uint64_t)n_genomes * rank_stride; i += blockDim.x) {
+            const uint32_t g = (uint32_t)(i / rank_stride), r = (uint32_t)(i % rank_stride);
+            sm_rank[i] = r < n_rows ? __ldg(ranks + (size_t)r * n_genomes + g) : kNoRank;
+        }
+    if (kSmemHist || kSmemRanks) __syncthreads();
+
+    const unsigned lane = threadIdx.x & 31;
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    const uint64_t warp0 = (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    for (uint32_t rb = 0; rb * 32 < n_rows; ++rb) {
+        const uint32_t row = rb * 32 + lane;
+        unsigned long long zero = 0;   // this lane's bin-0 count
+        for (uint64_t base = warp0 * 32; base < n_slots; base += warps * 32) {
+            const uint32_t head = base + lane < n_slots ? __ldg(&lh[base + lane].y) : kNil;
+            for (unsigned occ = __ballot_sync(0xffffffffu, head != kNil); occ; occ &= occ - 1) {
+                uint32_t at = __shfl_sync(0xffffffffu, head, __ffs(occ) - 1);
+                uint32_t best = kNoRank;
+                while (at != kNil) {   // the list, 32 nodes at a time: lane i keeps the i-th genome of the chunk
+                    uint32_t gl = 0;
+                    int na = 0;
+                    for (; na < 32 && at != kNil; ++na) {
+                        const PairNode nd = nodes[at];
+                        if (lane == (unsigned)na) gl = nd.genome;
+                        at = nd.next;
+                    }
+                    for (int i = 0; i < na; ++i) {
+                        const uint32_t g = __shfl_sync(0xffffffffu, gl, i);
+                        if (g >= n_genomes) continue;   // outside the caller's genome range: never read out of bounds
+                        uint32_t rk;
+                        if (kSmemRanks) rk = sm_rank[(size_t)g * rank_stride + row];
+                        else rk = row < n_rows ? __ldg(ranks + (size_t)row * n_genomes + g) : kNoRank;
+                        best = rk < best ? rk : best;
+                    }
+                }
+                if (best == 0) ++zero;
+                else if (best < n_genomes) {   // (kNoRank: no genome of the row holds the key; a rank >= n is not counted)
+                    if (kSmemHist) atomicAdd(&sm_hist[(size_t)row * hist_stride + best], 1u);
+                    else atomicAdd(&out[(size_t)row * n_genomes + best], 1ull);
+                }
+            }
+        }
+        if (row < n_rows && zero) atomicAdd(&out[(size_t)row * n_genomes], zero);
+    }
+    if (kSmemHist) {
+        __syncthreads();
+        for (uint64_t i = threadIdx.x; i < n_cells; i += blockDim.x) {
+            const uint64_t r = i / n_genomes, m = i % n_genomes;
+            const uint32_t v = sm_hist[r * hist_stride + m];
+            if (v) atomicAdd(&out[i], (unsigned long long)v);
+        }
+    }
+}
+
+constexpr size_t kRankSmemBytes = 128 * 1024;   // counters + transposed rank table, per CTA
+
+cudaError_t exact_first_rank_hist(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
+                                  const uint16_t *d_ranks, uint64_t n_rows, uint64_t *d_hist, int sm_count, cudaStream_t stream) {
+    if (n_genomes == 0 || n_rows == 0) return cudaSuccess;
+    const uint8_t *ws = static_cast<const uint8_t *>(d_ws);
+    const ExactWsHeader *hdr = static_cast<const ExactWsHeader *>(d_ws);
+    const uint2 *lh = reinterpret_cast<const uint2 *>(ws + pairs_lh_offset(k, capacity, max_streams));
+    const PairNode *nodes = reinterpret_cast<const PairNode *>(ws + pairs_node_offset(k, capacity, max_streams));
+    unsigned long long *out = reinterpret_cast<unsigned long long *>(d_hist);
+    const uint64_t n_slots = capacity + 1;
+    const uint32_t hist_stride = (uint32_t)(n_genomes | 1);                  // odd: one bank per row
+    const uint32_t rank_stride = (uint32_t)((n_rows + 31) / 32 * 32);        // whole row blocks, padded with kNoRank
+    const size_t hist_bytes = (size_t)n_rows * hist_stride * sizeof(uint32_t);
+    const size_t rank_bytes = (size_t)n_genomes * rank_stride * sizeof(uint16_t);
+    const bool smem_hist = hist_bytes <= kPairSmemBytes;
+    const bool smem_rank = (smem_hist ? hist_bytes : 0) + rank_bytes <= kRankSmemBytes;
+    const size_t smem = (smem_hist ? hist_bytes : 0) + (smem_rank ? rank_bytes : 0);
+    unsigned grid;
+    if (smem_hist) {
+        grid = (unsigned)(sm_count * 2);   // every CTA pays one pass over its counters at the start and one at the end
+    } else {
+        const uint64_t want = (n_slots + 255) / 256;   // one 32-slot group per warp
+        grid = (unsigned)(want < (uint64_t)sm_count * 16 ? (want ? want : 1) : (uint64_t)sm_count * 16);
+    }
+    auto launch = [&](auto kernel) -> cudaError_t {
+        if (smem > 48 * 1024) {
+            const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e != cudaSuccess) return e;
+        }
+        DD_COUNT_LAUNCH(), kernel<<<grid, 256, smem, stream>>>(hdr, lh, nodes, n_slots, (uint32_t)n_genomes, d_ranks,
+                                                              (uint32_t)n_rows, hist_stride, rank_stride, out);
+        return cudaGetLastError();
+    };
+    if (smem_hist && smem_rank) return launch(exact_first_rank_kernel<true, true>);
+    if (smem_hist) return launch(exact_first_rank_kernel<true, false>);
+    if (smem_rank) return launch(exact_first_rank_kernel<false, true>);
+    return launch(exact_first_rank_kernel<false, false>);
+}
+
 // Dense path: popc(A & B) over K5 presence bitmaps.  A CTA owns a tile of 8 row genomes x 8 column
 // genomes and a slice of the bitmap words: each word range of the 16 bitmaps is read once per tile
 // (from L2 when other tiles have just read it) and feeds 64 pair counters.

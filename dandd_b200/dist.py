@@ -227,10 +227,12 @@ class ExactWorkers:
     """`dandd tree --exact` under torchrun: rank 0 runs the (inherently sequential) tree logic; every
     exact count it needs is announced to the other ranks, all ranks insert their key range of the
     k-mer set (`shard=(rank, world)`) and the counts are summed.  Ranks > 0 sit in serve() until
-    rank 0 calls stop()."""
+    rank 0 calls stop().  Two kinds of request: the progressive counts of one FASTA list at one k ("exact"),
+    and the first-rank histograms of a rank table at several k ("hist", GpuSketchStore.exact_union_cards)."""
 
-    def __init__(self, counter):
+    def __init__(self, counter, hists=None):
         self.counter = counter          # callable(fastas, k, canon, shard) -> list of progressive counts (this rank's shard)
+        self.hists = hists              # callable(fastas, ranks, ks, canon, singles, shard) -> int64 [nk, R, n] (this rank's shard)
         self.rank, self.world = world()
         self.active = self.world > 1
 
@@ -247,6 +249,20 @@ class ExactWorkers:
             mine = mine.cuda()
         return [int(v) for v in sum_counts(mine).cpu().tolist()]
 
+    def rank_hists(self, fastas, ranks, ks, canon, singles=None):
+        """Called on rank 0: first-rank histograms int64 [nk, R, n], every rank running its key range."""
+        if not self.active:
+            return self.hists(fastas, ranks, ks, canon, singles, None)
+        broadcast_object(("hist", list(fastas), ranks, list(ks), bool(canon), singles))
+        return self._hist_collective(fastas, ranks, ks, canon, singles)
+
+    def _hist_collective(self, fastas, ranks, ks, canon, singles):
+        mine = torch.from_numpy(np.ascontiguousarray(self.hists(fastas, ranks, ks, canon, singles, (self.rank, self.world)),
+                                                     dtype=np.int64))
+        if dist.get_backend() == "nccl":
+            mine = mine.cuda()
+        return sum_counts(mine).cpu().numpy()
+
     def serve(self) -> int:
         """Ranks > 0: answer requests until rank 0 says stop; returns how many were served."""
         served = 0
@@ -254,7 +270,10 @@ class ExactWorkers:
             req = broadcast_object(None)
             if not req or req[0] == "stop":
                 return served
-            self._collective(req[1], req[2], req[3])
+            if req[0] == "hist":
+                self._hist_collective(*req[1:])
+            else:
+                self._collective(req[1], req[2], req[3])
             served += 1
 
     def stop(self) -> None:

@@ -454,6 +454,23 @@ class Engine:
             return out
         if k > 64 and n > 65536:
             raise DandDError("exact pairs above k = 64 take at most 65536 genomes per job")
+        part = torch.zeros(len(out), dtype=torch.int64, device=self.device)
+        for ws, cap, nodes in self._key_lists(seqs, k, canon, singles, shard, passes):
+            part.zero_()
+            check(self.lib.dd_exact_pairs_accumulate(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part.data_ptr(), self.stream),
+                  "dd_exact_pairs_accumulate")
+            got = part.cpu().numpy().view(np.uint64)
+            if (got == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
+                raise DandDError("exact pair table or node array overflowed; the single counts given understate the genomes")
+            out += got
+        return out
+
+    def _key_lists(self, seqs: Sequence[PackedSeq], k: int, canon: bool, singles: Sequence[int],
+                   shard: Optional[tuple] = None, passes: Optional[int] = None):
+        """The K7 sparse workspace, once per key-range pass: yields (workspace, capacity, max_nodes) after every
+        genome has pushed itself onto the list of every key of the pass it holds (genome g = seqs[g]).  The
+        caller reads the lists (K7 pair counts, K8 first-rank histograms) before asking for the next pass."""
+        n = len(seqs)
         srank, sworld = (int(shard[0]), int(shard[1])) if shard is not None else (0, 1)
         nsyms = [s.nsym for s in seqs]
         plan = plan_pair_passes(singles, k, lambda c, m: int(self.lib.dd_exact_pairs_workspace_bytes(k, c, m, n)),
@@ -461,24 +478,49 @@ class Engine:
         self.last_pair_plan = dict(plan, path="sparse")
         cap, nodes = plan["capacity"], plan["max_nodes"]
         ws = self._buf(plan["ws_bytes"], "exact_pairs")
-        part = torch.zeros(len(out), dtype=torch.int64, device=self.device)
         st = self.stream
-        for p in range(plan["passes"]):
-            sr, sw = pass_shard(srank, sworld, p, plan["passes"])
-            check(self.lib.dd_exact_pairs_begin(ws.data_ptr(), ws.numel(), k, cap, nodes, n, st), "dd_exact_pairs_begin")
-            for g, (s, ns) in enumerate(zip(seqs, nsyms)):
-                check(self.lib.dd_exact_pairs_insert_shard(s.codes.data_ptr(), s.invalid.data_ptr(), 0, ns, k, int(canon), g,
-                                                           ws.data_ptr(), ws.numel(), cap, nodes, n, sr, sw, st),
-                      "dd_exact_pairs_insert_shard")
+        try:
+            for p in range(plan["passes"]):
+                sr, sw = pass_shard(srank, sworld, p, plan["passes"])
+                check(self.lib.dd_exact_pairs_begin(ws.data_ptr(), ws.numel(), k, cap, nodes, n, st), "dd_exact_pairs_begin")
+                for g, (s, ns) in enumerate(zip(seqs, nsyms)):
+                    check(self.lib.dd_exact_pairs_insert_shard(s.codes.data_ptr(), s.invalid.data_ptr(), 0, ns, k, int(canon), g,
+                                                               ws.data_ptr(), ws.numel(), cap, nodes, n, sr, sw, st),
+                          "dd_exact_pairs_insert_shard")
+                yield ws, cap, nodes
+        finally:
+            del ws
+            self._ws.pop("exact_pairs", None)     # a pass may take half the device: not kept for later stages
+
+    # ---- K8 ---------------------------------------------------------------------------------
+    def exact_first_rank_hist(self, seqs: Sequence[PackedSeq], k: int, canon: bool, ranks,
+                              singles: Optional[Sequence[int]] = None, shard: Optional[tuple] = None,
+                              passes: Optional[int] = None) -> np.ndarray:
+        """hist uint64 [R, n] for a rank table `ranks` [R, n] (uint16; 0xFFFF = genome not in the row): hist[r][m] =
+        distinct k-mers of seqs whose minimum rank over the genomes holding them is m under row r.  A progressive
+        ordering's row holds each genome's position (prefix i: cumsum(hist[r])[i - 1]); a set's row holds 0 for its
+        members (its union: hist[r][0]).  One K7 list job at k (every genome read once per pass) and one K8 launch
+        per pass.  singles / shard / passes as for exact_pairs_sparse."""
+        n = len(seqs)
+        ranks = np.ascontiguousarray(ranks, dtype=np.uint16).reshape(-1, n)
+        rows = ranks.shape[0]
+        out = np.zeros((rows, n), dtype=np.uint64)
+        if n == 0 or rows == 0:
+            return out
+        if n > 65535:
+            raise DandDError("first-rank histograms take at most 65535 genomes per job (ranks are 16-bit)")
+        if singles is None:
+            singles = [self.exact_counts([s], k, canon, shard=shard)[0] for s in seqs]
+        d_ranks = torch.from_numpy(ranks.view(np.int16)).to(self.device)
+        part = torch.zeros((rows, n), dtype=torch.int64, device=self.device)
+        for ws, cap, nodes in self._key_lists(seqs, k, canon, singles, shard, passes):
             part.zero_()
-            check(self.lib.dd_exact_pairs_accumulate(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part.data_ptr(), st),
-                  "dd_exact_pairs_accumulate")
+            check(self.lib.dd_exact_first_rank_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, d_ranks.data_ptr(), rows,
+                                                    part.data_ptr(), self.stream), "dd_exact_first_rank_hist")
             got = part.cpu().numpy().view(np.uint64)
             if (got == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
-                raise DandDError("exact pair table or node array overflowed; the single counts given understate the genomes")
+                raise DandDError("exact k-mer table or node array overflowed; the single counts given understate the genomes")
             out += got
-        del ws
-        self._ws.pop("exact_pairs", None)     # a pass may take half the device: not kept for later stages
         return out
 
     def exact_pairs_dense(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,

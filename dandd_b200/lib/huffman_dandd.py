@@ -430,13 +430,14 @@ class DeltaTree:
         """--ksweep: every (inner node, k) cell of the tree is known before any parent is evaluated -- the
         shape depends on node sizes only, and a node's union is the max over its progeny LEAVES -- so all
         of them go to the device as one batched job (GpuSketchStore.union_many) instead of one launch per
-        node; the parents built below then find their sketch files and cardinalities in place.  HLL mode
-        only; the hill-climb visits k adaptively and keeps the per-node batches."""
+        node; the parents built below then find their sketch files and cardinalities in place.  Exact mode
+        takes the same cells to one first-rank histogram job per k (_prefetch_exact_sets).  The hill-climb
+        visits k adaptively and keeps the per-node batches."""
         sweep = self.experiment["ksweep"]
-        if (sweep is None or self.experiment["tool"] != "dashing" or self.experiment["lowmem"] or len(leaves) < 3
-                or not all(leaf.ngen == 1 for leaf in leaves) or os.environ.get("DANDD_B200_TREE_BATCH", "1") == "0"):
+        tool = self.experiment["tool"]
+        if sweep is None or self.experiment["lowmem"] or len(leaves) < 3 or not all(leaf.ngen == 1 for leaf in leaves):
             return
-        ks = list(range(max(1, int(sweep[0])), min(HLL_MAX_K, int(sweep[1])) + 1))
+        ks = list(range(max(1, int(sweep[0])), min(EXACT_MAX_K if tool == "kmc" else HLL_MAX_K, int(sweep[1])) + 1))
         plan = self.plan_tree([1] * len(leaves), nchildren)
         if len(plan) < 2 or not ks:
             return                      # a spider has one inner node: the per-node batch is already one launch
@@ -444,6 +445,11 @@ class DeltaTree:
             return                      # the reference's cursor arithmetic runs off the list for some (n, nchildren),
                                         # e.g. (4, 3) or (6, 4), and then fails naming a parent without members
                                         # (lib/huffman_dandd.py:412-438): leave that to _build_tree, same error
+        if tool == "kmc":
+            self._prefetch_exact_sets(leaves, [([leaves[i].fastas[0] for i in progeny], None, None) for progeny in plan], ks)
+            return
+        if tool != "dashing" or os.environ.get("DANDD_B200_TREE_BATCH", "1") == "0":
+            return
         probe = DashSketchObj(kval=0, sfp=SketchFilePath(filenames=[leaves[0].fastas[0]], kval=0, speciesinfo=self.speciesinfo,
                                                          experiment=self.experiment),
                               speciesinfo=self.speciesinfo, experiment=self.experiment)
@@ -468,6 +474,57 @@ class DeltaTree:
         for (members, out_paths), cards in zip(jobs, results):
             for k, card in cards.items():
                 self.speciesinfo.cardkey[out_paths[k]] = card
+
+    def _exact_set_path(self, fastas, k: int) -> str:
+        """Where SketchFilePath puts the exact database of the set `fastas` at k -- without registering the set's
+        names: the node that asks for the set later does that itself, in the order the per-union path does."""
+        spec = self.speciesinfo
+        files = sorted(os.path.basename(f) for f in fastas)
+        stored = spec.fastahex.get("".join(files)) or hex(sum(int(spec.fastahex[name], 16) for name in files))
+        nc = "" if self.experiment["canonicalize"] else "nc"
+        base = f"{stored[:15]}_{self.experiment['registers']}n{len(fastas)}k{k}{nc}"
+        return os.path.join(spec.sketchdir, "ngen" + str(len(fastas)), "k" + str(k), base)
+
+    def _prefetch_exact_sets(self, leaves: List[DeltaTreeNode], cells, ks: List[int], orderings=None) -> None:
+        """Exact mode: the union databases of many nodes x every k of `ks` from one batched device job per k
+        (K7 lists + K8 first-rank histograms, GpuSketchStore.exact_union_cards / exact_prefix_cards) instead of
+        one fresh k-mer set per (node, k).  leaves: the genomes, in index order.  cells: (fastas of the asking
+        node, o, i) -- with `orderings`, the node is the union of the first i genomes of orderings[o]; without,
+        it is the set of its fastas.  Only the descriptor files are written; the node objects built later find
+        them, read the counts back and issue no device work, so every file, name and cardinality comes out as on
+        the per-union path (DANDD_B200_EXACT_SET_BATCH=0), in the same order.  A descriptor lists its inputs in
+        the order of the asking node's fastas."""
+        if not ks or not cells or self.experiment["lowmem"] or os.environ.get("DANDD_B200_EXACT_SET_BATCH", "1") == "0":
+            return
+        todo, seen = {}, set()
+        for c, (fastas, _, _) in enumerate(cells):
+            for k in ks:
+                path = self._exact_set_path(fastas, k)
+                if path not in seen and not all(nonempty_file(path + ext) for ext in (".kmc_pre", ".kmc_suf")):
+                    seen.add(path)
+                    todo.setdefault(k, []).append((path, c))
+        if not todo:
+            return                      # a cached re-run: nothing to compute, and the store (CUDA start-up) is never created
+        store = get_store()
+        if not hasattr(store, "exact_union_cards") or not hasattr(getattr(store, "engine", None), "exact_first_rank_hist"):
+            return
+        ks = sorted(todo)
+        canon = bool(self.experiment["canonicalize"])
+        genomes = [leaf.fastas[0] for leaf in leaves]
+        singles = None                  # exact leaf counts on record size the job; else the store counts them
+        if all(k < len(leaf.ksketches) and leaf.ksketches[k] is not None for leaf in leaves for k in ks):
+            singles = [[int(leaf.ksketches[k].card) for k in ks] for leaf in leaves]
+        if orderings is None:
+            index = {f: g for g, f in enumerate(genomes)}
+            cards = store.exact_union_cards(genomes, [[index[f] for f in fastas] for fastas, _, _ in cells], ks, canon,
+                                            singles=singles)
+            count = lambda c, col: cards[c, col]                                                  # noqa: E731
+        else:
+            cards = store.exact_prefix_cards(genomes, orderings, ks, canon, singles=singles)
+            count = lambda c, col: cards[cells[c][1], cells[c][2] - 1, col]                       # noqa: E731
+        for col, k in enumerate(ks):
+            for path, c in todo[k]:
+                KMCSketchObj.write_db(path, k, canon, cells[c][0], int(count(c, col)), None)
 
     def fill_tree(self, padding=False) -> None:
         """Give every node a sketch at every k that is some node's argmax (hill-climb mode), or sweep
@@ -586,9 +643,20 @@ class DeltaTree:
         """K3: with a k sweep requested every (ordering, prefix, k) cell is known in advance, so all
         prefix unions -- cardinalities and sketch files -- come from one running-max pass per
         ordering, stored under the names the per-prefix SubSpiders will ask for; those then find
-        every file present and every cardinality cached and issue no further work.  HLL mode only
-        (exact mode and the hill-climb go through the per-node batches)."""
+        every file present and every cardinality cached and issue no further work.  Exact mode: the same cells
+        over the k range every prefix is swept at (the sweep, else the spider's own [mink, maxk]) come from one
+        first-rank histogram job per k (_prefetch_exact_sets).  HLL without a sweep goes through the per-node
+        batches."""
         sweep = self.experiment["ksweep"]
+        if self.experiment["tool"] == "kmc" and orderings:
+            lo, hi = sweep if sweep is not None else (self.mink, self.maxk)
+            by_fasta = {node.fastas[0]: node for node in self.leaf_nodes()}
+            cells = [([n.fastas[0] for n in self.nodes_from_fastas([self.fastas[j] for j in ordering[:i]])], o, i)
+                     for o, ordering in enumerate(orderings) for i in range(2, len(ordering) + 1) if i % step == 0]
+            self._prefetch_exact_sets([by_fasta[f] for f in self.fastas], cells,
+                                      list(range(max(1, int(lo)), min(EXACT_MAX_K, int(hi)) + 1)),
+                                      orderings=[list(o) for o in orderings])
+            return
         if sweep is None or self.experiment["tool"] != "dashing" or not orderings:
             return
         ks = list(range(max(1, int(sweep[0])), min(HLL_MAX_K, int(sweep[1])) + 1))

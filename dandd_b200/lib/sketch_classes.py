@@ -383,14 +383,16 @@ class KMCSketchObj(SketchObj):
     @classmethod
     def write_db(cls, full: str, kval: int, canon: bool, fastas, count: int, cardkey) -> None:
         """Write the descriptor pair of a set whose count is known at `full` + .kmc_pre/.kmc_suf and cache
-        the count (build_db, and the pairs a batched all-pairs job has already counted)."""
+        the count (build_db, and the pairs a batched all-pairs job has already counted).  cardkey=None: the
+        count is left for the object that later finds the descriptor to read back (_run_card)."""
         ensure_dir(os.path.dirname(full))
         body = (cls.MAGIC + f"k={kval}\ncanonical={int(canon)}\ntotal k-mers={count}\n".encode()
                 + "".join(f"input={f}\n" for f in fastas).encode())
         for ext in (".kmc_pre", ".kmc_suf"):
             with open(full + ext, "wb") as fh:
                 fh.write(body)
-        cardkey[full] = float(count)
+        if cardkey is not None:
+            cardkey[full] = float(count)
 
     def _run_leaf(self) -> None:
         self.build_db(self.sfp.full, self.kval, bool(self.experiment["canonicalize"]), self.sfp.ffiles,

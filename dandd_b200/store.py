@@ -11,6 +11,8 @@ progressive prefix unions and pairwise unions never re-read a file or re-sketch 
     dashing card                        -> card_of_file()
     kmc + kmc_tools info / complex      -> exact_count()        GPU k-mer set (bitmap / hash set)
     kmc_tools complex over all pairs    -> exact_pair_cards()   one pair-intersection job per k
+    kmc_tools complex over prefixes,    -> exact_prefix_cards() / exact_union_cards()
+      over tree nodes                                            one first-rank histogram job per k
 
 One store per process; it talks to one Engine (one GPU).  There is no CPU path here.
 """
@@ -489,6 +491,64 @@ class GpuSketchStore:
                                      "row": {f: g for g, f in enumerate(fastas)}, "singles": singles, "unions": unions}
         return singles.astype(np.float64), unions.astype(np.float64)
 
+    def exact_prefix_cards(self, fastas: Sequence[str], orderings, ks: Sequence[int], canon: bool,
+                           shard: Optional[Tuple[int, int]] = None, singles=None) -> np.ndarray:
+        """Exact counts of every prefix union of every ordering, at every k: int64 [n_orderings, n, nk], cell
+        [o, i - 1, c] = |fastas[orderings[o][0]] u .. u fastas[orderings[o][i - 1]]| at ks[c] (an ordering shorter
+        than n repeats its full union).  One batched device job per k (K7 lists + K8 first-rank histograms: every
+        FASTA read once per k, whatever the number of orderings).  singles [n, nk]: exact counts of the single
+        FASTAs if the caller has them on record (they size the job), else they are counted.  shard=(rank, world):
+        this rank's key range only.  An engine without the batched job counts ordering by ordering."""
+        n, ks = len(fastas), [int(k) for k in ks]
+        orderings = [[int(g) for g in o] for o in orderings]
+        out = np.zeros((len(orderings), n, len(ks)), dtype=np.int64)
+        if not hasattr(self.engine, "exact_first_rank_hist"):
+            for c, k in enumerate(ks):
+                for o, order in enumerate(orderings):
+                    if order:
+                        got = self.exact_prefix_counts([fastas[g] for g in order], k, canon)
+                        out[o, :len(got), c] = got
+                        out[o, len(got):, c] = got[-1]
+            return out
+        ranks = np.full((len(orderings), n), 0xFFFF, dtype=np.uint16)
+        for o, order in enumerate(orderings):
+            ranks[o, order[::-1]] = np.arange(len(order), dtype=np.uint16)[::-1]   # a genome listed twice keeps its first place
+        hist = self._rank_hists(fastas, ranks, ks, canon, shard, singles)
+        return np.cumsum(hist, axis=2).transpose(1, 2, 0).copy()
+
+    def exact_union_cards(self, fastas: Sequence[str], sets, ks: Sequence[int], canon: bool,
+                          shard: Optional[Tuple[int, int]] = None, singles=None) -> np.ndarray:
+        """Exact count of the union of every set of FASTAs (sets: lists of indices into fastas) at every k:
+        int64 [n_sets, nk].  One batched device job per k, as exact_prefix_cards; an engine without it counts
+        set by set."""
+        n, ks = len(fastas), [int(k) for k in ks]
+        sets = [[int(g) for g in s] for s in sets]
+        if not hasattr(self.engine, "exact_first_rank_hist"):
+            return np.array([[self.exact_count([fastas[g] for g in s], k, canon) if s else 0 for k in ks] for s in sets],
+                            dtype=np.int64).reshape(len(sets), len(ks))
+        ranks = np.full((len(sets), n), 0xFFFF, dtype=np.uint16)
+        for r, members in enumerate(sets):
+            ranks[r, members] = 0
+        hist = self._rank_hists(fastas, ranks, ks, canon, shard, singles)
+        return hist[:, :, 0].T.copy() if n else np.zeros((len(sets), len(ks)), dtype=np.int64)
+
+    def _rank_hists(self, fastas, ranks, ks, canon, shard, singles) -> np.ndarray:
+        """First-rank histograms int64 [nk, R, n], one engine job per k; all ranks helping under `tree --exact`
+        with several ranks (dist.ExactWorkers), else this process's key range `shard` (None: all keys)."""
+        self.stats["exact_calls"] += len(ks)
+        workers = self.exact_workers
+        if shard is None and workers is not None and workers.active:
+            return workers.rank_hists(list(fastas), ranks, list(ks), bool(canon), singles)
+        return self._rank_hists_shard(fastas, ranks, ks, canon, singles, shard)
+
+    def _rank_hists_shard(self, fastas, ranks, ks, canon, singles, shard) -> np.ndarray:
+        seqs = [self.packed(f) for f in fastas]
+        out = np.zeros((len(ks), ranks.shape[0], len(fastas)), dtype=np.int64)
+        for c, k in enumerate(ks):
+            s = None if singles is None else [int(v) for v in np.asarray(singles)[:, c]]
+            out[c] = self.engine.exact_first_rank_hist(seqs, int(k), bool(canon), ranks, singles=s, shard=shard).astype(np.int64)
+        return out
+
     def _exact_from_table(self, fastas, k, canon):
         tab = getattr(self, "exact_pair_table", None)
         if tab is None or tab["canon"] != bool(canon) or int(k) not in tab["col"] or not 1 <= len(fastas) <= 2:
@@ -509,7 +569,7 @@ class GpuSketchStore:
     def start_exact_workers(self):
         """Multi-rank exact mode (dandd_b200.dist.ExactWorkers): rank 0 keeps going, the others serve."""
         from dandd_b200 import dist as dd_dist
-        self.exact_workers = dd_dist.ExactWorkers(self._exact_shard_counts)
+        self.exact_workers = dd_dist.ExactWorkers(self._exact_shard_counts, self._rank_hists_shard)
         return self.exact_workers
 
 

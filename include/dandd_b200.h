@@ -303,6 +303,23 @@ DD_API int dd_exact_pair_popc(const void *d_row_ws, int64_t row0, int nr, const 
                               size_t ws_stride, int k, int64_t n_genomes, uint64_t *d_inter, dd_stream stream);
 
 /* ===========================================================================================
+ * K8  --exact unions of many genome sets at one k, from the K7 sparse workspace after every genome has
+ * been inserted with dd_exact_pairs_insert_shard (same workspace, same arguments).  d_ranks [n_rows]
+ * [n_genomes] u16: row r gives every genome a rank (ties allowed; 0xFFFF = not in the row's family; any
+ * other value must be below n_genomes, larger ones are not counted).  Adds into d_hist [n_rows][n_genomes]
+ * u64 (the caller zeroes it): hist[r][m] = number of distinct keys whose minimum rank over the genomes
+ * holding them, under row r, is m; a key no genome of the row holds is not counted.  So
+ *   - a progressive ordering (row = the position of every genome in it): the union of its first i genomes
+ *     holds sum(hist[r][0 .. i-1]) k-mers -- the prefix unions of `kmc_tools complex` in
+ *     lib/huffman_dandd.py:624-663;
+ *   - a set S (row = 0 for its members, 0xFFFF elsewhere): |union of S| = hist[r][0] -- a tree node.
+ * n_genomes <= 65535.  A full table or node array writes all-ones into every cell of d_hist.
+ * =========================================================================================== */
+DD_API int dd_exact_first_rank_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                                    uint32_t max_streams, int64_t n_genomes, const uint16_t *d_ranks, int64_t n_rows,
+                                    uint64_t *d_hist, dd_stream stream);
+
+/* ===========================================================================================
  * Host-buffer convenience path (what bench.py's e2e number times): one FASTA held in host memory
  * -> H2D copy -> K1 -> K2 -> K4 -> D2H of cardinalities (and registers if h_regs != NULL);
  * synchronises the stream before returning.  Equivalent to the reference running

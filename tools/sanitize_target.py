@@ -4,7 +4,8 @@
     compute-sanitizer --tool racecheck python tools/sanitize_target.py
 K1 (general + fast tiles, chunked), K2 (persistent small-k bitmap path, static k sets, generic mask,
 floor schedule), finalize, K3 byte + bit-plane kernels with the identical-prefix table, K4, K5 (bitmap,
-64-bit and 128-bit hash sets), K6, the poly-T pass.  Results are compared with the oracle so that a
+64-bit and 128-bit hash sets), K6, K7 lists with K8 first-rank histograms (shared and global counters), the
+poly-T pass.  Results are compared with the oracle so that a
 "clean" run is also a correct one."""
 import os
 import sys
@@ -56,6 +57,17 @@ def main():
     for k in (5, 12, 21, 32, 40, 64):
         got = eng.exact_counts([seq], k)
         assert got == [orc.exact_count([sym], k)] if k <= 32 else got[0] > 0, k
+    # K7 lists + K8 first-rank histograms: prefix unions of two orderings and one set, on both counter paths
+    texts = [to_fasta([(b"g", mutate(rng, anc, sub=0.05))]) for _ in range(4)]
+    gseqs = [eng.pack(t) for t in texts]
+    gsyms = [orc.fasta_symbols(t) for t in texts]
+    ranks = np.array([[0, 1, 2, 3], [3, 2, 1, 0], [0, 0xFFFF, 0, 0xFFFF]], dtype=np.uint16)
+    for k in (12, 21, 40):
+        for reps in (1, 2000):   # 3 rows: counters in shared memory; 6000 rows: global atomics
+            hist = eng.exact_first_rank_hist(gseqs, k, True, np.tile(ranks, (reps, 1)))[:3].astype(np.int64)
+            if k <= 32:
+                assert hist[0].cumsum().tolist() == [orc.exact_count(gsyms[:i + 1], k) for i in range(4)], k
+                assert hist[1].cumsum()[-1] == orc.exact_count(gsyms, k) and hist[2, 0] == orc.exact_count(gsyms[::2], k), k
     # A.6 pass
     eng.polyt_sentinel = True
     t2 = to_fasta([(b"t", np.full(300, ord("T"), dtype=np.uint8))])
