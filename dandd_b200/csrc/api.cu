@@ -500,6 +500,12 @@ int dd_exact_first_rank_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t 
             "dd_exact_first_rank_hist");
     return DD_OK;
 }
+int dd_exact_pairs_node_count(const void *d_ws, size_t ws_bytes, uint64_t *d_out, dd_stream stream) {
+    if (!d_ws || !d_out) return fail(DD_ERR_ARG, "dd_exact_pairs_node_count: null pointer");
+    if (ws_bytes < sizeof(dd::ExactWsHeader)) return fail(DD_ERR_WORKSPACE, "dd_exact_pairs_node_count: workspace %zu too small", ws_bytes);
+    DD_CUDA(dd::exact_pairs_node_count(d_ws, d_out, S(stream)), "dd_exact_pairs_node_count");
+    return DD_OK;
+}
 
 int dd_exact_pair_popc(const void *d_row_ws, int64_t row0, int nr, const void *d_col_ws, int64_t col0, int nc, size_t ws_stride,
                        int k, int64_t n_genomes, uint64_t *d_inter, dd_stream stream) {

@@ -397,6 +397,13 @@ cudaError_t exact_pairs_insert(const uint32_t *d_codes, const uint32_t *d_invali
                        max_streams, /*bitmap=*/false, shard_rank, shard_world, act, stream);
 }
 
+// PushGenome pushes one node per (genome, slot) and a key owns exactly one slot in all three layouts, so the
+// counter's growth over one genome's insert is that genome's distinct keys in the pass (the family job's singles).
+cudaError_t exact_pairs_node_count(const void *d_ws, uint64_t *d_out, cudaStream_t stream) {
+    const ExactWsHeader *hdr = static_cast<const ExactWsHeader *>(d_ws);
+    return cudaMemcpyAsync(d_out, &hdr->n_nodes, sizeof(uint64_t), cudaMemcpyDeviceToDevice, stream);
+}
+
 __device__ __forceinline__ uint64_t pair_row(uint64_t a, uint64_t b, uint64_t n) {  // a < b
     return a * (2 * n - a - 1) / 2 + (b - a - 1);
 }

@@ -98,6 +98,8 @@ cudaError_t exact_pairs_accumulate(const void *d_ws, int k, uint64_t capacity, u
 // ---- K8 (exact.cu): first-rank histograms over the K7 lists, ranks [n_rows][n_genomes] u16 -> hist [n_rows][n_genomes]
 cudaError_t exact_first_rank_hist(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
                                   const uint16_t *d_ranks, uint64_t n_rows, uint64_t *d_hist, int sm_count, cudaStream_t stream);
+// the node counter of a K7 sparse workspace (ExactWsHeader::n_nodes) -> *d_out, a copy on the stream
+cudaError_t exact_pairs_node_count(const void *d_ws, uint64_t *d_out, cudaStream_t stream);
 // Dense: K5 bitmap workspaces, ws_stride bytes apart, for genomes row0.. and col0..
 cudaError_t exact_pair_popc(const void *d_rows, int64_t row0, int nr, const void *d_cols, int64_t col0, int nc,
                             size_t ws_stride, int k, int64_t n_genomes, uint64_t *d_inter, int sm_count, cudaStream_t stream);

@@ -227,12 +227,14 @@ class ExactWorkers:
     """`dandd tree --exact` under torchrun: rank 0 runs the (inherently sequential) tree logic; every
     exact count it needs is announced to the other ranks, all ranks insert their key range of the
     k-mer set (`shard=(rank, world)`) and the counts are summed.  Ranks > 0 sit in serve() until
-    rank 0 calls stop().  Two kinds of request: the progressive counts of one FASTA list at one k ("exact"),
-    and the first-rank histograms of a rank table at several k ("hist", GpuSketchStore.exact_union_cards)."""
+    rank 0 calls stop().  Three kinds of request: the progressive counts of one FASTA list at one k ("exact"),
+    the first-rank histograms of a rank table at several k ("hist", GpuSketchStore.exact_union_cards), and the
+    single counts + first-rank histograms of a registered family at one k ("family", GpuSketchStore.exact_family)."""
 
-    def __init__(self, counter, hists=None):
+    def __init__(self, counter, hists=None, family=None):
         self.counter = counter          # callable(fastas, k, canon, shard) -> list of progressive counts (this rank's shard)
         self.hists = hists              # callable(fastas, ranks, ks, canon, singles, shard) -> int64 [nk, R, n] (this rank's shard)
+        self.family = family            # callable(fastas, ranks, k, canon, shard) -> (int64 [n], int64 [R, n]) (this rank's shard)
         self.rank, self.world = world()
         self.active = self.world > 1
 
@@ -263,6 +265,24 @@ class ExactWorkers:
             mine = mine.cuda()
         return sum_counts(mine).cpu().numpy()
 
+    def family_counts(self, fastas, ranks, k, canon):
+        """Called on rank 0: (singles int64 [n], first-rank histograms int64 [R, n]) at k, every rank running its key
+        range; one all_reduce of [n + R n] adds them up."""
+        if not self.active:
+            return self.family(fastas, ranks, k, canon, None)
+        broadcast_object(("family", list(fastas), ranks, int(k), bool(canon)))
+        return self._family_collective(fastas, ranks, k, canon)
+
+    def _family_collective(self, fastas, ranks, k, canon):
+        singles, hist = self.family(fastas, ranks, k, canon, (self.rank, self.world))
+        mine = torch.from_numpy(np.concatenate([np.asarray(singles, dtype=np.int64).reshape(-1),
+                                                np.asarray(hist, dtype=np.int64).reshape(-1)]))
+        if dist.get_backend() == "nccl":
+            mine = mine.cuda()
+        total = sum_counts(mine).cpu().numpy()
+        n = len(fastas)
+        return total[:n], total[n:].reshape(len(ranks), n)
+
     def serve(self) -> int:
         """Ranks > 0: answer requests until rank 0 says stop; returns how many were served."""
         served = 0
@@ -272,6 +292,8 @@ class ExactWorkers:
                 return served
             if req[0] == "hist":
                 self._hist_collective(*req[1:])
+            elif req[0] == "family":
+                self._family_collective(*req[1:])
             else:
                 self._collective(req[1], req[2], req[3])
             served += 1

@@ -466,10 +466,12 @@ class Engine:
         return out
 
     def _key_lists(self, seqs: Sequence[PackedSeq], k: int, canon: bool, singles: Sequence[int],
-                   shard: Optional[tuple] = None, passes: Optional[int] = None):
+                   shard: Optional[tuple] = None, passes: Optional[int] = None, node_counts: Optional[torch.Tensor] = None):
         """The K7 sparse workspace, once per key-range pass: yields (workspace, capacity, max_nodes) after every
         genome has pushed itself onto the list of every key of the pass it holds (genome g = seqs[g]).  The
-        caller reads the lists (K7 pair counts, K8 first-rank histograms) before asking for the next pass."""
+        caller reads the lists (K7 pair counts, K8 first-rank histograms) before asking for the next pass.
+        node_counts (int64 [n] on the device): the node counter after genome g's insert is copied to entry g
+        of every pass (dd_exact_pairs_node_count) -- its growth over genome g is |A_g n the pass's key range|."""
         n = len(seqs)
         srank, sworld = (int(shard[0]), int(shard[1])) if shard is not None else (0, 1)
         nsyms = [s.nsym for s in seqs]
@@ -487,6 +489,9 @@ class Engine:
                     check(self.lib.dd_exact_pairs_insert_shard(s.codes.data_ptr(), s.invalid.data_ptr(), 0, ns, k, int(canon), g,
                                                                ws.data_ptr(), ws.numel(), cap, nodes, n, sr, sw, st),
                           "dd_exact_pairs_insert_shard")
+                    if node_counts is not None:
+                        check(self.lib.dd_exact_pairs_node_count(ws.data_ptr(), ws.numel(), node_counts.data_ptr() + 8 * g, st),
+                              "dd_exact_pairs_node_count")
                 yield ws, cap, nodes
         finally:
             del ws
@@ -522,6 +527,42 @@ class Engine:
                 raise DandDError("exact k-mer table or node array overflowed; the single counts given understate the genomes")
             out += got
         return out
+
+    def exact_family_counts(self, seqs: Sequence[PackedSeq], k: int, canon: bool, ranks, shard: Optional[tuple] = None,
+                            passes: Optional[int] = None):
+        """(singles uint64 [n], hist uint64 [R, n]) in one job at k: hist as exact_first_rank_hist gives it for the rank
+        table `ranks` [R, n], and singles[g] = |A_g| (this rank's key range under `shard`).  Unlike
+        exact_first_rank_hist nothing is counted up front: the job is sized from the sequence lengths (length_bounds,
+        never below the real counts), and the singles come from the list-node counter -- every genome pushes one node
+        per key it holds, so the counter's growth over its insert is its count (dd_exact_pairs_node_count, summed
+        over passes).  One K7 list job and one K8 launch per pass, one device->host copy per pass."""
+        n = len(seqs)
+        ranks = np.ascontiguousarray(ranks, dtype=np.uint16).reshape(-1, n) if n else np.zeros((len(ranks), 0), np.uint16)
+        rows = ranks.shape[0]
+        singles = np.zeros(n, dtype=np.uint64)
+        hist = np.zeros((rows, n), dtype=np.uint64)
+        if n == 0:
+            return singles, hist
+        if n > 65535:
+            raise DandDError("family counts take at most 65535 genomes per job (ranks are 16-bit)")
+        world = int(shard[1]) if shard is not None else 1
+        bounds = length_bounds([s.nsym for s in seqs], k, world)
+        # with no row, one row that holds no genome: K8 still reports a full table or node array
+        table = ranks if rows else np.full((1, n), 0xFFFF, dtype=np.uint16)
+        d_ranks = torch.from_numpy(table.view(np.int16)).to(self.device)
+        cells = table.shape[0] * n
+        part = torch.zeros(cells + n, dtype=torch.int64, device=self.device)    # [hist cells | node counter after genome g]
+        for ws, cap, nodes in self._key_lists(seqs, k, canon, bounds, shard, passes, node_counts=part[cells:]):
+            part[:cells].zero_()
+            check(self.lib.dd_exact_first_rank_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, d_ranks.data_ptr(),
+                                                    table.shape[0], part.data_ptr(), self.stream), "dd_exact_first_rank_hist")
+            got = part.cpu().numpy().view(np.uint64)
+            if (got[:cells] == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
+                raise DandDError("exact k-mer table or node array overflowed; the length bounds understate the genomes")
+            if rows:
+                hist += got[:cells].reshape(rows, n)
+            singles += np.diff(got[cells:], prepend=np.uint64(0))
+        return singles, hist
 
     def exact_pairs_dense(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
                           block: Optional[int] = None) -> np.ndarray:
@@ -583,6 +624,14 @@ def dense_pairs(k: int, singles: Sequence[int], world: int = 1) -> bool:
         return False
     mean = float(np.mean(np.asarray(singles, dtype=np.float64))) * world
     return 4 ** k / DENSE_BITS_PER_KMER <= mean
+
+
+def length_bounds(nsyms: Sequence[int], k: int, world: int = 1) -> List[int]:
+    """Upper bounds of the single counts |A_g| from the sequence lengths, to size a job that has not counted them:
+    a genome holds at most one distinct k-mer per symbol and at most 4^k of them; a key-range shard of `world`
+    holds its share of those (the share's fluctuation is what plan_pair_passes' margin covers, as for passes)."""
+    cap = 4 ** int(k) if int(k) < 32 else None
+    return [-(-(min(int(s), cap) if cap else int(s)) // int(world)) for s in nsyms]
 
 
 def pass_shard(rank: int, world: int, p: int, passes: int) -> tuple:

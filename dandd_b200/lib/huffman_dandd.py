@@ -16,6 +16,7 @@ per-k SketchObj constructors that follow find everything cached.  Progressive un
 every ordering in a single launch (a running max: n sketch reads per ordering instead of the
 reference's n(n+1)/2).
 """
+import contextlib
 import csv
 import os
 import pickle
@@ -25,7 +26,7 @@ from math import factorial
 from random import sample, shuffle
 from typing import Dict, List, Set, Tuple
 
-from sketch_classes import DashSketchObj, KMCSketchObj, SketchFilePath, SketchObj, ensure_dir, nonempty_file  # noqa: F401
+from sketch_classes import DashSketchObj, KMCSketchObj, SketchFilePath, SketchObj, ensure_dir, exact_family, nonempty_file  # noqa: F401
 from species_specifics import SpeciesSpecifics
 
 from dandd_b200 import ingest, timing
@@ -324,8 +325,9 @@ class DeltaTree:
         self.speciesinfo = speciesinfo
         if self.experiment["verbose"]:
             print("Now making tree for fastas: " + ", ".join(fasta_files))
-        self._build_tree(fasta_files, nchildren)
-        self.fill_tree(padding=padding)
+        with self._exact_tree_family(fasta_files, nchildren):
+            self._build_tree(fasta_files, nchildren)
+            self.fill_tree(padding=padding)
         self.ngen = len(fasta_files)
         self.root = self._dt[-1]
         self.delta = self.root_delta()
@@ -474,6 +476,28 @@ class DeltaTree:
         for (members, out_paths), cards in zip(jobs, results):
             for k, card in cards.items():
                 self.speciesinfo.cardkey[out_paths[k]] = card
+
+    def _exact_climb(self) -> bool:
+        """Exact hill-climb whose genome sets may be registered as a family (sketch_classes.exact_family): not under
+        --ksweep (_prefetch_exact_sets batches those cells), --lowmem, or DANDD_B200_EXACT_SET_BATCH=0 (union by union)."""
+        return (self.experiment["tool"] == "kmc" and self.experiment["ksweep"] is None and not self.experiment["lowmem"]
+                and os.environ.get("DANDD_B200_EXACT_SET_BATCH", "1") != "0")
+
+    def _exact_tree_family(self, fastas, nchildren: int):
+        """Exact hill-climb: the climb picks k as it goes, but which sets it counts is fixed by the node sizes alone --
+        the leaves (sorted by size: every leaf holds one FASTA, so in the given order) and the inner nodes of
+        plan_tree.  They are registered for the whole build, fill_tree's argmax k included, and every k the climb
+        visits then costs one family job (GpuSketchStore.exact_family) instead of a fresh k-mer set per (node, k).
+        Shapes the reference cannot build register nothing, so that _build_tree reaches the same failure."""
+        if not self._exact_climb() or not fastas or (len(fastas) > 1 and int(nchildren) < 2):
+            return contextlib.nullcontext()
+        try:
+            plan = self.plan_tree([1] * len(fastas), int(nchildren))
+        except IndexError:
+            return contextlib.nullcontext()
+        if any(not progeny for progeny in plan):
+            return contextlib.nullcontext()
+        return exact_family(fastas, bool(self.experiment["canonicalize"]), sets=plan)
 
     def _exact_set_path(self, fastas, k: int) -> str:
         """Where SketchFilePath puts the exact database of the set `fastas` at k -- without registering the set's
@@ -626,17 +650,22 @@ class DeltaTree:
     def progressive_union(self, flist, orderings, step) -> Tuple[List[dict], List[dict]]:
         """For every ordering, delta (or the whole k sweep) of the union of its first i FASTAs,
         i = step, 2*step, ...  The pickles are saved after every ordering, as in the reference."""
-        smain = DeltaSpider(fasta_files=flist, speciesinfo=self.speciesinfo, experiment=self.experiment)
-        smain._prefetch_prefix_unions(orderings, step)
-        results, summary = [], []
-        for number, ordering in enumerate(orderings, start=1):
-            if self.experiment["verbose"]:
-                print(f"Now sweeping for ordering {number}")
-            rows, sweep_rows = smain.sketch_ordering(ordering, ordering_number=number, step=step)
-            results.extend(rows)
-            summary.extend(sweep_rows)
-            self.speciesinfo.save_references(fast=self.experiment["fast"])
-            self.speciesinfo.save_cardkey(tool=self.experiment["tool"], fast=self.experiment["fast"])
+        family = contextlib.nullcontext()
+        if self._exact_climb() and all(0 <= int(j) < len(flist) for ordering in orderings for j in ordering):
+            # every prefix the climbs count, the spider's union included (prefix n of any ordering)
+            family = exact_family(flist, bool(self.experiment["canonicalize"]), orderings=orderings)
+        with family:
+            smain = DeltaSpider(fasta_files=flist, speciesinfo=self.speciesinfo, experiment=self.experiment)
+            smain._prefetch_prefix_unions(orderings, step)
+            results, summary = [], []
+            for number, ordering in enumerate(orderings, start=1):
+                if self.experiment["verbose"]:
+                    print(f"Now sweeping for ordering {number}")
+                rows, sweep_rows = smain.sketch_ordering(ordering, ordering_number=number, step=step)
+                results.extend(rows)
+                summary.extend(sweep_rows)
+                self.speciesinfo.save_references(fast=self.experiment["fast"])
+                self.speciesinfo.save_cardkey(tool=self.experiment["tool"], fast=self.experiment["fast"])
         return results, summary
 
     def _prefetch_prefix_unions(self, orderings, step) -> None:

@@ -12,6 +12,7 @@ recorded in `.cmd` (it appears in DandD's CSV output and documents what was repl
     DashSketchObj             reference :302-373  (HyperLogLog, `dashing sketch|union|card`)
     KMCSketchObj              reference :377-465  (exact, `kmc`, `kmc_tools info|complex`)
 """
+import contextlib
 import glob
 import os
 
@@ -26,6 +27,38 @@ def get_store():
     torch and starting CUDA."""
     from dandd_b200.store import get_store as _get
     return _get()
+
+
+_family = None   # the exact family registered by the running hill-climb (exact_family), entered in the store on demand
+
+
+@contextlib.contextmanager
+def exact_family(genomes, canon: bool, sets=(), orderings=()):
+    """Register the genome sets an exact hill-climb is going to count (GpuSketchStore.exact_family: `sets` are index
+    lists into genomes, `orderings` index sequences whose prefixes are the sets).  Recorded here on the host: the
+    store is only given the family when a count is actually computed (KMCSketchObj.build_db), so a run served
+    from the sketch database never creates it.  While one family is registered another registers nothing."""
+    global _family
+    if _family is not None:
+        yield
+        return
+    _family = {"args": (list(genomes), bool(canon), [list(s) for s in sets], [list(o) for o in orderings]), "open": None}
+    try:
+        yield
+    finally:
+        fam, _family = _family, None
+        if fam["open"] is not None:
+            fam["open"].__exit__(None, None, None)
+
+
+def _store_with_family():
+    """get_store(), with the registered exact family handed to it first (stores without exact_family: never)."""
+    store = get_store()
+    if _family is not None and _family["open"] is None and hasattr(store, "exact_family"):
+        ctx = store.exact_family(*_family["args"])
+        ctx.__enter__()
+        _family["open"] = ctx
+    return store
 
 
 DASHINGLOC = "dashing"   # kept for API compatibility; only ever used inside the recorded .cmd text
@@ -376,7 +409,7 @@ class KMCSketchObj(SketchObj):
         """Count the distinct k-mers of the FASTA set on the GPU, write the descriptor pair at
         `full` + .kmc_pre/.kmc_suf and cache the count -- `kmc` (one FASTA) or `kmc_tools complex`
         (several) followed by `kmc_tools info`, in one step."""
-        count = get_store().exact_count(list(fastas), kval, canon)
+        count = _store_with_family().exact_count(list(fastas), kval, canon)
         cls.write_db(full, kval, canon, fastas, count, cardkey)
         return count
 

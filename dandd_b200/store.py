@@ -18,6 +18,7 @@ One store per process; it talks to one Engine (one GPU).  There is no CPU path h
 """
 import os
 from collections import OrderedDict
+from contextlib import contextmanager
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -27,6 +28,7 @@ from . import hllfile, ingest, timing
 from .engine import Engine, get_engine
 
 ALL_HLL_KS = tuple(range(1, 33))
+EXACT_MAX_K = 256   # KMC's own k limit, and the exact kernels'
 STREAM_MIN_BYTES = int(os.environ.get("DANDD_B200_STREAM_MIN", str(32 << 20)))   # larger FASTAs take the chunked pipeline
 
 
@@ -56,7 +58,9 @@ class GpuSketchStore:
         self._bytes = 0
         self.pair_table = None   # cardinalities of every two-leaf union, filled by one batched K6 job (pair_unions)
         self.exact_pair_table = None   # exact counts of every leaf and two-leaf union (exact_pair_cards, remember=True)
-        self.stats = {"leaf_passes": 0, "union_launches": 0, "files_written": 0, "files_read": 0, "exact_calls": 0}
+        self.exact_family_table = None   # the genome sets of a running exact hill-climb, counted per k (exact_family)
+        self.stats = {"leaf_passes": 0, "union_launches": 0, "files_written": 0, "files_read": 0, "exact_calls": 0,
+                      "exact_family_jobs": 0}
         self.exact_workers = None   # set by start_exact_workers() for `--exact` under torchrun
         self.stream_stats: List[dict] = []   # per streamed FASTA: stage times (read, blake2b, GPU span, wall)
 
@@ -450,9 +454,68 @@ class GpuSketchStore:
     def exact_count(self, fastas: Sequence[str], k: int, canon: bool) -> int:
         """Number of distinct (canonical) k-mers in the union of the FASTAs (KMC semantics)."""
         known = self._exact_from_table(fastas, k, canon)
+        if known is None:
+            known = self._exact_from_family(fastas, k, canon)
         if known is not None:
             return known
         return self.exact_prefix_counts(fastas, k, canon)[-1]
+
+    @contextmanager
+    def exact_family(self, genomes: Sequence[str], canon: bool, sets=(), orderings=()):
+        """While open, exact_count answers every genome of `genomes`, every set of `sets` (index lists into
+        genomes: tree nodes) and every prefix of every ordering of `orderings` (index sequences: progressive
+        orderings) from one family job per k (Engine.exact_family_counts: K7 lists + one K8 launch, the singles from
+        the list-node counter), run the first time any of them is asked for at that k and kept as a few integers per
+        (row, k).  For a caller that knows WHICH sets it will count but not at which k (the exact hill-climb).
+        Another set, another `canon`, a k outside 1..256 or an engine without the job keep the per-union path."""
+        genomes = [str(f) for f in genomes]
+        n = len(genomes)
+        sets = [[int(g) for g in s] for s in sets]
+        orderings = [[int(g) for g in o] for o in orderings]
+        ranks = np.full((len(sets) + len(orderings), n), 0xFFFF, dtype=np.uint16)
+        cells = {frozenset([f]): ("single", g, 0) for g, f in reversed(list(enumerate(genomes)))}
+        for r, members in enumerate(sets):
+            ranks[r, members] = 0
+            if members:
+                cells.setdefault(frozenset(genomes[g] for g in members), ("row", r, 1))
+        for o, order in enumerate(orderings):
+            r = len(sets) + o
+            ranks[r, order[::-1]] = np.arange(len(order), dtype=np.uint16)[::-1]   # a genome listed twice keeps its first place
+            for i in range(1, len(order) + 1):
+                cells.setdefault(frozenset(genomes[g] for g in order[:i]), ("row", r, i))
+        family = {"genomes": genomes, "canon": bool(canon), "ranks": ranks, "cells": cells, "counts": {}}
+        outer, self.exact_family_table = getattr(self, "exact_family_table", None), family
+        try:
+            yield family
+        finally:
+            self.exact_family_table = outer
+
+    def _exact_from_family(self, fastas, k, canon):
+        fam = getattr(self, "exact_family_table", None)
+        if fam is None or fam["canon"] != bool(canon) or not 1 <= int(k) <= EXACT_MAX_K \
+                or not hasattr(self.engine, "exact_family_counts"):
+            return None
+        cell = fam["cells"].get(frozenset(fastas))
+        if cell is None:
+            return None
+        got = fam["counts"].get(int(k))
+        if got is None:
+            self.stats["exact_calls"] += 1
+            self.stats["exact_family_jobs"] += 1
+            workers = self.exact_workers
+            if workers is not None and workers.active:
+                got = workers.family_counts(fam["genomes"], fam["ranks"], int(k), fam["canon"])
+            else:
+                got = self._family_shard(fam["genomes"], fam["ranks"], int(k), fam["canon"], None)
+            fam["counts"][int(k)] = got
+        singles, hist = got
+        kind, r, i = cell
+        return int(singles[r]) if kind == "single" else int(hist[r, :i].sum())
+
+    def _family_shard(self, fastas, ranks, k, canon, shard):
+        """Engine.exact_family_counts on this process's key range `shard` (None: all keys), as int64."""
+        singles, hist = self.engine.exact_family_counts([self.packed(f) for f in fastas], int(k), bool(canon), ranks, shard=shard)
+        return np.asarray(singles, dtype=np.int64), np.asarray(hist, dtype=np.int64)
 
     def exact_prefix_counts(self, fastas: Sequence[str], k: int, canon: bool) -> List[int]:
         self.stats["exact_calls"] += 1
@@ -569,7 +632,7 @@ class GpuSketchStore:
     def start_exact_workers(self):
         """Multi-rank exact mode (dandd_b200.dist.ExactWorkers): rank 0 keeps going, the others serve."""
         from dandd_b200 import dist as dd_dist
-        self.exact_workers = dd_dist.ExactWorkers(self._exact_shard_counts, self._rank_hists_shard)
+        self.exact_workers = dd_dist.ExactWorkers(self._exact_shard_counts, self._rank_hists_shard, self._family_shard)
         return self.exact_workers
 
 

@@ -318,6 +318,13 @@ DD_API int dd_exact_pair_popc(const void *d_row_ws, int64_t row0, int nr, const 
 DD_API int dd_exact_first_rank_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
                                     uint32_t max_streams, int64_t n_genomes, const uint16_t *d_ranks, int64_t n_rows,
                                     uint64_t *d_hist, dd_stream stream);
+/* The K7 sparse workspace's node counter, copied on the stream into the caller's device word d_out (u64; no
+ * kernel, no synchronisation).  dd_exact_pairs_insert_shard pushes exactly one node per (genome, key of the
+ * range) it holds, so the counter read after a genome's insert minus the one read before it is the number of
+ * distinct keys of that genome in the workspace's key range: the single counts |A_g| of a family job come
+ * from the lists themselves.  The counter keeps counting past max_nodes; such a job is reported full by
+ * dd_exact_pairs_accumulate / dd_exact_first_rank_hist. */
+DD_API int dd_exact_pairs_node_count(const void *d_ws, size_t ws_bytes, uint64_t *d_out, dd_stream stream);
 
 /* ===========================================================================================
  * Host-buffer convenience path (what bench.py's e2e number times): one FASTA held in host memory
