@@ -500,6 +500,17 @@ int dd_exact_first_rank_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t 
             "dd_exact_first_rank_hist");
     return DD_OK;
 }
+// ---- K9 ------------------------------------------------------------------------------------------
+int dd_exact_occupancy_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams,
+                            int64_t n_genomes, uint64_t *d_hist, uint64_t *d_priv, dd_stream stream) {
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, "dd_exact_occupancy_hist")) return rc;
+    if (n_genomes < 1 || n_genomes > 0xFFFFFFFFll)   // genome indices are u32
+        return fail(DD_ERR_ARG, "dd_exact_occupancy_hist: n_genomes=%lld outside [1,4294967295]", (long long)n_genomes);
+    if (!d_hist) return fail(DD_ERR_ARG, "dd_exact_occupancy_hist: null pointer");
+    DD_CUDA(dd::exact_occupancy_hist(d_ws, k, capacity, max_streams, (uint64_t)n_genomes, d_hist, d_priv, sm_count_now(), S(stream)),
+            "dd_exact_occupancy_hist");
+    return DD_OK;
+}
 int dd_exact_pairs_node_count(const void *d_ws, size_t ws_bytes, uint64_t *d_out, dd_stream stream) {
     if (!d_ws || !d_out) return fail(DD_ERR_ARG, "dd_exact_pairs_node_count: null pointer");
     if (ws_bytes < sizeof(dd::ExactWsHeader)) return fail(DD_ERR_WORKSPACE, "dd_exact_pairs_node_count: workspace %zu too small", ws_bytes);

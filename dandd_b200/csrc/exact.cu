@@ -629,6 +629,89 @@ cudaError_t exact_first_rank_hist(const void *d_ws, int k, uint64_t capacity, un
     return launch(exact_first_rank_kernel<false, false>);
 }
 
+// ---- K9: the sharing spectrum over the K7 lists ------------------------------------------------------
+// A key's list holds one node per genome that holds it, so its length is the key's sharing count c:
+// hist[c - 1] counts the keys held by exactly c genomes, priv[g] (optional) the keys held by genome g alone.
+// Only the length and, for a list of one, its genome are needed -- so unlike K7 and K8, where a warp walks
+// one list at a time with broadcast loads, every lane walks the list of its own slot: 32 independent pointer
+// chases per warp.  kSmem: both counter arrays fit in shared memory (u32), flushed once per CTA.
+template <bool kSmem>
+__global__ void __launch_bounds__(256)
+exact_occupancy_kernel(const ExactWsHeader *__restrict__ hdr, const uint2 *__restrict__ lh, const PairNode *__restrict__ nodes,
+                       uint64_t n_slots, uint64_t n_genomes, unsigned long long *hist, unsigned long long *priv) {
+    extern __shared__ uint32_t sm_occ[];
+    if (hdr->overflow) {   // a full table or node array: the marker, never a count
+        for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_genomes; i += (uint64_t)gridDim.x * blockDim.x) {
+            hist[i] = kEmptyKey;
+            if (priv) priv[i] = kEmptyKey;
+        }
+        return;
+    }
+    uint32_t *sm_hist = sm_occ, *sm_priv = sm_occ + n_genomes;
+    if (kSmem) {
+        for (uint64_t i = threadIdx.x; i < (priv ? 2 : 1) * n_genomes; i += blockDim.x) sm_occ[i] = 0;
+        __syncthreads();
+    }
+    const uint64_t threads = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n_slots; s += threads) {   // 32 slots per warp load
+        uint32_t at = __ldg(&lh[s].y);
+        uint64_t c = 0;
+        uint32_t only = 0;
+        while (at != kNil) {
+            const PairNode nd = nodes[at];
+            if (nd.genome < n_genomes) {   // outside the caller's genome range: never counted, never an address
+                only = nd.genome;
+                ++c;
+            }
+            at = nd.next;
+        }
+        if (c == 0 || c > n_genomes) continue;   // (c > n: a genome pushed twice, against the insert contract)
+        if (kSmem) {
+            atomicAdd(&sm_hist[c - 1], 1u);
+            if (priv && c == 1) atomicAdd(&sm_priv[only], 1u);
+        } else {
+            atomicAdd(&hist[c - 1], 1ull);
+            if (priv && c == 1) atomicAdd(&priv[only], 1ull);
+        }
+    }
+    if (kSmem) {
+        __syncthreads();
+        for (uint64_t i = threadIdx.x; i < n_genomes; i += blockDim.x) {
+            if (sm_hist[i]) atomicAdd(&hist[i], (unsigned long long)sm_hist[i]);
+            if (priv && sm_priv[i]) atomicAdd(&priv[i], (unsigned long long)sm_priv[i]);
+        }
+    }
+}
+
+cudaError_t exact_occupancy_hist(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
+                                 uint64_t *d_hist, uint64_t *d_priv, int sm_count, cudaStream_t stream) {
+    if (n_genomes == 0) return cudaSuccess;
+    const uint8_t *ws = static_cast<const uint8_t *>(d_ws);
+    const ExactWsHeader *hdr = static_cast<const ExactWsHeader *>(d_ws);
+    const uint2 *lh = reinterpret_cast<const uint2 *>(ws + pairs_lh_offset(k, capacity, max_streams));
+    const PairNode *nodes = reinterpret_cast<const PairNode *>(ws + pairs_node_offset(k, capacity, max_streams));
+    unsigned long long *hist = reinterpret_cast<unsigned long long *>(d_hist);
+    unsigned long long *priv = reinterpret_cast<unsigned long long *>(d_priv);
+    const uint64_t n_slots = capacity + 1;
+    const size_t smem = (size_t)(d_priv ? 2 : 1) * n_genomes * sizeof(uint32_t);
+    const uint64_t want = (n_slots + 255) / 256;   // one slot per thread
+    if (smem <= kPairSmemBytes) {
+        // a latency-bound walk wants full occupancy; every CTA pays one pass over its counters at each end
+        const uint64_t per_sm = smem <= 8 * 1024 ? 8 : 2;
+        const unsigned grid = (unsigned)(want < (uint64_t)sm_count * per_sm ? want : (uint64_t)sm_count * per_sm);
+        if (smem > 48 * 1024) {
+            const cudaError_t e = cudaFuncSetAttribute(exact_occupancy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                       (int)kPairSmemBytes);
+            if (e != cudaSuccess) return e;
+        }
+        DD_COUNT_LAUNCH(), exact_occupancy_kernel<true><<<grid, 256, smem, stream>>>(hdr, lh, nodes, n_slots, n_genomes, hist, priv);
+    } else {
+        const unsigned grid = (unsigned)(want < (uint64_t)sm_count * 16 ? want : (uint64_t)sm_count * 16);
+        DD_COUNT_LAUNCH(), exact_occupancy_kernel<false><<<grid, 256, 0, stream>>>(hdr, lh, nodes, n_slots, n_genomes, hist, priv);
+    }
+    return cudaGetLastError();
+}
+
 // Dense path: popc(A & B) over K5 presence bitmaps.  A CTA owns a tile of 8 row genomes x 8 column
 // genomes and a slice of the bitmap words: each word range of the 16 bitmaps is read once per tile
 // (from L2 when other tiles have just read it) and feeds 64 pair counters.

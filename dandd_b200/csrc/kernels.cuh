@@ -98,6 +98,10 @@ cudaError_t exact_pairs_accumulate(const void *d_ws, int k, uint64_t capacity, u
 // ---- K8 (exact.cu): first-rank histograms over the K7 lists, ranks [n_rows][n_genomes] u16 -> hist [n_rows][n_genomes]
 cudaError_t exact_first_rank_hist(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
                                   const uint16_t *d_ranks, uint64_t n_rows, uint64_t *d_hist, int sm_count, cudaStream_t stream);
+// ---- K9 (exact.cu): sharing spectrum over the K7 lists -> hist [n_genomes] (keys held by c = i + 1 genomes),
+// priv [n_genomes] or null (keys held by genome g alone)
+cudaError_t exact_occupancy_hist(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
+                                 uint64_t *d_hist, uint64_t *d_priv, int sm_count, cudaStream_t stream);
 // the node counter of a K7 sparse workspace (ExactWsHeader::n_nodes) -> *d_out, a copy on the stream
 cudaError_t exact_pairs_node_count(const void *d_ws, uint64_t *d_out, cudaStream_t stream);
 // Dense: K5 bitmap workspaces, ws_stride bytes apart, for genomes row0.. and col0..

@@ -564,6 +564,34 @@ class Engine:
             singles += np.diff(got[cells:], prepend=np.uint64(0))
         return singles, hist
 
+    # ---- K9 ---------------------------------------------------------------------------------
+    def exact_spectrum(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
+                       passes: Optional[int] = None):
+        """(hist, singles, priv), uint64 [n] each, in one job at k: hist[c - 1] = distinct k-mers held by exactly c of
+        seqs, singles[g] = |A_g|, priv[g] = k-mers held by seqs[g] alone (this rank's key range under `shard`).  Sized
+        from the sequence lengths and with the singles from the list-node counter, as exact_family_counts; one K7 list
+        job, one K9 launch and one device->host copy per pass."""
+        n = len(seqs)
+        hist, singles, priv = (np.zeros(n, dtype=np.uint64) for _ in range(3))
+        if n == 0:
+            return hist, singles, priv
+        if k > 64 and n > 65536:
+            raise DandDError("the exact spectrum above k = 64 takes at most 65536 genomes per job")
+        world = int(shard[1]) if shard is not None else 1
+        bounds = length_bounds([s.nsym for s in seqs], k, world)
+        part = torch.zeros(3 * n, dtype=torch.int64, device=self.device)    # [hist | priv | node counter after genome g]
+        for ws, cap, nodes in self._key_lists(seqs, k, canon, bounds, shard, passes, node_counts=part[2 * n:]):
+            part[:2 * n].zero_()
+            check(self.lib.dd_exact_occupancy_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part.data_ptr(),
+                                                   part.data_ptr() + 8 * n, self.stream), "dd_exact_occupancy_hist")
+            got = part.cpu().numpy().view(np.uint64)
+            if (got[:2 * n] == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
+                raise DandDError("exact k-mer table or node array overflowed; the length bounds understate the genomes")
+            hist += got[:n]
+            priv += got[n:2 * n]
+            singles += np.diff(got[2 * n:], prepend=np.uint64(0))
+        return hist, singles, priv
+
     def exact_pairs_dense(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
                           block: Optional[int] = None) -> np.ndarray:
         """The bitmap path of exact_pair_intersections (k <= DD_EXACT_BITMAP_MAXK): one K5 presence bitmap

@@ -612,6 +612,23 @@ class GpuSketchStore:
             out[c] = self.engine.exact_first_rank_hist(seqs, int(k), bool(canon), ranks, singles=s, shard=shard).astype(np.int64)
         return out
 
+    def exact_spectrum(self, fastas: Sequence[str], ks: Sequence[int], canon: bool,
+                       shard: Optional[Tuple[int, int]] = None) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """The sharing spectrum of the FASTAs at every k: (hist, singles, priv), int64 [nk, n] each; hist[c, i - 1] =
+        distinct k-mers held by exactly i of the FASTAs at ks[c], singles[c, g] = |fastas[g]|, priv[c, g] = k-mers only
+        fastas[g] holds.  One engine job per k (Engine.exact_spectrum: K7 lists + K9).  shard=(rank, world): this
+        rank's key range only; the ranks' results add up.  There is no per-union fallback: the spectrum has no cheap
+        equivalent in union counts."""
+        if not hasattr(self.engine, "exact_spectrum"):
+            raise RuntimeError("the exact sharing spectrum needs an engine with the spectrum job (Engine.exact_spectrum)")
+        n, ks = len(fastas), [int(k) for k in ks]
+        seqs = [self.packed(f) for f in fastas]
+        out = np.zeros((3, len(ks), n), dtype=np.int64)
+        for c, k in enumerate(ks):
+            self.stats["exact_calls"] += 1
+            out[:, c] = [np.asarray(a, dtype=np.int64) for a in self.engine.exact_spectrum(seqs, k, bool(canon), shard=shard)]
+        return out[0], out[1], out[2]
+
     def _exact_from_table(self, fastas, k, canon):
         tab = getattr(self, "exact_pair_table", None)
         if tab is None or tab["canon"] != bool(canon) or int(k) not in tab["col"] or not 1 <= len(fastas) <= 2:

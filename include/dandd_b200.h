@@ -327,6 +327,21 @@ DD_API int dd_exact_first_rank_hist(const void *d_ws, size_t ws_bytes, int k, ui
 DD_API int dd_exact_pairs_node_count(const void *d_ws, size_t ws_bytes, uint64_t *d_out, dd_stream stream);
 
 /* ===========================================================================================
+ * K9  --exact sharing spectrum at one k, from the K7 sparse workspace after every genome has been inserted
+ * with dd_exact_pairs_insert_shard (same workspace, same arguments).  A key's list holds one node per genome
+ * holding it, so its length is the key's sharing count c.  Adds into d_hist [n_genomes] u64 (the caller
+ * zeroes it): d_hist[c - 1] = number of distinct keys held by exactly c of the genomes 0 .. n_genomes-1; and,
+ * if d_priv is not NULL, into d_priv [n_genomes] u64: d_priv[g] = number of keys genome g alone holds.  Nodes
+ * of a genome index >= n_genomes are not counted.  1 <= n_genomes < 2^32.  With the singles |A_g| (the node
+ * counter, dd_exact_pairs_node_count) this gives the core / shell / cloud split of a collection and, in
+ * closed form, the mean union and intersection of the first m genomes over all n! orderings.  A full table
+ * or node array writes all-ones into every cell of d_hist (and of d_priv).
+ * =========================================================================================== */
+DD_API int dd_exact_occupancy_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                                   uint32_t max_streams, int64_t n_genomes, uint64_t *d_hist, uint64_t *d_priv,
+                                   dd_stream stream);
+
+/* ===========================================================================================
  * Host-buffer convenience path (what bench.py's e2e number times): one FASTA held in host memory
  * -> H2D copy -> K1 -> K2 -> K4 -> D2H of cardinalities (and registers if h_regs != NULL);
  * synchronises the stream before returning.  Equivalent to the reference running
