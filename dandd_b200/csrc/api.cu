@@ -85,6 +85,10 @@ int dd_set_option(const char *name, long value) {
         dd::g_midk = value != 0;
         return DD_OK;
     }
+    if (!strcmp(name, "sketch_sink")) {
+        dd::g_sink = value != 0;
+        return DD_OK;
+    }
     if (!strcmp(name, "prefix_planes")) {
         dd::g_prefix_planes = value != 0;
         return DD_OK;

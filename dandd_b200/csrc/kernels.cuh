@@ -24,9 +24,11 @@ cudaError_t pack_polyt_sentinel(const uint32_t *d_codes, uint32_t *d_invalid, co
                                 uint64_t sym_begin, uint64_t sym_end, size_t max_symbols, cudaStream_t stream);
 extern int g_polyt_sentinel;  // dd_set_option("polyt_sentinel"): the *_host entry points apply the pass
 
-// ---- K2 (sketch.cu).  Workspace = [SketchWsHeader | u16 accumulators [nk][2^p]]
+// ---- K2 (sketch.cu).  Workspace = [SketchWsHeader | scratch | u16 accumulators [nk][2^p] | rank-1 sink bitmaps
+// [nk][2^p/32] u32 | mid-k presence bitmaps]; register = max(accumulator, sink bit)
 extern int g_k_per_pass;
 extern int g_midk;
+extern int g_sink;
 struct SketchWsHeader {
     uint8_t floor[32];  // floor[k-1] <= min(register of k): updates with rank <= floor are no-ops
     uint32_t use_floor;

@@ -163,6 +163,75 @@ __device__ __forceinline__ uint64_t xorshr(uint64_t h) {
 #endif
 }
 
+// dd::wang64 (common.cuh) with the multiplications pinned to the FMA pipe
+__device__ __forceinline__ uint64_t wang64_fma(uint64_t v, uint64_t minus_one) {
+    uint64_t h = mad64x32(v, 0x1FFFFFu, minus_one);
+#if DD_XORSHIFT_ON_FMA
+    h = xorshr_fma<24>(h);
+    h = mul64x32(h, 265u);
+    h = xorshr_fma<14>(h);
+    h = mul64x32(h, 21u);
+    h = xorshr_fma<28>(h);
+#else
+    h = xorshr<24>(h);
+    h = mul64x32(h, 265u);
+    h = xorshr<14>(h);
+    h = mul64x32(h, 21u);
+    h = xorshr<28>(h);
+#endif
+    return mul64x32(h, 0x80000001u);
+}
+
+// Rank of a hash whose 32 bits below the register index are t (lo = its low word): clz(t) + 1 unless
+// they are all zero.
+__device__ __forceinline__ uint32_t rank_of(uint32_t t, uint32_t lo, int p) {
+    return t ? (uint32_t)__clz((int)t) + 1u : 33u + (uint32_t)__clz((int)((lo << p) | (1u << (p - 1))));
+}
+
+// acc[slot_off + register / 2] = max(.., rank) on the register's u16 half (register = hi >> (32 - p))
+__device__ __forceinline__ void red_max_register(uint32_t *acc, uint32_t slot_off, uint32_t hi, uint32_t rank, int p) {
+    // register idx = hi >> (32-p) lives in word idx>>1, half idx&1
+    const uint32_t val = rank << ((hi >> (28 - p)) & 16u);
+    uint32_t *word = acc + (slot_off + (hi >> (33 - p)));
+    asm volatile("{ .reg .b16 l, h; mov.b32 {l, h}, %1; red.global.max.noftz.v2.f16 [%0], {l, h}; }" ::"l"(word), "r"(val) : "memory");
+}
+
+// The packed words behind the 16 symbols of code word w: every window ending in it is two funnel
+// shifts over w0..w2 (r0..r2 = their reverse complements), its validity a ctz over i0:i1.  Only
+// symbols j_lo <= j < j_hi lie in the range being sketched; a word out of range has none.
+struct WordSpan {
+    uint32_t w0, w1, w2, r0, r1, r2, i0, i1;
+    uint32_t sm_base;
+    int j_lo, j_hi;
+    bool all_valid;
+};
+__device__ __forceinline__ WordSpan load_word(const uint32_t *codes, const uint32_t *invalid, uint64_t w, bool in_range,
+                                              uint64_t sym_begin, uint64_t sym_end) {
+    WordSpan s;
+    const uint64_t s0 = w << 4;
+    s.w0 = in_range ? __ldg(codes + w) : 0u;
+    s.w1 = in_range && w >= 1 ? __ldg(codes + w - 1) : 0u;
+    s.w2 = in_range && w >= 2 ? __ldg(codes + w - 2) : 0u;
+    const uint64_t iw = w >> 1;
+    s.i0 = in_range ? __ldg(invalid + iw) : 0xffffffffu;
+    s.i1 = in_range && iw >= 1 ? __ldg(invalid + iw - 1) : 0xffffffffu;  // before the stream: breaks
+    s.r0 = revcomp_word(s.w0);
+    s.r1 = revcomp_word(s.w1);
+    s.r2 = revcomp_word(s.w2);
+    s.all_valid = (s.i0 | s.i1) == 0u;
+    s.j_lo = sym_begin > s0 ? (int)(sym_begin - s0) : 0;
+    s.j_hi = !in_range ? 0 : (sym_end - s0 < 16 ? (int)(sym_end - s0) : 16);
+    s.sm_base = (uint32_t)(s0 & 31);
+    return s;
+}
+__device__ __forceinline__ Window span_window(const WordSpan &s, int j) { return window_at(s.w0, s.w1, s.w2, s.r0, s.r1, s.r2, j); }
+// valid symbols ending at symbol j of the word (0 outside the range)
+__device__ __forceinline__ int span_run(const WordSpan &s, int j) {
+    int run = s.all_valid ? 32 : valid_run(invalid_window(s.i0, s.i1, s.sm_base + (uint32_t)j));
+    if (j < s.j_lo || j >= s.j_hi) run = 0;
+    return run;
+}
+
 // Canonical (or forward) k-mer ending at the current symbol.  For K <= 16 the whole k-mer lives in
 // one 32-bit register: mask, shift and min are single instructions.
 template <int K, bool kCanon>
@@ -232,22 +301,7 @@ __device__ __forceinline__ void update_one_k(const Window &win, int run, uint32_
             return;
         }
     }
-    // dd::wang64 (common.cuh) with the multiplications pinned to the FMA pipe
-    uint64_t h = mad64x32(v, 0x1FFFFFu, minus_one);
-#if DD_XORSHIFT_ON_FMA
-    h = xorshr_fma<24>(h);
-    h = mul64x32(h, 265u);
-    h = xorshr_fma<14>(h);
-    h = mul64x32(h, 21u);
-    h = xorshr_fma<28>(h);
-#else
-    h = xorshr<24>(h);
-    h = mul64x32(h, 265u);
-    h = xorshr<14>(h);
-    h = mul64x32(h, 21u);
-    h = xorshr<28>(h);
-#endif
-    h = mul64x32(h, 0x80000001u);
+    const uint64_t h = wang64_fma(v, minus_one);
     const uint32_t hi = (uint32_t)(h >> 32), lo = (uint32_t)h;
     // t = the 32 bits below the register index; rank = clz(t) + 1 unless they are all zero
     const uint32_t t = __funnelshift_l(lo, hi, (uint32_t)p);
@@ -256,14 +310,10 @@ __device__ __forceinline__ void update_one_k(const Window &win, int run, uint32_
     if (__any_sync(0xffffffffu, pass))   // warp-uniform branch (no reconvergence barrier); the tail is predicated
 #endif
     if (pass) {
-        const uint32_t rank = t ? (uint32_t)__clz((int)t) + 1u : 33u + (uint32_t)__clz((int)((lo << p) | (1u << (p - 1))));
+        const uint32_t rank = rank_of(t, lo, p);
         if (rank > kc.floor[K - 1]) {
-            // register idx = hi >> (32-p) lives in word idx>>1, half idx&1
-            const uint32_t val = rank << ((hi >> (28 - p)) & 16u);
             const uint32_t slot_off = kStaticMask ? (uint32_t)__popc(kStaticMask & (bit - 1u)) << (p - 1) : off_k;
-            uint32_t *word = acc + (slot_off + (hi >> (33 - p)));
-            asm volatile("{ .reg .b16 l, h; mov.b32 {l, h}, %1; red.global.max.noftz.v2.f16 [%0], {l, h}; }" ::"l"(word), "r"(val)
-                         : "memory");
+            red_max_register(acc, slot_off, hi, rank, p);
         }
     }
     if (!kStaticMask) off_k += 1u << (p - 1);
@@ -278,6 +328,26 @@ __device__ __forceinline__ void update_all_k(std::integer_sequence<int, Ks...>, 
     (update_one_k<Ks + 1, kCanon, kStaticMask, kMidK>(win, run, kmask, kmask_run, p, acc, off_k, kc, s_seen, midk, midk_hi, minus_one), ...);
 }
 
+// per-k floors (indexed by k-1) and the remainder thresholds derived from them; the caller syncs
+__device__ __forceinline__ void load_kconsts(const SketchWsHeader *hdr, KConsts &kc) {
+    if (threadIdx.x < 32) {
+        const uint32_t f = hdr->floor[threadIdx.x];
+        kc.floor[threadIdx.x] = f;
+        kc.thresh[threadIdx.x] = f >= 32u ? 0u : 0xffffffffu >> f;
+    }
+}
+
+// [sym_begin, sym_end) of a launch: explicit, or read from the pack state on the device
+__device__ __forceinline__ void launch_range(const SketchArgs &a, uint64_t &sym_begin, uint64_t &sym_end) {
+    sym_begin = a.sym_begin;
+    sym_end = a.sym_end;
+    if (a.state) {   // the range of the last pack call; a.sym_begin / a.sym_end select a sub-range of it, relative to its start
+        const uint64_t first = a.state->prev_nsym, last = a.state->nsym;
+        sym_begin = first + a.sym_begin < last ? first + a.sym_begin : last;
+        sym_end = a.sym_end < last - first ? first + a.sym_end : last;
+    }
+}
+
 template <bool kCanon, uint32_t kStaticMask, int kThreads, bool kMidK = false>
 __global__ void __launch_bounds__(kThreads, min_ctas_for(kThreads)) sketch_allk_kernel(SketchArgs a) {
     extern __shared__ uint32_t s_seen[];  // presence bitmaps, only allocated when a k <= 9 is requested
@@ -286,53 +356,113 @@ __global__ void __launch_bounds__(kThreads, min_ctas_for(kThreads)) sketch_allk_
         for (uint32_t i = threadIdx.x; i < kBitmapWords; i += kThreads) s_seen[i] = 0u;
         __syncthreads();
     }
-    // per-k floors (indexed by k-1) and the remainder thresholds derived from them
     __shared__ KConsts kc;
-    if (threadIdx.x < 32) {
-        const uint32_t f = a.hdr->floor[threadIdx.x];
-        kc.floor[threadIdx.x] = f;
-        kc.thresh[threadIdx.x] = f >= 32u ? 0u : 0xffffffffu >> f;
-    }
+    load_kconsts(a.hdr, kc);
     __syncthreads();
     const uint64_t minus_one = ~0ull;   // (ptxas splits the addend off the IMAD.WIDE whether or not it can see its value)
     // k = 13 / 14 bitmaps: only those the header says were zeroed since dd_sketch_begin
     const int midk_hi = kMidK ? min(a.midk_hi, max(12, (int)a.hdr->pad[0])) : 0;
-    uint64_t sym_begin = a.sym_begin, sym_end = a.sym_end;
-    if (a.state) {   // the range of the last pack call; a.sym_begin / a.sym_end select a sub-range of it, relative to its start
-        const uint64_t first = a.state->prev_nsym, last = a.state->nsym;
-        sym_begin = first + a.sym_begin < last ? first + a.sym_begin : last;
-        sym_end = a.sym_end < last - first ? first + a.sym_end : last;
-    }
+    uint64_t sym_begin, sym_end;
+    launch_range(a, sym_begin, sym_end);
 
 #pragma unroll 1
     for (uint32_t tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
         const uint64_t w = (sym_begin >> 4) + (uint64_t)tile * kThreads + threadIdx.x;
-        const uint64_t s0 = w << 4;
         if ((uint64_t)((sym_begin >> 4) + (uint64_t)tile * kThreads) << 4 >= sym_end) break;  // CTA-uniform
-        const bool in_range = s0 < sym_end;   // lanes past the end stay in the loop, predicated off
-
-        const uint32_t w0 = in_range ? __ldg(a.codes + w) : 0u;
-        const uint32_t w1 = in_range && w >= 1 ? __ldg(a.codes + w - 1) : 0u;
-        const uint32_t w2 = in_range && w >= 2 ? __ldg(a.codes + w - 2) : 0u;
-        const uint64_t iw = w >> 1;
-        const uint32_t i0 = in_range ? __ldg(a.invalid + iw) : 0xffffffffu;
-        const uint32_t i1 = in_range && iw >= 1 ? __ldg(a.invalid + iw - 1) : 0xffffffffu;  // before the stream: breaks
-        const uint32_t r0 = revcomp_word(w0), r1 = revcomp_word(w1), r2 = revcomp_word(w2);
-        const bool all_valid = (i0 | i1) == 0u;
-
-        const int j_lo = sym_begin > s0 ? (int)(sym_begin - s0) : 0;
-        const int j_hi = !in_range ? 0 : (sym_end - s0 < 16 ? (int)(sym_end - s0) : 16);
-        const uint32_t sm_base = (uint32_t)(s0 & 31);
+        // lanes past the end stay in the loop, predicated off
+        const WordSpan ws = load_word(a.codes, a.invalid, w, (w << 4) < sym_end, sym_begin, sym_end);
 
 #pragma unroll 1
         for (int j = 0; j < 16; ++j) {
-            const Window win = window_at(w0, w1, w2, r0, r1, r2, j);
-            int run = all_valid ? 32 : valid_run(invalid_window(i0, i1, sm_base + (uint32_t)j));
-            if (j < j_lo || j >= j_hi) run = 0;
+            const Window win = span_window(ws, j);
+            const int run = span_run(ws, j);
             if (!__any_sync(0xffffffffu, run != 0)) continue;  // warp-uniform
             update_all_k<kCanon, kStaticMask, kMidK>(std::make_integer_sequence<int, 32>{}, win, run, a.kmask, a.kmask_run, a.p,
                                                      a.acc, kc, s_seen, a.midk, midk_hi, minus_one);
         }
+    }
+}
+
+// ---- rank-1 sink: one k per CTA, rank-1 updates absorbed in a shared-memory bitmap ---------------
+// Half of all updates have rank 1, and a rank-1 update can only raise a register from 0 to 1: all it
+// records is "some k-mer hit register r", one bit.  Before the floor schedule's first cut (floor 0)
+// every such update is a scattered L2 reduction -- the resource that bounds K2 on short genomes.  Here
+// a CTA owns one k over a contiguous slice of the stream and ORs its rank-1 updates into a 2^p-bit
+// bitmap in shared memory (128 KiB at p = 20); at the end only the non-zero words go to the
+// workspace's per-k sink bitmap with red.global.or.  Every such merge carries at least one rank-1
+// update, so the sink never issues more L2 reductions than the plain kernel.  The register is
+// max(acc, bit) -- finalize_kernel and floor_min_kernel read it so -- which keeps the result exact
+// under any floor (floor >= 1 drops rank 1 at the threshold already).  k <= 9 stays with the
+// presence-bitmap kernel.
+constexpr int kSinkThreads = 1024, kSinkMinK = kBitmapMaxK + 1, kSinkMaxP = 20;
+
+template <int K, bool kCanon>
+__device__ __forceinline__ void sink_slice(const SketchArgs &a, const KConsts &kc, uint32_t *s_bits, uint32_t slot_off,
+                                           uint64_t sym_begin, uint64_t sym_end, uint64_t w_lo, uint64_t w_hi) {
+    const uint64_t minus_one = ~0ull;
+    const int p = a.p;
+#pragma unroll 1
+    for (uint64_t base = w_lo; base < w_hi; base += kSinkThreads) {
+        const uint64_t w = base + threadIdx.x;
+        const WordSpan ws = load_word(a.codes, a.invalid, w, w < w_hi, sym_begin, sym_end);
+#pragma unroll 1
+        for (int j = 0; j < 16; ++j) {
+            const bool live = span_run(ws, j) >= K;
+            if (!__any_sync(0xffffffffu, live)) continue;  // warp-uniform
+            const uint64_t h = wang64_fma(kmer_of<K, kCanon>(span_window(ws, j)), minus_one);
+            const uint32_t hi = (uint32_t)(h >> 32), lo = (uint32_t)h;
+            const uint32_t t = __funnelshift_l(lo, hi, (uint32_t)p);
+            if (live && t <= kc.thresh[K - 1]) {
+                if ((int32_t)t < 0) {   // rank 1
+                    const uint32_t r = hi >> (32 - p);
+                    atomicOr(s_bits + (r >> 5), 1u << (r & 31u));
+                } else {
+                    const uint32_t rank = rank_of(t, lo, p);
+                    if (rank > kc.floor[K - 1]) red_max_register(a.acc, slot_off, hi, rank, p);
+                }
+            }
+        }
+    }
+}
+
+// CTA-uniform dispatch to the compile-time K of this CTA (immediate masks in kmer_of)
+template <bool kCanon, int... Ks>
+__device__ __forceinline__ void sink_dispatch(std::integer_sequence<int, Ks...>, int k, const SketchArgs &a, const KConsts &kc,
+                                              uint32_t *s_bits, uint32_t slot_off, uint64_t sym_begin, uint64_t sym_end,
+                                              uint64_t w_lo, uint64_t w_hi) {
+    ((k == Ks + kSinkMinK ? sink_slice<Ks + kSinkMinK, kCanon>(a, kc, s_bits, slot_off, sym_begin, sym_end, w_lo, w_hi) : void()), ...);
+}
+
+// grid = (k values of a.kmask_run, all >= kSinkMinK) x slices; dynamic shared memory = 2^p / 8 bytes
+template <bool kCanon>
+__global__ void __launch_bounds__(kSinkThreads, 1) sketch_sink_kernel(SketchArgs a, uint32_t *sink, uint32_t slices) {
+    extern __shared__ uint4 s_bits4[];
+    uint32_t *s_bits = reinterpret_cast<uint32_t *>(s_bits4);
+    const int p = a.p;
+    const uint32_t nwords = 1u << (p - 5);
+    for (uint32_t i = threadIdx.x; i < (nwords + 3) / 4; i += kSinkThreads) s_bits4[i] = make_uint4(0u, 0u, 0u, 0u);
+    __shared__ KConsts kc;
+    load_kconsts(a.hdr, kc);
+    __syncthreads();
+
+    // this CTA's k: the (blockIdx.x / slices)-th set bit of kmask_run; its table slot counts over kmask
+    uint32_t m = a.kmask_run;
+    for (uint32_t u = blockIdx.x / slices; u > 0; --u) m &= m - 1u;
+    const int k = __ffs((int)m);
+    const uint32_t slot = (uint32_t)__popc(a.kmask & ((1u << (k - 1)) - 1u));
+    // this CTA's slice: whole code words, so every symbol of the range belongs to exactly one slice
+    uint64_t sym_begin, sym_end;
+    launch_range(a, sym_begin, sym_end);
+    const uint64_t wb = sym_begin >> 4, we = sym_end > sym_begin ? (sym_end + 15) >> 4 : wb;
+    const uint64_t per = (we - wb + slices - 1) / slices, slice = blockIdx.x % slices;
+    const uint64_t w_lo = min(wb + slice * per, we), w_hi = min(w_lo + per, we);
+    sink_dispatch<kCanon>(std::make_integer_sequence<int, 33 - kSinkMinK>{}, k, a, kc, s_bits, slot << (p - 1), sym_begin, sym_end,
+                          w_lo, w_hi);
+    __syncthreads();
+    uint32_t *g = sink + (size_t)slot * nwords;
+    for (uint32_t i = threadIdx.x; i < nwords; i += kSinkThreads) {
+        const uint32_t v = s_bits[i];
+        if (v) atomicOr(g + i, v);
     }
 }
 
@@ -342,14 +472,25 @@ __global__ void midk_ready_kernel(SketchWsHeader *hdr, uint32_t k) {
 }
 
 // ---- per-slot min(register): the "floor" filter ---------------------------------------------------
-__global__ void __launch_bounds__(256) floor_min_kernel(const uint32_t *__restrict__ acc, int p, SketchWsHeader *hdr,
-                                                        uint32_t *scratch /*[nk]*/) {
-    // grid (slices, nk); scratch pre-set to 0xff.  acc rows are 2^p u16 registers = 2^(p-1) words.
+// Rank-1 sink bits as register values: bit i of x -> byte i (0 or 1), i < 4; -> u16 half i, i < 2.
+__device__ __forceinline__ uint32_t bits_to_bytes(uint32_t x) { return (x * 0x00204081u) & 0x01010101u; }
+__device__ __forceinline__ uint32_t bits_to_halves(uint32_t x) { return (x & 1u) | ((x & 2u) << 15); }
+
+__global__ void __launch_bounds__(256) floor_min_kernel(const uint32_t *__restrict__ acc, const uint32_t *__restrict__ sink, int p,
+                                                        SketchWsHeader *hdr, uint32_t *scratch /*[nk]*/) {
+    // grid (slices, nk); scratch pre-set to 0xff.  acc rows are 2^p u16 registers = 2^(p-1) words;
+    // register = max(acc, sink bit), byte i of a sink row holding the bits of registers 8i..8i+7.
     const size_t nwords = (size_t)1 << (p - 1);
     const uint32_t *t = acc + (size_t)blockIdx.y * nwords;
+    const uint8_t *bits = reinterpret_cast<const uint8_t *>(sink) + ((size_t)blockIdx.y << (p - 3));
     uint32_t mn = 0xffffu;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nwords / 4; i += (size_t)gridDim.x * blockDim.x) {
-        const uint4 v = reinterpret_cast<const uint4 *>(t)[i];
+        uint4 v = reinterpret_cast<const uint4 *>(t)[i];
+        const uint32_t b = bits[i];
+        v.x = __vmaxu2(v.x, bits_to_halves(b));
+        v.y = __vmaxu2(v.y, bits_to_halves(b >> 2));
+        v.z = __vmaxu2(v.z, bits_to_halves(b >> 4));
+        v.w = __vmaxu2(v.w, bits_to_halves(b >> 6));
         const uint32_t w = __vminu2(__vminu2(v.x, v.y), __vminu2(v.z, v.w));
         mn = min(mn, min(w & 0xffffu, w >> 16));
     }
@@ -372,13 +513,15 @@ constexpr int kFinOctPerThread = 30;                                   // 30 x 8
 constexpr int kFinChunk = kPhThreads * kFinOctPerThread * 8;           // registers per CTA
 
 __global__ void __launch_bounds__(kPhThreads)
-finalize_kernel(const uint32_t *__restrict__ acc, int p, uint8_t *__restrict__ regs, uint32_t *__restrict__ hist) {
+finalize_kernel(const uint32_t *__restrict__ acc, const uint32_t *__restrict__ sink, int p, uint8_t *__restrict__ regs,
+                uint32_t *__restrict__ hist) {
     __shared__ __align__(16) uint8_t s_hist[kPhBytes];
     const uint32_t slot = ph_slot();
     const size_t m = (size_t)1 << p;
     const int table = blockIdx.y;
-    // 8 u16 accumulators (one uint4) -> 8 u8 registers (one uint2)
+    // 8 u16 accumulators (one uint4) and one byte of rank-1 sink bits -> 8 u8 registers (one uint2)
     const uint4 *src = reinterpret_cast<const uint4 *>(acc + (size_t)table * (m / 2));
+    const uint8_t *bits = reinterpret_cast<const uint8_t *>(sink) + (size_t)table * (m / 8);
     uint2 *dst = reinterpret_cast<uint2 *>(regs + (size_t)table * m);
     if (hist) ph_zero(s_hist);
     __syncthreads();
@@ -390,7 +533,9 @@ finalize_kernel(const uint32_t *__restrict__ acc, int p, uint8_t *__restrict__ r
         if (q < noct) {
             const uint4 v = __ldcs(src + q);
             // bytes 0 and 2 of each word are the low bytes of its two u16 registers (ranks < 256)
-            const uint2 out = make_uint2(__byte_perm(v.x, v.y, 0x6420), __byte_perm(v.z, v.w, 0x6420));
+            const uint32_t b = __ldcs(bits + q);
+            const uint2 out = make_uint2(__vmaxu4(__byte_perm(v.x, v.y, 0x6420), bits_to_bytes(b & 15u)),
+                                         __vmaxu4(__byte_perm(v.z, v.w, 0x6420), bits_to_bytes(b >> 4)));
             dst[q] = out;
             if (hist) {
                 ph_add_word(s_hist, slot, out.x);
@@ -465,37 +610,66 @@ static unsigned persistent_grid(const SketchVariant &v, size_t smem) {
 }
 
 static size_t acc_bytes(int nk, int p) { return ((size_t)nk * sizeof(uint16_t) * ((size_t)1 << p) + 255) / 256 * 256; }
-size_t sketch_workspace_bytes(int nk, int p) {   // [header | scratch | accumulators | mid-k bitmaps]
-    return sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + (size_t)kMidKWords * sizeof(uint32_t);
-}
-static uint32_t *ws_midk(void *ws, int nk, int p) {
-    return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p));
+static size_t sink_bytes(int nk, int p) { return (((size_t)nk << (p - 3)) + 255) / 256 * 256; }   // [nk][2^p / 32] u32
+size_t sketch_workspace_bytes(int nk, int p) {   // [header | scratch | accumulators | rank-1 sink bitmaps | mid-k bitmaps]
+    return sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + sink_bytes(nk, p) + (size_t)kMidKWords * sizeof(uint32_t);
 }
 static SketchWsHeader *ws_hdr(void *ws) { return static_cast<SketchWsHeader *>(ws); }
 static uint32_t *ws_scratch(void *ws) { return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader)); }
 static uint32_t *ws_acc(void *ws) { return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader) + 256); }
+static uint32_t *ws_sink(void *ws, int nk, int p) {
+    return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p));
+}
+static uint32_t *ws_midk(void *ws, int nk, int p) {
+    return reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(ws_sink(ws, nk, p)) + sink_bytes(nk, p));
+}
 
 cudaError_t sketch_begin(void *d_ws, int nk, int p, cudaStream_t stream) {
-    // header, scratch, accumulators and the k <= 12 bitmaps; the 8 + 32 MiB of k = 13 / 14 are zeroed by the
-    // launch that first consults them (only streams longer than 4^13 symbols ever do)
-    return cudaMemsetAsync(d_ws, 0, sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + (size_t)midk_offset(13) * sizeof(uint32_t), stream);
+    // header, scratch, accumulators, sink bitmaps and the k <= 12 bitmaps; the 8 + 32 MiB of k = 13 / 14 are
+    // zeroed by the launch that first consults them (only streams longer than 4^13 symbols ever do)
+    return cudaMemsetAsync(d_ws, 0,
+                           sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + sink_bytes(nk, p) + (size_t)midk_offset(13) * sizeof(uint32_t),
+                           stream);
 }
 
 int g_midk = 1;   // dd_set_option("sketch_midk", 0/1): tuning knob, never changes results
+int g_sink = 1;   // dd_set_option("sketch_sink", 0/1): A/B switch for the rank-1 sink, never changes results
+
+// resident sink CTAs on this device (its SM count x CTAs per SM at 2^p/8 bytes of shared memory), cached
+static unsigned sink_resident(bool canon, int p) {
+    constexpr int kMaxDev = 64;
+    static unsigned cached[kMaxDev][2][kSinkMaxP + 1] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    unsigned local = 0;
+    unsigned &g = (dev >= 0 && dev < kMaxDev) ? cached[dev][canon ? 1 : 0][p] : local;
+    if (g == 0) {
+        const auto fn = canon ? sketch_sink_kernel<true> : sketch_sink_kernel<false>;
+        cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(((size_t)1 << kSinkMaxP) / 8));
+        int sms = 148, per_sm = 1;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kSinkThreads, ((size_t)1 << p) / 8);
+        g = (unsigned)(sms * (per_sm > 0 ? per_sm : 1));
+    }
+    return g;
+}
 
 static cudaError_t sketch_update_impl(const uint32_t *d_codes, const uint32_t *d_invalid, const dd_pack_state *d_state,
                                       uint64_t sym_begin, uint64_t sym_end, size_t max_new_symbols, uint32_t kmask, int p,
-                                      int canon, void *d_ws, int midk_hi, cudaStream_t stream);
+                                      int canon, void *d_ws, int midk_hi, bool sink, cudaStream_t stream);
 
 cudaError_t sketch_update(const uint32_t *d_codes, const uint32_t *d_invalid, const dd_pack_state *d_state,
                           uint64_t sym_begin, uint64_t sym_end, size_t max_new_symbols, uint32_t kmask, int p,
                           int canon, void *d_ws, cudaStream_t stream) {
-    return sketch_update_impl(d_codes, d_invalid, d_state, sym_begin, sym_end, max_new_symbols, kmask, p, canon, d_ws, 0, stream);
+    return sketch_update_impl(d_codes, d_invalid, d_state, sym_begin, sym_end, max_new_symbols, kmask, p, canon, d_ws, 0, false,
+                              stream);
 }
 
+// sink = the caller allows the rank-1 sink for this range (it ends before the first floor cut); it is used
+// for the k >= 10 of the mask when p fits the shared-memory bitmap and every CTA gets >= 2^p / 4 symbols
 static cudaError_t sketch_update_impl(const uint32_t *d_codes, const uint32_t *d_invalid, const dd_pack_state *d_state,
                                       uint64_t sym_begin, uint64_t sym_end, size_t max_new_symbols, uint32_t kmask, int p,
-                                      int canon, void *d_ws, int midk_hi, cudaStream_t stream) {
+                                      int canon, void *d_ws, int midk_hi, bool sink, cudaStream_t stream) {
     const bool midk = midk_hi >= 12;
     SketchArgs a;
     a.codes = d_codes;
@@ -527,6 +701,19 @@ static cudaError_t sketch_update_impl(const uint32_t *d_codes, const uint32_t *d
     // launch (2^(p+1) bytes per k) stay L2-resident; 0 = all k in one launch.
     const int per_pass = g_k_per_pass > 0 ? g_k_per_pass : 32;
     uint32_t todo = kmask;
+    const uint32_t sink_mask = kmask & ~kSmallKMask;
+    if (sink && sink_mask && p <= kSinkMaxP) {
+        const unsigned nk_sink = (unsigned)__builtin_popcount(sink_mask);
+        const unsigned resident = sink_resident(canon != 0, p);
+        const unsigned slices = resident / nk_sink > 0 ? resident / nk_sink : 1u;
+        if (nsym >= (size_t)slices * (((size_t)1 << p) / 4)) {
+            a.kmask_run = sink_mask;
+            const size_t smem = ((((size_t)1 << p) / 8) + 15) / 16 * 16;
+            const auto fn = canon ? sketch_sink_kernel<true> : sketch_sink_kernel<false>;
+            DD_COUNT_LAUNCH(), fn<<<nk_sink * slices, kSinkThreads, smem, stream>>>(a, ws_sink(d_ws, __builtin_popcount(kmask), p), slices);
+            todo &= kSmallKMask;
+        }
+    }
     while (todo) {
         uint32_t run = 0;
         for (int c = 0; c < per_pass && todo; ++c) {
@@ -591,8 +778,11 @@ cudaError_t sketch_update_sched(const uint32_t *d_codes, const uint32_t *d_inval
                     DD_COUNT_LAUNCH(), midk_ready_kernel<<<1, 1, 0, stream>>>(ws_hdr(d_ws), (uint32_t)k);
                 }
             }
+        // before the first cut the floor is 0 and half of all updates have rank 1: absorb them in the sink;
+        // past it the floor drops them for free and the plain kernels are the right ones
+        const bool sink = g_sink && at_end <= ((uint64_t)16 << p);
         if ((e = sketch_update_impl(d_codes, d_invalid, d_state, origin + pos, origin + upto, max_new_symbols, kmask, p, canon, d_ws,
-                                    midk_hi, stream)) != cudaSuccess)
+                                    midk_hi, sink, stream)) != cudaSuccess)
             return e;
         pos = upto;
         if (refresh) {
@@ -607,7 +797,8 @@ cudaError_t sketch_refresh_floor(void *d_ws, uint32_t kmask, int p, cudaStream_t
     const int nk = __builtin_popcount(kmask);
     cudaError_t e = cudaMemsetAsync(ws_scratch(d_ws), 0xff, 32 * sizeof(uint32_t), stream);
     if (e != cudaSuccess) return e;
-    DD_COUNT_LAUNCH(), floor_min_kernel<<<dim3(16, nk), 256, 0, stream>>>(ws_acc(d_ws), p, ws_hdr(d_ws), ws_scratch(d_ws));
+    DD_COUNT_LAUNCH(), floor_min_kernel<<<dim3(16, nk), 256, 0, stream>>>(ws_acc(d_ws), ws_sink(d_ws, nk, p), p, ws_hdr(d_ws),
+                                                                          ws_scratch(d_ws));
     DD_COUNT_LAUNCH(), floor_publish_kernel<<<1, 32, 0, stream>>>(ws_hdr(d_ws), ws_scratch(d_ws), kmask);
     return cudaGetLastError();
 }
@@ -618,7 +809,7 @@ cudaError_t sketch_end(void *d_ws, int nk, int p, uint8_t *d_regs, uint32_t *d_h
     if (d_hist && (e = cudaMemsetAsync(d_hist, 0, (size_t)nk * DD_HIST_BINS * sizeof(uint32_t), stream)) != cudaSuccess)
         return e;
     const unsigned slices = (unsigned)((((size_t)1 << p) + kFinChunk - 1) / kFinChunk);
-    DD_COUNT_LAUNCH(), finalize_kernel<<<dim3(slices, nk), kPhThreads, 0, stream>>>(ws_acc(d_ws), p, d_regs, d_hist);
+    DD_COUNT_LAUNCH(), finalize_kernel<<<dim3(slices, nk), kPhThreads, 0, stream>>>(ws_acc(d_ws), ws_sink(d_ws, nk, p), p, d_regs, d_hist);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     if (d_hist && d_cards) return mle_from_hist(d_hist, nk, p, d_cards, stream);
     return cudaSuccess;

@@ -63,7 +63,10 @@ DD_API int dd_init(int device);
  * kernel launch (0 = all in one), trading re-reads of the packed stream for L2 residency of the
  * accumulators.  "prefix_planes" = 0/1: dd_prefix_union_card uses the bit-sliced kernel (default 1)
  * or the byte kernel.  "sketch_midk" = 0/1: dd_sketch_update_sched lets pieces deep inside a long stream
- * consult L2-resident presence bitmaps for k = 10..12 before hashing (default 1).  "polyt_sentinel" = 0/1: the dd_*_host entry points apply dd_pack_polyt_sentinel
+ * consult L2-resident presence bitmaps for k = 10..12 before hashing (default 1).  "sketch_sink" = 0/1:
+ * dd_sketch_update_sched sketches the k >= 10 of pieces before the first floor cut (p <= 20) with one k per
+ * CTA, absorbing rank-1 updates in a shared-memory bitmap instead of L2 reductions (default 1; for A/B
+ * measurement).  "polyt_sentinel" = 0/1: the dd_*_host entry points apply dd_pack_polyt_sentinel
  * (this one DOES change results: it selects the SURVEY.md A.6 encoder behaviour; default 0). */
 DD_API int dd_set_option(const char *name, long value);
 DD_API int dd_device_info(int device, int *sm_count, int *cc_major, int *cc_minor, size_t *l2_bytes, size_t *total_mem);

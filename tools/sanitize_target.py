@@ -3,7 +3,7 @@
     compute-sanitizer --tool memcheck  python tools/sanitize_target.py
     compute-sanitizer --tool racecheck python tools/sanitize_target.py
 K1 (general + fast tiles, chunked), K2 (persistent small-k bitmap path, static k sets, generic mask,
-floor schedule), finalize, K3 byte + bit-plane kernels with the identical-prefix table, K4, K5 (bitmap,
+floor schedule, the rank-1 sink kernel with and without a small-k launch beside it), finalize, K3 byte + bit-plane kernels with the identical-prefix table, K4, K5 (bitmap,
 64-bit and 128-bit hash sets), K6, K7 lists with K8 first-rank histograms (shared and global counters), the
 poly-T pass.  Results are compared with the oracle so that a
 "clean" run is also a correct one."""
@@ -33,6 +33,9 @@ def main():
         regs, cards = eng.sketch(seq, ks, p=p)
         for i in (0, len(ks) - 1):
             assert np.array_equal(regs[i].cpu().numpy(), orc.hll_sketch(sym, ks[i], p)), ks[i]
+    regs, _ = eng.sketch(seq, list(range(10, 33)), p=16)     # rank-1 sink: whole stream before the first cut
+    assert np.array_equal(regs[0].cpu().numpy(), orc.hll_sketch(sym, 10, 16))
+    assert np.array_equal(regs[22].cpu().numpy(), orc.hll_sketch(sym, 32, 16))
     regs, _ = eng.sketch(seq, list(range(2, 33)), p=8, ranges=[(0, 5000), (5000, sym.size)], floor_every=4096)   # floor path on
     assert np.array_equal(regs[10].cpu().numpy(), orc.hll_sketch(sym, 12, 8))
     hregs, hcards = eng.sketch_fasta_host(txt, [11, 21], p=p)
