@@ -401,6 +401,39 @@ int dd_pairwise_union_card_planes(const uint32_t *d_planes, int n_genomes, int n
                                        nullptr, 0, stream);
 }
 
+// ---- K10 -----------------------------------------------------------------------------------------
+size_t dd_leave_out_workspace_bytes(int n_genomes, int nk) {
+    if (n_genomes < 1 || nk < 1) return 0;
+    return dd::leave_out_workspace_bytes(n_genomes, nk);
+}
+int dd_leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const int32_t *d_group, int n_groups,
+                      uint64_t reg_begin, uint64_t reg_end, uint32_t *d_hist, void *d_ws, size_t ws_bytes, dd_stream stream) {
+    const char *fn = "dd_leave_out_hist";
+    if (!d_regs || !d_group || !d_hist || !d_ws) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (bad_p(p)) return fail(DD_ERR_ARG, "%s: p=%d outside [5,26]", fn, p);
+    if (nk < 1 || nk > 65535) return fail(DD_ERR_ARG, "%s: nk=%d outside [1,65535]", fn, nk);
+    if (n_genomes < 1 || n_groups < 1 || n_groups > n_genomes || n_groups > 65535)   // group ids are u16 in the kernel
+        return fail(DD_ERR_ARG, "%s: need 1 <= n_groups (%d) <= min(n_genomes (%d), 65535)", fn, n_groups, n_genomes);
+    if ((int64_t)nk * (1 + (int64_t)n_groups) * DD_HIST_BINS > 0x7fffffffll)
+        return fail(DD_ERR_ARG, "%s: too many (k, row) histograms: %d x %d", fn, nk, 1 + n_groups);
+    if (reg_begin > reg_end || reg_end > ((uint64_t)1 << p) || (reg_begin & 15) || (reg_end & 15))
+        return fail(DD_ERR_ARG, "%s: register range [%llu,%llu) is not 16-aligned within [0,%llu]", fn,
+                    (unsigned long long)reg_begin, (unsigned long long)reg_end, (unsigned long long)1 << p);
+    if (reinterpret_cast<uintptr_t>(d_regs) & 15) return fail(DD_ERR_ARG, "%s: registers must be 16-byte aligned", fn);
+    if ((reinterpret_cast<uintptr_t>(d_ws) & 7) || (reinterpret_cast<uintptr_t>(d_hist) & 3))
+        return fail(DD_ERR_ARG, "%s: misaligned workspace or histogram", fn);
+    if (ws_bytes < dd::leave_out_workspace_bytes(n_genomes, nk))
+        return fail(DD_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, ws_bytes, dd::leave_out_workspace_bytes(n_genomes, nk));
+    std::vector<int32_t> group(n_genomes);   // ids index rows and shared counters: checked here, before any launch
+    DD_CUDA(cudaMemcpyAsync(group.data(), d_group, group.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, S(stream)), fn);
+    DD_CUDA(cudaStreamSynchronize(S(stream)), fn);
+    for (int g = 0; g < n_genomes; ++g)
+        if (group[g] < 0 || group[g] >= n_groups)
+            return fail(DD_ERR_ARG, "%s: genome %d has group %d outside [0,%d)", fn, g, group[g], n_groups);
+    DD_CUDA(dd::leave_out_hist(d_regs, n_genomes, nk, p, group.data(), n_groups, reg_begin, reg_end, d_hist, d_ws, S(stream)), fn);
+    return DD_OK;
+}
+
 // ---- K5 ------------------------------------------------------------------------------------------
 static int exact_check(int k, uint64_t capacity, const void *ws, size_t ws_bytes, const char *fn) {
     if (!ws) return fail(DD_ERR_ARG, "%s: null workspace", fn);

@@ -73,6 +73,12 @@ extern int g_prefix_planes;  // tuning knob: 1 = use the bit-plane kernel where 
 cudaError_t union_sets_hist(const uint8_t *const *d_members, int n_sets, int n_steps, int p, int final_only,
                             uint32_t *d_hist, uint8_t *d_unions, cudaStream_t stream);
 
+// ---- K10 (leaveout.cu): union and leave-one-group-out histograms, regs [n][nk][2^p] -> hist [nk][1 + G][64] (added to).
+// Workspace = [nk][64] u32 union part | [n] int2 members sorted by group.  h_group: host copy, ids in [0, G).
+size_t leave_out_workspace_bytes(int n_genomes, int nk);
+cudaError_t leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const int32_t *h_group, int n_groups,
+                           uint64_t reg_begin, uint64_t reg_end, uint32_t *d_hist, void *d_ws, cudaStream_t stream);
+
 // ---- K5 (exact.cu).  Workspace = [ExactWsHeader | bitmap or key table]
 struct ExactWsHeader {
     unsigned long long count;     // distinct keys inserted (hash-set mode; bitmap mode counts on demand)

@@ -396,6 +396,28 @@ class Engine:
         self._keep = pr
         return cards
 
+    # ---- K10 --------------------------------------------------------------------------------
+    def leave_out_hist(self, regs: torch.Tensor, group, n_groups: int, p: int, reg_range: Optional[tuple] = None,
+                       out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Register histograms int32 [nk, 1 + n_groups, 64] on the device: row 0 of the union of all genomes of regs
+        [n, nk, 2^p], row 1 + g of the union of every genome whose group[g'] != g (group: n ids in [0, n_groups)).
+        One read of the registers (K10).  reg_range=(begin, end): only those registers of every k (multiples of 16);
+        histograms of disjoint ranges add up.  out: an int32 [nk, 1 + n_groups, 64] tensor to ADD into."""
+        n, nk, m = regs.shape
+        assert m == 1 << p and regs.is_contiguous() and regs.dtype == torch.uint8
+        begin, end = reg_range if reg_range is not None else (0, m)
+        group = np.asarray(group, dtype=np.int32).reshape(-1)
+        if group.size != n:
+            raise DandDError("leave_out_hist: %d group ids for %d genomes" % (group.size, n))
+        d_group = torch.from_numpy(group).to(self.device)
+        if out is None:
+            out = torch.zeros((nk, 1 + int(n_groups), DD_HIST_BINS), dtype=torch.int32, device=self.device)
+        assert out.is_contiguous() and out.dtype == torch.int32 and out.numel() == nk * (1 + int(n_groups)) * DD_HIST_BINS
+        ws = self._buf(self.lib.dd_leave_out_workspace_bytes(n, nk), "leave_out")
+        check(self.lib.dd_leave_out_hist(regs.data_ptr(), n, nk, p, d_group.data_ptr(), int(n_groups), int(begin), int(end),
+                                         out.data_ptr(), ws.data_ptr(), ws.numel(), self.stream), "dd_leave_out_hist")
+        return out
+
     # ---- K5 ---------------------------------------------------------------------------------
     def exact_counts(self, seqs: Sequence[PackedSeq], k: int, canon: bool = True, capacity: Optional[int] = None,
                      shard: Optional[tuple] = None) -> List[int]:

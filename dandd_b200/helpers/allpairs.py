@@ -170,6 +170,27 @@ def mash_distances(j: np.ndarray, k) -> np.ndarray:
     return -np.asarray(list(map(math.log, (2.0 * j / (1.0 + j)).tolist()))).reshape(j.shape) / k
 
 
+def gather_leaf_registers(store, inputs: Sequence[str], ks: Sequence[int], p: int, canon: bool, owners, tag: str = "allpairs"):
+    """(regs, single): the registers uint8 [n, nk, 2^p] of every input on this rank's device, on every rank, and their
+    cardinalities float64 [n, nk] on the host.  Rank r sketches the inputs owners[r] lists (each once, all k) into its
+    slice of the job's array; one all-gather then gives every rank the whole array."""
+    import torch
+    from dandd_b200 import dist as dd_dist
+    from dandd_b200 import timing
+    rank, _ = dd_dist.world()
+    dev = getattr(getattr(store, "engine", None), "device", "cpu")
+    local = torch.empty((len(owners[rank]), len(ks), 1 << p), dtype=torch.uint8, device=dev)
+    local_cards = np.zeros((len(owners[rank]), len(ks)))
+    with timing.span(tag + "_sketch"):
+        for j, g in enumerate(owners[rank]):      # the registers land in their slice of the job's array
+            local_cards[j] = store.leaf_block(inputs[g], ks, p, canon, out=local[j])[1]
+    local_cards = torch.as_tensor(local_cards, dtype=torch.float64, device=dev)
+    with timing.span(tag + "_gather"):
+        regs = dd_dist.gather_registers(local, owners)                     # [n, nk, 2^p] on every rank
+        single = dd_dist.gather_cards(local_cards, owners).cpu().numpy()
+    return regs, single
+
+
 def card_table(tool: str, inputs: Sequence[str], names: Sequence[str], klist: Sequence[int], nest: int = 262144,
                extra: str = "", store=None, tile_pairs: int = 1 << 16) -> CardTable:
     """Every cardinality the reference's command list asks for, as one device job per rank.
@@ -207,16 +228,7 @@ def card_table(tool: str, inputs: Sequence[str], names: Sequence[str], klist: Se
     if tool == "dashing":
         p = int(math.log2(nest))
         uniq = sorted(set(ks))
-        dev = getattr(getattr(store, "engine", None), "device", "cpu")
-        local = torch.empty((len(owners[rank]), len(uniq), 1 << p), dtype=torch.uint8, device=dev)
-        local_cards = np.zeros((len(owners[rank]), len(uniq)))
-        with timing.span("allpairs_sketch"):
-            for j, g in enumerate(owners[rank]):      # the registers land in their slice of the job's array
-                local_cards[j] = store.leaf_block(inputs[g], uniq, p, canon, out=local[j])[1]
-        local_cards = torch.as_tensor(local_cards, dtype=torch.float64, device=dev)
-        with timing.span("allpairs_gather"):
-            regs = dd_dist.gather_registers(local, owners)                     # [n, nk, 2^p] on every rank
-            single = dd_dist.gather_cards(local_cards, owners).cpu().numpy()
+        regs, single = gather_leaf_registers(store, inputs, uniq, p, canon, owners)
         with timing.span("allpairs_pairs"):
             part = store.pair_cards(regs, mine, p, tile_pairs)
         col = [uniq.index(k) for k in ks]

@@ -629,6 +629,55 @@ class GpuSketchStore:
             out[:, c] = [np.asarray(a, dtype=np.int64) for a in self.engine.exact_spectrum(seqs, k, bool(canon), shard=shard)]
         return out[0], out[1], out[2]
 
+    def leave_out_cards(self, regs: torch.Tensor, group, n_groups: int, p: int,
+                        shard: Optional[Tuple[int, int]] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """HLL cardinalities of the union of all genomes of regs [n, nk, 2^p] and of the union without each group
+        (group: n ids in [0, n_groups)): float64 [nk] and [nk, n_groups].  One K10 read of the registers, then the MLE
+        of the nk (1 + n_groups) histograms; the histograms are the ones the per-union K3 path builds for the same
+        members, so the estimates are the same floats.  shard=(rank, world): this rank takes an equal slice of every
+        k's register range and one all_reduce(SUM) adds the histograms of all ranks (every rank holds all of regs)."""
+        from dandd_b200 import dist as dd_dist
+        nk, m = int(regs.shape[1]), 1 << p
+        vec = m // 16
+        rank, world = shard if shard is not None else (0, 1)
+        span = (vec * rank // world * 16, vec * (rank + 1) // world * 16)
+        hist = self.engine.leave_out_hist(regs, group, n_groups, p, reg_range=span)
+        self.stats["union_launches"] += 1
+        if world > 1:
+            hist = dd_dist.sum_counts(hist)
+        cards = self.engine.mle(hist, p).cpu().numpy().reshape(nk, 1 + int(n_groups))
+        return cards[:, 0].copy(), cards[:, 1:].copy()
+
+    def exact_leave_out(self, fastas: Sequence[str], ks: Sequence[int], canon: bool, group, n_groups: int,
+                        shard: Optional[Tuple[int, int]] = None) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """Exact counts of the union of the FASTAs and of the union without each group (group: one id in [0, n_groups)
+        per FASTA), and of every FASTA alone: int64 [nk], [nk, n_groups] and [nk, n].  One engine job per k: with one
+        FASTA per group the sharing-spectrum job (K9; without g = union - keys only g holds), else one first-rank job
+        (K8) whose row g ranks group g's members 1 and every other FASTA 0 (without g = bin 0, its novel keys bin 1).
+        shard=(rank, world): this rank's key range only; the ranks' results add up."""
+        n, ks, n_groups = len(fastas), [int(k) for k in ks], int(n_groups)
+        group = np.asarray(group, dtype=np.int64)
+        seqs = [self.packed(f) for f in fastas]
+        union = np.zeros(len(ks), dtype=np.int64)
+        without = np.zeros((len(ks), n_groups), dtype=np.int64)
+        singles = np.zeros((len(ks), n), dtype=np.int64)
+        singleton = n_groups == n and len(set(group.tolist())) == n
+        ranks = (group[None, :] == np.arange(n_groups)[:, None]).astype(np.uint16)
+        for c, k in enumerate(ks):
+            self.stats["exact_calls"] += 1
+            if singleton:
+                hist, singles[c], priv = (np.asarray(a, dtype=np.int64) for a in
+                                          self.engine.exact_spectrum(seqs, k, bool(canon), shard=shard))
+                union[c] = hist.sum()
+                without[c, group] = union[c] - priv
+            else:
+                s, hist = self.engine.exact_family_counts(seqs, k, bool(canon), ranks, shard=shard)
+                singles[c] = np.asarray(s, dtype=np.int64)
+                hist = np.asarray(hist, dtype=np.int64)
+                without[c] = hist[:, 0]
+                union[c] = hist[0, 0] + hist[0, 1]
+        return union, without, singles
+
     def _exact_from_table(self, fastas, k, canon):
         tab = getattr(self, "exact_pair_table", None)
         if tab is None or tab["canon"] != bool(canon) or int(k) not in tab["col"] or not 1 <= len(fastas) <= 2:

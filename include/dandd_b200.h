@@ -238,6 +238,26 @@ DD_API int dd_pairwise_union_card_planes(const uint32_t *d_planes, int n_genomes
                                   int64_t n_pairs, double *d_cards, uint32_t *d_hist, dd_stream stream);
 
 /* ===========================================================================================
+ * K10  leave-one-group-out unions (what lib/huffman_dandd.py:559-566 find_delta_delta asks per subset:
+ * a fresh SubSpider over the remaining genomes, climbed union by union).  One read of the registers gives
+ * the histograms of the union of all genomes and of the union of every genome outside each group.
+ *   d_regs  [n_genomes][nk][2^p] u8 (the layout of dd_pairwise_union_card), 16-byte aligned
+ *   d_group [n_genomes] int32, group of each genome in [0, n_groups), any order;
+ *           1 <= n_groups <= min(n_genomes, 65535).
+ *           It is read back to the host and checked before any launch (the call synchronises the stream).
+ *   [reg_begin, reg_end) register range of every k, multiples of 16, reg_end <= 2^p
+ *   d_hist  [nk][1 + n_groups][64] u32, ADDED to (the caller zeroes it): row 0 is the union of all genomes,
+ *           row 1 + g the union of every genome not in group g.  Calls over disjoint register ranges, on one
+ *           device or on several, add up to the histograms of the whole range.
+ *   d_ws    dd_leave_out_workspace_bytes(n_genomes, nk) bytes of scratch
+ * nk * (1 + n_groups) * 64 < 2^31.  Cardinalities: dd_mle_from_hist over the nk * (1 + n_groups) rows.
+ * =========================================================================================== */
+DD_API size_t dd_leave_out_workspace_bytes(int n_genomes, int nk);
+DD_API int dd_leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const int32_t *d_group, int n_groups,
+                             uint64_t reg_begin, uint64_t reg_end, uint32_t *d_hist, void *d_ws, size_t ws_bytes,
+                             dd_stream stream);
+
+/* ===========================================================================================
  * K5  --exact: number of distinct (canonical) k-mers, KMC semantics (SURVEY.md Appendix B).
  * Replaces `kmc -ci1 -cs2 -kK [-b] -fm ...` + `kmc_tools info` (lib/sketch_classes.py:389-399,
  * 434-449) and, by inserting several streams into one set, `kmc_tools complex` unions (:451-465).
