@@ -75,6 +75,10 @@ SIGNATURES = {
     "dd_exact_occupancy_hist": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _vp, _vp, _vp]),
     "dd_leave_out_workspace_bytes": (_sz, [_i, _i]),
     "dd_leave_out_hist": (_i, [_vp, _i, _i, _i, _vp, _i, _u64, _u64, _vp, _vp, _sz, _vp]),
+    "dd_greedy_workspace_bytes": (_sz, [_i]),
+    "dd_greedy_dense_hist": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _sz, _vp]),
+    "dd_greedy_compact": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i64, _vp, _sz, _vp]),
+    "dd_greedy_sparse_hist": (_i, [_vp, _i64, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _sz, _vp]),
     "dd_sketch_fasta_host_workspace_bytes": (_sz, [_sz, _i, _i]),
     "dd_sketch_fasta_host": (_i, [_vp, _sz, _u32, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "dd_sketch_fasta_host_async": (_i, [_vp, _sz, _u32, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -434,6 +434,82 @@ int dd_leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const
     return DD_OK;
 }
 
+// ---- K11 -----------------------------------------------------------------------------------------
+size_t dd_greedy_workspace_bytes(int n_cand) {
+    if (n_cand < 1) return 0;
+    return dd::greedy_workspace_bytes(n_cand);
+}
+// The checks every K11 entry shares; the candidates are host values, so no check waits for the device.
+static int greedy_check(const char *fn, const void *d_union, int n_genomes, int nk, int p, const int32_t *h_cand,
+                        int n_cand, const void *d_ws, size_t ws_bytes) {
+    if (!d_union || !h_cand || !d_ws) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (bad_p(p)) return fail(DD_ERR_ARG, "%s: p=%d outside [5,26]", fn, p);
+    if (nk < 1 || nk > 65535) return fail(DD_ERR_ARG, "%s: nk=%d outside [1,65535]", fn, nk);
+    if (n_genomes < 1 || n_cand < 1) return fail(DD_ERR_ARG, "%s: need n_genomes (%d) >= 1 and n_cand (%d) >= 1", fn, n_genomes, n_cand);
+    if ((int64_t)n_cand * nk * DD_HIST_BINS > 0x7fffffffll)
+        return fail(DD_ERR_ARG, "%s: too many (candidate, k) histograms: %d x %d", fn, n_cand, nk);
+    if (reinterpret_cast<uintptr_t>(d_union) & 15) return fail(DD_ERR_ARG, "%s: the union must be 16-byte aligned", fn);
+    if (reinterpret_cast<uintptr_t>(d_ws) & 15) return fail(DD_ERR_ARG, "%s: misaligned workspace", fn);
+    if (ws_bytes < dd::greedy_workspace_bytes(n_cand))
+        return fail(DD_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, ws_bytes, dd::greedy_workspace_bytes(n_cand));
+    std::vector<char> seen(n_genomes, 0);   // a candidate listed twice would compact one segment from two CTAs
+    for (int c = 0; c < n_cand; ++c) {
+        if (h_cand[c] < 0 || h_cand[c] >= n_genomes)
+            return fail(DD_ERR_ARG, "%s: candidate %d is genome %d, outside [0,%d)", fn, c, h_cand[c], n_genomes);
+        if (seen[h_cand[c]]++) return fail(DD_ERR_ARG, "%s: genome %d is listed twice", fn, h_cand[c]);
+    }
+    return DD_OK;
+}
+int dd_greedy_dense_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const uint8_t *d_union,
+                         const uint32_t *d_union_hist, const int32_t *h_cand, int n_cand, uint32_t *d_hist,
+                         uint32_t *d_live, void *d_ws, size_t ws_bytes, dd_stream stream) {
+    const char *fn = "dd_greedy_dense_hist";
+    if (!d_regs || !d_union_hist || !d_hist || !d_live) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (int r = greedy_check(fn, d_union, n_genomes, nk, p, h_cand, n_cand, d_ws, ws_bytes)) return r;
+    if (reinterpret_cast<uintptr_t>(d_regs) & 15) return fail(DD_ERR_ARG, "%s: registers must be 16-byte aligned", fn);
+    if ((reinterpret_cast<uintptr_t>(d_union_hist) | reinterpret_cast<uintptr_t>(d_hist) | reinterpret_cast<uintptr_t>(d_live)) & 3)
+        return fail(DD_ERR_ARG, "%s: misaligned histogram or live counts", fn);
+    DD_CUDA(dd::greedy_dense_hist(d_regs, nk, p, d_union, d_union_hist, h_cand, n_cand, d_hist, d_live, d_ws, S(stream)), fn);
+    return DD_OK;
+}
+int dd_greedy_compact(const uint8_t *d_regs, int n_genomes, int nk, int p, const uint8_t *d_union, const int32_t *h_cand,
+                      int n_cand, const int64_t *h_seg_off, int64_t *d_seg_off, uint32_t *d_seg_len, uint32_t *d_entries,
+                      int64_t n_entries, void *d_ws, size_t ws_bytes, dd_stream stream) {
+    const char *fn = "dd_greedy_compact";
+    if (!d_regs || !h_seg_off || !d_seg_off || !d_seg_len || (!d_entries && n_entries > 0))
+        return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (int r = greedy_check(fn, d_union, n_genomes, nk, p, h_cand, n_cand, d_ws, ws_bytes)) return r;
+    if (reinterpret_cast<uintptr_t>(d_regs) & 15) return fail(DD_ERR_ARG, "%s: registers must be 16-byte aligned", fn);
+    if ((reinterpret_cast<uintptr_t>(d_seg_off) & 7) || ((reinterpret_cast<uintptr_t>(d_seg_len) | reinterpret_cast<uintptr_t>(d_entries)) & 3))
+        return fail(DD_ERR_ARG, "%s: misaligned segment table or entries", fn);
+    const size_t n_seg = (size_t)n_genomes * nk;
+    if (h_seg_off[0] != 0) return fail(DD_ERR_ARG, "%s: segment offsets must start at 0", fn);
+    for (size_t s = 0; s < n_seg; ++s)
+        if (h_seg_off[s + 1] < h_seg_off[s]) return fail(DD_ERR_ARG, "%s: segment offsets decrease at %zu", fn, s);
+    if (h_seg_off[n_seg] > n_entries)
+        return fail(DD_ERR_ARG, "%s: segments need %lld entries, the buffer holds %lld", fn, (long long)h_seg_off[n_seg],
+                    (long long)n_entries);
+    DD_CUDA(dd::greedy_compact(d_regs, n_genomes, nk, p, d_union, h_cand, n_cand, h_seg_off, d_seg_off, d_seg_len, d_entries,
+                               d_ws, S(stream)), fn);
+    return DD_OK;
+}
+int dd_greedy_sparse_hist(uint32_t *d_entries, int64_t n_entries, const int64_t *d_seg_off, uint32_t *d_seg_len,
+                          int n_genomes, int nk, int p, const uint8_t *d_union, const uint32_t *d_union_hist,
+                          const int32_t *h_cand, int n_cand, uint32_t *d_hist, uint32_t *d_live, void *d_ws,
+                          size_t ws_bytes, dd_stream stream) {
+    const char *fn = "dd_greedy_sparse_hist";
+    if ((!d_entries && n_entries > 0) || n_entries < 0 || !d_seg_off || !d_seg_len || !d_union_hist || !d_hist || !d_live)
+        return fail(DD_ERR_ARG, "%s: null pointer or negative entry count", fn);
+    if (int r = greedy_check(fn, d_union, n_genomes, nk, p, h_cand, n_cand, d_ws, ws_bytes)) return r;
+    if ((reinterpret_cast<uintptr_t>(d_seg_off) & 7) ||
+        ((reinterpret_cast<uintptr_t>(d_seg_len) | reinterpret_cast<uintptr_t>(d_entries) | reinterpret_cast<uintptr_t>(d_union_hist) |
+          reinterpret_cast<uintptr_t>(d_hist) | reinterpret_cast<uintptr_t>(d_live)) & 3))
+        return fail(DD_ERR_ARG, "%s: misaligned segment table, entries, histogram or live counts", fn);
+    DD_CUDA(dd::greedy_sparse_hist(d_entries, n_entries, d_seg_off, d_seg_len, nk, p, d_union, d_union_hist, h_cand, n_cand,
+                                   d_hist, d_live, d_ws, S(stream)), fn);
+    return DD_OK;
+}
+
 // ---- K5 ------------------------------------------------------------------------------------------
 static int exact_check(int k, uint64_t capacity, const void *ws, size_t ws_bytes, const char *fn) {
     if (!ws) return fail(DD_ERR_ARG, "%s: null workspace", fn);

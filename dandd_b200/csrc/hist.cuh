@@ -28,16 +28,21 @@ __device__ __forceinline__ void ph_add_word(uint8_t *s_hist, uint32_t slot, uint
 #pragma unroll
     for (int b = 0; b < 4; ++b) s_hist[ph_bin((w >> (8 * b)) & 0xffu) * kPhThreads + slot]++;
 }
+// Bin b summed over the 256 threads, in every lane of the calling warp: a lane adds the 8 byte counters of one
+// 64-bit word with SWAR adds.
+__device__ __forceinline__ uint32_t ph_total(const uint8_t *s_hist, int b) {
+    const uint2 x = reinterpret_cast<const uint2 *>(s_hist + b * kPhThreads)[threadIdx.x & 31];
+    uint32_t s = (x.x & 0x00ff00ffu) + ((x.x >> 8) & 0x00ff00ffu) + (x.y & 0x00ff00ffu) + ((x.y >> 8) & 0x00ff00ffu);
+    s = (s & 0xffffu) + (s >> 16);
+    return __reduce_add_sync(0xffffffffu, s);
+}
 // Sum every bin over the 256 threads and add the totals to a global histogram row.  Each warp
-// takes 8 bins; a lane adds the 8 byte counters of one 64-bit word with SWAR adds.
+// takes 8 bins.
 __device__ __forceinline__ void ph_flush(const uint8_t *s_hist, uint32_t *g_hist) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll 2
     for (int b = warp; b < DD_HIST_BINS; b += kPhThreads / 32) {
-        const uint2 x = reinterpret_cast<const uint2 *>(s_hist + b * kPhThreads)[lane];
-        uint32_t s = (x.x & 0x00ff00ffu) + ((x.x >> 8) & 0x00ff00ffu) + (x.y & 0x00ff00ffu) + ((x.y >> 8) & 0x00ff00ffu);
-        s = (s & 0xffffu) + (s >> 16);
-        s = __reduce_add_sync(0xffffffffu, s);
+        const uint32_t s = ph_total(s_hist, b);
         if (lane == 0 && s) atomicAdd(&g_hist[b], s);
     }
 }

@@ -79,6 +79,20 @@ size_t leave_out_workspace_bytes(int n_genomes, int nk);
 cudaError_t leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const int32_t *h_group, int n_groups,
                            uint64_t reg_begin, uint64_t reg_end, uint32_t *d_hist, void *d_ws, cudaStream_t stream);
 
+// ---- K11 (greedy.cu): hist(max(U, g)) for every listed candidate g, regs [n][nk][2^p], U [nk][2^p] ->
+// hist [C][nk][64] and live [C][nk] (written).  Workspace = the candidate list.  h_cand / h_seg_off: host copies,
+// checked by the caller.
+size_t greedy_workspace_bytes(int n_cand);
+cudaError_t greedy_dense_hist(const uint8_t *d_regs, int nk, int p, const uint8_t *d_union, const uint32_t *d_uhist,
+                              const int32_t *h_cand, int n_cand, uint32_t *d_hist, uint32_t *d_live, void *d_ws,
+                              cudaStream_t stream);
+cudaError_t greedy_compact(const uint8_t *d_regs, int n_genomes, int nk, int p, const uint8_t *d_union,
+                           const int32_t *h_cand, int n_cand, const int64_t *h_seg_off, int64_t *d_seg_off,
+                           uint32_t *d_seg_len, uint32_t *d_entries, void *d_ws, cudaStream_t stream);
+cudaError_t greedy_sparse_hist(uint32_t *d_entries, int64_t n_entries, const int64_t *d_seg_off, uint32_t *d_seg_len,
+                               int nk, int p, const uint8_t *d_union, const uint32_t *d_uhist, const int32_t *h_cand,
+                               int n_cand, uint32_t *d_hist, uint32_t *d_live, void *d_ws, cudaStream_t stream);
+
 // ---- K5 (exact.cu).  Workspace = [ExactWsHeader | bitmap or key table]
 struct ExactWsHeader {
     unsigned long long count;     // distinct keys inserted (hash-set mode; bitmap mode counts on demand)

@@ -6,7 +6,7 @@ and stream semantics work as usual.  One Engine per process / per GPU."""
 import ctypes as C
 import os
 from dataclasses import dataclass
-from typing import Iterable, List, Optional, Sequence
+from typing import Iterable, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -417,6 +417,67 @@ class Engine:
         check(self.lib.dd_leave_out_hist(regs.data_ptr(), n, nk, p, d_group.data_ptr(), int(n_groups), int(begin), int(end),
                                          out.data_ptr(), ws.data_ptr(), ws.numel(), self.stream), "dd_leave_out_hist")
         return out
+
+    # ---- K11 --------------------------------------------------------------------------------
+    def cards_hist(self, regs: torch.Tensor, p: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(cards float64 [...], histograms int32 [..., 64]) of the sketches regs [..., 2^p] on the device (K4)."""
+        flat = regs.contiguous().view(-1, 1 << p)
+        hist = torch.empty((flat.shape[0], DD_HIST_BINS), dtype=torch.int32, device=self.device)
+        out = torch.empty(flat.shape[0], dtype=torch.float64, device=self.device)
+        check(self.lib.dd_card_ertl_mle(flat.data_ptr(), flat.shape[0], p, out.data_ptr(), hist.data_ptr(), self.stream),
+              "dd_card_ertl_mle")
+        return out.view(regs.shape[:-1]), hist.view(tuple(regs.shape[:-1]) + (DD_HIST_BINS,))
+
+    def greedy_dense_hist(self, regs: torch.Tensor, union: torch.Tensor, union_hist: torch.Tensor, cand, p: int):
+        """(hist int32 [C, nk, 64], live int32 [C, nk]) on the device: the histogram of max(union, regs[g]) and the
+        number of registers where regs[g] > union, for the C distinct genome indices `cand` (host), every k.  regs
+        [n, nk, 2^p], union [nk, 2^p], union_hist [nk, 64] (cards_hist of union).  Reads every register (K11 dense)."""
+        n, nk, m = regs.shape
+        assert m == 1 << p and regs.is_contiguous() and union.is_contiguous() and union_hist.is_contiguous()
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        hist = torch.empty((cand.size, nk, DD_HIST_BINS), dtype=torch.int32, device=self.device)
+        live = torch.empty((cand.size, nk), dtype=torch.int32, device=self.device)
+        ws = self._buf(self.lib.dd_greedy_workspace_bytes(cand.size), "greedy")
+        check(self.lib.dd_greedy_dense_hist(regs.data_ptr(), n, nk, p, union.data_ptr(), union_hist.data_ptr(),
+                                            cand.ctypes.data, cand.size, hist.data_ptr(), live.data_ptr(), ws.data_ptr(),
+                                            ws.numel(), self.stream), "dd_greedy_dense_hist")
+        return hist, live
+
+    def greedy_compact(self, regs: torch.Tensor, union: torch.Tensor, cand, seg_off, p: int) -> dict:
+        """The live registers (regs[g] > union) of the candidates `cand` as u32 entries `j << 6 | value` in segments
+        g * nk + k whose capacities are the host offsets seg_off [n * nk + 1] (K11 compaction).  Returns the sparse
+        state {"entries", "seg_off", "seg_len"} that greedy_sparse_hist reads and updates."""
+        n, nk, m = regs.shape
+        assert m == 1 << p and regs.is_contiguous() and union.is_contiguous()
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        seg_off = np.ascontiguousarray(seg_off, dtype=np.int64)
+        assert seg_off.size == n * nk + 1
+        total = int(seg_off[-1])
+        state = {"entries": torch.empty(max(total, 1), dtype=torch.int32, device=self.device), "n_entries": total,
+                 "seg_off": torch.empty(n * nk + 1, dtype=torch.int64, device=self.device),
+                 "seg_len": torch.empty(n * nk, dtype=torch.int32, device=self.device), "n": n}
+        ws = self._buf(self.lib.dd_greedy_workspace_bytes(cand.size), "greedy")
+        check(self.lib.dd_greedy_compact(regs.data_ptr(), n, nk, p, union.data_ptr(), cand.ctypes.data, cand.size,
+                                         seg_off.ctypes.data, state["seg_off"].data_ptr(), state["seg_len"].data_ptr(),
+                                         state["entries"].data_ptr(), total, ws.data_ptr(), ws.numel(), self.stream),
+              "dd_greedy_compact")
+        return state
+
+    def greedy_sparse_hist(self, state: dict, union: torch.Tensor, union_hist: torch.Tensor, cand, p: int):
+        """greedy_dense_hist from the sparse state of greedy_compact (K11 sparse): the entries no longer above union
+        are dropped for good, so every call must follow the previous one's union update."""
+        nk = union.shape[0]
+        assert union.shape[1] == 1 << p and union.is_contiguous() and union_hist.is_contiguous()
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        hist = torch.empty((cand.size, nk, DD_HIST_BINS), dtype=torch.int32, device=self.device)
+        live = torch.empty((cand.size, nk), dtype=torch.int32, device=self.device)
+        ws = self._buf(self.lib.dd_greedy_workspace_bytes(cand.size), "greedy")
+        check(self.lib.dd_greedy_sparse_hist(state["entries"].data_ptr(), state["n_entries"], state["seg_off"].data_ptr(),
+                                             state["seg_len"].data_ptr(), state["n"], nk, p, union.data_ptr(),
+                                             union_hist.data_ptr(), cand.ctypes.data, cand.size, hist.data_ptr(),
+                                             live.data_ptr(), ws.data_ptr(), ws.numel(), self.stream),
+              "dd_greedy_sparse_hist")
+        return hist, live
 
     # ---- K5 ---------------------------------------------------------------------------------
     def exact_counts(self, seqs: Sequence[PackedSeq], k: int, canon: bool = True, capacity: Optional[int] = None,

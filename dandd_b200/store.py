@@ -29,6 +29,10 @@ from .engine import Engine, get_engine
 
 ALL_HLL_KS = tuple(range(1, 33))
 EXACT_MAX_K = 256   # KMC's own k limit, and the exact kernels'
+# The greedy ordering compacts its live registers once 4 bytes per live register, times this, is at most what a
+# dense step reads (1 byte per register of every remaining candidate): sparse entries cost more than their 4 bytes
+# (a random L2 read of U, a write back, a CTA per segment).
+SPARSE_CROSS = 2
 STREAM_MIN_BYTES = int(os.environ.get("DANDD_B200_STREAM_MIN", str(32 << 20)))   # larger FASTAs take the chunked pipeline
 
 
@@ -647,6 +651,81 @@ class GpuSketchStore:
             hist = dd_dist.sum_counts(hist)
         cards = self.engine.mle(hist, p).cpu().numpy().reshape(nk, 1 + int(n_groups))
         return cards[:, 0].copy(), cards[:, 1:].copy()
+
+    def greedy_order(self, regs: torch.Tensor, ks: Sequence[int], p: int, steps: int, order: str = "max", first=(),
+                     shard: Optional[Tuple[int, int]] = None, budget: Optional[int] = None):
+        """Greedy ordering of the genomes of regs [n, nk, 2^p]: step t adds the genome g not chosen yet whose union with
+        the running union U has the largest (order="max") or smallest ("min") delta = max_k card_k / k, the lowest
+        index winning a tie; the genomes of `first` take the first steps as given.  Returns (order int64 [steps],
+        cards float64 [steps, nk] of U after each step, stats).  card_k(U u g) is the MLE of the histogram of max(U, g),
+        the histogram K3 builds for the same members, so the floats are those of a progressive replay of the order.
+
+        Every step runs K11 over the remaining candidates: dense (every register) until the live registers (g > U)
+        fit in 4-byte entries within `budget` (default: half of the free device memory) and take well under the
+        dense step's bytes, then one compaction and sparse steps over the live entries to the end; both give the
+        same histograms.  shard=(rank, world): rank r evaluates the candidates g = r (mod world), one
+        all_reduce(SUM) of the [n, nk] cards per step adds the ranks' rows, and every rank makes the same pick."""
+        if not hasattr(self.engine, "greedy_dense_hist"):
+            raise RuntimeError("the greedy ordering needs an engine with the K11 step (Engine.greedy_dense_hist)")
+        from dandd_b200 import dist as dd_dist
+        n, nk, m = (int(x) for x in regs.shape)
+        first = [int(g) for g in first]
+        assert m == 1 << p and order in ("max", "min") and len(first) <= steps <= n and len(set(first)) == len(first)
+        rank, world = shard if shard is not None else (0, 1)
+        dev = regs.device
+        if budget is None:
+            budget = self.engine._pairs_budget()
+        kdiv = torch.as_tensor(np.asarray(ks, dtype=np.float64), device=dev)
+        fill = float("-inf") if order == "max" else float("inf")
+        union = torch.zeros((nk, m), dtype=torch.uint8, device=dev)
+        _, uhist = self.engine.cards_hist(union, p)
+        cards = torch.empty((steps, nk), dtype=torch.float64, device=dev)
+        chosen = torch.zeros(n, dtype=torch.bool, device=dev)
+        left, picks, sparse = list(range(n)), [], None
+        stats = {"switch_step": None, "live": [], "dense_steps": 0, "sparse_steps": 0}
+        for t in range(steps):
+            mine = [g for g in left if g % world == rank]
+            if t < len(first):
+                pick_d = torch.tensor(first[t], device=dev)
+                live_left = torch.zeros((), dtype=torch.int64, device=dev)
+            else:
+                full = torch.zeros((n, nk), dtype=torch.float64, device=dev)
+                live_left = torch.zeros((), dtype=torch.int64, device=dev)
+                if mine:
+                    if sparse is None:
+                        hist, live = self.engine.greedy_dense_hist(regs, union, uhist, mine, p)
+                        stats["dense_steps"] += 1
+                    else:
+                        hist, live = self.engine.greedy_sparse_hist(sparse, union, uhist, mine, p)
+                        stats["sparse_steps"] += 1
+                    rows = torch.as_tensor(np.asarray(mine, dtype=np.int64), device=dev)
+                    full[rows] = self.engine.mle(hist, p)
+                if world > 1:
+                    full = dd_dist.sum_counts(full)
+                delta = (full / kdiv).amax(dim=1).masked_fill(chosen, fill)
+                pick_d = delta.argmax() if order == "max" else delta.argmin()   # the first extremum: the lowest index
+                if mine:
+                    live_left = live.to(torch.int64).sum() - (live.to(torch.int64) * (rows == pick_d)[:, None]).sum()
+            union = torch.maximum(union, regs.index_select(0, pick_d.view(1))[0])
+            chosen.index_fill_(0, pick_d.view(1), True)
+            ucards, uhist = self.engine.cards_hist(union, p)
+            cards[t] = ucards
+            pick, live_total = (int(x) for x in torch.stack([pick_d.to(torch.int64), live_left]).cpu())   # the one read
+            picks.append(pick)
+            left.remove(pick)
+            stats["live"].append(live_total if t >= len(first) else -1)
+            rest = [g for g in mine if g != pick]
+            if (sparse is None and t >= len(first) and t + 1 < steps and rest and 4 * live_total < budget
+                    and SPARSE_CROSS * 4 * live_total <= len(rest) * nk * m):
+                # the dense step's live counts bound the live registers of the grown union: segment capacities
+                counts = np.zeros((n, nk), dtype=np.int64)
+                counts[mine] = live.cpu().numpy()
+                counts[pick] = 0
+                off = np.concatenate([[0], np.cumsum(counts.reshape(-1))])
+                sparse = self.engine.greedy_compact(regs, union, rest, off, p)
+                stats["switch_step"] = t + 1
+        self.stats["union_launches"] += steps
+        return np.asarray(picks, dtype=np.int64), cards.cpu().numpy(), stats
 
     def exact_leave_out(self, fastas: Sequence[str], ks: Sequence[int], canon: bool, group, n_groups: int,
                         shard: Optional[Tuple[int, int]] = None) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:

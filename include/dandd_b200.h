@@ -258,6 +258,43 @@ DD_API int dd_leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p
                              dd_stream stream);
 
 /* ===========================================================================================
+ * K11  one step of a greedy ordering (a chosen ordering for `progressive -r`, lib/huffman_dandd.py:618-663
+ * orderings_list, where the reference would climb one SubSpider union per candidate per step).  U is the running
+ * union; for every listed candidate g and every k these give the histogram of max(U, g), as hist(U) plus one
+ * -1 / +1 pair per "live" register where g > U, and the number of live registers.
+ *   d_regs      [n_genomes][nk][2^p] u8 (the layout of dd_pairwise_union_card), 16-byte aligned
+ *   d_union     [nk][2^p] u8, 16-byte aligned; register values < 64
+ *   d_union_hist [nk][64] u32, the histogram of d_union (dd_card_ertl_mle's d_hist)
+ *   h_cand      [n_cand] int32 HOST array of distinct genome indices in [0, n_genomes); n_cand >= 1
+ *   d_hist      [n_cand][nk][64] u32, written: row (c, k) is the histogram of max(U, regs[h_cand[c]][k])
+ *   d_live      [n_cand][nk] u32, written: registers where regs[h_cand[c]][k] > U[k]
+ *   d_ws        dd_greedy_workspace_bytes(n_cand) bytes of scratch, 16-byte aligned
+ * n_cand * nk * 64 < 2^31.  Cardinalities: dd_mle_from_hist over the n_cand * nk rows.
+ *
+ * dd_greedy_dense_hist reads every register of every candidate.  dd_greedy_compact writes the live registers of
+ * every candidate as entries `j << 6 | value` (u32) into segment g * nk + k of d_entries:
+ *   h_seg_off   [n_genomes * nk + 1] int64 HOST offsets, starting at 0, non-decreasing, last <= n_entries;
+ *               the capacity of segment s is h_seg_off[s + 1] - h_seg_off[s] (live counts of an earlier U bound it)
+ *   d_seg_off   [n_genomes * nk + 1] int64, written: a device copy of h_seg_off
+ *   d_seg_len   [n_genomes * nk] u32, written: the live count of each listed segment, 0 elsewhere
+ * dd_greedy_sparse_hist then does a step from the segments alone: it drops the entries with value <= U[k][j],
+ * compacts the rest in place, sets d_seg_len to the kept count (also d_live) and counts their pairs.  A segment is
+ * clipped to its capacity and to the entry buffer.  Both sparse and dense give the same d_hist and d_live.
+ * =========================================================================================== */
+DD_API size_t dd_greedy_workspace_bytes(int n_cand);
+DD_API int dd_greedy_dense_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const uint8_t *d_union,
+                                const uint32_t *d_union_hist, const int32_t *h_cand, int n_cand, uint32_t *d_hist,
+                                uint32_t *d_live, void *d_ws, size_t ws_bytes, dd_stream stream);
+DD_API int dd_greedy_compact(const uint8_t *d_regs, int n_genomes, int nk, int p, const uint8_t *d_union,
+                             const int32_t *h_cand, int n_cand, const int64_t *h_seg_off, int64_t *d_seg_off,
+                             uint32_t *d_seg_len, uint32_t *d_entries, int64_t n_entries, void *d_ws, size_t ws_bytes,
+                             dd_stream stream);
+DD_API int dd_greedy_sparse_hist(uint32_t *d_entries, int64_t n_entries, const int64_t *d_seg_off, uint32_t *d_seg_len,
+                                 int n_genomes, int nk, int p, const uint8_t *d_union, const uint32_t *d_union_hist,
+                                 const int32_t *h_cand, int n_cand, uint32_t *d_hist, uint32_t *d_live, void *d_ws,
+                                 size_t ws_bytes, dd_stream stream);
+
+/* ===========================================================================================
  * K5  --exact: number of distinct (canonical) k-mers, KMC semantics (SURVEY.md Appendix B).
  * Replaces `kmc -ci1 -cs2 -kK [-b] -fm ...` + `kmc_tools info` (lib/sketch_classes.py:389-399,
  * 434-449) and, by inserting several streams into one set, `kmc_tools complex` unions (:451-465).
