@@ -532,33 +532,37 @@ class Engine:
         """The co-occurrence-list path of exact_pair_intersections, in `passes` key-range passes (default:
         as few as fit the memory budget, plan_pair_passes)."""
         n = len(seqs)
-        out = np.zeros(n * (n - 1) // 2, dtype=np.uint64)
         if n < 2:
-            return out
+            return np.zeros(n * (n - 1) // 2, dtype=np.uint64)
         if k > 64 and n > 65536:
             raise DandDError("exact pairs above k = 64 take at most 65536 genomes per job")
-        part = torch.zeros(len(out), dtype=torch.int64, device=self.device)
-        for ws, cap, nodes in self._key_lists(seqs, k, canon, singles, shard, passes):
-            part.zero_()
-            check(self.lib.dd_exact_pairs_accumulate(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part.data_ptr(), self.stream),
+
+        def launch(ws, cap, nodes, part):
+            check(self.lib.dd_exact_pairs_accumulate(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part, self.stream),
                   "dd_exact_pairs_accumulate")
-            got = part.cpu().numpy().view(np.uint64)
-            if (got == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
-                raise DandDError("exact pair table or node array overflowed; the single counts given understate the genomes")
-            out += got
+
+        out, _ = self._list_job(seqs, k, canon, singles, shard, passes, n * (n - 1) // 2, False, launch,
+                                "exact pair table or node array overflowed; the single counts given understate the genomes")
         return out
 
-    def _key_lists(self, seqs: Sequence[PackedSeq], k: int, canon: bool, singles: Sequence[int],
-                   shard: Optional[tuple] = None, passes: Optional[int] = None, node_counts: Optional[torch.Tensor] = None):
-        """The K7 sparse workspace, once per key-range pass: yields (workspace, capacity, max_nodes) after every
-        genome has pushed itself onto the list of every key of the pass it holds (genome g = seqs[g]).  The
-        caller reads the lists (K7 pair counts, K8 first-rank histograms) before asking for the next pass.
-        node_counts (int64 [n] on the device): the node counter after genome g's insert is copied to entry g
-        of every pass (dd_exact_pairs_node_count) -- its growth over genome g is |A_g n the pass's key range|."""
+    def _list_job(self, seqs: Sequence[PackedSeq], k: int, canon: bool, sizes: Sequence[int], shard: Optional[tuple],
+                  passes: Optional[int], cells: int, node_counts: bool, launch, overflow: str):
+        """One job over the K7 co-occurrence lists, in key-range passes (plan_pair_passes over `sizes`: the exact
+        singles, or length bounds that never understate them).  Every pass, each genome pushes itself onto the list
+        of every key of the pass it holds (genome g = seqs[g]); then launch(workspace, capacity, max_nodes, out_ptr)
+        adds the pass's result into `cells` zeroed int64 cells on the device, and one copy brings them to the host.
+        An all-ones cell means the table or node array overflowed: DandDError(overflow).  Returns (the cells summed
+        over the passes, uint64; with node_counts, |A_g| per genome, uint64 [n], else None): the list-node counter is
+        read after every genome's insert (dd_exact_pairs_node_count), and its growth over genome g is
+        |A_g n the pass's key range|."""
         n = len(seqs)
         srank, sworld = (int(shard[0]), int(shard[1])) if shard is not None else (0, 1)
         nsyms = [s.nsym for s in seqs]
-        plan = plan_pair_passes(singles, k, lambda c, m: int(self.lib.dd_exact_pairs_workspace_bytes(k, c, m, n)),
+        # [cells | node counter after genome g]
+        part = torch.zeros(cells + (n if node_counts else 0), dtype=torch.int64, device=self.device)
+        out = np.zeros(cells, dtype=np.uint64)
+        singles = np.zeros(n, dtype=np.uint64) if node_counts else None
+        plan = plan_pair_passes(sizes, k, lambda c, m: int(self.lib.dd_exact_pairs_workspace_bytes(k, c, m, n)),
                                 self._pairs_budget(), passes)
         self.last_pair_plan = dict(plan, path="sparse")
         cap, nodes = plan["capacity"], plan["max_nodes"]
@@ -572,13 +576,28 @@ class Engine:
                     check(self.lib.dd_exact_pairs_insert_shard(s.codes.data_ptr(), s.invalid.data_ptr(), 0, ns, k, int(canon), g,
                                                                ws.data_ptr(), ws.numel(), cap, nodes, n, sr, sw, st),
                           "dd_exact_pairs_insert_shard")
-                    if node_counts is not None:
-                        check(self.lib.dd_exact_pairs_node_count(ws.data_ptr(), ws.numel(), node_counts.data_ptr() + 8 * g, st),
-                              "dd_exact_pairs_node_count")
-                yield ws, cap, nodes
+                    if node_counts:
+                        check(self.lib.dd_exact_pairs_node_count(ws.data_ptr(), ws.numel(), part.data_ptr() + 8 * (cells + g),
+                                                                 st), "dd_exact_pairs_node_count")
+                part[:cells].zero_()
+                launch(ws, cap, nodes, part.data_ptr())
+                got = part.cpu().numpy().view(np.uint64)
+                if (got[:cells] == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
+                    raise DandDError(overflow)
+                out += got[:cells]
+                if node_counts:
+                    singles += np.diff(got[cells:], prepend=np.uint64(0))
+            return out, singles
         finally:
             del ws
             self._ws.pop("exact_pairs", None)     # a pass may take half the device: not kept for later stages
+
+    def _first_rank_launch(self, k: int, n: int, ranks: np.ndarray):
+        """The K8 launch of _list_job for the rank table `ranks` [R, n] (uint16 on the host; copied to the device here)."""
+        d_ranks = torch.from_numpy(ranks.view(np.int16)).to(self.device)
+        return lambda ws, cap, nodes, part: check(
+            self.lib.dd_exact_first_rank_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, d_ranks.data_ptr(), ranks.shape[0],
+                                              part, self.stream), "dd_exact_first_rank_hist")
 
     # ---- K8 ---------------------------------------------------------------------------------
     def exact_first_rank_hist(self, seqs: Sequence[PackedSeq], k: int, canon: bool, ranks,
@@ -592,24 +611,15 @@ class Engine:
         n = len(seqs)
         ranks = np.ascontiguousarray(ranks, dtype=np.uint16).reshape(-1, n)
         rows = ranks.shape[0]
-        out = np.zeros((rows, n), dtype=np.uint64)
         if n == 0 or rows == 0:
-            return out
+            return np.zeros((rows, n), dtype=np.uint64)
         if n > 65535:
             raise DandDError("first-rank histograms take at most 65535 genomes per job (ranks are 16-bit)")
         if singles is None:
             singles = [self.exact_counts([s], k, canon, shard=shard)[0] for s in seqs]
-        d_ranks = torch.from_numpy(ranks.view(np.int16)).to(self.device)
-        part = torch.zeros((rows, n), dtype=torch.int64, device=self.device)
-        for ws, cap, nodes in self._key_lists(seqs, k, canon, singles, shard, passes):
-            part.zero_()
-            check(self.lib.dd_exact_first_rank_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, d_ranks.data_ptr(), rows,
-                                                    part.data_ptr(), self.stream), "dd_exact_first_rank_hist")
-            got = part.cpu().numpy().view(np.uint64)
-            if (got == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
-                raise DandDError("exact k-mer table or node array overflowed; the single counts given understate the genomes")
-            out += got
-        return out
+        hist, _ = self._list_job(seqs, k, canon, singles, shard, passes, rows * n, False, self._first_rank_launch(k, n, ranks),
+                                 "exact k-mer table or node array overflowed; the single counts given understate the genomes")
+        return hist.reshape(rows, n)
 
     def exact_family_counts(self, seqs: Sequence[PackedSeq], k: int, canon: bool, ranks, shard: Optional[tuple] = None,
                             passes: Optional[int] = None):
@@ -622,30 +632,18 @@ class Engine:
         n = len(seqs)
         ranks = np.ascontiguousarray(ranks, dtype=np.uint16).reshape(-1, n) if n else np.zeros((len(ranks), 0), np.uint16)
         rows = ranks.shape[0]
-        singles = np.zeros(n, dtype=np.uint64)
-        hist = np.zeros((rows, n), dtype=np.uint64)
         if n == 0:
-            return singles, hist
+            return np.zeros(n, dtype=np.uint64), np.zeros((rows, n), dtype=np.uint64)
         if n > 65535:
             raise DandDError("family counts take at most 65535 genomes per job (ranks are 16-bit)")
         world = int(shard[1]) if shard is not None else 1
         bounds = length_bounds([s.nsym for s in seqs], k, world)
         # with no row, one row that holds no genome: K8 still reports a full table or node array
         table = ranks if rows else np.full((1, n), 0xFFFF, dtype=np.uint16)
-        d_ranks = torch.from_numpy(table.view(np.int16)).to(self.device)
-        cells = table.shape[0] * n
-        part = torch.zeros(cells + n, dtype=torch.int64, device=self.device)    # [hist cells | node counter after genome g]
-        for ws, cap, nodes in self._key_lists(seqs, k, canon, bounds, shard, passes, node_counts=part[cells:]):
-            part[:cells].zero_()
-            check(self.lib.dd_exact_first_rank_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, d_ranks.data_ptr(),
-                                                    table.shape[0], part.data_ptr(), self.stream), "dd_exact_first_rank_hist")
-            got = part.cpu().numpy().view(np.uint64)
-            if (got[:cells] == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
-                raise DandDError("exact k-mer table or node array overflowed; the length bounds understate the genomes")
-            if rows:
-                hist += got[:cells].reshape(rows, n)
-            singles += np.diff(got[cells:], prepend=np.uint64(0))
-        return singles, hist
+        launch = self._first_rank_launch(k, n, table)
+        hist, singles = self._list_job(seqs, k, canon, bounds, shard, passes, table.size, True, launch,
+                                       "exact k-mer table or node array overflowed; the length bounds understate the genomes")
+        return singles, hist.reshape(-1, n)[:rows]
 
     # ---- K9 ---------------------------------------------------------------------------------
     def exact_spectrum(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
@@ -655,25 +653,20 @@ class Engine:
         from the sequence lengths and with the singles from the list-node counter, as exact_family_counts; one K7 list
         job, one K9 launch and one device->host copy per pass."""
         n = len(seqs)
-        hist, singles, priv = (np.zeros(n, dtype=np.uint64) for _ in range(3))
         if n == 0:
-            return hist, singles, priv
+            return tuple(np.zeros(n, dtype=np.uint64) for _ in range(3))
         if k > 64 and n > 65536:
             raise DandDError("the exact spectrum above k = 64 takes at most 65536 genomes per job")
         world = int(shard[1]) if shard is not None else 1
         bounds = length_bounds([s.nsym for s in seqs], k, world)
-        part = torch.zeros(3 * n, dtype=torch.int64, device=self.device)    # [hist | priv | node counter after genome g]
-        for ws, cap, nodes in self._key_lists(seqs, k, canon, bounds, shard, passes, node_counts=part[2 * n:]):
-            part[:2 * n].zero_()
-            check(self.lib.dd_exact_occupancy_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part.data_ptr(),
-                                                   part.data_ptr() + 8 * n, self.stream), "dd_exact_occupancy_hist")
-            got = part.cpu().numpy().view(np.uint64)
-            if (got[:2 * n] == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
-                raise DandDError("exact k-mer table or node array overflowed; the length bounds understate the genomes")
-            hist += got[:n]
-            priv += got[n:2 * n]
-            singles += np.diff(got[2 * n:], prepend=np.uint64(0))
-        return hist, singles, priv
+
+        def launch(ws, cap, nodes, part):      # cells [hist | priv]
+            check(self.lib.dd_exact_occupancy_hist(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, part, part + 8 * n,
+                                                   self.stream), "dd_exact_occupancy_hist")
+
+        got, singles = self._list_job(seqs, k, canon, bounds, shard, passes, 2 * n, True, launch,
+                                      "exact k-mer table or node array overflowed; the length bounds understate the genomes")
+        return got[:n], singles, got[n:]
 
     def exact_pairs_dense(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
                           block: Optional[int] = None) -> np.ndarray:

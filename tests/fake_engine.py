@@ -110,8 +110,107 @@ class FakeEngine:
                 cards[j, i] = orc.card(np.maximum(h[a, i], h[b, i]), p)
         return cards
 
+    def mle(self, hist, p):
+        flat = hist.reshape(-1, 64).numpy()
+        return torch.tensor([orc.ertl_mle(row.astype(np.uint32), p) for row in flat], dtype=torch.float64).view(hist.shape[:-1])
+
     def exact_counts(self, seqs, k, canon=True, capacity=None, shard=None):
         self.calls["exact_counts"] += 1
         if shard is not None and shard[0] != 0:      # (the oracle has no key-range filter: rank 0 counts everything)
             return [0] * len(seqs)
         return [orc.exact_count([s.sym for s in seqs[:i + 1]], int(k), canon) for i in range(len(seqs))]
+
+
+LIST_JOBS = ("exact_pair_intersections", "exact_first_rank_hist", "exact_family_counts", "exact_spectrum")
+
+
+def _absent(job):
+    def get(self):
+        raise AttributeError(job)
+    return property(get)
+
+
+class ListJobEngine(FakeEngine):
+    """FakeEngine plus the jobs Engine runs over the K7 co-occurrence lists (LIST_JOBS), all read off one table of
+    which genomes hold each distinct k-mer, from oracle k-mer sets (rank 0 holds every key, as in
+    FakeEngine.exact_counts).  Records the genome count of every per-union count and the k of every family job."""
+
+    def __init__(self):
+        super().__init__()
+        self.calls.update(dict.fromkeys(LIST_JOBS, 0))
+        self.union_sizes = []           # len(seqs) of every exact_counts call
+        self.family_ks = []             # k of every exact_family_counts call
+        self._held = {}
+
+    @classmethod
+    def only(cls, *jobs):
+        """This double offering only the list jobs `jobs`.  The store takes a job's batched path when its engine has
+        the method (hasattr), else the per-union path: the other jobs are hidden as an engine without them lacks them."""
+        hidden = {job: _absent(job) for job in LIST_JOBS if job not in jobs}
+        return type("%s.only(%s)" % (cls.__name__, ", ".join(jobs)), (cls,), hidden)
+
+    def exact_counts(self, seqs, k, canon=True, capacity=None, shard=None):
+        self.union_sizes.append(len(seqs))
+        return super().exact_counts(seqs, k, canon, capacity, shard)
+
+    def _holders(self, seqs, k, canon):
+        """bool [distinct k-mers of seqs, n]: which genomes hold each k-mer.  Cached per (seqs, k, canon); the cache
+        keeps the seqs, so their ids stay theirs."""
+        key = (tuple(id(s) for s in seqs), int(k), bool(canon))
+        if key not in self._held:
+            sets = [np.unique(orc.kmers(s.sym, int(k), canon)) for s in seqs]
+            keys, row = np.unique(np.concatenate([np.zeros(0, np.uint64)] + sets), return_inverse=True)
+            held = np.zeros((keys.size, len(seqs)), dtype=bool)
+            held[row, np.repeat(np.arange(len(seqs)), [a.size for a in sets])] = True
+            self._held[key] = (list(seqs), held)
+        return self._held[key][1]
+
+    def _first_rank(self, held, ranks):
+        """hist uint64 [R, n]: hist[r][m] = k-mers whose least rank over their holders is m under row r."""
+        n = held.shape[1]
+        hist = np.zeros(ranks.shape, dtype=np.uint64)
+        for r, row in enumerate(ranks):
+            m = np.where(held, row, 0xFFFF).min(axis=1)
+            hist[r] = np.bincount(m[m < n], minlength=n)
+        return hist
+
+    def exact_pair_intersections(self, seqs, k, canon=True, singles=None, shard=None):
+        self.calls["exact_pair_intersections"] += 1
+        n = len(seqs)
+        if shard is not None and shard[0] != 0:
+            return np.zeros(n * (n - 1) // 2, dtype=np.uint64)
+        held = self._holders(seqs, k, canon).astype(np.uint64)
+        assert singles is None or list(singles) == held.sum(axis=0).tolist()
+        return (held.T @ held)[np.triu_indices(n, 1)]
+
+    def exact_first_rank_hist(self, seqs, k, canon, ranks, singles=None, shard=None, passes=None):
+        self.calls["exact_first_rank_hist"] += 1
+        ranks = np.asarray(ranks, dtype=np.uint16).reshape(-1, len(seqs))
+        if shard is not None and shard[0] != 0:
+            return np.zeros(ranks.shape, dtype=np.uint64)
+        held = self._holders(seqs, k, canon)
+        assert singles is None or list(singles) == held.sum(axis=0).tolist()
+        return self._first_rank(held, ranks)
+
+    def exact_family_counts(self, seqs, k, canon, ranks, shard=None, passes=None):
+        from dandd_b200.engine import length_bounds
+        self.calls["exact_family_counts"] += 1
+        self.family_ks.append(int(k))
+        n = len(seqs)
+        ranks = np.asarray(ranks, dtype=np.uint16).reshape(-1, n)
+        if shard is not None and shard[0] != 0:
+            return np.zeros(n, dtype=np.uint64), np.zeros(ranks.shape, dtype=np.uint64)
+        held = self._holders(seqs, k, canon)
+        singles = held.sum(axis=0).astype(np.uint64)
+        assert all(b >= c for b, c in zip(length_bounds([s.nsym for s in seqs], k), singles))   # the job is never undersized
+        return singles, self._first_rank(held, ranks)
+
+    def exact_spectrum(self, seqs, k, canon, shard=None, passes=None):
+        self.calls["exact_spectrum"] += 1
+        n = len(seqs)
+        if shard is not None and shard[0] != 0:
+            return tuple(np.zeros(n, dtype=np.uint64) for _ in range(3))
+        held = self._holders(seqs, k, canon)
+        holders = held.sum(axis=1)
+        hist = np.bincount(holders, minlength=n + 1)[1:].astype(np.uint64)
+        return hist, held.sum(axis=0).astype(np.uint64), held[holders == 1].sum(axis=0).astype(np.uint64)

@@ -7,65 +7,15 @@ import pickle
 import random
 import socket
 
-import numpy as np
 import pytest
 
 from dandd_b200 import store as ddstore
-from tests.fake_engine import FakeEngine
+from tests.fake_engine import ListJobEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-
-class FamilyFakeEngine(FakeEngine):
-    """FakeEngine plus Engine.exact_family_counts, from oracle k-mer sets (rank 0 holds every key, as in
-    FakeEngine.exact_counts).  Records the genome count of every per-union count and the k of every family job."""
-
-    def __init__(self):
-        super().__init__()
-        self.calls["exact_family_counts"] = 0
-        self.union_sizes = []           # len(seqs) of every exact_counts call
-        self.family_ks = []             # k of every exact_family_counts call
-        self._sets = {}
-
-    def exact_counts(self, seqs, k, canon=True, capacity=None, shard=None):
-        self.union_sizes.append(len(seqs))
-        return super().exact_counts(seqs, k, canon, capacity, shard)
-
-    def _kmers(self, s, k, canon):
-        from oracle import pyoracle as orc
-        key = (id(s), int(k), bool(canon))
-        if key not in self._sets:
-            self._sets[key] = (s, set(orc.kmers(s.sym, int(k), canon).tolist()))
-        return self._sets[key][1]
-
-    def exact_family_counts(self, seqs, k, canon, ranks, shard=None, passes=None):
-        from dandd_b200.engine import length_bounds
-        self.calls["exact_family_counts"] += 1
-        self.family_ks.append(int(k))
-        n = len(seqs)
-        ranks = np.asarray(ranks, dtype=np.uint16).reshape(-1, n)
-        singles = np.zeros(n, dtype=np.uint64)
-        hist = np.zeros(ranks.shape, dtype=np.uint64)
-        if shard is not None and shard[0] != 0:
-            return singles, hist
-        sets = [self._kmers(s, k, canon) for s in seqs]
-        singles[:] = [len(s) for s in sets]
-        assert all(b >= c for b, c in zip(length_bounds([s.nsym for s in seqs], k), singles))   # the job is never undersized
-        holders = {}
-        for g, s in enumerate(sets):
-            for x in s:
-                holders.setdefault(x, []).append(g)
-        for r in range(ranks.shape[0]):
-            for gs in holders.values():
-                m = min(int(ranks[r, g]) for g in gs)
-                if m < n:
-                    hist[r, m] += 1
-        return singles, hist
-
-
-class NoFamilyEngine(FamilyFakeEngine):
-    """The same double without the family job (hasattr is what the store looks at)."""
-    exact_family_counts = property(lambda self: (_ for _ in ()).throw(AttributeError("exact_family_counts")))
+FamilyFakeEngine = ListJobEngine.only("exact_family_counts")
+NoFamilyEngine = ListJobEngine.only()           # the same double without the family job
 
 
 def _content(obj, path=()):

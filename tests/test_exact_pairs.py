@@ -11,22 +11,9 @@ from dandd_b200 import engine as E
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import allpairs
 from tests import allpairs_cases as cases
-from tests.fake_engine import FakeEngine
+from tests.fake_engine import FakeEngine, ListJobEngine
 
-
-class PairFakeEngine(FakeEngine):
-    """FakeEngine plus Engine.exact_pair_intersections, from oracle k-mer sets (rank 0 holds every key, as in
-    FakeEngine.exact_counts)."""
-
-    def exact_pair_intersections(self, seqs, k, canon=True, singles=None, shard=None):
-        from oracle import pyoracle as orc
-        self.calls["exact_pair_intersections"] = self.calls.get("exact_pair_intersections", 0) + 1
-        n = len(seqs)
-        if shard is not None and shard[0] != 0:
-            return np.zeros(n * (n - 1) // 2, dtype=np.uint64)
-        sets = [set(orc.kmers(s.sym, int(k), canon).tolist()) for s in seqs]
-        assert singles is None or list(singles) == [len(s) for s in sets]
-        return np.array([len(sets[a] & sets[b]) for a in range(n) for b in range(a + 1, n)], dtype=np.uint64)
+PairFakeEngine = ListJobEngine.only("exact_pair_intersections")
 
 
 CASE = {"genomes": 5, "length": 2500, "seed": 31, "sub": 0.05, "klist": [9, 13, 21, 32], "nest": 4096, "extra": ""}

@@ -10,33 +10,10 @@ import numpy as np
 import pytest
 
 from dandd_b200 import store as ddstore
-from tests.fake_engine import FakeEngine
+from tests.fake_engine import FakeEngine, ListJobEngine
 
-
-class SetFakeEngine(FakeEngine):
-    """FakeEngine plus Engine.exact_first_rank_hist, from oracle k-mer sets (rank 0 holds every key, as in
-    FakeEngine.exact_counts)."""
-
-    def exact_first_rank_hist(self, seqs, k, canon, ranks, singles=None, shard=None, passes=None):
-        from oracle import pyoracle as orc
-        self.calls["exact_first_rank_hist"] = self.calls.get("exact_first_rank_hist", 0) + 1
-        n = len(seqs)
-        ranks = np.asarray(ranks, dtype=np.uint16).reshape(-1, n)
-        hist = np.zeros(ranks.shape, dtype=np.uint64)
-        if shard is not None and shard[0] != 0:
-            return hist
-        sets = [set(orc.kmers(s.sym, int(k), canon).tolist()) for s in seqs]
-        assert singles is None or list(singles) == [len(s) for s in sets]
-        holders = {}
-        for g, s in enumerate(sets):
-            for x in s:
-                holders.setdefault(x, []).append(g)
-        for r in range(ranks.shape[0]):
-            for gs in holders.values():
-                m = min(int(ranks[r, g]) for g in gs)
-                if m < n:
-                    hist[r, m] += 1
-        return hist
+# the first-rank job alone: without the family job, a hill-climb's cells stay per union
+SetFakeEngine = ListJobEngine.only("exact_first_rank_hist")
 
 
 def _symbols_sets(fastas, k):

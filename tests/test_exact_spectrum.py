@@ -17,33 +17,11 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import spectrum
-from tests.test_exact_sets import SetFakeEngine
+from tests.fake_engine import ListJobEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-
-class SpectrumFakeEngine(SetFakeEngine):
-    """SetFakeEngine (exact counts and first-rank histograms) plus Engine.exact_spectrum, from oracle k-mer sets (rank 0
-    holds every key, as in FakeEngine.exact_counts)."""
-
-    def exact_spectrum(self, seqs, k, canon, shard=None, passes=None):
-        from oracle import pyoracle as orc
-        self.calls["exact_spectrum"] = self.calls.get("exact_spectrum", 0) + 1
-        n = len(seqs)
-        hist, singles, priv = (np.zeros(n, dtype=np.uint64) for _ in range(3))
-        if shard is not None and shard[0] != 0:
-            return hist, singles, priv
-        sets = [set(orc.kmers(s.sym, int(k), canon).tolist()) for s in seqs]
-        singles[:] = [len(s) for s in sets]
-        holders = {}
-        for g, s in enumerate(sets):
-            for x in s:
-                holders.setdefault(x, []).append(g)
-        for gs in holders.values():
-            hist[len(gs) - 1] += 1
-            if len(gs) == 1:
-                priv[gs[0]] += 1
-        return hist, singles, priv
+SpectrumFakeEngine = ListJobEngine.only("exact_first_rank_hist", "exact_spectrum")
 
 
 def _read_tsv(path):
@@ -185,7 +163,7 @@ def test_integer_identities(tmp_path, canon):
 def test_store_refuses_an_engine_without_the_job(tmp_path):
     from tests.util import make_dataset
     files = make_dataset(str(tmp_path / "d"), 2, 500, seed=1)
-    st = ddstore.GpuSketchStore(engine=SetFakeEngine())
+    st = ddstore.GpuSketchStore(engine=ListJobEngine.only("exact_first_rank_hist")())
     with pytest.raises(RuntimeError, match="spectrum"):
         st.exact_spectrum(files, [5], True)
 

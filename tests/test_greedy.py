@@ -13,7 +13,7 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import greedy
-from tests.test_leaveout import LeaveOutFakeEngine
+from tests.fake_engine import ListJobEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BINS = 64
@@ -132,8 +132,8 @@ def test_sparse_rule_follows_union_updates():
 
 
 # ---------------------------------------------------------------- the store's loop on an engine double
-class GreedyFakeEngine(LeaveOutFakeEngine):
-    """LeaveOutFakeEngine plus the K11 methods as the numpy restatement above, and Engine.cards_hist."""
+class GreedyFakeEngine(ListJobEngine):
+    """ListJobEngine plus the K11 methods as the numpy restatement above, and Engine.cards_hist."""
 
     def cards_hist(self, regs, p):
         import torch
@@ -229,7 +229,7 @@ def test_store_loop_equals_brute_force(clustered, monkeypatch, mode, order, firs
 
 def test_store_refuses_an_engine_without_the_step():
     import torch
-    st = ddstore.GpuSketchStore(engine=LeaveOutFakeEngine())
+    st = ddstore.GpuSketchStore(engine=ListJobEngine())
     with pytest.raises(RuntimeError, match="K11"):
         st.greedy_order(torch.zeros((2, 1, 32), dtype=torch.uint8), [3], 5, 2)
 

@@ -12,7 +12,7 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import leaveout
-from tests.test_exact_spectrum import SpectrumFakeEngine
+from tests.fake_engine import ListJobEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BINS = 64
@@ -57,9 +57,8 @@ def streaming_hist(regs, group, n_groups, order=None):
     return out
 
 
-class LeaveOutFakeEngine(SpectrumFakeEngine):
-    """SpectrumFakeEngine plus Engine.leave_out_hist (explicit maxima), Engine.mle (the oracle's estimator) and
-    Engine.exact_family_counts (oracle k-mer sets; rank 0 holds every key, as in FakeEngine.exact_counts)."""
+class LeaveOutFakeEngine(ListJobEngine):
+    """ListJobEngine plus Engine.leave_out_hist (explicit maxima)."""
 
     def leave_out_hist(self, regs, group, n_groups, p, reg_range=None, out=None):
         import torch
@@ -68,22 +67,6 @@ class LeaveOutFakeEngine(SpectrumFakeEngine):
         assert begin % 16 == 0 and end % 16 == 0
         got = torch.from_numpy(brute_hist(regs.numpy(), group, n_groups, begin, end).astype(np.int32))
         return got if out is None else out.add_(got)
-
-    def mle(self, hist, p):
-        import torch
-        from oracle import pyoracle as orc
-        flat = hist.reshape(-1, BINS).numpy()
-        return torch.tensor([orc.ertl_mle(row.astype(np.uint32), p) for row in flat], dtype=torch.float64).view(hist.shape[:-1])
-
-    def exact_family_counts(self, seqs, k, canon, ranks, shard=None, passes=None):
-        from oracle import pyoracle as orc
-        self.calls["exact_family_counts"] = self.calls.get("exact_family_counts", 0) + 1
-        n = len(seqs)
-        singles = np.zeros(n, dtype=np.uint64)
-        if shard is not None and shard[0] != 0:
-            return singles, np.zeros((len(ranks), n), dtype=np.uint64)
-        singles[:] = [len(set(orc.kmers(s.sym, int(k), canon).tolist())) for s in seqs]
-        return singles, self.exact_first_rank_hist(seqs, k, canon, ranks)
 
 
 # ---------------------------------------------------------------- the streaming rule
@@ -222,12 +205,11 @@ def test_kmc_contribution_equals_find_delta_delta(tmp_path):
     import dandd_b200
     from tests.host_harness import run_dandd
     from tests.util import make_dataset
-    from tests.test_exact_climb import FamilyFakeEngine
     data = str(tmp_path / "data")
     fastas = make_dataset(data, 4, 2500, seed=31)
     (union, without), _ = _run(["-d", data, "--tool", "kmc", "--mink", "2", "--maxk", "20", "--name", str(tmp_path / "run")])
     ks = list(range(2, 21))
-    st = ddstore.GpuSketchStore(engine=FamilyFakeEngine())
+    st = ddstore.GpuSketchStore(engine=ListJobEngine.only("exact_family_counts")())    # as test_exact_climb climbs
     ddstore.set_store(st)
     try:
         run_dandd(["tree", "-d", data, "-s", "ex", "-o", str(tmp_path / "out"), "--exact"])
