@@ -10,6 +10,7 @@ LIB_PATH = os.path.join(_HERE, "libdandd_b200.so")
 
 DD_HIST_BINS = 64
 DD_EXACT_BITMAP_MAXK = 16
+DD_COVER_PART_BYTES = 64
 ABI_VERSION = 2
 DD_PACK_FLAG_OVERFLOW, DD_PACK_FLAG_FASTQ = 1, 2
 DD_ERR_FORMAT = -5
@@ -73,6 +74,9 @@ SIGNATURES = {
     "dd_exact_first_rank_hist": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _vp, _i64, _vp, _vp]),
     "dd_exact_pairs_node_count": (_i, [_vp, _sz, _vp, _vp]),
     "dd_exact_occupancy_hist": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _vp, _vp, _vp]),
+    "dd_exact_cover_count": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _vp, _vp]),
+    "dd_exact_cover_emit": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _u64, _u64, _vp, _vp, _vp, _vp, _vp]),
+    "dd_exact_cover_step": (_i, [_vp, _i, _i64, _i64, _vp, _sz, _vp]),
     "dd_leave_out_workspace_bytes": (_sz, [_i, _i]),
     "dd_leave_out_hist": (_i, [_vp, _i, _i, _i, _vp, _i, _u64, _u64, _vp, _vp, _sz, _vp]),
     "dd_greedy_workspace_bytes": (_sz, [_i]),

@@ -624,6 +624,67 @@ int dd_exact_occupancy_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t c
             "dd_exact_occupancy_hist");
     return DD_OK;
 }
+// ---- K12 -----------------------------------------------------------------------------------------
+static bool misaligned(const void *p, uintptr_t a) { return reinterpret_cast<uintptr_t>(p) & (a - 1); }
+int dd_exact_cover_count(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams,
+                         uint64_t *d_counts, dd_stream stream) {
+    const char *fn = "dd_exact_cover_count";
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, fn)) return rc;
+    if (!d_counts) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (misaligned(d_counts, 8)) return fail(DD_ERR_ARG, "%s: misaligned counts", fn);
+    DD_CUDA(dd::exact_cover_count(d_ws, k, capacity, max_streams, d_counts, sm_count_now(), S(stream)), fn);
+    return DD_OK;
+}
+int dd_exact_cover_emit(void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams,
+                        int64_t n_genomes, uint64_t n_keys, uint64_t n_nodes, uint32_t *d_offsets, uint16_t *d_holders,
+                        uint32_t *d_key_of_node, uint64_t *d_status, dd_stream stream) {
+    const char *fn = "dd_exact_cover_emit";
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, fn)) return rc;
+    if (n_genomes < 1 || n_genomes > 0xFFFF)   // holders are u16
+        return fail(DD_ERR_ARG, "%s: n_genomes=%lld outside [1,65535]", fn, (long long)n_genomes);
+    if (n_keys > 0xFFFFFFFFull) return fail(DD_ERR_ARG, "%s: %llu keys, key ids are u32", fn, (unsigned long long)n_keys);
+    if (n_nodes >= 0xFFFFFFFFull) return fail(DD_ERR_ARG, "%s: %llu nodes, offsets are u32", fn, (unsigned long long)n_nodes);
+    if (!d_offsets || !d_status || (n_nodes > 0 && (!d_holders || !d_key_of_node))) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (misaligned(d_offsets, 4) || misaligned(d_holders, 2) || misaligned(d_key_of_node, 4) || misaligned(d_status, 8))
+        return fail(DD_ERR_ARG, "%s: misaligned offsets, holders, key ids or status", fn);
+    DD_CUDA(dd::exact_cover_emit(d_ws, k, capacity, max_streams, (uint32_t)n_genomes, n_keys, n_nodes, d_offsets, d_holders,
+                                 d_key_of_node, d_status, sm_count_now(), S(stream)), fn);
+    return DD_OK;
+}
+int dd_exact_cover_step(const dd_cover_part *h_parts, int n_parts, int64_t n_genomes, int64_t genome, void *d_ws,
+                        size_t ws_bytes, dd_stream stream) {
+    static_assert(sizeof(dd_cover_part) == DD_COVER_PART_BYTES && sizeof(dd::CoverPart) == DD_COVER_PART_BYTES,
+                  "cover part descriptors are 64 bytes on both sides");
+    const char *fn = "dd_exact_cover_step";
+    if (!h_parts || !d_ws) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (misaligned(d_ws, 16)) return fail(DD_ERR_ARG, "%s: misaligned workspace", fn);
+    if (n_parts < 1 || n_parts > 65535) return fail(DD_ERR_ARG, "%s: n_parts=%d outside [1,65535]", fn, n_parts);
+    if (n_genomes < 1 || n_genomes > 0xFFFF) return fail(DD_ERR_ARG, "%s: n_genomes=%lld outside [1,65535]", fn, (long long)n_genomes);
+    if (genome < 0 || genome >= n_genomes)
+        return fail(DD_ERR_ARG, "%s: genome %lld outside [0,%lld)", fn, (long long)genome, (long long)n_genomes);
+    if (ws_bytes < (size_t)n_parts * DD_COVER_PART_BYTES)
+        return fail(DD_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, ws_bytes, (size_t)n_parts * DD_COVER_PART_BYTES);
+    std::vector<dd::CoverPart> parts(n_parts);
+    for (int i = 0; i < n_parts; ++i) {
+        const dd_cover_part &p = h_parts[i];
+        if (!p.d_offsets || !p.d_covered || !p.d_lost || !p.h_node_start || (p.n_nodes > 0 && (!p.d_holders || !p.d_key_of_node)))
+            return fail(DD_ERR_ARG, "%s: part %d: null pointer", fn, i);
+        if (misaligned(p.d_offsets, 4) || misaligned(p.d_holders, 2) || misaligned(p.d_key_of_node, 4) || misaligned(p.d_lost, 8))
+            return fail(DD_ERR_ARG, "%s: part %d: misaligned offsets, holders, key ids or counters", fn, i);
+        if (p.n_keys > 0xFFFFFFFFull || p.n_nodes >= 0xFFFFFFFFull)
+            return fail(DD_ERR_ARG, "%s: part %d: %llu keys, %llu nodes (key ids and offsets are u32)", fn, i,
+                        (unsigned long long)p.n_keys, (unsigned long long)p.n_nodes);
+        const uint64_t b = p.h_node_start[genome], e = p.h_node_start[genome + 1];
+        if (b > e || e > p.n_nodes)
+            return fail(DD_ERR_ARG, "%s: part %d: genome %lld has nodes [%llu,%llu), outside [0,%llu] or decreasing", fn, i,
+                        (long long)genome, (unsigned long long)b, (unsigned long long)e, (unsigned long long)p.n_nodes);
+        parts[i] = dd::CoverPart{p.d_offsets, p.d_holders, p.d_key_of_node, p.d_covered,
+                                 reinterpret_cast<unsigned long long *>(p.d_lost), b, e, 0};
+    }
+    DD_CUDA(dd::exact_cover_step(parts.data(), n_parts, (uint32_t)n_genomes, d_ws, sm_count_now(), S(stream)), fn);
+    return DD_OK;
+}
+
 int dd_exact_pairs_node_count(const void *d_ws, size_t ws_bytes, uint64_t *d_out, dd_stream stream) {
     if (!d_ws || !d_out) return fail(DD_ERR_ARG, "dd_exact_pairs_node_count: null pointer");
     if (ws_bytes < sizeof(dd::ExactWsHeader)) return fail(DD_ERR_WORKSPACE, "dd_exact_pairs_node_count: workspace %zu too small", ws_bytes);

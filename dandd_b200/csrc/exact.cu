@@ -67,10 +67,6 @@ struct CountFresh {  // K5: distinct keys
     }
 };
 
-constexpr uint32_t kNil = 0xFFFFFFFFu;
-struct PairNode {
-    uint32_t genome, next;
-};
 // K7: slot s keeps (last genome pushed, head of its node list) in lh[s]; the all-ones key, which cannot
 // live in the table, uses the extra slot lh[capacity].  Genomes are inserted one after another, so the
 // first thread of genome g to reach a slot is the one whose exchange returns something other than g.
@@ -361,10 +357,10 @@ cudaError_t exact_count(void *d_ws, int k, uint64_t capacity, uint64_t *d_count,
 // for every two genomes on one list -- sum over keys of occ(occ-1)/2 increments.
 static size_t pairs_key_bytes(int k, uint64_t capacity) { return (size_t)capacity * (k > 32 ? 2 : 1) * sizeof(unsigned long long); }
 static size_t pairs_stream_bytes(int k, unsigned max_streams) { return k > 64 ? (size_t)max_streams * sizeof(const uint32_t *) : 0; }
-static size_t pairs_lh_offset(int k, uint64_t capacity, unsigned max_streams) {
+size_t pairs_lh_offset(int k, uint64_t capacity, unsigned max_streams) {
     return 256 + pairs_key_bytes(k, capacity) + pairs_stream_bytes(k, max_streams);
 }
-static size_t pairs_node_offset(int k, uint64_t capacity, unsigned max_streams) {
+size_t pairs_node_offset(int k, uint64_t capacity, unsigned max_streams) {
     return pairs_lh_offset(k, capacity, max_streams) + (size_t)(capacity + 1) * sizeof(uint2);
 }
 size_t exact_pairs_workspace_bytes(int k, uint64_t capacity, uint64_t max_nodes, unsigned max_streams) {

@@ -101,6 +101,8 @@ struct ExactWsHeader {
     unsigned long long cur_stream;  // k > 64: index (in the stream table) of the stream being inserted
     unsigned long long n_streams;   // k > 64: streams registered so far
     unsigned long long n_nodes;     // K7: co-occurrence nodes pushed so far
+    unsigned long long cover_cursor;  // K12 emit: (keys << 32) | nodes reserved so far
+    unsigned long long cover_bad;     // K12 emit: a reservation did not fit the caller's buffers, or a genome >= n
 };
 size_t exact_workspace_bytes(int k, uint64_t capacity);
 cudaError_t exact_begin(void *d_ws, int k, uint64_t capacity, cudaStream_t stream);
@@ -110,6 +112,12 @@ cudaError_t exact_insert(const uint32_t *d_codes, const uint32_t *d_invalid, uin
 cudaError_t exact_count(void *d_ws, int k, uint64_t capacity, uint64_t *d_count, cudaStream_t stream);
 
 // ---- K7 (exact.cu): pair intersections.  Sparse: [ExactWsHeader | key table | streams | (last, head) | nodes]
+constexpr uint32_t kNil = 0xFFFFFFFFu;
+struct PairNode {
+    uint32_t genome, next;
+};
+size_t pairs_lh_offset(int k, uint64_t capacity, unsigned max_streams);     // the (last, head) u32 pairs, capacity + 1
+size_t pairs_node_offset(int k, uint64_t capacity, unsigned max_streams);   // the PairNode array
 size_t exact_pairs_workspace_bytes(int k, uint64_t capacity, uint64_t max_nodes, unsigned max_streams);
 cudaError_t exact_pairs_begin(void *d_ws, int k, uint64_t capacity, unsigned max_streams, cudaStream_t stream);
 cudaError_t exact_pairs_insert(const uint32_t *d_codes, const uint32_t *d_invalid, uint64_t sym_begin, uint64_t sym_end, int k,
@@ -129,5 +137,27 @@ cudaError_t exact_pairs_node_count(const void *d_ws, uint64_t *d_out, cudaStream
 // Dense: K5 bitmap workspaces, ws_stride bytes apart, for genomes row0.. and col0..
 cudaError_t exact_pair_popc(const void *d_rows, int64_t row0, int nr, const void *d_cols, int64_t col0, int nc,
                             size_t ws_stride, int k, int64_t n_genomes, uint64_t *d_inter, int sm_count, cudaStream_t stream);
+
+// ---- K12 (cover.cu): the exact greedy cover index over the K7 lists.  count: d_counts[2] = (distinct keys, nodes),
+// all-ones on a full table or node array.  emit: offsets [n_keys + 1] u32, holders [n_nodes] u16, key_of_node
+// [n_nodes] u32; d_status[2] = (keys, nodes) written, or all-ones.  step: one launch over the parts (device
+// descriptors in d_parts) adds, for every key of the picked genome's node range not covered yet, 1 to lost[h] of
+// every holder h.
+struct CoverPart {
+    const uint32_t *offsets;
+    const uint16_t *holders;
+    const uint32_t *key_of_node;
+    uint8_t *covered;
+    unsigned long long *lost;   // [n_genomes], added to
+    uint64_t node_begin, node_end;
+    uint64_t pad;
+};
+cudaError_t exact_cover_count(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t *d_counts,
+                              int sm_count, cudaStream_t stream);
+cudaError_t exact_cover_emit(void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint32_t n_genomes, uint64_t n_keys,
+                             uint64_t n_nodes, uint32_t *d_offsets, uint16_t *d_holders, uint32_t *d_key_of_node,
+                             uint64_t *d_status, int sm_count, cudaStream_t stream);
+cudaError_t exact_cover_step(const CoverPart *h_parts, int n_parts, uint32_t n_genomes, void *d_ws, int sm_count,
+                             cudaStream_t stream);
 
 }  // namespace dd

@@ -12,7 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import DD_HIST_BINS, DD_PACK_FLAG_FASTQ, DD_PACK_FLAG_OVERFLOW, DandDError, check
+from ._lib import DD_COVER_PART_BYTES, DD_HIST_BINS, DD_PACK_FLAG_FASTQ, DD_PACK_FLAG_OVERFLOW, DandDError, check
 
 
 class FastqInput(DandDError):
@@ -546,7 +546,7 @@ class Engine:
         return out
 
     def _list_job(self, seqs: Sequence[PackedSeq], k: int, canon: bool, sizes: Sequence[int], shard: Optional[tuple],
-                  passes: Optional[int], cells: int, node_counts: bool, launch, overflow: str):
+                  passes: Optional[int], cells: int, node_counts: bool, launch, overflow: str, after=None):
         """One job over the K7 co-occurrence lists, in key-range passes (plan_pair_passes over `sizes`: the exact
         singles, or length bounds that never understate them).  Every pass, each genome pushes itself onto the list
         of every key of the pass it holds (genome g = seqs[g]); then launch(workspace, capacity, max_nodes, out_ptr)
@@ -554,7 +554,8 @@ class Engine:
         An all-ones cell means the table or node array overflowed: DandDError(overflow).  Returns (the cells summed
         over the passes, uint64; with node_counts, |A_g| per genome, uint64 [n], else None): the list-node counter is
         read after every genome's insert (dd_exact_pairs_node_count), and its growth over genome g is
-        |A_g n the pass's key range|."""
+        |A_g n the pass's key range|.  after(workspace, capacity, max_nodes, got), if given, runs at the end of every pass
+        while its lists are still in the workspace; got is the pass's copy (uint64 [cells | node counter after genome g])."""
         n = len(seqs)
         srank, sworld = (int(shard[0]), int(shard[1])) if shard is not None else (0, 1)
         nsyms = [s.nsym for s in seqs]
@@ -585,6 +586,8 @@ class Engine:
                 if (got[:cells] == np.uint64(0xFFFFFFFFFFFFFFFF)).any():
                     raise DandDError(overflow)
                 out += got[:cells]
+                if after is not None:
+                    after(ws, cap, nodes, got)
                 if node_counts:
                     singles += np.diff(got[cells:], prepend=np.uint64(0))
             return out, singles
@@ -667,6 +670,71 @@ class Engine:
         got, singles = self._list_job(seqs, k, canon, bounds, shard, passes, 2 * n, True, launch,
                                       "exact k-mer table or node array overflowed; the length bounds understate the genomes")
         return got[:n], singles, got[n:]
+
+    # ---- K12 --------------------------------------------------------------------------------
+    def exact_cover_index(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
+                          passes: Optional[int] = None) -> dict:
+        """The greedy cover index of seqs at k (K12), one part per key-range pass, resident on the device:
+        {"k", "n", "parts": [{"offsets", "holders", "key_of_node", "covered", "n_keys", "n_nodes", "node_start"}],
+        "singles": uint64 [n] (|A_g|), "keys": distinct keys (|union of all|), "bytes": device bytes of the parts}
+        (this rank's key range under `shard`).  One K7 list job: after every pass's inserts, a count of its keys and
+        nodes is read back and the pass's index is allocated to exactly that and emitted from the lists; node_start
+        [n + 1] (host) holds the node counter before every genome's insert, so genome g's keys in the part are
+        key_of_node[node_start[g]:node_start[g + 1]].  Raises DandDError for a full table or node array, and torch's
+        OutOfMemoryError when the index does not fit."""
+        n = len(seqs)
+        if not 1 <= n <= 65535:
+            raise DandDError("the exact cover index takes 1..65535 genomes per job (holders are 16-bit), got %d" % n)
+        world = int(shard[1]) if shard is not None else 1
+        bounds = length_bounds([s.nsym for s in seqs], k, world)
+        parts = []
+
+        def count(ws, cap, nodes, part):      # cells [distinct keys, nodes]
+            check(self.lib.dd_exact_cover_count(ws.data_ptr(), ws.numel(), k, cap, nodes, n, part, self.stream),
+                  "dd_exact_cover_count")
+
+        def emit(ws, cap, nodes, got):
+            n_keys, n_nodes = int(got[0]), int(got[1])
+            dev = self.device
+            part = {"offsets": torch.empty(n_keys + 1, dtype=torch.int32, device=dev),
+                    "holders": torch.empty(max(n_nodes, 1), dtype=torch.int16, device=dev),
+                    "key_of_node": torch.empty(max(n_nodes, 1), dtype=torch.int32, device=dev),
+                    "covered": torch.zeros(max(n_keys, 1), dtype=torch.uint8, device=dev),
+                    "n_keys": n_keys, "n_nodes": n_nodes,
+                    "node_start": np.concatenate([[0], got[2:]]).astype(np.uint64)}
+            status = torch.empty(2, dtype=torch.int64, device=dev)
+            check(self.lib.dd_exact_cover_emit(ws.data_ptr(), ws.numel(), k, cap, nodes, n, n, n_keys, n_nodes,
+                                               part["offsets"].data_ptr(), part["holders"].data_ptr(),
+                                               part["key_of_node"].data_ptr(), status.data_ptr(), self.stream),
+                  "dd_exact_cover_emit")
+            if status.cpu().numpy().view(np.uint64).tolist() != [n_keys, n_nodes]:
+                raise DandDError("exact cover index at k=%d: the lists did not match their count" % k)
+            parts.append(part)
+
+        got, singles = self._list_job(seqs, k, canon, bounds, shard, passes, 2, True, count,
+                                      "exact k-mer table or node array overflowed; the length bounds understate the genomes",
+                                      after=emit)
+        nbytes = sum(sum(part[t].numel() * part[t].element_size() for t in ("offsets", "holders", "key_of_node", "covered"))
+                     for part in parts)
+        return {"k": int(k), "n": n, "parts": parts, "singles": singles, "keys": int(got[0]), "bytes": nbytes}
+
+    def exact_cover_step(self, indices: Sequence[dict], genome: int, lost: torch.Tensor) -> None:
+        """Genome `genome` joins the union (K12): for every part of every index (one per k, from exact_cover_index), the
+        keys of the genome not covered yet are covered and add 1 to lost[c][h] of every genome h holding them, c the
+        index's position.  lost: int64 [len(indices), n] on the device, added to.  One launch, no synchronisation."""
+        n = int(indices[0]["n"])
+        assert lost.dtype == torch.int64 and lost.is_contiguous() and tuple(lost.shape) == (len(indices), n)
+        table = np.zeros((sum(len(ix["parts"]) for ix in indices), DD_COVER_PART_BYTES // 8), dtype=np.uint64)
+        i = 0
+        for c, ix in enumerate(indices):
+            for part in ix["parts"]:
+                table[i] = [part["offsets"].data_ptr(), part["holders"].data_ptr(), part["key_of_node"].data_ptr(),
+                            part["covered"].data_ptr(), lost[c].data_ptr(), part["n_keys"], part["n_nodes"],
+                            part["node_start"].ctypes.data]
+                i += 1
+        ws = self._buf(table.shape[0] * DD_COVER_PART_BYTES, "cover_step")
+        check(self.lib.dd_exact_cover_step(table.ctypes.data, table.shape[0], n, int(genome), ws.data_ptr(), ws.numel(),
+                                           self.stream), "dd_exact_cover_step")
 
     def exact_pairs_dense(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
                           block: Optional[int] = None) -> np.ndarray:

@@ -5,20 +5,26 @@ Step t adds the genome not chosen yet whose union with the genomes chosen so far
 or the smallest (--order min), the lowest input index winning a tie; genomes listed in --first take the first steps
 in the order given.  delta is the maximum over the swept k of card / k, the first k winning a tie.  The greedy
 growth curve is the upper edge of the band `dandd progressive` samples (--order min gives a lower curve), and its
-first m genomes answer "which m assemblies capture most of the diversity".  Every step evaluates every remaining
-candidate on the HLL registers resident on the device (store.greedy_order, K11): the time grows with steps x n.
+first m genomes answer "which m assemblies capture most of the diversity".
+  --tool dashing  every step evaluates every remaining candidate on the HLL registers resident on the device
+                  (store.greedy_order, K11): the time grows with steps x n.
+  --tool kmc      exact distinct k-mer counts (store.exact_greedy_order, K12): a cover index per k is built once and
+                  held on the device (about 6 bytes per (genome, distinct k-mer) plus 5 per distinct k-mer, per k);
+                  then every step is one device launch over all k, and the whole order costs one visit per holder of
+                  every k-mer.  Late in an order the candidates differ by few novel k-mers, which HLL estimates blur;
+                  these counts do not.  At most 65535 inputs; k up to 256; --registers is not used.
 
 Inputs are listed as `dandd tree` lists them (-d DATADIR or -f LIST, sorted); genome i is index i of that list and
 names are the FASTA base names, which must be distinct.  --first names input base names, one per line.  Written
-into --name (a directory that must not exist yet), tab-separated, floats by repr:
+into --name (a directory that must not exist yet), tab-separated, floats by repr, integer cards for kmc:
   order.tsv       step  genome  forced  delta  k  gain  fraction   gain = delta - delta before the step (0 before
                                                                      the first), fraction = delta / delta(all inputs)
   growth.tsv      ngen  k  card  delta_pos                          the union of the first ngen genomes, every k
   collection.tsv  ngen  delta  k                                    the union of all inputs
   ordering.pickle {tuple(order)}: `dandd progressive -d <tree of the same inputs> -r DIR/ordering.pickle --ksweep`
                   replays it (-n 0; with --steps n, -n 30 adds random orderings beside it).
-Under torchrun every rank sketches its share of the genomes and evaluates its share of the candidates, and rank 0
-writes."""
+Under torchrun every rank sketches its share of the genomes and evaluates its share of the candidates (dashing) or
+indexes its key range of every genome (kmc), and rank 0 writes."""
 import argparse
 import os
 import pickle
@@ -28,6 +34,8 @@ from typing import List, Sequence
 import numpy as np
 
 HLL_MAX_K = 32       # Dashing's
+EXACT_MAX_K = 256    # KMC's
+EXACT_MAX_N = 65535  # the cover index keeps genome ids in 16 bits
 
 
 def get_store():
@@ -56,7 +64,9 @@ def write_outputs(directory: str, names: Sequence[str], ks: Sequence[int], order
     """order.tsv, growth.tsv, collection.tsv and ordering.pickle from order [steps], cards [steps, nk] (the union
     after each step) and all_cards [nk] (the union of every input)."""
     from dandd_b200.helpers.leaveout import best_k
-    cards = np.asarray(cards, dtype=np.float64)
+    cards = np.asarray(cards)
+    if cards.dtype.kind not in "iu":      # integer (exact) cards stay integers
+        cards = cards.astype(np.float64)
     d_all, k_all = best_k(ks, np.asarray(all_cards, dtype=np.float64))
     d_all = float(d_all)
     rows = {"order.tsv": ["step\tgenome\tforced\tdelta\tk\tgain\tfraction"], "growth.tsv": ["ngen\tk\tcard\tdelta_pos"],
@@ -83,7 +93,9 @@ def parse_arguments(argv=None):
     src = parser.add_mutually_exclusive_group()
     src.add_argument("-d", "--datadir", dest="genomedir", default=None, help="directory of FASTA files (every file is an input)")
     src.add_argument("-f", "--fastas", dest="flist_loc", default=None, help="file listing one FASTA path per line")
-    parser.add_argument("--mink", type=int, default=2, help="smallest k (1..%d)" % HLL_MAX_K)
+    parser.add_argument("--tool", choices=["dashing", "kmc"], default="dashing",
+                        help="dashing: HLL estimates (default); kmc: exact distinct k-mer counts")
+    parser.add_argument("--mink", type=int, default=2, help="smallest k (1..%d for dashing, 1..%d for kmc)" % (HLL_MAX_K, EXACT_MAX_K))
     parser.add_argument("--maxk", type=int, default=32, help="largest k")
     parser.add_argument("--registers", type=int, default=20, help="log2 of the number of HLL registers")
     parser.add_argument("--no-canon", dest="canon", action="store_false", help="count k-mers as read, not canonical")
@@ -103,11 +115,13 @@ def _inputs(args):
     if not (args.genomedir or args.flist_loc):
         return None, "give the inputs: -d DATADIR or -f LIST"
     for flag, k in (("--mink", args.mink), ("--maxk", args.maxk)):
-        if not 1 <= k <= HLL_MAX_K:
+        if args.tool == "dashing" and not 1 <= k <= HLL_MAX_K:
             return None, "%s %d is outside 1..%d" % (flag, k, HLL_MAX_K)
+        if args.tool == "kmc" and not 1 <= k <= EXACT_MAX_K:
+            return None, "%s %d is outside 1..%d for kmc" % (flag, k, EXACT_MAX_K)
     if args.mink > args.maxk:
         return None, "--mink %d is above --maxk %d" % (args.mink, args.maxk)
-    if not 5 <= args.registers <= 26:
+    if args.tool == "dashing" and not 5 <= args.registers <= 26:
         return None, "--registers %d is outside 5..26" % args.registers
     try:
         fastas = list_fastas(args.genomedir, args.flist_loc)
@@ -119,6 +133,8 @@ def _inputs(args):
         return None, "input names must be distinct: %s" % dup
     if len(names) < 2:
         return None, "an ordering needs at least 2 inputs, got %d" % len(names)
+    if args.tool == "kmc" and len(names) > EXACT_MAX_N:
+        return None, "--tool kmc orders at most %d inputs, got %d" % (EXACT_MAX_N, len(names))
     first: List[int] = []
     if args.first:
         try:
@@ -151,16 +167,23 @@ def go(argv=None):
     try:
         store = get_store()
         from dandd_b200 import ingest
-        from dandd_b200.helpers.allpairs import gather_leaf_registers
-        owners = [[g for g in range(n) if g % world == r] for r in range(world)]
-        ingest.prefetch([fastas[g] for g in owners[rank]], want_digest=False)
-        regs, _ = gather_leaf_registers(store, fastas, ks, args.registers, args.canon, owners, tag="greedy")
-        with timing.span("greedy_order"):
-            order, cards, stats = store.greedy_order(regs, ks, args.registers, steps, order=args.order, first=first,
-                                                     shard=shard)
-        with timing.span("greedy_collection"):
-            engine = store.engine
-            all_cards = engine.cards(engine.union([regs[g] for g in range(n)]), args.registers).cpu().numpy()
+        if args.tool == "kmc":
+            ingest.prefetch(fastas, want_digest=False)          # every rank indexes its key range of every genome
+            with timing.span("greedy_order"):
+                order, cards, stats = store.exact_greedy_order(fastas, ks, args.canon, steps, order=args.order, first=first,
+                                                               shard=shard)
+            all_cards = np.asarray(stats["distinct_keys"], dtype=np.int64)   # the index's keys: |union of all|
+        else:
+            from dandd_b200.helpers.allpairs import gather_leaf_registers
+            owners = [[g for g in range(n) if g % world == r] for r in range(world)]
+            ingest.prefetch([fastas[g] for g in owners[rank]], want_digest=False)
+            regs, _ = gather_leaf_registers(store, fastas, ks, args.registers, args.canon, owners, tag="greedy")
+            with timing.span("greedy_order"):
+                order, cards, stats = store.greedy_order(regs, ks, args.registers, steps, order=args.order, first=first,
+                                                         shard=shard)
+            with timing.span("greedy_collection"):
+                engine = store.engine
+                all_cards = engine.cards(engine.union([regs[g] for g in range(n)]), args.registers).cpu().numpy()
         if rank == 0:
             with timing.span("greedy_outputs"):
                 write_outputs(args.name, names, ks, order, len(first), cards, all_cards)

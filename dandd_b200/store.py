@@ -36,6 +36,14 @@ SPARSE_CROSS = 2
 STREAM_MIN_BYTES = int(os.environ.get("DANDD_B200_STREAM_MIN", str(32 << 20)))   # larger FASTAs take the chunked pipeline
 
 
+def greedy_pick(cards: torch.Tensor, kdiv: torch.Tensor, chosen: torch.Tensor, order: str) -> torch.Tensor:
+    """One greedy step's pick, on the device: the genome not `chosen` whose delta = max_k cards[g, k] / k is the largest
+    (order="max") or the smallest ("min"), the lowest index winning a tie.  cards float64 [n, nk], kdiv the ks [nk]."""
+    fill = float("-inf") if order == "max" else float("inf")
+    delta = (cards / kdiv).amax(dim=1).masked_fill(chosen, fill)
+    return delta.argmax() if order == "max" else delta.argmin()   # the first extremum: the lowest index
+
+
 def read_fasta_bytes(path: str) -> bytes:
     """Whole FASTA as bytes; .gz is inflated on the host (dashing/kmc read .gz transparently).
     Served from the background ingest pool when the file was prefetched."""
@@ -676,7 +684,6 @@ class GpuSketchStore:
         if budget is None:
             budget = self.engine._pairs_budget()
         kdiv = torch.as_tensor(np.asarray(ks, dtype=np.float64), device=dev)
-        fill = float("-inf") if order == "max" else float("inf")
         union = torch.zeros((nk, m), dtype=torch.uint8, device=dev)
         _, uhist = self.engine.cards_hist(union, p)
         cards = torch.empty((steps, nk), dtype=torch.float64, device=dev)
@@ -702,8 +709,7 @@ class GpuSketchStore:
                     full[rows] = self.engine.mle(hist, p)
                 if world > 1:
                     full = dd_dist.sum_counts(full)
-                delta = (full / kdiv).amax(dim=1).masked_fill(chosen, fill)
-                pick_d = delta.argmax() if order == "max" else delta.argmin()   # the first extremum: the lowest index
+                pick_d = greedy_pick(full, kdiv, chosen, order)
                 if mine:
                     live_left = live.to(torch.int64).sum() - (live.to(torch.int64) * (rows == pick_d)[:, None]).sum()
             union = torch.maximum(union, regs.index_select(0, pick_d.view(1))[0])
@@ -726,6 +732,69 @@ class GpuSketchStore:
                 stats["switch_step"] = t + 1
         self.stats["union_launches"] += steps
         return np.asarray(picks, dtype=np.int64), cards.cpu().numpy(), stats
+
+    def exact_greedy_order(self, fastas: Sequence[str], ks: Sequence[int], canon: bool, steps: int, order: str = "max",
+                           first=(), shard: Optional[Tuple[int, int]] = None):
+        """The greedy ordering of greedy_order by exact counts: step t adds the FASTA whose union with the ones chosen
+        so far has the largest (order="max") or smallest ("min") delta = max_k |U u g|_k / k, the lowest index winning
+        a tie; `first` takes the first steps as given.  Returns (order int64 [steps], cards int64 [steps, nk] of U
+        after each step, stats {"index_bytes": per k, "distinct_keys": per k, |union of all FASTAs|}).
+
+        A cover index per k (Engine.exact_cover_index, K12) is built first and held on the device for the call:
+        |U u g| = |U| + |A_g| - lost[g], lost[g] = |A_g n U|.  Every step computes the [n, nk] candidate counts on the
+        device, picks, reads the pick (the one device->host read) and runs one K12 step over every k, which adds the
+        keys the pick covers to lost.  shard=(rank, world): this rank's key range; one all_reduce(SUM) of the
+        candidate counts per step adds the ranks' shares (every key belongs to one rank, so |U|, |A_g| and lost[g] all
+        add), and every rank makes the same pick."""
+        if not hasattr(self.engine, "exact_cover_index"):
+            raise RuntimeError("the exact greedy ordering needs an engine with the K12 cover index (Engine.exact_cover_index)")
+        from dandd_b200 import dist as dd_dist
+        n, ks = len(fastas), [int(k) for k in ks]
+        first = [int(g) for g in first]
+        assert order in ("max", "min") and len(first) <= steps <= n and len(set(first)) == len(first)
+        world = shard[1] if shard is not None else 1
+        dev = self.engine.device
+        seqs = [self.packed(f) for f in fastas]
+        indices, held = [], 0
+        try:
+            with timing.span("exact_cover_index"):
+                for k in ks:
+                    try:
+                        ix = self.engine.exact_cover_index(seqs, k, bool(canon), shard=shard)
+                    except torch.OutOfMemoryError as err:
+                        raise RuntimeError("the exact greedy index does not fit the device: out of memory at k=%d with %d "
+                                           "bytes of index held for the k before it; use fewer k or more ranks"
+                                           % (k, held)) from err
+                    indices.append(ix)
+                    held += ix["bytes"]
+                    self.stats["exact_calls"] += 1
+            kdiv = torch.as_tensor(np.asarray(ks, dtype=np.float64), device=dev)
+            singles = torch.as_tensor(np.stack([ix["singles"].astype(np.int64) for ix in indices], axis=1), device=dev)
+            lost = torch.zeros((len(ks), n), dtype=torch.int64, device=dev)
+            union = torch.zeros(len(ks), dtype=torch.int64, device=dev)
+            cards = torch.empty((steps, len(ks)), dtype=torch.int64, device=dev)
+            chosen = torch.zeros(n, dtype=torch.bool, device=dev)
+            picks = []
+            for t in range(steps):
+                mine = union + singles - lost.T                      # [n, nk]: this rank's share of |U u g|
+                full = dd_dist.sum_counts(mine.clone()) if world > 1 else mine
+                if t < len(first):
+                    pick_d = torch.tensor(first[t], device=dev)
+                else:
+                    pick_d = greedy_pick(full.to(torch.float64), kdiv, chosen, order)
+                cards[t] = full.index_select(0, pick_d.view(1))[0]
+                union = mine.index_select(0, pick_d.view(1))[0]
+                chosen.index_fill_(0, pick_d.view(1), True)
+                picks.append(int(pick_d))                            # the one read
+                if t + 1 < steps:
+                    self.engine.exact_cover_step(indices, picks[-1], lost)
+            keys = torch.as_tensor(np.asarray([ix["keys"] for ix in indices], dtype=np.int64), device=dev)
+            if world > 1:
+                keys = dd_dist.sum_counts(keys)
+            stats = {"index_bytes": [int(ix["bytes"]) for ix in indices], "distinct_keys": keys.cpu().numpy().tolist()}
+            return np.asarray(picks, dtype=np.int64), cards.cpu().numpy(), stats
+        finally:
+            indices.clear()                                          # the index lives for this call only
 
     def exact_leave_out(self, fastas: Sequence[str], ks: Sequence[int], canon: bool, group, n_groups: int,
                         shard: Optional[Tuple[int, int]] = None) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:

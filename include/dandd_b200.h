@@ -402,6 +402,51 @@ DD_API int dd_exact_occupancy_hist(const void *d_ws, size_t ws_bytes, int k, uin
                                    dd_stream stream);
 
 /* ===========================================================================================
+ * K12  the exact greedy cover index (a chosen ordering for `progressive -r`, lib/huffman_dandd.py:618-663
+ * orderings_list, by exact counts: the greedy order where the reference would count one `kmc_tools complex` union
+ * per remaining candidate per step).  With A_g genome g's distinct keys and U the union of the genomes chosen so
+ * far, |U u A_g| = |U| + |A_g| - lost[g], lost[g] = |A_g n U|; when g* joins U, every key of A_g* not covered yet
+ * becomes covered and adds 1 to lost[h] of every genome h holding it.
+ * The index of one part (one k, one key-range pass) is built from the K7 sparse workspace after every genome has
+ * been inserted with dd_exact_pairs_insert_shard as genome g (same workspace, same arguments):
+ *   dd_exact_cover_count  writes d_counts [2] u64: the distinct keys of the workspace and its list nodes (one per
+ *                         (genome, key)), so the caller allocates the index exactly; all-ones for a full table or
+ *                         node array.
+ *   dd_exact_cover_emit   writes the index: d_offsets [n_keys + 1] u32, a key-major CSR over d_holders [n_nodes]
+ *                         u16 (the genomes holding each key), and d_key_of_node [n_nodes] u32 (the key id of every
+ *                         list node).  Genome g's nodes are the range between the node counter read before and
+ *                         after its insert (dd_exact_pairs_node_count): that range is g's key list.  d_status [2]
+ *                         u64 is written: (n_keys, n_nodes), or all-ones if the table or node array was full, the
+ *                         lists did not match the counts given, or a list holds a genome >= n_genomes -- never a
+ *                         partial index.  1 <= n_genomes <= 65535; n_keys < 2^32; n_nodes < 2^32 - 1.
+ *   dd_exact_cover_step   one launch over the n_parts parts (for example every (k, pass) of an ordering): for the
+ *                         picked genome's nodes [h_node_start[genome], h_node_start[genome + 1]) of each part it
+ *                         marks the keys not covered yet covered and adds 1 to d_lost[h] (u64, [n_genomes]) of every
+ *                         holder h of each of them.  h_parts is a HOST array, checked before any launch: pointers
+ *                         and alignment, 0 <= genome < n_genomes <= 65535, n_keys < 2^32, and node starts that do
+ *                         not decrease over the pick and fit n_nodes.  d_ws: n_parts * DD_COVER_PART_BYTES bytes,
+ *                         16-byte aligned (the descriptors are staged there).  d_covered [n_keys] u8 starts zeroed.
+ * =========================================================================================== */
+typedef struct dd_cover_part {
+    const uint32_t *d_offsets;      /* [n_keys + 1] */
+    const uint16_t *d_holders;      /* [n_nodes] */
+    const uint32_t *d_key_of_node;  /* [n_nodes] */
+    uint8_t *d_covered;             /* [n_keys] */
+    uint64_t *d_lost;               /* [n_genomes], added to */
+    uint64_t n_keys, n_nodes;
+    const uint64_t *h_node_start;   /* HOST [n_genomes + 1]: the node counter before each genome's insert, then after the last */
+} dd_cover_part;
+#define DD_COVER_PART_BYTES 64
+DD_API int dd_exact_cover_count(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                                uint32_t max_streams, uint64_t *d_counts, dd_stream stream);
+DD_API int dd_exact_cover_emit(void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                               uint32_t max_streams, int64_t n_genomes, uint64_t n_keys, uint64_t n_nodes,
+                               uint32_t *d_offsets, uint16_t *d_holders, uint32_t *d_key_of_node, uint64_t *d_status,
+                               dd_stream stream);
+DD_API int dd_exact_cover_step(const dd_cover_part *h_parts, int n_parts, int64_t n_genomes, int64_t genome,
+                               void *d_ws, size_t ws_bytes, dd_stream stream);
+
+/* ===========================================================================================
  * Host-buffer convenience path (what bench.py's e2e number times): one FASTA held in host memory
  * -> H2D copy -> K1 -> K2 -> K4 -> D2H of cardinalities (and registers if h_regs != NULL);
  * synchronises the stream before returning.  Equivalent to the reference running
