@@ -74,6 +74,7 @@ SIGNATURES = {
     "dd_exact_first_rank_hist": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _vp, _i64, _vp, _vp]),
     "dd_exact_pairs_node_count": (_i, [_vp, _sz, _vp, _vp]),
     "dd_exact_occupancy_hist": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _vp, _vp, _vp]),
+    "dd_exact_query_counts": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _i64, _vp, _vp, _vp, _vp]),
     "dd_exact_cover_count": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _vp, _vp]),
     "dd_exact_cover_emit": (_i, [_vp, _sz, _i, _u64, _u64, _u32, _i64, _u64, _u64, _vp, _vp, _vp, _vp, _vp]),
     "dd_exact_cover_step": (_i, [_vp, _i, _i64, _i64, _vp, _sz, _vp]),

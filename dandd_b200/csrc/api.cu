@@ -624,6 +624,27 @@ int dd_exact_occupancy_hist(const void *d_ws, size_t ws_bytes, int k, uint64_t c
             "dd_exact_occupancy_hist");
     return DD_OK;
 }
+// ---- K13 -----------------------------------------------------------------------------------------
+int dd_exact_query_counts(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams,
+                          int64_t n_refs, int64_t n_queries, uint64_t *d_inter, uint64_t *d_shared, uint64_t *d_union,
+                          dd_stream stream) {
+    const char *fn = "dd_exact_query_counts";
+    if (int rc = pairs_check(k, capacity, max_nodes, max_streams, d_ws, ws_bytes, fn)) return rc;
+    if (!d_inter || !d_shared || !d_union) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (n_refs < 1 || n_queries < 1) return fail(DD_ERR_ARG, "%s: n_refs=%lld n_queries=%lld, both must be >= 1", fn,
+                                                 (long long)n_refs, (long long)n_queries);
+    if (n_refs + n_queries > 0xFFFFFFFFll)   // genome indices are u32, 0xFFFFFFFF is the end of a list
+        return fail(DD_ERR_ARG, "%s: n_refs + n_queries=%lld above 4294967295", fn, (long long)(n_refs + n_queries));
+    if (n_refs * n_queries > DD_QUERY_MAX_CELLS)
+        return fail(DD_ERR_ARG, "%s: n_queries * n_refs=%lld above %lld cells", fn, (long long)(n_refs * n_queries),
+                    (long long)DD_QUERY_MAX_CELLS);
+    if (k > 64 && n_refs + n_queries > 65536)   // every genome is one stream of the k > 64 key references
+        return fail(DD_ERR_ARG, "%s: above k = 64 n_refs + n_queries=%lld above 65536", fn, (long long)(n_refs + n_queries));
+    DD_CUDA(dd::exact_query_counts(d_ws, k, capacity, max_streams, (uint32_t)n_refs, (uint32_t)n_queries, d_inter, d_shared,
+                                   d_union, sm_count_now(), S(stream)),
+            fn);
+    return DD_OK;
+}
 // ---- K12 -----------------------------------------------------------------------------------------
 static bool misaligned(const void *p, uintptr_t a) { return reinterpret_cast<uintptr_t>(p) & (a - 1); }
 int dd_exact_cover_count(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes, uint32_t max_streams,

@@ -708,6 +708,142 @@ cudaError_t exact_occupancy_hist(const void *d_ws, int k, uint64_t capacity, uns
     return cudaGetLastError();
 }
 
+// ---- K13: query genomes against a reference collection over the K7 lists -------------------------------
+// Genomes 0 .. R-1 are the references, R .. R+Q-1 the queries.  Per key: union_R += 1 if a reference holds it,
+// shared[q] += 1 for every query on such a list, inter[q][r] += 1 for every (query, reference) pair on it --
+// occ + q_on * r_on work per key where K7 pays occ(occ-1)/2.
+// The walk depends on the list order: PushGenome links every node at the list head, and genomes are inserted
+// one after another in id order, so every list is in DECREASING genome order -- its query nodes come before its
+// reference nodes.  A list whose head is a reference holds no query (one node load), and the references that
+// pair with a chunk of queries are those after the chunk's queries: one walk of the rest of the list per chunk.
+// Queries go in chunks of <= 32, one per lane, broadcast by shuffle while every lane owns one reference node,
+// so the lanes of a warp hit one counter row at distinct columns.  kSmem: the Q*R + Q counters fit in shared
+// memory (u32) and each CTA flushes them once; union_R is a per-lane register count, flushed once.
+template <bool kSmem>
+__global__ void __launch_bounds__(256)
+exact_query_kernel(const ExactWsHeader *__restrict__ hdr, const uint2 *__restrict__ lh, const PairNode *__restrict__ nodes,
+                   uint64_t n_slots, uint32_t n_refs, uint32_t n_queries, unsigned long long *inter,
+                   unsigned long long *shared, unsigned long long *union_r) {
+    extern __shared__ uint32_t sm_q[];
+    const uint64_t n_inter = (uint64_t)n_queries * n_refs;
+    if (hdr->overflow) {   // a full table or node array: the marker, never a count
+        for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_inter + n_queries + 1;
+             i += (uint64_t)gridDim.x * blockDim.x) {
+            if (i < n_inter) inter[i] = kEmptyKey;
+            else if (i < n_inter + n_queries) shared[i - n_inter] = kEmptyKey;
+            else *union_r = kEmptyKey;
+        }
+        return;
+    }
+    if (kSmem) {
+        for (uint64_t i = threadIdx.x; i < n_inter + n_queries; i += blockDim.x) sm_q[i] = 0;
+        __syncthreads();
+    }
+    const uint32_t n_all = n_refs + n_queries;
+    const unsigned lane = threadIdx.x & 31;
+    unsigned long long keys_r = 0;   // lane 0's union_R count
+    auto add_pair = [&](uint32_t q, uint32_t r) {   // q: a query index, r: a reference genome
+        const uint64_t c = (uint64_t)q * n_refs + r;
+        if (kSmem) atomicAdd(&sm_q[c], 1u);
+        else atomicAdd(&inter[c], 1ull);
+    };
+    // up to 32 nodes from `at`, lane j keeps the j-th genome (kNil past the chunk); returns the node after it
+    auto load = [&](uint32_t at, uint32_t &g) {
+        g = kNil;
+        for (unsigned i = 0; i < 32 && at != kNil; ++i) {
+            const PairNode nd = nodes[at];
+            if (lane == i) g = nd.genome;
+            at = nd.next;
+        }
+        return at;
+    };
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    for (uint64_t base = ((uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 32; base < n_slots; base += warps * 32) {
+        // 32 slots per coalesced load; the warp then walks the lists of the occupied ones one by one
+        const uint32_t head = base + lane < n_slots ? __ldg(&lh[base + lane].y) : kNil;
+        for (unsigned occ = __ballot_sync(0xffffffffu, head != kNil); occ; occ &= occ - 1) {
+            uint32_t at = __shfl_sync(0xffffffffu, head, __ffs(occ) - 1);
+            if (nodes[at].genome < n_refs) {   // a reference at the head: no query on this list
+                keys_r += lane == 0;
+                continue;
+            }
+            bool has_ref = false;
+            while (at != kNil) {
+                uint32_t gq;
+                const uint32_t after = load(at, gq);
+                const bool is_q = gq >= n_refs && gq < n_all, is_r = gq < n_refs;
+                const unsigned qm = __ballot_sync(0xffffffffu, is_q), rm = __ballot_sync(0xffffffffu, is_r);
+                if (qm) {
+                    // the references of this chunk (after its queries), then every later chunk
+                    bool own_r = is_r;
+                    uint32_t gr = gq, b_at = after;
+                    for (;;) {
+                        has_ref |= __any_sync(0xffffffffu, own_r);
+                        for (unsigned m = qm; m; m &= m - 1) {
+                            const uint32_t q = __shfl_sync(0xffffffffu, gq, __ffs(m) - 1) - n_refs;
+                            if (own_r) add_pair(q, gr);
+                        }
+                        if (b_at == kNil) break;
+                        b_at = load(b_at, gr);
+                        own_r = gr < n_refs;
+                    }
+                    if (has_ref && is_q) {
+                        if (kSmem) atomicAdd(&sm_q[n_inter + (gq - n_refs)], 1u);
+                        else atomicAdd(&shared[gq - n_refs], 1ull);
+                    }
+                }
+                if (rm) {   // references began in this chunk: no query follows (decreasing order)
+                    has_ref = true;
+                    break;
+                }
+                at = after;
+            }
+            keys_r += lane == 0 && has_ref;
+        }
+    }
+    if (keys_r) atomicAdd(union_r, keys_r);
+    if (kSmem) {
+        __syncthreads();
+        for (uint64_t i = threadIdx.x; i < n_inter + n_queries; i += blockDim.x) {
+            const uint32_t v = sm_q[i];
+            if (!v) continue;
+            if (i < n_inter) atomicAdd(&inter[i], (unsigned long long)v);
+            else atomicAdd(&shared[i - n_inter], (unsigned long long)v);
+        }
+    }
+}
+
+cudaError_t exact_query_counts(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint32_t n_refs,
+                               uint32_t n_queries, uint64_t *d_inter, uint64_t *d_shared, uint64_t *d_union, int sm_count,
+                               cudaStream_t stream) {
+    const uint8_t *ws = static_cast<const uint8_t *>(d_ws);
+    const ExactWsHeader *hdr = static_cast<const ExactWsHeader *>(d_ws);
+    const uint2 *lh = reinterpret_cast<const uint2 *>(ws + pairs_lh_offset(k, capacity, max_streams));
+    const PairNode *nodes = reinterpret_cast<const PairNode *>(ws + pairs_node_offset(k, capacity, max_streams));
+    auto *inter = reinterpret_cast<unsigned long long *>(d_inter);
+    auto *shared = reinterpret_cast<unsigned long long *>(d_shared);
+    auto *union_r = reinterpret_cast<unsigned long long *>(d_union);
+    const uint64_t n_slots = capacity + 1;
+    const size_t smem = ((size_t)n_queries * n_refs + n_queries) * sizeof(uint32_t);
+    if (smem <= kPairSmemBytes) {
+        if (smem > 48 * 1024) {
+            const cudaError_t e = cudaFuncSetAttribute(exact_query_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                       (int)kPairSmemBytes);
+            if (e != cudaSuccess) return e;
+        }
+        // few CTAs: every CTA pays one pass over the counters at the start and one at the end
+        const unsigned grid = (unsigned)(sm_count * 2);
+        DD_COUNT_LAUNCH(), exact_query_kernel<true><<<grid, 256, smem, stream>>>(hdr, lh, nodes, n_slots, n_refs, n_queries,
+                                                                                 inter, shared, union_r);
+    } else {
+        const uint64_t want = (n_slots + 255) / 256;   // one 32-slot group per warp
+        const unsigned grid = (unsigned)(want < (uint64_t)sm_count * 16 ? (want ? want : 1) : (uint64_t)sm_count * 16);
+        DD_COUNT_LAUNCH(), exact_query_kernel<false><<<grid, 256, 0, stream>>>(hdr, lh, nodes, n_slots, n_refs, n_queries,
+                                                                               inter, shared, union_r);
+    }
+    return cudaGetLastError();
+}
+
 // Dense path: popc(A & B) over K5 presence bitmaps.  A CTA owns a tile of 8 row genomes x 8 column
 // genomes and a slice of the bitmap words: each word range of the 16 bitmaps is read once per tile
 // (from L2 when other tiles have just read it) and feeds 64 pair counters.

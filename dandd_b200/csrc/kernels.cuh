@@ -132,6 +132,11 @@ cudaError_t exact_first_rank_hist(const void *d_ws, int k, uint64_t capacity, un
 // priv [n_genomes] or null (keys held by genome g alone)
 cudaError_t exact_occupancy_hist(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint64_t n_genomes,
                                  uint64_t *d_hist, uint64_t *d_priv, int sm_count, cudaStream_t stream);
+// ---- K13 (exact.cu): genomes 0..R-1 references, R..R+Q-1 queries on the K7 lists -> inter [Q][R], shared [Q]
+// (keys of q a reference holds), *d_union (keys some reference holds); added to
+cudaError_t exact_query_counts(const void *d_ws, int k, uint64_t capacity, unsigned max_streams, uint32_t n_refs,
+                               uint32_t n_queries, uint64_t *d_inter, uint64_t *d_shared, uint64_t *d_union, int sm_count,
+                               cudaStream_t stream);
 // the node counter of a K7 sparse workspace (ExactWsHeader::n_nodes) -> *d_out, a copy on the stream
 cudaError_t exact_pairs_node_count(const void *d_ws, uint64_t *d_out, cudaStream_t stream);
 // Dense: K5 bitmap workspaces, ws_stride bytes apart, for genomes row0.. and col0..

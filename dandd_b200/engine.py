@@ -671,6 +671,33 @@ class Engine:
                                       "exact k-mer table or node array overflowed; the length bounds understate the genomes")
         return got[:n], singles, got[n:]
 
+    # ---- K13 --------------------------------------------------------------------------------
+    def exact_query_counts(self, seqs: Sequence[PackedSeq], n_refs: int, k: int, canon: bool, shard: Optional[tuple] = None,
+                           passes: Optional[int] = None):
+        """(singles uint64 [R + Q], inter uint64 [Q, R], shared uint64 [Q], union_R int) in one job at k, where seqs[:n_refs]
+        are the R references and seqs[n_refs:] the Q queries: singles[g] = |A_g|, inter[q, r] = |A_q n A_r| (query q is
+        seqs[R + q]), shared[q] = |A_q n U_R| and union_R = |U_R|, U_R the union of the references (this rank's key range
+        under `shard`).  So |U_R u A_q| = union_R + |A_q| - shared[q].  Sized from the sequence lengths and with the
+        singles from the list-node counter, as exact_family_counts; one K7 list job, one K13 launch and one
+        device->host copy per pass."""
+        n, R = len(seqs), int(n_refs)
+        Q = n - R
+        if R < 1 or Q < 1:
+            raise DandDError("query counts need at least one reference and one query, got %d and %d" % (R, Q))
+        if k > 64 and n > 65536:
+            raise DandDError("query counts above k = 64 take at most 65536 genomes per job")
+        world = int(shard[1]) if shard is not None else 1
+        bounds = length_bounds([s.nsym for s in seqs], k, world)
+        cells = Q * R
+
+        def launch(ws, cap, nodes, part):      # cells [inter | shared | union_R]
+            check(self.lib.dd_exact_query_counts(ws.data_ptr(), ws.numel(), k, cap, nodes, n, R, Q, part, part + 8 * cells,
+                                                 part + 8 * (cells + Q), self.stream), "dd_exact_query_counts")
+
+        got, singles = self._list_job(seqs, k, canon, bounds, shard, passes, cells + Q + 1, True, launch,
+                                      "exact k-mer table or node array overflowed; the length bounds understate the genomes")
+        return singles, got[:cells].reshape(Q, R), got[cells:cells + Q], int(got[-1])
+
     # ---- K12 --------------------------------------------------------------------------------
     def exact_cover_index(self, seqs: Sequence[PackedSeq], k: int, canon: bool, shard: Optional[tuple] = None,
                           passes: Optional[int] = None) -> dict:

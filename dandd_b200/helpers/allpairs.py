@@ -133,13 +133,12 @@ class CardTable:
         d1, _, k1 = self._best(self.single)
         d12, _, k12 = self._best(self.pair)
         a, b = self.pairs[:, 0], self.pairs[:, 1]
-        return (d1[a] + d1[b] - d12) / d12, k1[a], k1[b], k12
+        return jaccard_of(d1[a], d1[b], d12), k1[a], k1[b], k12
 
     def j_values(self, target_k: int) -> np.ndarray:
         """J at one k per pair of self.pairs."""
         c = self.ks.index(target_k)
-        ab = self.pair[:, c]
-        return (self.single[self.pairs[:, 0], c] + self.single[self.pairs[:, 1], c] - ab) / ab
+        return jaccard_of(self.single[self.pairs[:, 0], c], self.single[self.pairs[:, 1], c], self.pair[:, c])
 
     def j_summary(self, target_k: int) -> List[tuple]:
         """j_summarize(self.results(), target_k)."""
@@ -267,6 +266,12 @@ def _gather_objects(obj, world):
 
 
 # ---------------------------------------------------------------- the reference's summaries, on tuple lists
+def jaccard_of(a, b, ab):
+    """(a + b - ab) / ab: the Jaccard index from the sizes of two sets and of their union; over deltas instead of
+    sizes, KIJ (helpers/allpairs.py:121-179).  Scalars or numpy arrays."""
+    return (a + b - ab) / ab
+
+
 def delta_summarize(results):
     """[(tool, name1, name2, k, card)] -> [(tool, name1, name2, delta, card, k)] sorted by the names:
     the largest card/k per (tool, name1, name2); the first k seen wins a tie (helpers/allpairs.py:103-118)."""
@@ -290,7 +295,7 @@ def kij_summarize(delta_summary):
     out = []
     for a, b in itertools.combinations(alone, 2):
         (da, ka), (db, kb), (dab, kab) = alone[a], alone[b], together[frozenset((a, b))]
-        out.append((tool, a, b, 0, (da + db - dab) / dab, ka, kb, kab))
+        out.append((tool, a, b, 0, jaccard_of(da, db, dab), ka, kb, kab))
     return out
 
 
@@ -308,8 +313,7 @@ def j_summarize(results, target_k):
             together[frozenset((name1, name2))] = card
     out = []
     for a, b in itertools.combinations(alone, 2):
-        ab = together[frozenset((a, b))]
-        out.append((tool, a, b, target_k, (alone[a] + alone[b] - ab) / ab, None, None, None))
+        out.append((tool, a, b, target_k, jaccard_of(alone[a], alone[b], together[frozenset((a, b))]), None, None, None))
     return out
 
 

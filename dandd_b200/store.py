@@ -826,6 +826,68 @@ class GpuSketchStore:
                 union[c] = hist[0, 0] + hist[0, 1]
         return union, without, singles
 
+    def exact_query_cards(self, ref_fastas: Sequence[str], query_fastas: Sequence[str], ks: Sequence[int], canon: bool,
+                          shard: Optional[Tuple[int, int]] = None):
+        """Exact counts of query FASTAs against a collection of reference FASTAs at every k, int64: (ref_single [nk, R],
+        query_single [nk, Q], union_R [nk] = |U_R|, with_q [nk, Q] = |U_R u A_q|, pair_union [nk, Q, R] = |A_q u A_r|),
+        U_R the union of the references.  One engine job per k (Engine.exact_query_counts: K7 lists + K13).
+        shard=(rank, world): this rank's key range only; the ranks' results add up.  There is no per-union fallback:
+        it would cost Q (R + 1) union counts per k."""
+        if not hasattr(self.engine, "exact_query_counts"):
+            raise RuntimeError("exact query counts need an engine with the query job (Engine.exact_query_counts)")
+        R, Q, ks = len(ref_fastas), len(query_fastas), [int(k) for k in ks]
+        seqs = [self.packed(f) for f in list(ref_fastas) + list(query_fastas)]
+        singles = np.zeros((len(ks), R + Q), dtype=np.int64)
+        union = np.zeros(len(ks), dtype=np.int64)
+        with_q = np.zeros((len(ks), Q), dtype=np.int64)
+        pair = np.zeros((len(ks), Q, R), dtype=np.int64)
+        for c, k in enumerate(ks):
+            self.stats["exact_calls"] += 1
+            s, inter, shared, union[c] = self.engine.exact_query_counts(seqs, R, k, bool(canon), shard=shard)
+            singles[c] = np.asarray(s, dtype=np.int64)
+            with_q[c] = union[c] + singles[c, R:] - np.asarray(shared, dtype=np.int64)
+            pair[c] = singles[c, R:, None] + singles[c, None, :R] - np.asarray(inter, dtype=np.int64)
+        return singles[:, :R].copy(), singles[:, R:].copy(), union, with_q, pair
+
+    def query_cards(self, regs: torch.Tensor, n_refs: int, p: int, shard: Optional[Tuple[int, int]] = None):
+        """HLL cardinalities of query_cards' quantities from regs [R + Q, nk, 2^p] (references first, then queries):
+        (ref_single [nk, R], query_single [nk, Q], union_R [nk], with_q [nk, Q], pair_union [nk, Q, R]) float64.  The
+        union of the references and its histogram come from K3 and K4; card(max(U_R, q)) for every query from one K11
+        dense step with the queries as candidates; the Q x R pair cards from pair_cards (K6).  The histograms are the
+        ones the per-union K3 path builds for the same members, so the estimates are the same floats.
+        shard=(rank, world): rank r takes the queries q = r (mod world), and one all_reduce(SUM) adds the ranks' rows
+        (a row no rank owns is 0.0; rank 0 gives the references' rows); every rank holds all of regs."""
+        from dandd_b200 import dist as dd_dist
+        n, nk = int(regs.shape[0]), int(regs.shape[1])
+        R = int(n_refs)
+        Q = n - R
+        rank, world = shard if shard is not None else (0, 1)
+        mine = [q for q in range(Q) if q % world == rank]
+        eng, dev = self.engine, regs.device
+        union = eng.union([regs[r] for r in range(R)])
+        ucards, uhist = eng.cards_hist(union, p)
+        singles = eng.cards(regs, p)
+        # [union_R | ref singles | query singles | with_q | pair cards], float64 [nk, 1 + R + 2Q + QR] on the device
+        out = torch.zeros((nk, 1 + R + 2 * Q + Q * R), dtype=torch.float64, device=dev)
+        if rank == 0:
+            out[:, 0] = ucards
+            out[:, 1:1 + R] = singles[:R].T
+        if mine:
+            rows = torch.as_tensor(np.asarray(mine, dtype=np.int64), device=dev)
+            out[:, 1 + R + rows] = singles[R + rows].T
+            hist, _ = eng.greedy_dense_hist(regs, union, uhist, [R + q for q in mine], p)
+            out[:, 1 + R + Q + rows] = eng.mle(hist, p).T
+            pairs = np.array([(r, R + q) for q in mine for r in range(R)], dtype=np.int64)
+            cells = np.array([q * R + r for q in mine for r in range(R)], dtype=np.int64)
+            got = torch.as_tensor(self.pair_cards(regs, pairs, p), device=dev)
+            out[:, 1 + R + 2 * Q + torch.as_tensor(cells, device=dev)] = got.T
+        self.stats["union_launches"] += 2
+        if world > 1:
+            out = dd_dist.sum_counts(out)
+        out = out.cpu().numpy()
+        return (out[:, 1:1 + R].copy(), out[:, 1 + R:1 + R + Q].copy(), out[:, 0].copy(), out[:, 1 + R + Q:1 + R + 2 * Q].copy(),
+                out[:, 1 + R + 2 * Q:].reshape(nk, Q, R).copy())
+
     def _exact_from_table(self, fastas, k, canon):
         tab = getattr(self, "exact_pair_table", None)
         if tab is None or tab["canon"] != bool(canon) or int(k) not in tab["col"] or not 1 <= len(fastas) <= 2:

@@ -402,6 +402,27 @@ DD_API int dd_exact_occupancy_hist(const void *d_ws, size_t ws_bytes, int k, uin
                                    dd_stream stream);
 
 /* ===========================================================================================
+ * K13  --exact query genomes against a reference collection at one k, from the K7 sparse workspace after the
+ * n_refs references have been inserted with dd_exact_pairs_insert_shard as genomes 0 .. n_refs-1 and then the
+ * n_queries queries as genomes n_refs .. n_refs+n_queries-1, in that order (same workspace, same arguments).
+ * With A_g genome g's distinct keys and U_R the union of the references, adds into caller-zeroed u64 arrays:
+ *   d_inter  [n_queries][n_refs]  inter[q][r] = |A_q n A_r|   (query q is genome n_refs + q)
+ *   d_shared [n_queries]          shared[q]   = |A_q n U_R|
+ *   d_union  [1]                  |U_R|
+ * With the singles |A_g| (the node counter, dd_exact_pairs_node_count): |U_R u A_q| = |U_R| + |A_q| - shared[q]
+ * and |A_q u A_r| = |A_q| + |A_r| - inter[q][r].  It stands in for the reference's `kmc_tools complex` union +
+ * `kmc_tools info` per query (the collection plus the query) and per (query, reference) pair.  The kernel relies
+ * on the insert order: every list holds its genomes in decreasing order, queries first.  Nodes of a genome
+ * index >= n_refs + n_queries are not counted.  n_refs >= 1, n_queries >= 1, n_refs + n_queries < 2^32 (at most
+ * 65536 above k = 64), n_queries * n_refs <= DD_QUERY_MAX_CELLS.  A full table or node array writes all-ones into
+ * every cell of d_inter, d_shared and d_union: never a partial count.
+ * =========================================================================================== */
+#define DD_QUERY_MAX_CELLS (1ll << 32)
+DD_API int dd_exact_query_counts(const void *d_ws, size_t ws_bytes, int k, uint64_t capacity, uint64_t max_nodes,
+                                 uint32_t max_streams, int64_t n_refs, int64_t n_queries, uint64_t *d_inter,
+                                 uint64_t *d_shared, uint64_t *d_union, dd_stream stream);
+
+/* ===========================================================================================
  * K12  the exact greedy cover index (a chosen ordering for `progressive -r`, lib/huffman_dandd.py:618-663
  * orderings_list, by exact counts: the greedy order where the reference would count one `kmc_tools complex` union
  * per remaining candidate per step).  With A_g genome g's distinct keys and U the union of the genomes chosen so
