@@ -93,6 +93,10 @@ int dd_set_option(const char *name, long value) {
         dd::g_prefix_planes = value != 0;
         return DD_OK;
     }
+    if (!strcmp(name, "prefix_lattice")) {
+        dd::g_prefix_lattice = value != 0;
+        return DD_OK;
+    }
     if (!strcmp(name, "polyt_sentinel")) {
         dd::g_polyt_sentinel = value != 0;
         return DD_OK;
@@ -327,11 +331,19 @@ int dd_prefix_union_card(const uint8_t *d_regs, const int32_t *d_order, int n_or
         return fail(DD_ERR_ARG, "dd_prefix_union_card: bad argument");
     const size_t rows = (size_t)n_ord * (final_only ? 1 : n_steps) * nk;
     if (rows > 0x7fffffff) return fail(DD_ERR_ARG, "dd_prefix_union_card: too many (ordering, step, k) rows");
-    if (!d_unions && d_ws && dd::g_prefix_planes && dd::planes_supported(p)) {
+    // pairs (two steps, final union only) never use the identical-prefix table: planes alone
+    const bool pairs_only = final_only && n_steps == 2;
+    if (!d_unions && d_ws && dd::g_prefix_lattice && !pairs_only && dd::lattice_supported(n_genomes, p)) {
         void *base = reinterpret_cast<void *>(align_up(reinterpret_cast<uintptr_t>(d_ws), 256));
         const size_t lost = (size_t)(static_cast<uint8_t *>(base) - static_cast<uint8_t *>(d_ws));
-        // pairs (two steps, final union only) never use the identical-prefix table: planes alone
-        const bool pairs_only = final_only && n_steps == 2;
+        const size_t need = dd::prefix_lattice_workspace_bytes(n_ord, n_steps, n_genomes, nk);
+        if (ws_bytes < lost + need)
+            return fail(DD_ERR_WORKSPACE, "dd_prefix_union_card: workspace %zu < %zu", ws_bytes, need + 256);
+        DD_CUDA(dd::prefix_union_hist_lattice(d_regs, d_order, n_ord, n_steps, n_genomes, nk, p, final_only, d_hist, base, S(stream)),
+                "dd_prefix_union_card(lattice)");
+    } else if (!d_unions && d_ws && dd::g_prefix_planes && dd::planes_supported(p)) {
+        void *base = reinterpret_cast<void *>(align_up(reinterpret_cast<uintptr_t>(d_ws), 256));
+        const size_t lost = (size_t)(static_cast<uint8_t *>(base) - static_cast<uint8_t *>(d_ws));
         const size_t need = dd::prefix_union_workspace_bytes(pairs_only ? 0 : n_ord, pairs_only ? 0 : n_steps, n_genomes, nk, p);
         if (ws_bytes < lost + need - 256)
             return fail(DD_ERR_WORKSPACE, "dd_prefix_union_card: workspace %zu < %zu", ws_bytes, need);

@@ -376,10 +376,13 @@ size_t planes_bytes(int64_t n_sketches, int p) { return (size_t)n_sketches * kPl
 static size_t dedup_bytes(int n_ord, int n_steps) {
     return (size_t)n_ord * n_steps * (sizeof(unsigned long long) + sizeof(int32_t));
 }
-// scratch of the register-input entry: [planes | identical-prefix masks | representatives]
+// scratch of the register-input entry: [planes | identical-prefix masks | representatives], or the subset
+// table of lattice.cu, whichever is larger where that path applies
 size_t prefix_union_workspace_bytes(int n_ord, int n_steps, int n_genomes, int nk, int p) {
     const size_t pl = (planes_bytes((int64_t)n_genomes * nk, p) + 255) / 256 * 256;
-    return pl + (dedup_bytes(n_ord, n_steps) + 255) / 256 * 256 + 256;
+    const size_t planes_path = pl + (dedup_bytes(n_ord, n_steps) + 255) / 256 * 256;
+    const size_t lattice_path = lattice_supported(n_genomes, p) ? prefix_lattice_workspace_bytes(n_ord, n_steps, n_genomes, nk) : 0;
+    return (planes_path > lattice_path ? planes_path : lattice_path) + 256;
 }
 
 cudaError_t to_planes(const uint8_t *d_regs, int64_t n_sketches, int p, uint32_t *d_planes, cudaStream_t stream) {

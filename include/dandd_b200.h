@@ -62,7 +62,9 @@ DD_API int dd_init(int device);
 /* Tuning knobs (never change results).  "sketch_k_per_pass" = n: K2 updates at most n k values per
  * kernel launch (0 = all in one), trading re-reads of the packed stream for L2 residency of the
  * accumulators.  "prefix_planes" = 0/1: dd_prefix_union_card uses the bit-sliced kernel (default 1)
- * or the byte kernel.  "sketch_midk" = 0/1: dd_sketch_update_sched lets pieces deep inside a long stream
+ * or the byte kernel.  "prefix_lattice" = 0/1: dd_prefix_union_card answers index-mode jobs of at most 12
+ * genomes from a per-k subset table built in one pass over the registers (default 1; for A/B measurement:
+ * 0 sends them to the bit-sliced kernel).  "sketch_midk" = 0/1: dd_sketch_update_sched lets pieces deep inside a long stream
  * consult L2-resident presence bitmaps for k = 10..12 before hashing (default 1).  "sketch_sink" = 0/1:
  * dd_sketch_update_sched sketches the k >= 10 of pieces before the first floor cut (p <= 20) with one k per
  * CTA, absorbing rank-1 updates in a shared-memory bitmap instead of L2 reductions (default 1; for A/B
@@ -202,8 +204,10 @@ DD_API int dd_union_sets_card(const uint8_t *const *d_members, int n_sets, int n
                               double *d_cards, uint32_t *d_hist, uint8_t *d_unions, dd_stream stream);
 DD_API int dd_union_max(const uint8_t *const *d_in, int n_in, size_t len, uint8_t *d_out, dd_stream stream);
 /* Scratch: (d_ws, ws_bytes) sized by dd_prefix_union_workspace_bytes() lets the call use the bit-plane
- * kernel (it holds the transposed sketches and the identical-prefix table); with d_ws == NULL, or when
- * d_unions != NULL, the byte kernel runs, which needs no scratch. */
+ * kernel (it holds the transposed sketches and the identical-prefix table) or, for n_genomes <= 12 and
+ * p >= 12 except pairs (final_only with two steps), the subset table ([nk][64][2^n_genomes] u32): every
+ * prefix union of every ordering is then read from one pass over the registers.  With d_ws == NULL, or
+ * when d_unions != NULL, the byte kernel runs, which needs no scratch. */
 DD_API size_t dd_prefix_union_workspace_bytes(int n_ord, int n_steps, int n_genomes, int nk, int p);
 DD_API int dd_prefix_union_card(const uint8_t *d_regs, const int32_t *d_order, int n_ord, int n_steps, int n_genomes,
                          int nk, int p, int final_only, double *d_cards, uint32_t *d_hist, uint8_t *d_unions,
