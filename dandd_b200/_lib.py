@@ -52,6 +52,7 @@ SIGNATURES = {
     "dd_sketch_end": (_i, [_vp, _sz, _i, _i, _vp, _vp, _vp, _vp]),
     "dd_card_ertl_mle": (_i, [_vp, _i, _i, _vp, _vp, _vp]),
     "dd_mle_from_hist": (_i, [_vp, _i, _i, _vp, _vp]),
+    "dd_mle_from_hist_f64": (_i, [_vp, _i, _i, _vp, _vp]),
     "dd_union_max": (_i, [_vp, _i, _sz, _vp, _vp]),
     "dd_prefix_union_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
     "dd_prefix_union_card": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
@@ -80,6 +81,8 @@ SIGNATURES = {
     "dd_exact_cover_step": (_i, [_vp, _i, _i64, _i64, _vp, _sz, _vp]),
     "dd_leave_out_workspace_bytes": (_sz, [_i, _i]),
     "dd_leave_out_hist": (_i, [_vp, _i, _i, _i, _vp, _i, _u64, _u64, _vp, _vp, _sz, _vp]),
+    "dd_register_spectrum_workspace_bytes": (_sz, [_i, _i]),
+    "dd_register_spectrum": (_i, [_vp, _i, _i, _i, _u64, _u64, _vp, _vp, _sz, _vp]),
     "dd_greedy_workspace_bytes": (_sz, [_i]),
     "dd_greedy_dense_hist": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _sz, _vp]),
     "dd_greedy_compact": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i64, _vp, _sz, _vp]),

@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdandd_b200.so")
-SOURCES = ["pack.cu", "sketch.cu", "card.cu", "planes.cu", "lattice.cu", "exact.cu", "leaveout.cu", "greedy.cu", "cover.cu", "api.cu"]
+SOURCES = ["pack.cu", "sketch.cu", "card.cu", "planes.cu", "lattice.cu", "exact.cu", "leaveout.cu", "greedy.cu", "cover.cu", "spectrum.cu", "api.cu"]
 HEADERS = ["common.cuh", "kernels.cuh", "hist.cuh", "swar.cuh", os.path.join("..", "..", "include", "dandd_b200.h")]
 NVCC_FLAGS = ["-std=c++17", "-O3", "-lineinfo", "-gencode", "arch=compute_100a,code=sm_100a",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"] + os.environ.get("DD_NVCC_EXTRA", "").split()

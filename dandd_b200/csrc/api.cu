@@ -293,6 +293,13 @@ int dd_mle_from_hist(const uint32_t *d_hist, int nsk, int p, double *d_cards, dd
     return DD_OK;
 }
 
+int dd_mle_from_hist_f64(const double *d_hist, int nsk, int p, double *d_cards, dd_stream stream) {
+    if (nsk == 0) return DD_OK;
+    if (!d_hist || !d_cards || nsk < 0 || bad_p(p)) return fail(DD_ERR_ARG, "dd_mle_from_hist_f64: bad argument");
+    DD_CUDA(dd::mle_from_hist_f64(d_hist, nsk, p, d_cards, S(stream)), "dd_mle_from_hist_f64");
+    return DD_OK;
+}
+
 int dd_union_max(const uint8_t *const *d_in, int n_in, size_t len, uint8_t *d_out, dd_stream stream) {
     if (!d_in || !d_out || n_in < 1) return fail(DD_ERR_ARG, "dd_union_max: bad argument");
     if ((reinterpret_cast<uintptr_t>(d_out) & 15) != 0) return fail(DD_ERR_ARG, "dd_union_max: output must be 16-byte aligned");
@@ -443,6 +450,33 @@ int dd_leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const
         if (group[g] < 0 || group[g] >= n_groups)
             return fail(DD_ERR_ARG, "%s: genome %d has group %d outside [0,%d)", fn, g, group[g], n_groups);
     DD_CUDA(dd::leave_out_hist(d_regs, n_genomes, nk, p, group.data(), n_groups, reg_begin, reg_end, d_hist, d_ws, S(stream)), fn);
+    return DD_OK;
+}
+
+// ---- K14 -----------------------------------------------------------------------------------------
+size_t dd_register_spectrum_workspace_bytes(int n_genomes, int nk) {
+    if (n_genomes < 1 || n_genomes > 65535 || nk < 1 || nk > 65535) return 0;
+    return dd::register_spectrum_workspace_bytes(n_genomes, nk);
+}
+int dd_register_spectrum(const uint8_t *d_regs, int n_genomes, int nk, int p, uint64_t reg_begin, uint64_t reg_end,
+                         uint32_t *d_spec, void *d_ws, size_t ws_bytes, dd_stream stream) {
+    const char *fn = "dd_register_spectrum";
+    if (!d_regs || !d_spec || !d_ws) return fail(DD_ERR_ARG, "%s: null pointer", fn);
+    if (bad_p(p)) return fail(DD_ERR_ARG, "%s: p=%d outside [5,26]", fn, p);
+    if (nk < 1 || nk > 65535) return fail(DD_ERR_ARG, "%s: nk=%d outside [1,65535]", fn, nk);
+    if (n_genomes < 1 || n_genomes > 65535)   // the value counters are u16
+        return fail(DD_ERR_ARG, "%s: n_genomes=%d outside [1,65535]", fn, n_genomes);
+    if ((int64_t)nk * DD_HIST_BINS * n_genomes > 0x7fffffffll)
+        return fail(DD_ERR_ARG, "%s: too many (k, value, count) cells: %d x 64 x %d", fn, nk, n_genomes);
+    if (reg_begin > reg_end || reg_end > ((uint64_t)1 << p) || (reg_begin & 15) || (reg_end & 15))
+        return fail(DD_ERR_ARG, "%s: register range [%llu,%llu) is not 16-aligned within [0,%llu]", fn,
+                    (unsigned long long)reg_begin, (unsigned long long)reg_end, (unsigned long long)1 << p);
+    if (reinterpret_cast<uintptr_t>(d_regs) & 15) return fail(DD_ERR_ARG, "%s: registers must be 16-byte aligned", fn);
+    if ((reinterpret_cast<uintptr_t>(d_ws) & 3) || (reinterpret_cast<uintptr_t>(d_spec) & 3))
+        return fail(DD_ERR_ARG, "%s: misaligned workspace or table", fn);
+    if (ws_bytes < dd::register_spectrum_workspace_bytes(n_genomes, nk))
+        return fail(DD_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, ws_bytes, dd::register_spectrum_workspace_bytes(n_genomes, nk));
+    DD_CUDA(dd::register_spectrum(d_regs, n_genomes, nk, p, reg_begin, reg_end, d_spec, d_ws, S(stream)), fn);
     return DD_OK;
 }
 

@@ -75,15 +75,18 @@ __device__ __forceinline__ double mle_h(double t) {
     }
     return 1.0 - t / expm1(t);
 }
-__device__ double ertl_mle_warp(uint32_t c_lo, uint32_t c_hi, int p, int lane) {
+// T = uint32_t: integer histograms; T = double: fractional ones (mean histograms, K14).  The arithmetic is the same
+// for both: every count is read as a double.
+template <typename T>
+__device__ double ertl_mle_warp(T c_lo, T c_hi, int p, int lane) {
     const unsigned full = 0xffffffffu;
     const int q = 64 - p;
     const double m = ldexp(1.0, p);
     auto count_at = [&](int j) { return __shfl_sync(full, j < 32 ? c_lo : c_hi, j & 31); };
     const double c0 = (double)count_at(0), ctop_reg = (double)count_at(q + 1);
     if (ctop_reg == m) return INFINITY;  // every register saturated
-    unsigned long long nz = (unsigned long long)__ballot_sync(full, c_lo != 0u) |
-                            ((unsigned long long)__ballot_sync(full, c_hi != 0u) << 32);
+    unsigned long long nz = (unsigned long long)__ballot_sync(full, c_lo != T(0)) |
+                            ((unsigned long long)__ballot_sync(full, c_hi != T(0)) << 32);
     if (q + 2 < 64) nz &= (1ull << (q + 2)) - 1ull;
     if (nz == 0ull) return nan("");      // not a histogram of 2^p registers
     const int lo = __ffsll((long long)nz) - 1, hi = 63 - __clzll((long long)nz);
@@ -117,12 +120,13 @@ __device__ double ertl_mle_warp(uint32_t c_lo, uint32_t c_hi, int p, int lane) {
 }
 
 constexpr int kMleWarps = 4;
+template <typename T>
 __global__ void __launch_bounds__(32 * kMleWarps)
-mle_kernel(const uint32_t *__restrict__ hist, int nsk, int p, double *__restrict__ cards) {
+mle_kernel(const T *__restrict__ hist, int nsk, int p, double *__restrict__ cards) {
     const int lane = threadIdx.x & 31;
     const int i = blockIdx.x * kMleWarps + (threadIdx.x >> 5);
     if (i >= nsk) return;  // whole warps leave together
-    const uint32_t *row = hist + (size_t)i * DD_HIST_BINS;
+    const T *row = hist + (size_t)i * DD_HIST_BINS;
     const double card = ertl_mle_warp(row[lane], row[lane + 32], p, lane);
     if (lane == 0) cards[i] = card;
 }
@@ -253,6 +257,12 @@ cudaError_t card_hist(const uint8_t *d_regs, int nsk, int p, uint32_t *d_hist, c
 }
 
 cudaError_t mle_from_hist(const uint32_t *d_hist, int nsk, int p, double *d_cards, cudaStream_t stream) {
+    if (nsk == 0) return cudaSuccess;
+    DD_COUNT_LAUNCH(), mle_kernel<<<(nsk + kMleWarps - 1) / kMleWarps, 32 * kMleWarps, 0, stream>>>(d_hist, nsk, p, d_cards);
+    return cudaGetLastError();
+}
+
+cudaError_t mle_from_hist_f64(const double *d_hist, int nsk, int p, double *d_cards, cudaStream_t stream) {
     if (nsk == 0) return cudaSuccess;
     DD_COUNT_LAUNCH(), mle_kernel<<<(nsk + kMleWarps - 1) / kMleWarps, 32 * kMleWarps, 0, stream>>>(d_hist, nsk, p, d_cards);
     return cudaGetLastError();

@@ -54,6 +54,8 @@ cudaError_t sketch_end(void *d_ws, int nk, int p, uint8_t *d_regs, uint32_t *d_h
 // ---- K3 / K4 / K6 (card.cu)
 cudaError_t card_hist(const uint8_t *d_regs, int nsk, int p, uint32_t *d_hist, cudaStream_t stream);
 cudaError_t mle_from_hist(const uint32_t *d_hist, int nsk, int p, double *d_cards, cudaStream_t stream);
+// the same estimator on fractional counts (mean histograms); on integer counts the same floats as mle_from_hist
+cudaError_t mle_from_hist_f64(const double *d_hist, int nsk, int p, double *d_cards, cudaStream_t stream);
 cudaError_t union_max(const uint8_t *const *d_in, int n_in, size_t len, uint8_t *d_out, cudaStream_t stream);
 cudaError_t prefix_union_hist(const uint8_t *d_regs, const int32_t *d_order, int n_ord, int n_steps, int n_genomes,
                               int nk, int p, int final_only, uint32_t *d_hist, uint8_t *d_unions,
@@ -85,6 +87,13 @@ cudaError_t union_sets_hist(const uint8_t *const *d_members, int n_sets, int n_s
 size_t leave_out_workspace_bytes(int n_genomes, int nk);
 cudaError_t leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const int32_t *h_group, int n_groups,
                            uint64_t reg_begin, uint64_t reg_end, uint32_t *d_hist, void *d_ws, cudaStream_t stream);
+
+// ---- K14 (spectrum.cu): register sharing spectrum, regs [n][nk][2^p] -> spec [nk][64][n] u32 (added to); entry
+// (k, v, c - 1) counts the registers of [reg_begin, reg_end) where exactly c genomes are >= v.  Workspace = the
+// difference table [nk][64][n] u32.
+size_t register_spectrum_workspace_bytes(int n_genomes, int nk);
+cudaError_t register_spectrum(const uint8_t *d_regs, int n_genomes, int nk, int p, uint64_t reg_begin, uint64_t reg_end,
+                              uint32_t *d_spec, void *d_ws, cudaStream_t stream);
 
 // ---- K11 (greedy.cu): hist(max(U, g)) for every listed candidate g, regs [n][nk][2^p], U [nk][2^p] ->
 // hist [C][nk][64] and live [C][nk] (written).  Workspace = the candidate list.  h_cand / h_seg_off: host copies,

@@ -225,6 +225,14 @@ class Engine:
         check(self.lib.dd_mle_from_hist(flat.data_ptr(), flat.shape[0], p, out.data_ptr(), self.stream), "dd_mle_from_hist")
         return out.view(hist.shape[:-1])
 
+    def mle_f64(self, hist: torch.Tensor, p: int) -> torch.Tensor:
+        """Ertl-MLE cardinalities from fractional register histograms [..., 64] (float64, device): the estimator of mle(),
+        on mean histograms.  On integer counts the floats are mle()'s."""
+        flat = hist.to(self.device, torch.float64).contiguous().view(-1, DD_HIST_BINS)
+        out = torch.empty(flat.shape[0], dtype=torch.float64, device=self.device)
+        check(self.lib.dd_mle_from_hist_f64(flat.data_ptr(), flat.shape[0], p, out.data_ptr(), self.stream), "dd_mle_from_hist_f64")
+        return out.view(hist.shape[:-1])
+
     def _update_from_state(self, seq, kmask, p, canon, ws, st):
         # the pack state says [prev_nsym, nsym); for a whole-stream sketch rewind prev_nsym to 0
         state = seq.state.clone()
@@ -416,6 +424,25 @@ class Engine:
         ws = self._buf(self.lib.dd_leave_out_workspace_bytes(n, nk), "leave_out")
         check(self.lib.dd_leave_out_hist(regs.data_ptr(), n, nk, p, d_group.data_ptr(), int(n_groups), int(begin), int(end),
                                          out.data_ptr(), ws.data_ptr(), ws.numel(), self.stream), "dd_leave_out_hist")
+        return out
+
+    # ---- K14 --------------------------------------------------------------------------------
+    def register_spectrum(self, regs: torch.Tensor, p: int, reg_range: Optional[tuple] = None,
+                          out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The register sharing spectrum int32 [nk, 64, n] on the device of regs [n, nk, 2^p]: entry (k, v, c - 1) counts
+        the registers where exactly c genomes hold a value >= v (values clamped at 63; row v = 0 is 0).  One read of the
+        registers (K14).  reg_range=(begin, end): only those registers of every k (multiples of 16); tables of disjoint
+        ranges add up.  out: an int32 [nk, 64, n] tensor to ADD into (the counts are u32 in the kernel; they stay below
+        2^p <= 2^26)."""
+        n, nk, m = regs.shape
+        assert m == 1 << p and regs.is_contiguous() and regs.dtype == torch.uint8
+        begin, end = reg_range if reg_range is not None else (0, m)
+        if out is None:
+            out = torch.zeros((nk, DD_HIST_BINS, n), dtype=torch.int32, device=self.device)
+        assert out.is_contiguous() and out.dtype == torch.int32 and out.numel() == nk * DD_HIST_BINS * n
+        ws = self._buf(self.lib.dd_register_spectrum_workspace_bytes(n, nk), "register_spectrum")
+        check(self.lib.dd_register_spectrum(regs.data_ptr(), n, nk, p, int(begin), int(end), out.data_ptr(), ws.data_ptr(),
+                                            ws.numel(), self.stream), "dd_register_spectrum")
         return out
 
     # ---- K11 --------------------------------------------------------------------------------

@@ -50,6 +50,20 @@ def read_fasta_bytes(path: str) -> bytes:
     return ingest.fasta_bytes(path)
 
 
+def mean_prefix_hist(spec: torch.Tensor, p: int) -> torch.Tensor:
+    """float64 [nk, n, 64] on spec's device: row (k, m - 1) is the mean register histogram of the union of the first m
+    genomes over all n! orderings, from the register sharing spectrum spec [nk, 64, n] (Engine.register_spectrum).
+    cnt>=(v) = sum_c spec[k][v][c - 1] hit(c, m) as one float64 product, bin v = cnt>=(v) - cnt>=(v + 1) with
+    cnt>=(0) = 2^p.  A bin whose rounding falls below 0 is set to 0."""
+    from dandd_b200.helpers.spectrum import hit_weights
+    n = int(spec.shape[2])
+    w = torch.as_tensor(hit_weights(n), dtype=torch.float64, device=spec.device)     # [c, m]
+    ge = torch.matmul(spec.to(torch.float64), w)                                       # [nk, 64, m]
+    ge[:, 0, :] = float(1 << p)
+    hist = ge - torch.cat([ge[:, 1:, :], torch.zeros_like(ge[:, :1, :])], dim=1)
+    return hist.clamp_(min=0.0).transpose(1, 2).contiguous()
+
+
 class GpuSketchStore:
     def __init__(self, engine: Engine = None, prefetch_all_k: bool = True, cache_bytes: int = 64 << 30,
                  hll_compresslevel: int = None, union_files: str = None):
@@ -659,6 +673,28 @@ class GpuSketchStore:
             hist = dd_dist.sum_counts(hist)
         cards = self.engine.mle(hist, p).cpu().numpy().reshape(nk, 1 + int(n_groups))
         return cards[:, 0].copy(), cards[:, 1:].copy()
+
+    def register_spectrum_cards(self, regs: torch.Tensor, p: int,
+                                shard: Optional[Tuple[int, int]] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """The register sharing spectrum of regs [n, nk, 2^p] and the growth curve averaged over all n! orderings: (T int64
+        [nk, 64, n], cards float64 [nk, n]).  T[k][v][c - 1] counts the registers where exactly c genomes are >= v (K14,
+        one read of the registers).  cards[k][m - 1] is the Ertl MLE of the mean register histogram of the union of the
+        first m genomes over all orderings: cnt>=(v) = sum_c T[k][v][c] hit(c, m) (helpers/spectrum.py hit_weights) in
+        float64 on the device, a difference over v, then the MLE of the nk n rows.  It is not the mean of per-ordering
+        MLEs (max, MLE and mean do not commute).  m = n gives the union's histogram, so its card is the union's.
+        shard=(rank, world): this rank takes an equal slice of every k's register range and one all_reduce(SUM) adds the
+        tables of all ranks (every rank holds all of regs)."""
+        from dandd_b200 import dist as dd_dist
+        n, nk, m = (int(x) for x in regs.shape)
+        vec = m // 16
+        rank, world = shard if shard is not None else (0, 1)
+        span = (vec * rank // world * 16, vec * (rank + 1) // world * 16)
+        spec = self.engine.register_spectrum(regs, p, reg_range=span)
+        self.stats["union_launches"] += 1
+        if world > 1:
+            spec = dd_dist.sum_counts(spec)
+        cards = self.engine.mle_f64(mean_prefix_hist(spec, p), p).cpu().numpy().reshape(nk, n)
+        return spec.cpu().numpy().astype(np.int64), cards
 
     def greedy_order(self, regs: torch.Tensor, ks: Sequence[int], p: int, steps: int, order: str = "max", first=(),
                      shard: Optional[Tuple[int, int]] = None, budget: Optional[int] = None):

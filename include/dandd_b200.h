@@ -176,6 +176,9 @@ DD_API int dd_sketch_end(void *d_ws, size_t ws_bytes, int nk, int p, uint8_t *d_
 DD_API int dd_card_ertl_mle(const uint8_t *d_regs, int nsk, int p, double *d_cards, uint32_t *d_hist, dd_stream stream);
 /* Estimator alone, from histograms (host-callable building block; also used by K3/K6). */
 DD_API int dd_mle_from_hist(const uint32_t *d_hist, int nsk, int p, double *d_cards, dd_stream stream);
+/* The same estimator on fractional counts, d_hist [nsk][64] f64 (mean histograms: K14).  On integer counts it gives
+ * the floats dd_mle_from_hist gives. */
+DD_API int dd_mle_from_hist_f64(const double *d_hist, int nsk, int p, double *d_cards, dd_stream stream);
 
 /* ===========================================================================================
  * K3  unions.
@@ -260,6 +263,25 @@ DD_API size_t dd_leave_out_workspace_bytes(int n_genomes, int nk);
 DD_API int dd_leave_out_hist(const uint8_t *d_regs, int n_genomes, int nk, int p, const int32_t *d_group, int n_groups,
                              uint64_t reg_begin, uint64_t reg_end, uint32_t *d_hist, void *d_ws, size_t ws_bytes,
                              dd_stream stream);
+
+/* ===========================================================================================
+ * K14  register sharing spectrum (what `progressive -n N` samples from the orderings lib/huffman_dandd.py:618-663 climbs
+ * one union at a time, averaged over all n! orderings).  For register r and value v let c_v(r) = #{g : x_g(r) >= v};
+ * the union of a subset S has max >= v at r exactly when S meets those c_v(r) genomes, so the mean register histogram
+ * of the m-prefix union over all orderings follows from T[k][v][c] = #{r : c_v(r) = c} in closed form.  One read of
+ * the registers.
+ *   d_regs  [n_genomes][nk][2^p] u8 (the layout of dd_pairwise_union_card), 16-byte aligned; 1 <= n_genomes <= 65535
+ *   [reg_begin, reg_end) register range of every k, multiples of 16, reg_end <= 2^p
+ *   d_spec  [nk][64][n_genomes] u32, ADDED to (the caller zeroes it): entry (k, v, c - 1) = T[k][v][c] over the range;
+ *           row v = 0 stays 0.  Values are clamped at 63 as dd_card_ertl_mle's histogram clamps them, so row v sums to
+ *           the union's registers >= v.  Calls over disjoint register ranges, on one device or on several, add up.
+ *   d_ws    dd_register_spectrum_workspace_bytes(n_genomes, nk) bytes of scratch, 4-byte aligned
+ * nk * 64 * n_genomes < 2^31.  Every argument is checked before any launch.  Cardinalities: the mean histograms
+ * (helpers/spectrum.py hit_weights) through dd_mle_from_hist_f64.
+ * =========================================================================================== */
+DD_API size_t dd_register_spectrum_workspace_bytes(int n_genomes, int nk);
+DD_API int dd_register_spectrum(const uint8_t *d_regs, int n_genomes, int nk, int p, uint64_t reg_begin, uint64_t reg_end,
+                                uint32_t *d_spec, void *d_ws, size_t ws_bytes, dd_stream stream);
 
 /* ===========================================================================================
  * K11  one step of a greedy ordering (a chosen ordering for `progressive -r`, lib/huffman_dandd.py:618-663
