@@ -469,10 +469,7 @@ class DeltaTree:
             targets.append(paths)
         if not jobs:
             return                      # a cached re-run: nothing to compute, and the store (CUDA start-up) is never created
-        store = get_store()
-        if not hasattr(store, "union_many"):
-            return
-        results = store.union_many(jobs, int(self.experiment["registers"]))
+        results = get_store().union_many(jobs, int(self.experiment["registers"]))
         for (members, out_paths), cards in zip(jobs, results):
             for k, card in cards.items():
                 self.speciesinfo.cardkey[out_paths[k]] = card
@@ -530,7 +527,7 @@ class DeltaTree:
         if not todo:
             return                      # a cached re-run: nothing to compute, and the store (CUDA start-up) is never created
         store = get_store()
-        if not hasattr(store, "exact_union_cards") or not hasattr(getattr(store, "engine", None), "exact_first_rank_hist"):
+        if not hasattr(store, "exact_union_cards"):
             return
         ks = sorted(todo)
         canon = bool(self.experiment["canonicalize"])
@@ -901,8 +898,6 @@ class DeltaTree:
                     raise KeyError("this store has no batched exact pair job")     # -> the object path
                 return store.exact_pair_cards([leaf.fastas[0] for leaf in leaves], ks, bool(self.experiment["canonicalize"]),
                                               remember=True)[1]
-            if not hasattr(store, "pair_unions"):
-                raise KeyError("this store has no batched pair job")       # -> the object path, pair by pair
             return store.pair_unions({k: [leaf.ksketches[k].sketch for leaf in leaves] for k in ks}, registers)
         return _PairTable(ks, compute)
 

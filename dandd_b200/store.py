@@ -493,7 +493,7 @@ class GpuSketchStore:
         orderings) from one family job per k (Engine.exact_family_counts: K7 lists + one K8 launch, the singles from
         the list-node counter), run the first time any of them is asked for at that k and kept as a few integers per
         (row, k).  For a caller that knows WHICH sets it will count but not at which k (the exact hill-climb).
-        Another set, another `canon`, a k outside 1..256 or an engine without the job keep the per-union path."""
+        Another set, another `canon` or a k outside 1..256 keep the per-union path."""
         genomes = [str(f) for f in genomes]
         n = len(genomes)
         sets = [[int(g) for g in s] for s in sets]
@@ -518,8 +518,7 @@ class GpuSketchStore:
 
     def _exact_from_family(self, fastas, k, canon):
         fam = getattr(self, "exact_family_table", None)
-        if fam is None or fam["canon"] != bool(canon) or not 1 <= int(k) <= EXACT_MAX_K \
-                or not hasattr(self.engine, "exact_family_counts"):
+        if fam is None or fam["canon"] != bool(canon) or not 1 <= int(k) <= EXACT_MAX_K:
             return None
         cell = fam["cells"].get(frozenset(fastas))
         if cell is None:
@@ -554,27 +553,18 @@ class GpuSketchStore:
         """Exact counts of every FASTA and of the union of every pair, at every k: (singles [n, nk],
         unions [n(n-1)/2, nk]) float64, pairs (0,1), (0,2) .. (n-2,n-1).  One batched device job per k
         (K7: every genome read once per k, |A u B| = |A| + |B| - |A n B| in integers).  shard=(rank, world):
-        this rank's key range only; the ranks' results add up to the whole counts.  An engine without
-        the batched job answers pair by pair through exact_count.  With `remember`, later exact_count
-        calls for one or two of these FASTAs at these k are answered from the table."""
+        this rank's key range only; the ranks' results add up to the whole counts.  With `remember`, later
+        exact_count calls for one or two of these FASTAs at these k are answered from the table."""
         n, ks = len(fastas), [int(k) for k in ks]
         singles = np.zeros((n, len(ks)), dtype=np.int64)
         unions = np.zeros((n * (n - 1) // 2, len(ks)), dtype=np.int64)
-        batched = getattr(self.engine, "exact_pair_intersections", None)
-        if batched is None:
-            if shard is not None and shard[0] != 0:     # (the per-pair path counts whole sets: rank 0 holds them)
-                return singles.astype(np.float64), unions.astype(np.float64)
-            for c, k in enumerate(ks):
-                singles[:, c] = [self.exact_count([f], k, canon) for f in fastas]
-                unions[:, c] = [self.exact_count([fastas[a], fastas[b]], k, canon) for a, b in zip(*np.triu_indices(n, 1))]
-        else:
-            seqs = [self.packed(f) for f in fastas]
-            iu = np.triu_indices(n, 1)
-            for c, k in enumerate(ks):
-                self.stats["exact_calls"] += 1
-                singles[:, c] = [self.engine.exact_counts([s], k, canon, shard=shard)[0] for s in seqs]
-                inter = batched(seqs, k, canon, singles[:, c].tolist(), shard=shard).astype(np.int64)
-                unions[:, c] = singles[iu[0], c] + singles[iu[1], c] - inter
+        seqs = [self.packed(f) for f in fastas]
+        iu = np.triu_indices(n, 1)
+        for c, k in enumerate(ks):
+            self.stats["exact_calls"] += 1
+            singles[:, c] = [self.engine.exact_counts([s], k, canon, shard=shard)[0] for s in seqs]
+            inter = self.engine.exact_pair_intersections(seqs, k, canon, singles[:, c].tolist(), shard=shard).astype(np.int64)
+            unions[:, c] = singles[iu[0], c] + singles[iu[1], c] - inter
         if remember:
             self.exact_pair_table = {"n": n, "canon": bool(canon), "col": {k: c for c, k in enumerate(ks)},
                                      "row": {f: g for g, f in enumerate(fastas)}, "singles": singles, "unions": unions}
@@ -587,18 +577,9 @@ class GpuSketchStore:
         than n repeats its full union).  One batched device job per k (K7 lists + K8 first-rank histograms: every
         FASTA read once per k, whatever the number of orderings).  singles [n, nk]: exact counts of the single
         FASTAs if the caller has them on record (they size the job), else they are counted.  shard=(rank, world):
-        this rank's key range only.  An engine without the batched job counts ordering by ordering."""
+        this rank's key range only."""
         n, ks = len(fastas), [int(k) for k in ks]
         orderings = [[int(g) for g in o] for o in orderings]
-        out = np.zeros((len(orderings), n, len(ks)), dtype=np.int64)
-        if not hasattr(self.engine, "exact_first_rank_hist"):
-            for c, k in enumerate(ks):
-                for o, order in enumerate(orderings):
-                    if order:
-                        got = self.exact_prefix_counts([fastas[g] for g in order], k, canon)
-                        out[o, :len(got), c] = got
-                        out[o, len(got):, c] = got[-1]
-            return out
         ranks = np.full((len(orderings), n), 0xFFFF, dtype=np.uint16)
         for o, order in enumerate(orderings):
             ranks[o, order[::-1]] = np.arange(len(order), dtype=np.uint16)[::-1]   # a genome listed twice keeps its first place
@@ -608,13 +589,9 @@ class GpuSketchStore:
     def exact_union_cards(self, fastas: Sequence[str], sets, ks: Sequence[int], canon: bool,
                           shard: Optional[Tuple[int, int]] = None, singles=None) -> np.ndarray:
         """Exact count of the union of every set of FASTAs (sets: lists of indices into fastas) at every k:
-        int64 [n_sets, nk].  One batched device job per k, as exact_prefix_cards; an engine without it counts
-        set by set."""
+        int64 [n_sets, nk].  One batched device job per k, as exact_prefix_cards."""
         n, ks = len(fastas), [int(k) for k in ks]
         sets = [[int(g) for g in s] for s in sets]
-        if not hasattr(self.engine, "exact_first_rank_hist"):
-            return np.array([[self.exact_count([fastas[g] for g in s], k, canon) if s else 0 for k in ks] for s in sets],
-                            dtype=np.int64).reshape(len(sets), len(ks))
         ranks = np.full((len(sets), n), 0xFFFF, dtype=np.uint16)
         for r, members in enumerate(sets):
             ranks[r, members] = 0
@@ -645,8 +622,6 @@ class GpuSketchStore:
         fastas[g] holds.  One engine job per k (Engine.exact_spectrum: K7 lists + K9).  shard=(rank, world): this
         rank's key range only; the ranks' results add up.  There is no per-union fallback: the spectrum has no cheap
         equivalent in union counts."""
-        if not hasattr(self.engine, "exact_spectrum"):
-            raise RuntimeError("the exact sharing spectrum needs an engine with the spectrum job (Engine.exact_spectrum)")
         n, ks = len(fastas), [int(k) for k in ks]
         seqs = [self.packed(f) for f in fastas]
         out = np.zeros((3, len(ks), n), dtype=np.int64)
@@ -709,8 +684,6 @@ class GpuSketchStore:
         dense step's bytes, then one compaction and sparse steps over the live entries to the end; both give the
         same histograms.  shard=(rank, world): rank r evaluates the candidates g = r (mod world), one
         all_reduce(SUM) of the [n, nk] cards per step adds the ranks' rows, and every rank makes the same pick."""
-        if not hasattr(self.engine, "greedy_dense_hist"):
-            raise RuntimeError("the greedy ordering needs an engine with the K11 step (Engine.greedy_dense_hist)")
         from dandd_b200 import dist as dd_dist
         n, nk, m = (int(x) for x in regs.shape)
         first = [int(g) for g in first]
@@ -782,8 +755,6 @@ class GpuSketchStore:
         keys the pick covers to lost.  shard=(rank, world): this rank's key range; one all_reduce(SUM) of the
         candidate counts per step adds the ranks' shares (every key belongs to one rank, so |U|, |A_g| and lost[g] all
         add), and every rank makes the same pick."""
-        if not hasattr(self.engine, "exact_cover_index"):
-            raise RuntimeError("the exact greedy ordering needs an engine with the K12 cover index (Engine.exact_cover_index)")
         from dandd_b200 import dist as dd_dist
         n, ks = len(fastas), [int(k) for k in ks]
         first = [int(g) for g in first]
@@ -869,8 +840,6 @@ class GpuSketchStore:
         U_R the union of the references.  One engine job per k (Engine.exact_query_counts: K7 lists + K13).
         shard=(rank, world): this rank's key range only; the ranks' results add up.  There is no per-union fallback:
         it would cost Q (R + 1) union counts per k."""
-        if not hasattr(self.engine, "exact_query_counts"):
-            raise RuntimeError("exact query counts need an engine with the query job (Engine.exact_query_counts)")
         R, Q, ks = len(ref_fastas), len(query_fastas), [int(k) for k in ks]
         seqs = [self.packed(f) for f in list(ref_fastas) + list(query_fastas)]
         singles = np.zeros((len(ks), R + Q), dtype=np.int64)

@@ -1,7 +1,7 @@
 """Exact hill-climb unions from one family job per visited k, on the CPU: `tree --exact` and `progressive --exact`
-without --ksweep through the real store on an oracle-backed engine double that offers Engine.exact_family_counts,
-against the per-union path (DANDD_B200_EXACT_SET_BATCH=0) -- every file byte for byte, and the call accounting; the
-paths that keep counting union by union; a cached re-run; two gloo ranks; the family's lifetime; the ABI entry."""
+without --ksweep through the real store on the oracle-backed engine double, against the per-union path
+(DANDD_B200_EXACT_SET_BATCH=0) -- every file byte for byte, and the call accounting; the paths that keep counting union
+by union; a cached re-run; two gloo ranks; the family's lifetime; the ABI entry."""
 import os
 import pickle
 import random
@@ -10,12 +10,9 @@ import socket
 import pytest
 
 from dandd_b200 import store as ddstore
-from tests.fake_engine import ListJobEngine
+from tests.fake_engine import FakeEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-FamilyFakeEngine = ListJobEngine.only("exact_family_counts")
-NoFamilyEngine = ListJobEngine.only()           # the same double without the family job
 
 
 def _content(obj, path=()):
@@ -55,13 +52,13 @@ def _assert_same(a, b):
         assert a[key] == b[key], key
 
 
-def _run(tmp, argvs, batch, ngen=5, engine=FamilyFakeEngine, env=None):
+def _run(tmp, argvs, batch, ngen=5, env=None):
     """The dandd commands on a fresh dataset through the real store on the double; returns the files left behind,
     per command (store exact calls, per-union engine counts by genome count, family-job ks), and the store."""
     from tests.host_harness import run_dandd
     from tests.util import make_dataset
     make_dataset(os.path.join(tmp, "data"), ngen, 3000, seed=23)
-    st = ddstore.GpuSketchStore(engine=engine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     saved = {key: os.environ.get(key) for key in ["DANDD_B200_EXACT_SET_BATCH"] + list(env or {})}
     os.environ["DANDD_B200_EXACT_SET_BATCH"] = "1" if batch else "0"
@@ -155,14 +152,12 @@ def test_progressive_exact_hillclimb_equals_the_per_union_path(tmp_path, variant
         _check_accounting(on, off)
 
 
-@pytest.mark.parametrize("how", ["lowmem", "switch_off", "no_method"])
+@pytest.mark.parametrize("how", ["lowmem", "switch_off"])
 def test_per_union_path_kept(tmp_path, how):
-    """--lowmem, DANDD_B200_EXACT_SET_BATCH=0 and an engine without the family job count union by union, with the
-    same calls as the per-union path."""
+    """--lowmem and DANDD_B200_EXACT_SET_BATCH=0 count union by union, with the same calls as the per-union path."""
     argv = [TREE + ["-n", "2", "-k", "6"] + (["--lowmem"] if how == "lowmem" else []),
             PROG + ["-n", "2"] + (["--lowmem"] if how == "lowmem" else [])]
-    engine = NoFamilyEngine if how == "no_method" else FamilyFakeEngine
-    a, calls_a, _ = _run(str(tmp_path / "a"), argv, how != "switch_off", engine=engine)
+    a, calls_a, _ = _run(str(tmp_path / "a"), argv, how != "switch_off")
     b, calls_b, _ = _run(str(tmp_path / "b"), argv, False)
     _assert_same(a, b)
     for on, off in zip(calls_a, calls_b):
@@ -227,7 +222,7 @@ def test_store_family_counts(tmp_path):
     from tests.oracle_store import _read_fasta
     from tests.util import make_dataset
     fastas = make_dataset(str(tmp_path / "d"), 5, 2000, seed=4)
-    st = ddstore.GpuSketchStore(engine=FamilyFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     sets, orderings = [[0, 2], [1, 3, 4]], [[4, 1, 0, 3, 2], [2, 2, 0]]
     syms = [orc.fasta_symbols(_read_fasta(f)) for f in fastas]
     with st.exact_family(fastas, True, sets=sets, orderings=orderings):
@@ -254,7 +249,7 @@ def _tree_worker(rank, world, port, tmp):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
                       LOCAL_RANK=str(rank))
     from tests.host_harness import run_dandd
-    st = ddstore.GpuSketchStore(engine=FamilyFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     run_dandd([a.replace("<tmp>", tmp) for a in TREE + ["-n", "2", "-k", "6"]])
     with open(os.path.join(tmp, "family%d" % rank), "w") as fh:

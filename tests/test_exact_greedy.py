@@ -1,7 +1,8 @@
-"""Exact greedy ordering (`helpers/greedy.py --tool kmc`, K12) on the CPU: a numpy restatement of the cover index's
-emit and step, checked after every step of random orders against |A_h n U|; the store's loop on an engine double
-against a brute-force greedy over oracle k-mer sets; the command line end to end with the `dandd tree --exact` +
-`progressive --ksweep -r ordering.pickle` replay on the oracle store; refusals, two gloo ranks and the ABI entries."""
+"""Exact greedy ordering (`helpers/greedy.py --tool kmc`, K12) on the CPU: the numpy restatement of the cover index's
+emit and step (tests/fake_engine.py), checked after every step of random orders against |A_h n U|; the store's loop on the
+engine double against a brute-force greedy over oracle k-mer sets; the command line end to end with the `dandd tree
+--exact` + `progressive --ksweep -r ordering.pickle` replay on the oracle store; refusals, two gloo ranks and the ABI
+entries."""
 import os
 import pickle
 import re
@@ -12,45 +13,12 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import greedy
-from tests.fake_engine import ListJobEngine
+from tests.fake_engine import FakeEngine, emit_rule, kmer_keys, step_rule
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-# ---------------------------------------------------------------- numpy restatement of K12
-def emit_rule(held, rng):
-    """The index of one part from its holder matrix held bool [keys, n], as K7 + K12 build it: genomes push one node per
-    key they hold, one genome after another (in any order within a genome), and keys take ids in any order.
-    Returns {"offsets", "holders", "key_of_node", "node_start", "n_keys", "n_nodes"}."""
-    n_keys, n = held.shape
-    node_key, node_genome, node_start = [], [], [0]
-    for g in range(n):
-        keys = np.flatnonzero(held[:, g])
-        node_key += rng.permutation(keys).tolist()
-        node_genome += [g] * keys.size
-        node_start.append(len(node_key))
-    node_key, node_genome = np.asarray(node_key, dtype=np.int64), np.asarray(node_genome, dtype=np.int64)
-    slot_to_id = rng.permutation(n_keys)                     # the reservation order of the occupied slots
-    key_of_node = slot_to_id[node_key] if node_key.size else node_key
-    order = np.argsort(key_of_node, kind="stable")
-    counts = np.bincount(key_of_node, minlength=n_keys)
-    offsets = np.concatenate([[0], np.cumsum(counts)])
-    return {"offsets": offsets, "holders": node_genome[order], "key_of_node": key_of_node,
-            "node_start": np.asarray(node_start, dtype=np.int64), "n_keys": n_keys, "n_nodes": node_key.size,
-            "covered": np.zeros(n_keys, dtype=bool)}
-
-
-def step_rule(part, genome, lost):
-    """Genome `genome` joins the union: its keys not covered yet are covered, and each adds 1 to lost[h] of every holder h."""
-    for node in range(part["node_start"][genome], part["node_start"][genome + 1]):
-        key = part["key_of_node"][node]
-        if part["covered"][key]:
-            continue
-        part["covered"][key] = True
-        for h in part["holders"][part["offsets"][key]:part["offsets"][key + 1]]:
-            lost[h] += 1
-
-
+# ---------------------------------------------------------------- the numpy restatement of K12
 def _held_cases():
     rng = np.random.default_rng(5)
     out = []
@@ -86,30 +54,7 @@ def test_lost_is_the_overlap_with_the_union(held):
             assert lost.tolist() == (held & union[:, None]).sum(axis=0).tolist()
 
 
-# ---------------------------------------------------------------- the store's loop on an engine double
-class CoverFakeEngine(ListJobEngine):
-    """ListJobEngine plus Engine.exact_cover_index / exact_cover_step as the numpy restatement above, built from the
-    double's holder table (rank 0 holds every key); `passes` key-range parts per k."""
-    passes = 1
-
-    def exact_cover_index(self, seqs, k, canon, shard=None, passes=None):
-        self.calls["exact_cover_index"] = self.calls.get("exact_cover_index", 0) + 1
-        held = self._holders(seqs, k, canon)
-        if shard is not None and shard[0] != 0:
-            held = held[:0]
-        rng = np.random.default_rng(int(k))
-        parts = [emit_rule(held[np.arange(held.shape[0]) % self.passes == p], rng) for p in range(self.passes)]
-        return {"k": int(k), "n": len(seqs), "parts": parts, "singles": held.sum(axis=0).astype(np.uint64),
-                "keys": int(held.shape[0]), "bytes": int(6 * held.sum() + 5 * held.shape[0])}
-
-    def exact_cover_step(self, indices, genome, lost):
-        self.calls["exact_cover_step"] = self.calls.get("exact_cover_step", 0) + 1
-        view = lost.numpy()
-        for c, ix in enumerate(indices):
-            for part in ix["parts"]:
-                step_rule(part, genome, view[c])
-
-
+# ---------------------------------------------------------------- the store's loop on the engine double
 def _syms(fastas):
     from oracle import pyoracle as orc
     from tests.oracle_store import _read_fasta
@@ -118,8 +63,7 @@ def _syms(fastas):
 
 def brute_exact_greedy(fastas, ks, steps, order="max", first=(), canon=True):
     """(order, cards [steps, nk]) from explicit k-mer sets: the lowest index wins a tie."""
-    from oracle import pyoracle as orc
-    sets = [[set(orc.kmers(s, k, canon).tolist()) for k in ks] for s in _syms(fastas)]
+    sets = [[set(kmer_keys(s, k, canon).tolist()) for k in ks] for s in _syms(fastas)]
     union = [set() for _ in ks]
     picks, cards = [], []
     for t in range(steps):
@@ -157,7 +101,8 @@ def clustered(tmp_path_factory):
                                                ("max", (), 3)])
 def test_store_loop_equals_brute_force(clustered, order, first, steps, passes):
     ks = [3, 5, 8, 11]
-    eng = type("Passes", (CoverFakeEngine,), {"passes": passes})()
+    eng = FakeEngine()
+    eng.passes = passes
     st = ddstore.GpuSketchStore(engine=eng)
     got, cards, stats = st.exact_greedy_order(clustered, ks, True, steps, order=order, first=first)
     want, want_cards = brute_exact_greedy(clustered, ks, steps, order, first)
@@ -169,30 +114,24 @@ def test_store_loop_equals_brute_force(clustered, order, first, steps, passes):
         assert got.tolist().index(1) < got.tolist().index(6)     # the duplicate: the lower index first
 
 
-def test_store_refuses_an_engine_without_the_index(clustered):
-    st = ddstore.GpuSketchStore(engine=ListJobEngine())
-    with pytest.raises(RuntimeError, match="K12"):
-        st.exact_greedy_order(clustered[:2], [5], True, 2)
-
-
 def test_out_of_memory_names_the_k_and_the_bytes_held(clustered):
     import torch
 
-    class Full(CoverFakeEngine):
+    class Full(FakeEngine):
         def exact_cover_index(self, seqs, k, canon, shard=None, passes=None):
             if k == 8:
                 raise torch.OutOfMemoryError("CUDA out of memory")
             return super().exact_cover_index(seqs, k, canon, shard, passes)
 
     st = ddstore.GpuSketchStore(engine=Full())
-    held = sum(CoverFakeEngine().exact_cover_index([st.packed(f) for f in clustered], k, True)["bytes"] for k in (3, 5))
+    held = sum(FakeEngine().exact_cover_index([st.packed(f) for f in clustered], k, True)["bytes"] for k in (3, 5))
     with pytest.raises(RuntimeError, match=r"k=8 with %d bytes.*fewer k or more ranks" % held):
         st.exact_greedy_order(clustered, [3, 5, 8], True, 3)
 
 
 # ---------------------------------------------------------------- the command line
-def _run(argv, engine=CoverFakeEngine):
-    st = ddstore.GpuSketchStore(engine=engine())
+def _run(argv):
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         return greedy.go(argv), st

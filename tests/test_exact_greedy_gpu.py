@@ -9,7 +9,8 @@ import pickle
 import numpy as np
 import pytest
 
-from tests.test_exact_greedy import _read_tsv, emit_rule, step_rule
+from tests.fake_engine import emit_rule, step_rule
+from tests.test_exact_greedy import _read_tsv
 from tests.test_exact_pairs_gpu import _genomes
 from tests.test_exact_sets_gpu import _holders
 

@@ -1,6 +1,6 @@
-"""Exact all pairs (K7) on the CPU: the store's batched exact_pair_cards and `allpairs --tool kmc` against the
-per-pair path, with an oracle-backed engine double that offers the batched job, and the key-range pass
-planner of the sparse path."""
+"""Exact all pairs (K7) on the CPU: the store's batched exact_pair_cards on the oracle-backed engine double and
+`allpairs --tool kmc` against the per-pair path of the oracle store, and the key-range pass planner of the sparse
+path."""
 import os
 import socket
 
@@ -11,16 +11,15 @@ from dandd_b200 import engine as E
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import allpairs
 from tests import allpairs_cases as cases
-from tests.fake_engine import FakeEngine, ListJobEngine
-
-PairFakeEngine = ListJobEngine.only("exact_pair_intersections")
-
+from tests.fake_engine import FakeEngine
+from tests.oracle_store import OracleStore
 
 CASE = {"genomes": 5, "length": 2500, "seed": 31, "sub": 0.05, "klist": [9, 13, 21, 32], "nest": 4096, "extra": ""}
 
 
-def _run_allpairs(tmp, engine, case=CASE):
-    st = ddstore.GpuSketchStore(engine=engine)
+def _run_allpairs(tmp, st=None, case=CASE):
+    """`allpairs --tool kmc` through `st` (default: the real store on the engine double)."""
+    st = st or ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         _, dataset = cases.write_dataset(str(tmp), case)
@@ -36,9 +35,10 @@ def _run_allpairs(tmp, engine, case=CASE):
 
 
 def test_allpairs_kmc_files_equal_the_per_pair_path(tmp_path):
-    """The batched job writes the same bytes as one exact count per pair and k, in O(k) store calls."""
-    batched, st_b, files_b = _run_allpairs(tmp_path / "batched", PairFakeEngine())
-    per_pair, st_p, files_p = _run_allpairs(tmp_path / "per_pair", FakeEngine())
+    """The batched job writes the same bytes as one exact count per pair and k (the oracle store has no batched job), in
+    O(k) store calls."""
+    batched, st_b, files_b = _run_allpairs(tmp_path / "batched")
+    per_pair, st_p, files_p = _run_allpairs(tmp_path / "per_pair", OracleStore())
     assert files_b == files_p and len(files_b) == 2 + 2 * (1 + len(CASE["klist"]))
     assert np.array_equal(batched.single, per_pair.single) and np.array_equal(batched.pair, per_pair.pair)
     n, nk = CASE["genomes"], len(CASE["klist"])
@@ -48,7 +48,7 @@ def test_allpairs_kmc_files_equal_the_per_pair_path(tmp_path):
 
 
 def test_store_remembers_the_table(tmp_path):
-    eng = PairFakeEngine()
+    eng = FakeEngine()
     st = ddstore.GpuSketchStore(engine=eng)
     inputs = cases.make_dataset(str(tmp_path), 4, 2000, seed=5, sub=0.1)
     single, union = st.exact_pair_cards(inputs, [11, 17], True, remember=True)
@@ -69,8 +69,8 @@ def _free_port():
 def _worker(rank, world, port, tmp):
     import torch.distributed as dist
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
-    table, st, _ = _run_allpairs(os.path.join(tmp, "r%d" % rank), PairFakeEngine())
-    single, union = ddstore.GpuSketchStore(engine=PairFakeEngine()).exact_pair_cards(
+    table, st, _ = _run_allpairs(os.path.join(tmp, "r%d" % rank))
+    single, union = ddstore.GpuSketchStore(engine=FakeEngine()).exact_pair_cards(
         cases.make_dataset(os.path.join(tmp, "r%d" % rank, "data"), CASE["genomes"], CASE["length"], seed=CASE["seed"],
                            sub=CASE["sub"]), CASE["klist"], True)
     assert np.array_equal(table.single, single) and np.array_equal(table.pair, union)   # the ranks' shards summed
@@ -85,7 +85,7 @@ def test_two_ranks(tmp_path):
     mp.spawn(_worker, args=(2, _free_port(), str(tmp_path)), nprocs=2, join=True)
     assert os.path.exists(tmp_path / "ok0") and os.path.exists(tmp_path / "ok1")
     assert open(tmp_path / "r0" / "card.tsv", "rb").read() == \
-        _run_allpairs(tmp_path / "one", PairFakeEngine())[2]["card.tsv"]
+        _run_allpairs(tmp_path / "one")[2]["card.tsv"]
 
 
 @pytest.mark.parametrize("passes,world", [(1, 1), (3, 1), (1, 4), (3, 2), (5, 3)])
@@ -126,7 +126,7 @@ def _kij_exact_run(tmp, table):
     import pickle
     from tests.host_harness import run_dandd
     from tests.util import make_dataset
-    st = ddstore.GpuSketchStore(engine=PairFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     data = make_dataset(os.path.join(tmp, "data"), 6, 4000, seed=17)
     out = os.path.join(tmp, "out")

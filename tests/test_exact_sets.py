@@ -1,7 +1,6 @@
 """Exact unions of many genome sets (K8) on the CPU: `progressive --exact` and `tree --exact --ksweep` through the
-real store on an oracle-backed engine double that offers the first-rank histogram job, against the per-union
-path (DANDD_B200_EXACT_SET_BATCH=0); the histogram -> prefix / set count arithmetic of the store; a cached re-run;
-two gloo ranks."""
+real store on the oracle-backed engine double, against the per-union path (DANDD_B200_EXACT_SET_BATCH=0); the
+histogram -> prefix / set count arithmetic of the store; a cached re-run; two gloo ranks."""
 import os
 import random
 import socket
@@ -10,10 +9,8 @@ import numpy as np
 import pytest
 
 from dandd_b200 import store as ddstore
-from tests.fake_engine import FakeEngine, ListJobEngine
-
-# the first-rank job alone: without the family job, a hill-climb's cells stay per union
-SetFakeEngine = ListJobEngine.only("exact_first_rank_hist")
+from tests.fake_engine import FakeEngine
+from tests.test_exact_climb import _check_accounting
 
 
 def _symbols_sets(fastas, k):
@@ -40,7 +37,7 @@ def test_histograms_give_prefix_and_set_counts(tmp_path):
     orderings = [list(rng.permutation(n)) for _ in range(4)] + [[3, 1], [n - 1, 0, 2], [2, 2, 4], []]
     sets = [sorted(rng.choice(n, int(rng.integers(1, n + 1)), replace=False).tolist()) for _ in range(6)] + [[n - 1], [0], []]
     ks = [5, 11, 21]
-    st = ddstore.GpuSketchStore(engine=SetFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     pre = st.exact_prefix_cards(fastas, orderings, ks, True)
     uni = st.exact_union_cards(fastas, sets, ks, True)
     assert pre.shape == (len(orderings), n, len(ks)) and uni.shape == (len(sets), len(ks))
@@ -53,10 +50,6 @@ def test_histograms_give_prefix_and_set_counts(tmp_path):
                 assert pre[o, i, c] == want, (o, i, k)
         for s, members in enumerate(sets):
             assert uni[s, c] == len(set().union(*[kset[g] for g in members])), (s, k)
-    # an engine without the batched job: the same numbers, counted union by union
-    plain = ddstore.GpuSketchStore(engine=FakeEngine())
-    assert np.array_equal(plain.exact_prefix_cards(fastas, orderings, ks, True), pre)
-    assert np.array_equal(plain.exact_union_cards(fastas, sets, ks, True), uni)
     # singles on record size the job (the double checks they are the exact leaf counts)
     singles = np.array([[len(s) for s in _symbols_sets(fastas, k)] for k in ks]).T
     assert np.array_equal(st.exact_union_cards(fastas, sets, ks, True, singles=singles), uni)
@@ -95,21 +88,23 @@ def _snapshot(root):
 
 
 def _run(tmp, argvs, batch):
-    """The dandd commands on a fresh dataset through the real store on SetFakeEngine; returns the files left behind
-    and the exact store calls of each command."""
+    """The dandd commands on a fresh dataset through the real store on FakeEngine; returns the files left behind,
+    per command (store exact calls, per-union engine counts by genome count, family-job ks), and the store."""
     from tests.host_harness import run_dandd
     from tests.util import make_dataset
     make_dataset(os.path.join(tmp, "data"), 5, 4000, seed=17)
-    st = ddstore.GpuSketchStore(engine=SetFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     os.environ["DANDD_B200_EXACT_SET_BATCH"] = "1" if batch else "0"
     calls = []
     try:
         for argv in argvs:
             random.seed(3)                    # the same orderings in both runs
-            before = st.stats["exact_calls"]
+            before = (st.stats["exact_calls"], len(st.engine.union_sizes), len(st.engine.family_ks))
             run_dandd([a.replace("<tmp>", tmp) for a in argv])
-            calls.append(st.stats["exact_calls"] - before)
+            calls.append({"exact_calls": st.stats["exact_calls"] - before[0],
+                          "unions": st.engine.union_sizes[before[1]:],
+                          "family_ks": st.engine.family_ks[before[2]:]})
     finally:
         os.environ.pop("DANDD_B200_EXACT_SET_BATCH", None)
         ddstore.set_store(None)
@@ -130,7 +125,8 @@ def _assert_same(a, b):
 @pytest.mark.parametrize("mode", ["ksweep", "hillclimb"])
 def test_progressive_exact_equals_the_per_union_path(tmp_path, mode):
     """`progressive --exact` (several orderings, --step 2) leaves every CSV, descriptor and pickle byte for byte as
-    the per-union path does; with a sweep the prefix unions cost one store call per k."""
+    the per-union path does; with a sweep the prefix unions cost one store call per k, without one the hill-climb's
+    cells one family job per k it visits."""
     tree = TREE + SWEEP
     prog = PROG + (SWEEP if mode == "ksweep" else ["-s", "hc"])
     a, calls_a, st = _run(str(tmp_path / "a"), [tree, prog], True)
@@ -139,9 +135,10 @@ def test_progressive_exact_equals_the_per_union_path(tmp_path, mode):
     assert any("/ngen4/" in f and f.endswith(".kmc_pre") for f in a)            # prefix descriptors were written
     if mode == "ksweep":
         # 3 orderings x prefixes {2, 4} of 5 genomes x 4 k on the per-union path, 4 with one job per k
-        assert calls_a[1] == 4 and calls_b[1] > 4 and st.engine.calls["exact_first_rank_hist"] == 4
+        assert calls_a[1]["exact_calls"] == 4 and calls_b[1]["exact_calls"] > 4 and st.engine.calls["exact_first_rank_hist"] == 4
     else:
-        assert calls_a == calls_b                                                  # cells found by the hill-climb stay per union
+        assert calls_a[0] == calls_b[0]                                            # the tree: a spider, per union
+        _check_accounting(calls_a[1], calls_b[1])
 
 
 @pytest.mark.parametrize("nchildren", ["2", "3"])
@@ -151,7 +148,7 @@ def test_tree_exact_ksweep_equals_the_per_union_path(tmp_path, nchildren):
     b, calls_b, _ = _run(str(tmp_path / "b"), [argv], False)
     _assert_same(a, b)
     assert st.engine.calls["exact_first_rank_hist"] == 4
-    assert calls_a[0] == 5 * 4 + 4 < calls_b[0]                               # leaves one by one, inner nodes one job per k
+    assert calls_a[0]["exact_calls"] == 5 * 4 + 4 < calls_b[0]["exact_calls"]     # leaves one by one, inner nodes one job per k
 
 
 def test_cached_rerun_never_creates_the_store(tmp_path):
@@ -185,7 +182,7 @@ def _tree_worker(rank, world, port, tmp):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
                       LOCAL_RANK=str(rank))
     from tests.host_harness import run_dandd
-    st = ddstore.GpuSketchStore(engine=SetFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     run_dandd([a.replace("<tmp>", tmp) for a in TREE + SWEEP + ["-n", "2"]])
     with open(os.path.join(tmp, "hist%d" % rank), "w") as fh:

@@ -1,7 +1,7 @@
 """The exact sharing spectrum and the all-orderings mean growth curve (dandd_b200/helpers/spectrum.py) on the CPU: the
 closed forms against brute force and exact rationals; `growth.tsv` against `dandd progressive --exact --ksweep` over
 all n! orderings through the real store; the integer identities of the spectrum; the command line's refusals and two
-gloo ranks; the ABI entry.  The store runs on an oracle-backed engine double that offers Engine.exact_spectrum."""
+gloo ranks; the ABI entry.  The store runs on the oracle-backed engine double."""
 import csv
 import itertools
 import math
@@ -17,11 +17,9 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import spectrum
-from tests.fake_engine import ListJobEngine
+from tests.fake_engine import FakeEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-SpectrumFakeEngine = ListJobEngine.only("exact_first_rank_hist", "exact_spectrum")
 
 
 def _read_tsv(path):
@@ -67,8 +65,8 @@ def test_delta_of_the_mean_curve_takes_the_first_k_on_a_tie():
 
 
 # ---------------------------------------------------------------- against progressive over all n! orderings
-def _spectrum_run(tmp, argv, engine=SpectrumFakeEngine):
-    st = ddstore.GpuSketchStore(engine=engine())
+def _spectrum_run(tmp, argv):
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         return spectrum.go(argv), st
@@ -91,7 +89,7 @@ def test_growth_equals_the_mean_over_all_orderings(tmp_path, ngen, canon):
     orderings = os.path.join(tmp, "all.pickle")
     with open(orderings, "wb") as fh:
         pickle.dump(set(itertools.permutations(range(ngen))), fh)
-    st = ddstore.GpuSketchStore(engine=SpectrumFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         random.seed(3)
@@ -139,7 +137,7 @@ def test_integer_identities(tmp_path, canon):
         dst.write(src.read())
     with open(os.path.join(data, "z_empty.fasta"), "wb") as fh:
         fh.write(b">nothing\nACGNNN\n")
-    st = ddstore.GpuSketchStore(engine=SpectrumFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     files = sorted(os.path.join(data, f) for f in os.listdir(data))
     ks = [1, 2, 5, 9, 14]
     hist, singles, priv = st.exact_spectrum(files, ks, canon)
@@ -158,14 +156,6 @@ def test_integer_identities(tmp_path, canon):
         copy = files.index(os.path.join(data, "h_copy.fasta"))
         assert priv[c, 0] == priv[c, copy] == 0
     assert singles[ks.index(5):, -1].tolist() == [0, 0, 0] and singles[0, -1] > 0     # "ACG": k-mers up to k = 3 only
-
-
-def test_store_refuses_an_engine_without_the_job(tmp_path):
-    from tests.util import make_dataset
-    files = make_dataset(str(tmp_path / "d"), 2, 500, seed=1)
-    st = ddstore.GpuSketchStore(engine=ListJobEngine.only("exact_first_rank_hist")())
-    with pytest.raises(RuntimeError, match="spectrum"):
-        st.exact_spectrum(files, [5], True)
 
 
 # ---------------------------------------------------------------- command line

@@ -1,7 +1,7 @@
-"""Greedy ordering (dandd_b200/helpers/greedy.py, K11) on the CPU: a numpy restatement of the dense correction rule,
-the compaction and the sparse filter against explicit bincount(max(U, g)); the store's greedy loop on an engine double
-against a brute-force greedy over oracle registers; the command line end to end (file formats, the `dandd
-progressive -r ordering.pickle --ksweep` replay on the oracle store, refusals, two gloo ranks); the ABI entries."""
+"""Greedy ordering (dandd_b200/helpers/greedy.py, K11) on the CPU: the numpy restatement of the dense correction rule,
+the compaction and the sparse filter (tests/fake_engine.py) against explicit bincount(max(U, g)); the store's greedy loop
+on the engine double against a brute-force greedy over oracle registers; the command line end to end (file formats, the
+`dandd progressive -r ordering.pickle --ksweep` replay on the oracle store, refusals, two gloo ranks); the ABI entries."""
 import csv
 import os
 import pickle
@@ -13,73 +13,12 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import greedy
-from tests.fake_engine import ListJobEngine
+from tests.fake_engine import FakeEngine, compact_rule, dense_rule, hist_of, sparse_rule
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BINS = 64
 
 
-# ---------------------------------------------------------------- numpy restatement of K11
-def hist_of(u):
-    """int64 [nk, 64] histograms of registers u [nk, m]."""
-    return np.stack([np.bincount(np.minimum(row, BINS - 1), minlength=BINS) for row in np.asarray(u).astype(np.int64)])
-
-
-def dense_rule(regs, union, uhist, cand):
-    """(hist [C, nk, 64], live [C, nk]): hist(U) plus -1 at U[j] and +1 at g[j] for every register where g > U."""
-    regs, union = np.asarray(regs).astype(np.int64), np.asarray(union).astype(np.int64)
-    nk = union.shape[0]
-    hist = np.zeros((len(cand), nk, BINS), dtype=np.int64)
-    live = np.zeros((len(cand), nk), dtype=np.int64)
-    for c, g in enumerate(cand):
-        for k in range(nk):
-            up = regs[g, k] > union[k]
-            hist[c, k] = uhist[k]
-            np.subtract.at(hist[c, k], union[k][up], 1)
-            np.add.at(hist[c, k], regs[g, k][up], 1)
-            live[c, k] = up.sum()
-    return hist, live
-
-
-def compact_rule(regs, union, cand, seg_off):
-    """The sparse state: entries `j << 6 | value` of every live register in segment g * nk + k, within capacity."""
-    regs, union = np.asarray(regs).astype(np.int64), np.asarray(union).astype(np.int64)
-    n, nk, _ = regs.shape
-    seg_off = np.asarray(seg_off, dtype=np.int64)
-    entries = np.zeros(int(seg_off[-1]), dtype=np.int64)
-    seg_len = np.zeros(n * nk, dtype=np.int64)
-    for g in cand:
-        for k in range(nk):
-            s = g * nk + k
-            j = np.nonzero(regs[g, k] > union[k])[0]
-            cap = seg_off[s + 1] - seg_off[s]
-            entries[seg_off[s]:seg_off[s] + min(cap, j.size)] = ((j << 6) | regs[g, k][j])[:cap]
-            seg_len[s] = j.size
-    return {"entries": entries, "seg_off": seg_off, "seg_len": seg_len, "nk": nk}
-
-
-def sparse_rule(state, union, uhist, cand):
-    """The sparse step: drop the entries with value <= U[k][j], keep the rest in place, count their pairs."""
-    union = np.asarray(union).astype(np.int64)
-    nk = state["nk"]
-    hist = np.zeros((len(cand), nk, BINS), dtype=np.int64)
-    live = np.zeros((len(cand), nk), dtype=np.int64)
-    for c, g in enumerate(cand):
-        for k in range(nk):
-            s = g * nk + k
-            off = state["seg_off"][s]
-            n_len = min(state["seg_len"][s], state["seg_off"][s + 1] - off)
-            seg = state["entries"][off:off + n_len]
-            v, j = seg & 63, seg >> 6
-            keep = v > union[k][j]
-            state["entries"][off:off + keep.sum()] = seg[keep]
-            state["seg_len"][s] = live[c, k] = keep.sum()
-            hist[c, k] = uhist[k]
-            np.subtract.at(hist[c, k], union[k][j[keep]], 1)
-            np.add.at(hist[c, k], v[keep], 1)
-    return hist, live
-
-
+# ---------------------------------------------------------------- the numpy restatement of K11
 def explicit(regs, union, cand):
     regs, union = np.asarray(regs), np.asarray(union)
     hist = np.stack([hist_of(np.maximum(union, regs[g])) for g in cand])
@@ -131,35 +70,7 @@ def test_sparse_rule_follows_union_updates():
     assert state["seg_len"][7 * nk:8 * nk].tolist() == [0] * nk      # genome 7 == genome 1: nothing left
 
 
-# ---------------------------------------------------------------- the store's loop on an engine double
-class GreedyFakeEngine(ListJobEngine):
-    """ListJobEngine plus the K11 methods as the numpy restatement above, and Engine.cards_hist."""
-
-    def cards_hist(self, regs, p):
-        import torch
-        h = torch.from_numpy(hist_of(regs.numpy().reshape(-1, 1 << p)).astype(np.int32))
-        return self.mle(h, p).view(regs.shape[:-1]), h.view(tuple(regs.shape[:-1]) + (BINS,))
-
-    def greedy_dense_hist(self, regs, union, union_hist, cand, p):
-        import torch
-        self.calls["greedy_dense"] = self.calls.get("greedy_dense", 0) + 1
-        h, live = dense_rule(regs.numpy(), union.numpy(), union_hist.numpy(), list(cand))
-        return torch.from_numpy(h.astype(np.int32)), torch.from_numpy(live.astype(np.int32))
-
-    def greedy_compact(self, regs, union, cand, seg_off, p):
-        self.calls["greedy_compact"] = self.calls.get("greedy_compact", 0) + 1
-        return compact_rule(regs.numpy(), union.numpy(), list(cand), seg_off)
-
-    def greedy_sparse_hist(self, state, union, union_hist, cand, p):
-        import torch
-        self.calls["greedy_sparse"] = self.calls.get("greedy_sparse", 0) + 1
-        h, live = sparse_rule(state, union.numpy(), union_hist.numpy(), list(cand))
-        return torch.from_numpy(h.astype(np.int32)), torch.from_numpy(live.astype(np.int32))
-
-    def _pairs_budget(self):
-        return 1 << 40
-
-
+# ---------------------------------------------------------------- the store's loop on the engine double
 def brute_greedy(regs, ks, p, steps, order="max", first=()):
     """(order, cards [steps, nk]) by explicit unions and the oracle's estimator; the lowest index wins a tie."""
     from oracle import pyoracle as orc
@@ -209,7 +120,7 @@ def clustered(tmp_path_factory):
 def test_store_loop_equals_brute_force(clustered, monkeypatch, mode, order, first, steps):
     import torch
     regs, ks, p = clustered
-    st = ddstore.GpuSketchStore(engine=GreedyFakeEngine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     if mode == "sparse":                                            # compact right after the first evaluated step
         monkeypatch.setattr(ddstore, "SPARSE_CROSS", 0)
     got, cards, stats = st.greedy_order(torch.from_numpy(regs), ks, p, steps, order=order, first=first,
@@ -227,16 +138,9 @@ def test_store_loop_equals_brute_force(clustered, monkeypatch, mode, order, firs
         assert got.tolist().index(1) < got.tolist().index(6)     # the duplicate: the lower index first
 
 
-def test_store_refuses_an_engine_without_the_step():
-    import torch
-    st = ddstore.GpuSketchStore(engine=ListJobEngine())
-    with pytest.raises(RuntimeError, match="K11"):
-        st.greedy_order(torch.zeros((2, 1, 32), dtype=torch.uint8), [3], 5, 2)
-
-
 # ---------------------------------------------------------------- the command line
-def _run(argv, engine=GreedyFakeEngine):
-    st = ddstore.GpuSketchStore(engine=engine())
+def _run(argv):
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         return greedy.go(argv), st

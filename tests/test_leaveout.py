@@ -12,25 +12,9 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import leaveout
-from tests.fake_engine import ListJobEngine
+from tests.fake_engine import BINS, FakeEngine, brute_hist
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BINS = 64
-
-
-def brute_hist(regs, group, n_groups, begin=0, end=None):
-    """int64 [nk, 1 + G, 64]: row 0 the histogram of the union of all genomes, row 1 + g of the union of every genome
-    outside group g (explicit maxima; no genome left: all zeros), registers [begin, end) of every k."""
-    regs = np.asarray(regs)[:, :, begin:end]
-    group = np.asarray(group)
-    n, nk, m = regs.shape
-    out = np.zeros((nk, 1 + n_groups, BINS), dtype=np.int64)
-    for g in range(-1, n_groups):
-        keep = group != g
-        u = regs[keep].max(axis=0) if keep.any() else np.zeros((nk, m), dtype=np.uint8)
-        for c in range(nk):
-            out[c, 1 + g] = np.bincount(np.minimum(u[c], BINS - 1), minlength=BINS)
-    return out
 
 
 def streaming_hist(regs, group, n_groups, order=None):
@@ -57,18 +41,6 @@ def streaming_hist(regs, group, n_groups, order=None):
     return out
 
 
-class LeaveOutFakeEngine(ListJobEngine):
-    """ListJobEngine plus Engine.leave_out_hist (explicit maxima)."""
-
-    def leave_out_hist(self, regs, group, n_groups, p, reg_range=None, out=None):
-        import torch
-        self.calls["leave_out_hist"] = self.calls.get("leave_out_hist", 0) + 1
-        begin, end = reg_range if reg_range is not None else (0, 1 << p)
-        assert begin % 16 == 0 and end % 16 == 0
-        got = torch.from_numpy(brute_hist(regs.numpy(), group, n_groups, begin, end).astype(np.int32))
-        return got if out is None else out.add_(got)
-
-
 # ---------------------------------------------------------------- the streaming rule
 @pytest.mark.parametrize("case", ["ties", "duplicates", "zeros"])
 @pytest.mark.parametrize("n", [1, 2, 3, 7, 12])
@@ -92,8 +64,8 @@ def test_streaming_rule_equals_explicit_maxima(case, n):
 
 
 # ---------------------------------------------------------------- the command line
-def _run(argv, engine=LeaveOutFakeEngine):
-    st = ddstore.GpuSketchStore(engine=engine())
+def _run(argv):
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         return leaveout.go(argv), st
@@ -209,7 +181,7 @@ def test_kmc_contribution_equals_find_delta_delta(tmp_path):
     fastas = make_dataset(data, 4, 2500, seed=31)
     (union, without), _ = _run(["-d", data, "--tool", "kmc", "--mink", "2", "--maxk", "20", "--name", str(tmp_path / "run")])
     ks = list(range(2, 21))
-    st = ddstore.GpuSketchStore(engine=ListJobEngine.only("exact_family_counts")())    # as test_exact_climb climbs
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         run_dandd(["tree", "-d", data, "-s", "ex", "-o", str(tmp_path / "out"), "--exact"])

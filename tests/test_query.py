@@ -13,14 +13,14 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import query
-from tests.query_engine import QueryFakeEngine
+from tests.fake_engine import FakeEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 FILES = ("union.tsv", "collection.tsv", "with.tsv", "delta.tsv", "pairs.tsv", "kij.tsv")
 
 
-def _run(argv, engine=QueryFakeEngine):
-    st = ddstore.GpuSketchStore(engine=engine())
+def _run(argv):
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         return query.go(argv), st
@@ -225,13 +225,6 @@ def test_genome_count_limits(tmp_path, monkeypatch):
         _run(argv + ["--tool", "kmc", "--maxk", "65"])
     _run(argv + ["--tool", "kmc", "--mink", "60", "--maxk", "64"])       # up to k = 64 the count is not limited
     assert query.MAX_CELLS == 1 << 32 == _header_define("DD_QUERY_MAX_CELLS")
-
-
-def test_store_refuses_an_engine_without_the_job():
-    from tests.fake_engine import FakeEngine
-    st = ddstore.GpuSketchStore(engine=FakeEngine())
-    with pytest.raises(RuntimeError, match="Engine.exact_query_counts"):
-        st.exact_query_cards(["a"], ["b"], [5], True)
 
 
 # ---------------------------------------------------------------- two ranks

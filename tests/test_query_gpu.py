@@ -147,11 +147,11 @@ def _tables(name):
 
 @pytest.mark.parametrize("tool", ["dashing", "kmc"])
 def test_helper_matches_the_cpu_double(tmp_path, tool):
-    """The helper on the real engine and on QueryFakeEngine: kmc files identical, dashing numbers within 1e-9."""
+    """The helper on the real engine and on FakeEngine: kmc files identical, dashing numbers within 1e-9."""
     import shutil
     from dandd_b200 import store as ddstore
     from dandd_b200.helpers import query
-    from tests.query_engine import QueryFakeEngine
+    from tests.fake_engine import FakeEngine
     from tests.util import make_dataset
     refs = make_dataset(str(tmp_path / "refs"), 4, 2500, seed=41, prefix="r")
     make_dataset(str(tmp_path / "queries"), 2, 2500, seed=41, sub=0.08, prefix="q")
@@ -159,7 +159,7 @@ def test_helper_matches_the_cpu_double(tmp_path, tool):
     argv = ["-d", str(tmp_path / "refs"), "-q", str(tmp_path / "queries"), "--tool", tool, "--mink", "4", "--maxk", "12",
             "--registers", "12"]
     runs = {}
-    for label, store in (("gpu", ddstore.GpuSketchStore()), ("cpu", ddstore.GpuSketchStore(engine=QueryFakeEngine()))):
+    for label, store in (("gpu", ddstore.GpuSketchStore()), ("cpu", ddstore.GpuSketchStore(engine=FakeEngine()))):
         ddstore.set_store(store)
         try:
             query.go(argv + ["--name", str(tmp_path / label)])

@@ -13,8 +13,7 @@ import pytest
 
 from dandd_b200 import store as ddstore
 from dandd_b200.helpers import spectrum
-from tests.fake_engine import ListJobEngine
-from tests.register_spectrum_engine import BINS, RegisterSpectrumFakeEngine, ertl_mle_float, spectrum_numpy
+from tests.fake_engine import BINS, FakeEngine, ertl_mle_float, spectrum_numpy
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -96,8 +95,8 @@ def test_mean_histogram_equals_the_average_over_every_subset(n):
 
 
 # ---------------------------------------------------------------- the command line
-def _run(argv, engine=RegisterSpectrumFakeEngine):
-    st = ddstore.GpuSketchStore(engine=engine())
+def _run(argv):
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     ddstore.set_store(st)
     try:
         return spectrum.go(argv), st
@@ -200,8 +199,7 @@ def test_kmc_takes_k_above_32_and_ignores_registers(tmp_path):
     from tests.util import make_dataset
     data = str(tmp_path / "data")
     make_dataset(data, 2, 800, seed=2)
-    engine = ListJobEngine.only("exact_spectrum")
-    _run(["-d", data, "--mink", "40", "--maxk", "41", "--registers", "4", "--name", str(tmp_path / "run")], engine=engine)
+    _run(["-d", data, "--mink", "40", "--maxk", "41", "--registers", "4", "--name", str(tmp_path / "run")])
     assert sorted(os.listdir(str(tmp_path / "run"))) == ["delta.tsv", "genomes.tsv", "growth.tsv", "spectrum.tsv"]
 
 
@@ -209,13 +207,12 @@ def test_default_tool_is_the_exact_one(tmp_path):
     from tests.util import make_dataset
     data = str(tmp_path / "data")
     fastas = make_dataset(data, 4, 1500, seed=6)
-    engine = ListJobEngine.only("exact_spectrum")
     common = ["-d", data, "--mink", "3", "--maxk", "8", "--no-canon"]
     plain, kmc, direct = str(tmp_path / "plain"), str(tmp_path / "kmc"), str(tmp_path / "direct")
-    _run(common + ["--name", plain], engine=engine)
-    _run(common + ["--tool", "kmc", "--name", kmc], engine=engine)
+    _run(common + ["--name", plain])
+    _run(common + ["--tool", "kmc", "--name", kmc])
     os.makedirs(direct)
-    st = ddstore.GpuSketchStore(engine=engine())
+    st = ddstore.GpuSketchStore(engine=FakeEngine())
     hist, singles, priv = st.exact_spectrum(sorted(fastas), list(range(3, 9)), False)
     spectrum.write_outputs(direct, [os.path.basename(f) for f in sorted(fastas)], list(range(3, 9)), hist, singles, priv)
     for fn in ("spectrum.tsv", "genomes.tsv", "growth.tsv", "delta.tsv"):

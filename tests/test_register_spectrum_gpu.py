@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.register_spectrum_engine import ertl_mle_float
+from tests.fake_engine import ertl_mle_float
 
 pytestmark = pytest.mark.gpu
 BINS = 64
@@ -170,7 +170,7 @@ def test_command_line_on_the_engine(tmp_path):
     from dandd_b200.helpers import spectrum
     from oracle import pyoracle as orc
     from tests.oracle_store import _read_fasta
-    from tests.register_spectrum_engine import spectrum_numpy
+    from tests.fake_engine import spectrum_numpy
     from tests.util import make_dataset
     data = str(tmp_path / "data")
     n, p, lo, hi = 7, 14, 12, 18

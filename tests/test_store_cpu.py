@@ -140,6 +140,25 @@ def test_allpairs_exact(tmp_path, real_store):
         str(tmp_path), lambda fastas, k: orc.exact_count([orc.fasta_symbols(open(f, "rb").read()) for f in fastas], k, True))
 
 
+def test_engine_and_double_have_everything_the_store_reads():
+    """Every attribute the store reads off its engine (`self.engine.X`, `_store.engine.X`, `eng.X`) exists on Engine (a
+    class attribute or one its methods set on self) and on FakeEngine: the store calls the engine's jobs without probing
+    for them, and the CPU tests run the paths the device runs."""
+    import ast
+    import inspect
+    from dandd_b200.engine import Engine
+    used = {node.attr for node in ast.walk(ast.parse(inspect.getsource(ddstore))) if isinstance(node, ast.Attribute)
+            and (isinstance(node.value, ast.Attribute) and node.value.attr == "engine"
+                 or isinstance(node.value, ast.Name) and node.value.id == "eng")}
+    on_self = {node.attr for node in ast.walk(ast.parse(inspect.getsource(Engine)))
+               if isinstance(node, ast.Attribute) and isinstance(node.ctx, ast.Store) and isinstance(node.value, ast.Name)
+               and node.value.id == "self"}
+    assert {"exact_pair_intersections", "exact_family_counts", "greedy_dense_hist", "device"} <= used
+    assert sorted(a for a in used if not hasattr(Engine, a) and a not in on_self) == []
+    fake = FakeEngine()
+    assert sorted(a for a in used if not hasattr(fake, a)) == []
+
+
 # ---- the streaming branch of the store (files above STREAM_MIN_BYTES) on CPU doubles -----------------------
 class _OracleLib:
     """The slice of the C ABI that dandd_b200/streaming.py drives, answered by the oracle: the text given to
