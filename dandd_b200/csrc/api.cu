@@ -343,7 +343,7 @@ int dd_prefix_union_card(const uint8_t *d_regs, const int32_t *d_order, int n_or
     if (!d_unions && d_ws && dd::g_prefix_lattice && !pairs_only && dd::lattice_supported(n_genomes, p)) {
         void *base = reinterpret_cast<void *>(align_up(reinterpret_cast<uintptr_t>(d_ws), 256));
         const size_t lost = (size_t)(static_cast<uint8_t *>(base) - static_cast<uint8_t *>(d_ws));
-        const size_t need = dd::prefix_lattice_workspace_bytes(n_ord, n_steps, n_genomes, nk);
+        const size_t need = dd::prefix_lattice_workspace_bytes(n_ord, n_steps, n_genomes, nk, p);
         if (ws_bytes < lost + need)
             return fail(DD_ERR_WORKSPACE, "dd_prefix_union_card: workspace %zu < %zu", ws_bytes, need + 256);
         DD_CUDA(dd::prefix_union_hist_lattice(d_regs, d_order, n_ord, n_steps, n_genomes, nk, p, final_only, d_hist, base, S(stream)),

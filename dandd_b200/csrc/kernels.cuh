@@ -73,9 +73,10 @@ cudaError_t prefix_union_hist_planes(const uint8_t *d_regs, const int32_t *d_ord
                                      int nk, int p, int final_only, uint32_t *d_hist, void *d_ws, cudaStream_t stream);
 extern int g_prefix_planes;  // tuning knob: 1 = use the bit-plane kernel where it applies (default)
 // lattice.cu: the same contract for index-mode jobs of n_genomes <= 12, one pass over the registers whatever the
-// number of orderings.  Workspace = [difference table [nk][64][2^n] u32 | set of every (ordering, step)]
+// number of orderings.  Workspace = [subset table [nk][64][2^n] u32 | one slab [V][2^n] u32 per level-pass CTA |
+// set of every (ordering, step)]
 bool lattice_supported(int n_genomes, int p);
-size_t prefix_lattice_workspace_bytes(int n_ord, int n_steps, int n_genomes, int nk);
+size_t prefix_lattice_workspace_bytes(int n_ord, int n_steps, int n_genomes, int nk, int p);
 cudaError_t prefix_union_hist_lattice(const uint8_t *d_regs, const int32_t *d_order, int n_ord, int n_steps, int n_genomes,
                                       int nk, int p, int final_only, uint32_t *d_hist, void *d_ws, cudaStream_t stream);
 extern int g_prefix_lattice;  // A/B switch: 1 = use the subset table where it applies (default)

@@ -381,7 +381,7 @@ static size_t dedup_bytes(int n_ord, int n_steps) {
 size_t prefix_union_workspace_bytes(int n_ord, int n_steps, int n_genomes, int nk, int p) {
     const size_t pl = (planes_bytes((int64_t)n_genomes * nk, p) + 255) / 256 * 256;
     const size_t planes_path = pl + (dedup_bytes(n_ord, n_steps) + 255) / 256 * 256;
-    const size_t lattice_path = lattice_supported(n_genomes, p) ? prefix_lattice_workspace_bytes(n_ord, n_steps, n_genomes, nk) : 0;
+    const size_t lattice_path = lattice_supported(n_genomes, p) ? prefix_lattice_workspace_bytes(n_ord, n_steps, n_genomes, nk, p) : 0;
     return (planes_path > lattice_path ? planes_path : lattice_path) + 256;
 }
 
