@@ -24,15 +24,18 @@ cudaError_t pack_polyt_sentinel(const uint32_t *d_codes, uint32_t *d_invalid, co
                                 uint64_t sym_begin, uint64_t sym_end, size_t max_symbols, cudaStream_t stream);
 extern int g_polyt_sentinel;  // dd_set_option("polyt_sentinel"): the *_host entry points apply the pass
 
-// ---- K2 (sketch.cu).  Workspace = [SketchWsHeader | scratch | u16 accumulators [nk][2^p] | rank-1 sink bitmaps
-// [nk][2^p/32] u32 | mid-k presence bitmaps]; register = max(accumulator, sink bit)
+// ---- K2 (sketch.cu).  Workspace = [SketchWsHeader | scratch | u16 accumulators [nk][2^p] | slab-written flags |
+// mid-k presence bitmaps | rank-1 sink slabs, one 2^p-bit bitmap per sink CTA]; register = max(accumulator, OR of
+// its k's slabs)
 extern int g_k_per_pass;
 extern int g_midk;
 extern int g_sink;
 struct SketchWsHeader {
     uint8_t floor[32];  // floor[k-1] <= min(register of k): updates with rank <= floor are no-ops
     uint32_t use_floor;
-    uint32_t pad[7];
+    uint32_t sink_slices;  // slabs per k of the sink launches into this workspace (0: none ran)
+    uint32_t sink_first;   // table slot of their first k; the slabs of slot t start at (t - sink_first) x sink_slices
+    uint32_t pad[5];
 };
 size_t sketch_workspace_bytes(int nk, int p);
 cudaError_t sketch_begin(void *d_ws, int nk, int p, cudaStream_t stream);

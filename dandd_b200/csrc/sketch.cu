@@ -205,16 +205,28 @@ struct WordSpan {
     int j_lo, j_hi;
     bool all_valid;
 };
-__device__ __forceinline__ WordSpan load_word(const uint32_t *codes, const uint32_t *invalid, uint64_t w, bool in_range,
-                                              uint64_t sym_begin, uint64_t sym_end) {
+// the five loads behind code word w, apart from what is computed from them (so that they can be issued a tile early)
+struct RawWord {
+    uint32_t w0, w1, w2, i0, i1;
+};
+__device__ __forceinline__ RawWord load_raw(const uint32_t *codes, const uint32_t *invalid, uint64_t w, bool in_range) {
+    RawWord r;
+    r.w0 = in_range ? __ldg(codes + w) : 0u;
+    r.w1 = in_range && w >= 1 ? __ldg(codes + w - 1) : 0u;
+    r.w2 = in_range && w >= 2 ? __ldg(codes + w - 2) : 0u;
+    const uint64_t iw = w >> 1;
+    r.i0 = in_range ? __ldg(invalid + iw) : 0xffffffffu;
+    r.i1 = in_range && iw >= 1 ? __ldg(invalid + iw - 1) : 0xffffffffu;  // before the stream: breaks
+    return r;
+}
+__device__ __forceinline__ WordSpan span_of(const RawWord &r, uint64_t w, bool in_range, uint64_t sym_begin, uint64_t sym_end) {
     WordSpan s;
     const uint64_t s0 = w << 4;
-    s.w0 = in_range ? __ldg(codes + w) : 0u;
-    s.w1 = in_range && w >= 1 ? __ldg(codes + w - 1) : 0u;
-    s.w2 = in_range && w >= 2 ? __ldg(codes + w - 2) : 0u;
-    const uint64_t iw = w >> 1;
-    s.i0 = in_range ? __ldg(invalid + iw) : 0xffffffffu;
-    s.i1 = in_range && iw >= 1 ? __ldg(invalid + iw - 1) : 0xffffffffu;  // before the stream: breaks
+    s.w0 = r.w0;
+    s.w1 = r.w1;
+    s.w2 = r.w2;
+    s.i0 = r.i0;
+    s.i1 = r.i1;
     s.r0 = revcomp_word(s.w0);
     s.r1 = revcomp_word(s.w1);
     s.r2 = revcomp_word(s.w2);
@@ -223,6 +235,10 @@ __device__ __forceinline__ WordSpan load_word(const uint32_t *codes, const uint3
     s.j_hi = !in_range ? 0 : (sym_end - s0 < 16 ? (int)(sym_end - s0) : 16);
     s.sm_base = (uint32_t)(s0 & 31);
     return s;
+}
+__device__ __forceinline__ WordSpan load_word(const uint32_t *codes, const uint32_t *invalid, uint64_t w, bool in_range,
+                                              uint64_t sym_begin, uint64_t sym_end) {
+    return span_of(load_raw(codes, invalid, w, in_range), w, in_range, sym_begin, sym_end);
 }
 __device__ __forceinline__ Window span_window(const WordSpan &s, int j) { return window_at(s.w0, s.w1, s.w2, s.r0, s.r1, s.r2, j); }
 // valid symbols ending at symbol j of the word (0 outside the range)
@@ -388,38 +404,62 @@ __global__ void __launch_bounds__(kThreads, min_ctas_for(kThreads)) sketch_allk_
 // records is "some k-mer hit register r", one bit.  Before the floor schedule's first cut (floor 0)
 // every such update is a scattered L2 reduction -- the resource that bounds K2 on short genomes.  Here
 // a CTA owns one k over a contiguous slice of the stream and ORs its rank-1 updates into a 2^p-bit
-// bitmap in shared memory (128 KiB at p = 20); at the end only the non-zero words go to the
-// workspace's per-k sink bitmap with red.global.or.  Every such merge carries at least one rank-1
-// update, so the sink never issues more L2 reductions than the plain kernel.  The register is
-// max(acc, bit) -- finalize_kernel and floor_min_kernel read it so -- which keeps the result exact
-// under any floor (floor >= 1 drops rank 1 at the threshold already).  k <= 9 stays with the
-// presence-bitmap kernel.
+// bitmap in shared memory (128 KiB at p = 20); rank >= 2 goes to L2 as in the plain kernel.  At the end
+// the CTA stores its bitmap whole to its own slab of the workspace (no merge reductions), and a CTA of a
+// later launch into the same workspace starts from its slab.  The register is max(acc, OR of k's slabs)
+// -- finalize_kernel and floor_min_kernel read it so -- which keeps the result exact whichever kernel
+// sketched which piece.  k <= 9 stays with the presence-bitmap kernel.
+//
+// The sink only runs at floor 0 (sketch_update_sched), so it has no threshold or floor test.  A warp whose 32 words are all in range and hold no break runs its 16 symbols unrolled, with no
+// per-symbol validity test; the next tile's words are loaded before the current tile is hashed.
 constexpr int kSinkThreads = 1024, kSinkMinK = kBitmapMaxK + 1, kSinkMaxP = 20;
+// u32 words of one slab (the 2^p-bit bitmap, whole uint4s)
+__host__ __device__ constexpr uint32_t sink_slab_words(int p) { return ((1u << (p - 5)) + 3u) & ~3u; }
+
+// one (symbol, k) update at floor 0; acc_k = k's accumulator row, s_bits the bitmap's shared-window address.  The rank
+// is computed without a branch (clz(0) = 32, so the t == 0 case only adds the low word's clz).  The shared-memory OR
+// and the REDG each sit behind a short BSSY/BRA/BSYNC: ptxas wraps every predicated ATOMS or REDG so, even one
+// written as a PTX predicate.  Both are spelled out in PTX on a 32-bit register index, 3 SASS instructions per update
+// fewer than atomicOr and red_max_register on a 64-bit slot offset.
+template <int K, bool kCanon>
+__device__ __forceinline__ void sink_update(const Window &win, bool live, uint32_t s_bits, uint32_t *acc_k, int p) {
+    const uint64_t h = wang64_fma(kmer_of<K, kCanon>(win), ~0ull);
+    const uint32_t hi = (uint32_t)(h >> 32), lo = (uint32_t)h;
+    const uint32_t t = __funnelshift_l(lo, hi, (uint32_t)p);
+    const uint32_t r = hi >> (32 - p);
+    const uint32_t low = (uint32_t)__clz((int)((lo << p) | (1u << (p - 1))));
+    const uint32_t rank = (uint32_t)__clz((int)t) + 1u + (t == 0u ? low : 0u);
+    const bool one = (int32_t)t < 0;   // rank 1
+    if (live && one) asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(s_bits + ((r >> 3) & ~3u)), "r"(1u << (r & 31u)) : "memory");
+    if (live && !one) {
+        const uint32_t val = rank << ((hi >> (28 - p)) & 16u);   // register r's u16 half of word r / 2
+        asm volatile("{ .reg .b16 l, h; .reg .b64 a; mad.wide.u32 a, %1, 4, %0; mov.b32 {l, h}, %2; red.global.max.noftz.v2.f16 [a], {l, h}; }"
+                     ::"l"(acc_k), "r"(hi >> (33 - p)), "r"(val)
+                     : "memory");
+    }
+}
 
 template <int K, bool kCanon>
-__device__ __forceinline__ void sink_slice(const SketchArgs &a, const KConsts &kc, uint32_t *s_bits, uint32_t slot_off,
-                                           uint64_t sym_begin, uint64_t sym_end, uint64_t w_lo, uint64_t w_hi) {
-    const uint64_t minus_one = ~0ull;
+__device__ __forceinline__ void sink_slice(const SketchArgs &a, uint32_t s_bits, uint32_t *acc_k, uint64_t sym_begin,
+                                           uint64_t sym_end, uint64_t w_lo, uint64_t w_hi) {
     const int p = a.p;
+    RawWord next = load_raw(a.codes, a.invalid, w_lo + threadIdx.x, w_lo + threadIdx.x < w_hi);
 #pragma unroll 1
     for (uint64_t base = w_lo; base < w_hi; base += kSinkThreads) {
         const uint64_t w = base + threadIdx.x;
-        const WordSpan ws = load_word(a.codes, a.invalid, w, w < w_hi, sym_begin, sym_end);
+        const RawWord cur = next;
+        next = load_raw(a.codes, a.invalid, w + kSinkThreads, w + kSinkThreads < w_hi);
+        const WordSpan ws = span_of(cur, w, w < w_hi, sym_begin, sym_end);
+        const bool full = w < w_hi && ws.all_valid && ws.j_lo == 0 && ws.j_hi == 16;   // every symbol ends a valid 32-mer
+        if (__all_sync(0xffffffffu, full)) {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) sink_update<K, kCanon>(span_window(ws, j), true, s_bits, acc_k, p);
+        } else {
 #pragma unroll 1
-        for (int j = 0; j < 16; ++j) {
-            const bool live = span_run(ws, j) >= K;
-            if (!__any_sync(0xffffffffu, live)) continue;  // warp-uniform
-            const uint64_t h = wang64_fma(kmer_of<K, kCanon>(span_window(ws, j)), minus_one);
-            const uint32_t hi = (uint32_t)(h >> 32), lo = (uint32_t)h;
-            const uint32_t t = __funnelshift_l(lo, hi, (uint32_t)p);
-            if (live && t <= kc.thresh[K - 1]) {
-                if ((int32_t)t < 0) {   // rank 1
-                    const uint32_t r = hi >> (32 - p);
-                    atomicOr(s_bits + (r >> 5), 1u << (r & 31u));
-                } else {
-                    const uint32_t rank = rank_of(t, lo, p);
-                    if (rank > kc.floor[K - 1]) red_max_register(a.acc, slot_off, hi, rank, p);
-                }
+            for (int j = 0; j < 16; ++j) {
+                const bool live = span_run(ws, j) >= K;
+                if (!__any_sync(0xffffffffu, live)) continue;  // warp-uniform
+                sink_update<K, kCanon>(span_window(ws, j), live, s_bits, acc_k, p);
             }
         }
     }
@@ -427,22 +467,23 @@ __device__ __forceinline__ void sink_slice(const SketchArgs &a, const KConsts &k
 
 // CTA-uniform dispatch to the compile-time K of this CTA (immediate masks in kmer_of)
 template <bool kCanon, int... Ks>
-__device__ __forceinline__ void sink_dispatch(std::integer_sequence<int, Ks...>, int k, const SketchArgs &a, const KConsts &kc,
-                                              uint32_t *s_bits, uint32_t slot_off, uint64_t sym_begin, uint64_t sym_end,
-                                              uint64_t w_lo, uint64_t w_hi) {
-    ((k == Ks + kSinkMinK ? sink_slice<Ks + kSinkMinK, kCanon>(a, kc, s_bits, slot_off, sym_begin, sym_end, w_lo, w_hi) : void()), ...);
+__device__ __forceinline__ void sink_dispatch(std::integer_sequence<int, Ks...>, int k, const SketchArgs &a, uint32_t s_bits,
+                                              uint32_t *acc_k, uint64_t sym_begin, uint64_t sym_end, uint64_t w_lo, uint64_t w_hi) {
+    ((k == Ks + kSinkMinK ? sink_slice<Ks + kSinkMinK, kCanon>(a, s_bits, acc_k, sym_begin, sym_end, w_lo, w_hi) : void()), ...);
 }
 
-// grid = (k values of a.kmask_run, all >= kSinkMinK) x slices; dynamic shared memory = 2^p / 8 bytes
+// grid = (k values of a.kmask_run, all >= kSinkMinK) x slices, CTA b owning slab b; dynamic shared memory = one slab.
+// written[b] != 0: slab b holds the bits of an earlier launch into this workspace.
 template <bool kCanon>
-__global__ void __launch_bounds__(kSinkThreads, 1) sketch_sink_kernel(SketchArgs a, uint32_t *sink, uint32_t slices) {
+__global__ void __launch_bounds__(kSinkThreads, 1) sketch_sink_kernel(SketchArgs a, uint32_t *slabs, uint32_t *written,
+                                                                        uint32_t slices, SketchWsHeader *hdr) {
     extern __shared__ uint4 s_bits4[];
     uint32_t *s_bits = reinterpret_cast<uint32_t *>(s_bits4);
     const int p = a.p;
-    const uint32_t nwords = 1u << (p - 5);
-    for (uint32_t i = threadIdx.x; i < (nwords + 3) / 4; i += kSinkThreads) s_bits4[i] = make_uint4(0u, 0u, 0u, 0u);
-    __shared__ KConsts kc;
-    load_kconsts(a.hdr, kc);
+    const uint32_t n4 = sink_slab_words(p) / 4;
+    uint4 *slab = reinterpret_cast<uint4 *>(slabs + (size_t)blockIdx.x * sink_slab_words(p));
+    const bool carry = written[blockIdx.x] != 0u;
+    for (uint32_t i = threadIdx.x; i < n4; i += kSinkThreads) s_bits4[i] = carry ? __ldcs(slab + i) : make_uint4(0u, 0u, 0u, 0u);
     __syncthreads();
 
     // this CTA's k: the (blockIdx.x / slices)-th set bit of kmask_run; its table slot counts over kmask
@@ -456,13 +497,15 @@ __global__ void __launch_bounds__(kSinkThreads, 1) sketch_sink_kernel(SketchArgs
     const uint64_t wb = sym_begin >> 4, we = sym_end > sym_begin ? (sym_end + 15) >> 4 : wb;
     const uint64_t per = (we - wb + slices - 1) / slices, slice = blockIdx.x % slices;
     const uint64_t w_lo = min(wb + slice * per, we), w_hi = min(w_lo + per, we);
-    sink_dispatch<kCanon>(std::make_integer_sequence<int, 33 - kSinkMinK>{}, k, a, kc, s_bits, slot << (p - 1), sym_begin, sym_end,
-                          w_lo, w_hi);
+    sink_dispatch<kCanon>(std::make_integer_sequence<int, 33 - kSinkMinK>{}, k, a, (uint32_t)__cvta_generic_to_shared(s_bits),
+                          a.acc + ((size_t)slot << (p - 1)), sym_begin, sym_end, w_lo, w_hi);
     __syncthreads();
-    uint32_t *g = sink + (size_t)slot * nwords;
-    for (uint32_t i = threadIdx.x; i < nwords; i += kSinkThreads) {
-        const uint32_t v = s_bits[i];
-        if (v) atomicOr(g + i, v);
+    // evict-first stores: the slabs are read once, by finalize, and must not push the accumulators out of L2
+    for (uint32_t i = threadIdx.x; i < n4; i += kSinkThreads) __stcs(slab + i, s_bits4[i]);
+    if (threadIdx.x == 0) {
+        written[blockIdx.x] = 1u;
+        hdr->sink_slices = slices;                              // the same values from every CTA and launch
+        hdr->sink_first = (uint32_t)__popc(a.kmask & kSmallKMask);   // table slot of the first sink k
     }
 }
 
@@ -476,17 +519,45 @@ __global__ void midk_ready_kernel(SketchWsHeader *hdr, uint32_t k) {
 __device__ __forceinline__ uint32_t bits_to_bytes(uint32_t x) { return (x * 0x00204081u) & 0x01010101u; }
 __device__ __forceinline__ uint32_t bits_to_halves(uint32_t x) { return (x & 1u) | ((x & 2u) << 15); }
 
-__global__ void __launch_bounds__(256) floor_min_kernel(const uint32_t *__restrict__ acc, const uint32_t *__restrict__ sink, int p,
-                                                        SketchWsHeader *hdr, uint32_t *scratch /*[nk]*/) {
+// The first sink slab of table slot `table`, or null unless a sink launch has run into this workspace and the slot is
+// one of its k.
+__device__ __forceinline__ uint32_t *sink_slabs_of(uint32_t *slabs, const SketchWsHeader *hdr, uint32_t table, int p) {
+    const uint32_t slices = hdr->sink_slices, first = hdr->sink_first;
+    return slices != 0u && table >= first ? slabs + (size_t)(table - first) * slices * sink_slab_words(p) : nullptr;
+}
+
+// ORs every sink k's slabs into its first one, so that floor_min_kernel and finalize_kernel read one bitmap per k
+// (byte i holding the bits of registers 8i..8i+7).  Done in a pass of its own: finalize's threads, each with 30
+// octets in turn, would wait for every slab load one after the other.  grid (uint4s of a slab / 256, nk)
+__global__ void __launch_bounds__(256) sink_merge_kernel(uint32_t *slabs, const SketchWsHeader *hdr, int p) {
+    uint4 *s = reinterpret_cast<uint4 *>(sink_slabs_of(slabs, hdr, blockIdx.y, p));
+    const uint32_t slices = hdr->sink_slices, n4 = sink_slab_words(p) / 4, i = blockIdx.x * 256u + threadIdx.x;
+    if (!s || slices < 2u || i >= n4) return;
+    uint4 v = s[i];
+#pragma unroll 4
+    for (uint32_t c = 1; c < slices; ++c) {
+        const uint4 x = __ldcs(s + (size_t)c * n4 + i);
+        v = make_uint4(v.x | x.x, v.y | x.y, v.z | x.z, v.w | x.w);
+    }
+    s[i] = v;
+}
+static cudaError_t sink_merge(uint32_t *slabs, const SketchWsHeader *hdr, int nk, int p, cudaStream_t stream) {
+    if (p > kSinkMaxP) return cudaSuccess;   // no sink, no slabs
+    DD_COUNT_LAUNCH(), sink_merge_kernel<<<dim3((sink_slab_words(p) / 4 + 255) / 256, nk), 256, 0, stream>>>(slabs, hdr, p);
+    return cudaGetLastError();
+}
+
+__global__ void __launch_bounds__(256) floor_min_kernel(const uint32_t *__restrict__ acc, uint32_t *__restrict__ slabs, int p,
+                                                        const SketchWsHeader *hdr, uint32_t *scratch /*[nk]*/) {
     // grid (slices, nk); scratch pre-set to 0xff.  acc rows are 2^p u16 registers = 2^(p-1) words;
-    // register = max(acc, sink bit), byte i of a sink row holding the bits of registers 8i..8i+7.
+    // register = max(acc, sink bit).
     const size_t nwords = (size_t)1 << (p - 1);
     const uint32_t *t = acc + (size_t)blockIdx.y * nwords;
-    const uint8_t *bits = reinterpret_cast<const uint8_t *>(sink) + ((size_t)blockIdx.y << (p - 3));
+    const uint8_t *bits = reinterpret_cast<const uint8_t *>(sink_slabs_of(slabs, hdr, blockIdx.y, p));   // merged
     uint32_t mn = 0xffffu;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nwords / 4; i += (size_t)gridDim.x * blockDim.x) {
         uint4 v = reinterpret_cast<const uint4 *>(t)[i];
-        const uint32_t b = bits[i];
+        const uint32_t b = bits ? bits[i] : 0u;
         v.x = __vmaxu2(v.x, bits_to_halves(b));
         v.y = __vmaxu2(v.y, bits_to_halves(b >> 2));
         v.z = __vmaxu2(v.z, bits_to_halves(b >> 4));
@@ -513,15 +584,15 @@ constexpr int kFinOctPerThread = 30;                                   // 30 x 8
 constexpr int kFinChunk = kPhThreads * kFinOctPerThread * 8;           // registers per CTA
 
 __global__ void __launch_bounds__(kPhThreads)
-finalize_kernel(const uint32_t *__restrict__ acc, const uint32_t *__restrict__ sink, int p, uint8_t *__restrict__ regs,
-                uint32_t *__restrict__ hist) {
+finalize_kernel(const uint32_t *__restrict__ acc, uint32_t *__restrict__ slabs, const SketchWsHeader *hdr, int p,
+                uint8_t *__restrict__ regs, uint32_t *__restrict__ hist) {
     __shared__ __align__(16) uint8_t s_hist[kPhBytes];
     const uint32_t slot = ph_slot();
     const size_t m = (size_t)1 << p;
     const int table = blockIdx.y;
     // 8 u16 accumulators (one uint4) and one byte of rank-1 sink bits -> 8 u8 registers (one uint2)
     const uint4 *src = reinterpret_cast<const uint4 *>(acc + (size_t)table * (m / 2));
-    const uint8_t *bits = reinterpret_cast<const uint8_t *>(sink) + (size_t)table * (m / 8);
+    const uint8_t *bits = reinterpret_cast<const uint8_t *>(sink_slabs_of(slabs, hdr, (uint32_t)table, p));   // merged
     uint2 *dst = reinterpret_cast<uint2 *>(regs + (size_t)table * m);
     if (hist) ph_zero(s_hist);
     __syncthreads();
@@ -533,7 +604,7 @@ finalize_kernel(const uint32_t *__restrict__ acc, const uint32_t *__restrict__ s
         if (q < noct) {
             const uint4 v = __ldcs(src + q);
             // bytes 0 and 2 of each word are the low bytes of its two u16 registers (ranks < 256)
-            const uint32_t b = __ldcs(bits + q);
+            const uint32_t b = bits ? __ldcs(bits + q) : 0u;
             const uint2 out = make_uint2(__vmaxu4(__byte_perm(v.x, v.y, 0x6420), bits_to_bytes(b & 15u)),
                                          __vmaxu4(__byte_perm(v.z, v.w, 0x6420), bits_to_bytes(b >> 4)));
             dst[q] = out;
@@ -609,49 +680,71 @@ static unsigned persistent_grid(const SketchVariant &v, size_t smem) {
     return g;
 }
 
-static size_t acc_bytes(int nk, int p) { return ((size_t)nk * sizeof(uint16_t) * ((size_t)1 << p) + 255) / 256 * 256; }
-static size_t sink_bytes(int nk, int p) { return (((size_t)nk << (p - 3)) + 255) / 256 * 256; }   // [nk][2^p / 32] u32
-size_t sketch_workspace_bytes(int nk, int p) {   // [header | scratch | accumulators | rank-1 sink bitmaps | mid-k bitmaps]
-    return sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + sink_bytes(nk, p) + (size_t)kMidKWords * sizeof(uint32_t);
-}
-static SketchWsHeader *ws_hdr(void *ws) { return static_cast<SketchWsHeader *>(ws); }
-static uint32_t *ws_scratch(void *ws) { return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader)); }
-static uint32_t *ws_acc(void *ws) { return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader) + 256); }
-static uint32_t *ws_sink(void *ws, int nk, int p) {
-    return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p));
-}
-static uint32_t *ws_midk(void *ws, int nk, int p) {
-    return reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(ws_sink(ws, nk, p)) + sink_bytes(nk, p));
-}
-
-cudaError_t sketch_begin(void *d_ws, int nk, int p, cudaStream_t stream) {
-    // header, scratch, accumulators, sink bitmaps and the k <= 12 bitmaps; the 8 + 32 MiB of k = 13 / 14 are
-    // zeroed by the launch that first consults them (only streams longer than 4^13 symbols ever do)
-    return cudaMemsetAsync(d_ws, 0,
-                           sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + sink_bytes(nk, p) + (size_t)midk_offset(13) * sizeof(uint32_t),
-                           stream);
-}
-
 int g_midk = 1;   // dd_set_option("sketch_midk", 0/1): tuning knob, never changes results
 int g_sink = 1;   // dd_set_option("sketch_sink", 0/1): A/B switch for the rank-1 sink, never changes results
 
-// resident sink CTAs on this device (its SM count x CTAs per SM at 2^p/8 bytes of shared memory), cached
+// resident sink CTAs on this device (its SM count x CTAs per SM at one slab of shared memory), cached
 static unsigned sink_resident(bool canon, int p) {
     constexpr int kMaxDev = 64;
     static unsigned cached[kMaxDev][2][kSinkMaxP + 1] = {};
     int dev = 0;
-    cudaGetDevice(&dev);
+    if (cudaGetDevice(&dev) != cudaSuccess) cudaGetLastError();
     unsigned local = 0;
     unsigned &g = (dev >= 0 && dev < kMaxDev) ? cached[dev][canon ? 1 : 0][p] : local;
     if (g == 0) {
         const auto fn = canon ? sketch_sink_kernel<true> : sketch_sink_kernel<false>;
-        cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(((size_t)1 << kSinkMaxP) / 8));
-        int sms = 148, per_sm = 1;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kSinkThreads, ((size_t)1 << p) / 8);
+        int sms = 148, per_sm = 1;   // (no device: a B200's count, for the workspace size alone)
+        if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sink_slab_words(kSinkMaxP) * 4)) != cudaSuccess ||
+            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kSinkThreads, sink_slab_words(p) * 4) != cudaSuccess) {
+            cudaGetLastError();
+            return 148;
+        }
         g = (unsigned)(sms * (per_sm > 0 ? per_sm : 1));
     }
     return g;
+}
+// CTAs (and slabs) per k of a sink launch over nk_sink k values: the resident CTAs shared among them
+static unsigned sink_slices(bool canon, int p, unsigned nk_sink) {
+    const unsigned resident = sink_resident(canon, p);
+    return resident / nk_sink > 0 ? resident / nk_sink : 1u;
+}
+// slabs of a workspace: nk_sink x sink_slices(nk_sink) <= max(resident, nk) for any launch into it
+static size_t sink_slab_count(int nk, int p) {
+    if (p > kSinkMaxP) return 0;
+    const size_t resident = max(sink_resident(true, p), sink_resident(false, p));
+    return max(resident, (size_t)nk);
+}
+
+static size_t round256(size_t b) { return (b + 255) / 256 * 256; }
+static size_t acc_bytes(int nk, int p) { return round256((size_t)nk * sizeof(uint16_t) * ((size_t)1 << p)); }
+static size_t written_bytes(int nk, int p) { return round256(sink_slab_count(nk, p) * sizeof(uint32_t)); }
+static constexpr size_t kMidKBytes = (size_t)kMidKWords * sizeof(uint32_t);
+// [header | scratch | accumulators | slab-written flags | mid-k bitmaps | rank-1 sink slabs [k][slice][2^p / 32] u32]
+size_t sketch_workspace_bytes(int nk, int p) {
+    return sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + written_bytes(nk, p) + kMidKBytes +
+           sink_slab_count(nk, p) * sink_slab_words(p) * sizeof(uint32_t);
+}
+static SketchWsHeader *ws_hdr(void *ws) { return static_cast<SketchWsHeader *>(ws); }
+static uint32_t *ws_scratch(void *ws) { return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader)); }
+static uint32_t *ws_acc(void *ws) { return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader) + 256); }
+static uint32_t *ws_written(void *ws, int nk, int p) {
+    return reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p));
+}
+static uint32_t *ws_midk(void *ws, int nk, int p) {
+    return reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(ws_written(ws, nk, p)) + written_bytes(nk, p));
+}
+static uint32_t *ws_slabs(void *ws, int nk, int p) {
+    return reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(ws_midk(ws, nk, p)) + kMidKBytes);
+}
+
+cudaError_t sketch_begin(void *d_ws, int nk, int p, cudaStream_t stream) {
+    // header, scratch, accumulators, slab-written flags and the k <= 12 bitmaps; the 8 + 32 MiB of k = 13 / 14
+    // are zeroed by the launch that first consults them (only streams longer than 4^13 symbols ever do), and a
+    // slab is only read once its flag says a sink CTA has written it
+    return cudaMemsetAsync(d_ws, 0,
+                           sizeof(SketchWsHeader) + 256 + acc_bytes(nk, p) + written_bytes(nk, p) + (size_t)midk_offset(13) * sizeof(uint32_t),
+                           stream);
 }
 
 static cudaError_t sketch_update_impl(const uint32_t *d_codes, const uint32_t *d_invalid, const dd_pack_state *d_state,
@@ -704,13 +797,13 @@ static cudaError_t sketch_update_impl(const uint32_t *d_codes, const uint32_t *d
     const uint32_t sink_mask = kmask & ~kSmallKMask;
     if (sink && sink_mask && p <= kSinkMaxP) {
         const unsigned nk_sink = (unsigned)__builtin_popcount(sink_mask);
-        const unsigned resident = sink_resident(canon != 0, p);
-        const unsigned slices = resident / nk_sink > 0 ? resident / nk_sink : 1u;
+        const unsigned slices = sink_slices(canon != 0, p, nk_sink);
         if (nsym >= (size_t)slices * (((size_t)1 << p) / 4)) {
+            const int nk = __builtin_popcount(kmask);
             a.kmask_run = sink_mask;
-            const size_t smem = ((((size_t)1 << p) / 8) + 15) / 16 * 16;
             const auto fn = canon ? sketch_sink_kernel<true> : sketch_sink_kernel<false>;
-            DD_COUNT_LAUNCH(), fn<<<nk_sink * slices, kSinkThreads, smem, stream>>>(a, ws_sink(d_ws, __builtin_popcount(kmask), p), slices);
+            DD_COUNT_LAUNCH(), fn<<<nk_sink * slices, kSinkThreads, sink_slab_words(p) * sizeof(uint32_t), stream>>>(
+                a, ws_slabs(d_ws, nk, p), ws_written(d_ws, nk, p), slices, ws_hdr(d_ws));
             todo &= kSmallKMask;
         }
     }
@@ -779,7 +872,9 @@ cudaError_t sketch_update_sched(const uint32_t *d_codes, const uint32_t *d_inval
                 }
             }
         // before the first cut the floor is 0 and half of all updates have rank 1: absorb them in the sink;
-        // past it the floor drops them for free and the plain kernels are the right ones
+        // past it the floor drops them for free and the plain kernels are the right ones.  The sink kernel has no
+        // floor test, which stays exact even under a floor raised by hand: a floor is a minimum register, so an
+        // update of rank <= floor cannot raise any register.
         const bool sink = g_sink && at_end <= ((uint64_t)16 << p);
         if ((e = sketch_update_impl(d_codes, d_invalid, d_state, origin + pos, origin + upto, max_new_symbols, kmask, p, canon, d_ws,
                                     midk_hi, sink, stream)) != cudaSuccess)
@@ -797,7 +892,8 @@ cudaError_t sketch_refresh_floor(void *d_ws, uint32_t kmask, int p, cudaStream_t
     const int nk = __builtin_popcount(kmask);
     cudaError_t e = cudaMemsetAsync(ws_scratch(d_ws), 0xff, 32 * sizeof(uint32_t), stream);
     if (e != cudaSuccess) return e;
-    DD_COUNT_LAUNCH(), floor_min_kernel<<<dim3(16, nk), 256, 0, stream>>>(ws_acc(d_ws), ws_sink(d_ws, nk, p), p, ws_hdr(d_ws),
+    if ((e = sink_merge(ws_slabs(d_ws, nk, p), ws_hdr(d_ws), nk, p, stream)) != cudaSuccess) return e;
+    DD_COUNT_LAUNCH(), floor_min_kernel<<<dim3(16, nk), 256, 0, stream>>>(ws_acc(d_ws), ws_slabs(d_ws, nk, p), p, ws_hdr(d_ws),
                                                                           ws_scratch(d_ws));
     DD_COUNT_LAUNCH(), floor_publish_kernel<<<1, 32, 0, stream>>>(ws_hdr(d_ws), ws_scratch(d_ws), kmask);
     return cudaGetLastError();
@@ -808,8 +904,10 @@ cudaError_t sketch_end(void *d_ws, int nk, int p, uint8_t *d_regs, uint32_t *d_h
     cudaError_t e;
     if (d_hist && (e = cudaMemsetAsync(d_hist, 0, (size_t)nk * DD_HIST_BINS * sizeof(uint32_t), stream)) != cudaSuccess)
         return e;
+    if ((e = sink_merge(ws_slabs(d_ws, nk, p), ws_hdr(d_ws), nk, p, stream)) != cudaSuccess) return e;
     const unsigned slices = (unsigned)((((size_t)1 << p) + kFinChunk - 1) / kFinChunk);
-    DD_COUNT_LAUNCH(), finalize_kernel<<<dim3(slices, nk), kPhThreads, 0, stream>>>(ws_acc(d_ws), ws_sink(d_ws, nk, p), p, d_regs, d_hist);
+    DD_COUNT_LAUNCH(), finalize_kernel<<<dim3(slices, nk), kPhThreads, 0, stream>>>(ws_acc(d_ws), ws_slabs(d_ws, nk, p), ws_hdr(d_ws), p, d_regs,
+                                                                                        d_hist);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     if (d_hist && d_cards) return mle_from_hist(d_hist, nk, p, d_cards, stream);
     return cudaSuccess;

@@ -7,7 +7,12 @@ For each static-k-set instantiation of sketch_allk_kernel<canon=true> the unroll
 delimited by the hash's first multiply (`IMAD.WIDE.U32 ..., 0x1fffff`); inside a block the update
 tail (rank, register index, address, REDG) sits behind the branch that follows the threshold
 compare, so   always-executed = block length - tail length.
-Writes profiles/r02_k2_sass.json and profiles/r02_k2_sass.md (one k block, annotated)."""
+Writes profiles/r02_k2_sass.json and profiles/r02_k2_sass.md (one k block, annotated).
+
+--sink instead counts sketch_sink_kernel<canon=true>: on the all-valid warp path a k's 16 symbols are unrolled,
+one hash per symbol, and every warp runs both the rank-1 and the rank >= 2 side of the tail, so the distance
+between consecutive hashes of one unrolled run is the instructions a warp executes per (symbol, k).  That count
+goes into profiles/r15_k2_sink.json ("sass_sink_all_valid"), next to the kernel's measured times."""
 import json
 import os
 import re
@@ -26,9 +31,42 @@ def blocks_of(ins):
     return [(a + 1, b + 1) for a, b in zip(reds, reds[1:])]
 
 
+def instructions(body):
+    return [mm.group(1).strip() for ln in body if (mm := re.match(r"\s+/\*[0-9a-f]{4,}\*/\s+(.*?);", ln))]
+
+
+def sink_counts(sass, heads):
+    for n, h in enumerate(heads):
+        if "sketch_sink_kernelILb1E" not in sass[h]:
+            continue
+        ins = instructions(sass[h:heads[n + 1] if n + 1 < len(heads) else len(sass)])
+        hashes = [i for i, t in enumerate(ins) if "IMAD.WIDE.U32" in t and "0x1fffff" in t]
+        gaps = [b - a for a, b in zip(hashes, hashes[1:])]
+        # an unrolled run: a k's 16 hashes, 15 gaps, of which scheduling makes the first and last differ; the
+        # per-symbol path has one hash per k, so 10 equal gaps in a row only occur inside a run
+        runs = [gaps[i:i + 10] for i in range(len(gaps) - 9)
+                if len(set(gaps[i:i + 10])) == 1 and (i == 0 or gaps[i - 1] != gaps[i])]
+        per = statistics.median(r[0] for r in runs)
+        return {"kernel_instructions": len(ins), "hash_sites": len(hashes), "unrolled_runs": len(runs),
+                "instr_per_update_all_valid": per, "bssy": sum("BSSY" in t for t in ins),
+                "atoms_or": sum("ATOMS.OR" in t for t in ins), "redg": sum("REDG" in t for t in ins),
+                "how": "tools/k2_sass_count.py --sink on dandd_b200/build/sketch.o (cuobjdump -sass): median distance between "
+                       "consecutive hashes of the unrolled all-valid runs of sketch_sink_kernel<true>"}
+    raise SystemExit("sketch_sink_kernel<true> not found in " + OBJ)
+
+
 def main():
     sass = subprocess.check_output(["cuobjdump", "-sass", OBJ], text=True).split("\n")
     heads = [i for i, ln in enumerate(sass) if "Function :" in ln]
+    if "--sink" in sys.argv:
+        counts = sink_counts(sass, heads)
+        path = os.path.join(ROOT, "profiles", "r15_k2_sink.json")
+        report = json.load(open(path)) if os.path.exists(path) else {}
+        report["sass_sink_all_valid"] = counts
+        with open(path, "w") as fh:
+            json.dump(report, fh, indent=1)
+        print(json.dumps(counts, indent=1))
+        return 0
     out, listing = {}, []
     for n, h in enumerate(heads):
         name = sass[h]
@@ -36,7 +74,7 @@ def main():
         if not m or m.group(1) not in VARIANTS:
             continue
         body = sass[h:heads[n + 1] if n + 1 < len(heads) else len(sass)]
-        ins = [mm.group(1).strip() for ln in body if (mm := re.match(r"\s+/\*[0-9a-f]{4,}\*/\s+(.*?);", ln))]
+        ins = instructions(body)
         lengths, always, chosen = [], [], None
         for a, b in blocks_of(ins):
             blk = ins[a:b]

@@ -1,11 +1,16 @@
 #!/usr/bin/env python
 """A/B of K2's rank-1 sink (dd_set_option("sketch_sink", 1/0)) in one process, rounds alternated:
-  * serialised K2 time per config-2 genome (CUDA events around dd_sketch_update_sched, 12 genomes);
+  * serialised K2 time per config-2 genome (CUDA events around dd_sketch_update_sched, 12 genomes); at
+    config 2 that call is one sketch_sink_kernel launch, so with the sink on this is the sink kernel's time;
   * the bench-shaped step: 12 genomes on 2 streams (pack + K2 + finalize), leaf MLE, prefix unions;
   * one 100 Mbp and one 1 Gbp stream at k = 2..32, p = 20, which cross the first floor cut early and
     must not regress.
-Also records the card, its power limit and SM clock, and the static SASS of one k block of the sink
-kernel (cuobjdump on dandd_b200/build/sketch.o, when available).  Writes --out (JSON)."""
+Also records the card, its power limit and SM clock, the static SASS of one k block of the sink
+kernel (cuobjdump on dandd_b200/build/sketch.o, when available), the device time of every launch of
+one bench-shaped step under torch.profiler (a run of its own), and the rank >= 2 updates of one bench
+genome counted on the CPU with the oracle (the L2 reductions the sink cannot absorb).
+--lib loads another build of the library (e.g. a one-off variant of the sink kernel); --sink-only then
+records just the serialised per-genome K2 time with the sink on.  Writes --out (JSON)."""
 import argparse
 import json
 import os
@@ -52,6 +57,39 @@ def sink_sass():
     return None
 
 
+def rank2_updates(text, ks, p):
+    """(updates, updates of rank >= 2) of one genome over ks: every valid canonical k-mer is one update, and its
+    rank is >= 2 exactly when the hash bit just below the p register bits is 0."""
+    from oracle import pyoracle as orc
+    from oracle.ref_numpy import wang_np
+    sym = orc.fasta_symbols(text)
+    total = high = 0
+    for k in ks:
+        h = wang_np(orc.kmers(sym, k, True))
+        total += int(h.size)
+        high += int(np.count_nonzero(((h >> np.uint64(63 - p)) & np.uint64(1)) == 0))
+    return total, high
+
+
+def step_launches(step, torch):
+    """Device time of every kernel and memset of one step, under torch.profiler: {name: {calls, total_ms}}."""
+    from torch.profiler import ProfilerActivity, profile
+    step()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        step()
+        torch.cuda.synchronize()
+    out = {}
+    for ev in prof.key_averages():
+        t = getattr(ev, "device_time_total", None)
+        if t is None:
+            t = ev.cuda_time_total
+        if t <= 0 or ev.key.startswith("cuda"):
+            continue
+        out[ev.key] = {"calls": ev.count, "total_ms": t / 1e3}
+    return dict(sorted(out.items(), key=lambda kv: -kv[1]["total_ms"]))
+
+
 def long_fasta(n, seed):
     rng = np.random.default_rng(seed)
     s = bench.ACGT[rng.integers(0, 4, n, dtype=np.uint8)]
@@ -66,16 +104,24 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r07_k2_sink.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r15_k2_sink.json"))
+    ap.add_argument("--lib", default=None, help="load this build of libdandd_b200.so instead of the in-tree one")
+    ap.add_argument("--sink-only", action="store_true", help="only the serialised per-genome K2 time, sink on")
     args = ap.parse_args()
     import torch
-    from dandd_b200 import build
-    build.build()
+    from dandd_b200 import _lib
+    if args.lib:
+        _lib.LIB_PATH = os.path.abspath(args.lib)
+    else:
+        from dandd_b200 import build
+        build.build()
     from dandd_b200._lib import check
     from dandd_b200.engine import Engine
     eng = Engine(0)
     dev = eng.device
-    report = {"card": card_info(), "sass_sink_kernel_canon": sink_sass(), "rounds": args.rounds}
+    report = {"card": card_info(), "lib": _lib.LIB_PATH if args.lib else "in-tree", "rounds": args.rounds}
+    if not args.lib:
+        report["sass_sink_kernel_canon"] = sink_sass()
 
     def set_sink(on):
         check(eng.lib.dd_set_option(b"sketch_sink", int(on)), "dd_set_option")
@@ -130,6 +176,28 @@ def main():
         eng._update_from_state = orig_update
         return [a.elapsed_time(b) for a, b in events]
 
+    def write(rep):
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as fh:
+            json.dump(rep, fh, indent=1)
+
+    set_sink(1)
+    k2_serial()
+    if args.sink_only:
+        per = [statistics.median(k2_serial()) for _ in range(args.rounds)]
+        report["sink_ms_per_genome"] = {"median": statistics.median(per), "min": min(per), "max": max(per), "all": per,
+                                        "how": "median over the 12 genomes of CUDA events around each serialised call, per round"}
+        write(report)
+        print(json.dumps(report, indent=1))
+        return
+    report["step_launches"] = step_launches(step, torch)
+    per = [statistics.median(k2_serial()) for _ in range(args.rounds)]
+    report["sink_ms_per_genome"] = {"median": statistics.median(per), "min": min(per), "max": max(per), "all": per,
+                                    "how": "median over the 12 genomes of CUDA events around each serialised call, per round"}
+    total, high = rank2_updates(texts[0][0], bench.KS, bench.P)
+    report["bench_genome0_updates"] = {"all": total, "rank_ge2": high,
+                                       "rank_ge2_ms_at_187_g_per_s": high / 187e9 * 1e3}
+
     longs = {}
     for name, n in (("100mbp", 100_000_000), ("1gbp", 1_000_000_000)):
         txt = long_fasta(n, seed=7 if n < 10**9 else 8)
@@ -175,11 +243,9 @@ def main():
     report["updates_per_genome"] = updates
     report["update_rate_g_per_s"] = {arm: updates / (report[arm]["k2_ms_per_genome"]["median"] / 1e3) / 1e9
                                      for arm in ("sink_on", "sink_off")}
-    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-    with open(args.out, "w") as fh:
-        json.dump(report, fh, indent=1)
-    print(json.dumps({key: report[key] for key in ("card", "ratio_on_over_off", "identical_outputs_on_off", "update_rate_g_per_s")},
-                     indent=1))
+    write(report)
+    print(json.dumps({key: report[key] for key in ("card", "sink_ms_per_genome", "bench_genome0_updates", "ratio_on_over_off",
+                                                   "identical_outputs_on_off", "update_rate_g_per_s")}, indent=1))
 
 
 if __name__ == "__main__":
